@@ -23,14 +23,41 @@ Differences a caller can observe (all documented in INTEGRATION.md):
     everything (the geometrically correct image, not the reference's);
   * `cuda_devices=[0, 1, ...]` renders every frame on several GPUs of the box through the same call
     (b200rt_multi_*): bit-identical with the reference generator, equal up to the order of the float additions
-    with `rng_mode = RNG_PHILOX`.
+    with `rng_mode = RNG_PHILOX`;
+  * `adaptive = dict(rel_error=..., min_spp=16, check_every=8, floor=0.05)` (the keys of Context.render_adaptive) lets
+    each pixel stop sampling once its estimated error is below the tolerance, with the caller's spp as the maximum;
+    `last_spp` then holds the (height, width) map of samples taken.  B200RT_ADAPTIVE=rel_error[,min_spp[,check_every]]
+    in the environment sets it for callers that never touch the attribute.  One GPU only.
 """
+import math
 import os
 import warnings
 
 import numpy as np
 
 from . import _capi
+
+
+def adaptive_from_env(text):
+    """The `adaptive` dict that B200RT_ADAPTIVE=rel_error[,min_spp[,check_every]] stands for; ValueError if malformed."""
+    usage = f"B200RT_ADAPTIVE={text!r}: expected rel_error[,min_spp[,check_every]], e.g. 0.02 or 0.02,16,8"
+    parts = [p.strip() for p in str(text).split(",")]
+    if not 1 <= len(parts) <= 3 or "" in parts:
+        raise ValueError(usage)
+    try:
+        rel_error = float(parts[0])
+        ints = [int(p) for p in parts[1:]]
+    except ValueError:
+        raise ValueError(usage) from None
+    if not math.isfinite(rel_error) or rel_error < 0:
+        raise ValueError(usage + " (rel_error must be finite and >= 0)")
+    if ints and ints[0] < 2:
+        raise ValueError(usage + " (min_spp must be >= 2)")
+    if len(ints) > 1 and ints[1] < 1:
+        raise ValueError(usage + " (check_every must be >= 1)")
+    ad = {"rel_error": rel_error}
+    ad.update(zip(("min_spp", "check_every"), ints))
+    return ad
 
 
 class KernelLauncher(object):
@@ -57,12 +84,19 @@ class KernelLauncher(object):
         #                                 walks them (drops included); "nodrop": keep the fast, complete traversal
         self.sample_streams = 0      # RNG_PHILOX only: -1 automatic, N > 1 concurrent sample ranges on each GPU (b200rt.h)
         self.collect_stats = False
+        # None: every pixel takes spp samples (the reference's image); a dict: adaptive sampling (module docstring)
+        self.adaptive = adaptive_from_env(os.environ["B200RT_ADAPTIVE"]) if os.environ.get("B200RT_ADAPTIVE") else None
+        self.last_spp = None
         self.last_stats = None
         self._warned_deep = False
 
     # reference KernelLauncher.py:33
     def launch_Raytracing(self, h_img_out, h_vertex_p, h_vertex_n, h_vertex_uv, h_face_data, h_material_data,
                           h_light_data, h_BVH, h_cam, h_envData, imgDim, spp, maxBounce, h_IBL):
+        if self.adaptive is not None and isinstance(self._ctx, _capi.MultiContext):
+            raise ValueError("adaptive sampling renders on one GPU: its stopping rule needs each pixel's samples in one "
+                             f"sequence, which a split over cuda_devices={self._ctx.devices} would cut apart; set "
+                             "launcher.adaptive = None or use one device")
         cam = np.ascontiguousarray(h_cam, dtype=np.float32).reshape(-1)
         if cam.size < 10:
             raise ValueError("h_cam must hold 10 floats (main.py:59-61)")
@@ -98,7 +132,12 @@ class KernelLauncher(object):
         opts = _capi.make_opts(rng_mode=self.rng_mode, traversal=traversal, stack_cap=self.stack_cap,
                                seed=self.seed, collect_stats=self.collect_stats, sample_streams=self.sample_streams)
         out = h_img_out.reshape(-1)[:imgDim * 3]
-        self._ctx.render(cam[:10], h_envData, width, height, int(spp), int(maxBounce), out=out, opts=opts)
+        if self.adaptive is not None:
+            img, self.last_spp, _ = self._ctx.render_adaptive(cam[:10], h_envData, width, height, int(spp), int(maxBounce),
+                                                              opts=opts, **self.adaptive)
+            out[:] = img.reshape(-1)
+        else:
+            self._ctx.render(cam[:10], h_envData, width, height, int(spp), int(maxBounce), out=out, opts=opts)
         self.last_stats = self._ctx.stats()
 
     # reference KernelLauncher.py:90

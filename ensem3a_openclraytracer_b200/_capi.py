@@ -45,10 +45,16 @@ class Stats(ctypes.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_ if not k.startswith("reserved")}
 
 
+class Adaptive(ctypes.Structure):
+    """b200rt_adaptive: the stopping rule of adaptive sampling (include/b200rt.h)."""
+    _fields_ = [("min_spp", ctypes.c_int32), ("check_every", ctypes.c_int32), ("rel_error", ctypes.c_float),
+                ("floor", ctypes.c_float)]
+
+
 # every symbol include/b200rt.h declares (tests/test_abi.py checks the header against this list)
 SYMBOLS = [
     "b200rt_default_opts", "b200rt_create", "b200rt_destroy", "b200rt_last_error", "b200rt_set_scene",
-    "b200rt_set_materials", "b200rt_set_ibl", "b200rt_render", "b200rt_render_rgb8", "b200rt_render_device", "b200rt_finalize_device",
+    "b200rt_set_materials", "b200rt_set_ibl", "b200rt_render", "b200rt_render_adaptive", "b200rt_render_rgb8", "b200rt_render_device", "b200rt_finalize_device",
     "b200rt_reduce_finalize_device", "b200rt_sync", "b200rt_set_stream", "b200rt_invalidate", "b200rt_primary_hits", "b200rt_trace_rays",
     "b200rt_img_processing", "b200rt_get_stats", "b200rt_math_probe", "b200rt_philox_probe", "b200rt_alloc",
     "b200rt_free", "b200rt_ipc_export",
@@ -89,6 +95,8 @@ def load_library():
     lib.b200rt_set_materials.argtypes = [vp, vp, i64]
     lib.b200rt_set_ibl.argtypes = [vp, vp, i32, i32]
     lib.b200rt_render.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), vp]
+    lib.b200rt_render_adaptive.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), ctypes.POINTER(Adaptive),
+                                           vp, vp, vp]
     lib.b200rt_render_device.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), vp]
     lib.b200rt_render_rgb8.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), vp]
     lib.b200rt_finalize_device.argtypes = [vp, vp, vp, i64, i32]
@@ -277,6 +285,25 @@ class Context:
         self._check(self._lib.b200rt_render(self._h, _ptr(cam_), _ptr(env_), int(width), int(height), int(spp),
                                             int(max_bounce), ctypes.byref(o), _ptr(out)), "b200rt_render")
         return out
+
+    def render_adaptive(self, cam, env, width, height, spp, max_bounce, rel_error, min_spp=16, check_every=8, floor=0.05,
+                        opts=None):
+        """Adaptive sampling (b200rt_render_adaptive): every pixel takes at least min_spp and at most spp samples and
+        stops once the standard error of its mean luminance is at most rel_error * max(min(mean, 1), floor).
+        Returns (image (H, W, 3) float32, samples taken (H, W) int32, standard error (H, W) float32)."""
+        cam_, env_ = _f32(cam), _f32(env)
+        if cam_.size != 10 or env_.size != 5:
+            raise B200RTError("cam must hold 10 floats and envData 5 (main.py:59-61,72-73)")
+        h, w = int(height), int(width)
+        img = np.zeros((h, w, 3), dtype=np.float32)
+        spp_map = np.zeros((h, w), dtype=np.int32)
+        err_map = np.zeros((h, w), dtype=np.float32)
+        ad = Adaptive(int(min_spp), int(check_every), float(rel_error), float(floor))
+        o = opts if opts is not None else make_opts()
+        self._check(self._lib.b200rt_render_adaptive(self._h, _ptr(cam_), _ptr(env_), w, h, int(spp), int(max_bounce),
+                                                     ctypes.byref(o), ctypes.byref(ad), _ptr(img), _ptr(spp_map),
+                                                     _ptr(err_map)), "b200rt_render_adaptive")
+        return img, spp_map, err_map
 
     def render_rgb8(self, cam, env, width, height, spp, max_bounce, opts=None):
         """(height, width, 3) uint8 image, quantised on the device like FileManager.saveImg does on the host."""

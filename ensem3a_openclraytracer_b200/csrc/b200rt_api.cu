@@ -80,6 +80,9 @@ struct b200rt_ctx {
   DevBuf d_prim_dirk, d_prim_tri, d_out, d_misc, d_tmp_a, d_tmp_b;
   DevBuf d_pA, d_pB, d_pC, d_pHit, d_list0, d_list1, d_cnt;  // wavefront path state (rt_kernels.cuh)
   DevBuf d_slots, d_part_count;                               // order-preserving list compaction
+  DevBuf d_welford, d_ad_spp, d_ad_err;                       // adaptive sampling (AdaptArgs)
+  unsigned int *h_live = nullptr;   // adaptive sampling: pinned, the path-list length after each of the two batches in flight
+  cudaEvent_t ev_batch[2] = {nullptr, nullptr};
   DeviceCounters *d_counters = nullptr;
 
   b200rt_stats stats;
@@ -280,6 +283,7 @@ void fill_args(b200rt_ctx *c, const FrameParams &F, const b200rt_opts &o, float 
   A->refill_min = c->refill_min;
   A->tri_quorum = c->tri_quorum;
   A->validate = 0;
+  A->ad = AdaptArgs();
 }
 
 // The fast path needs a strict two-child tree with nested boxes; any other tree is walked in reference order.  When
@@ -383,7 +387,7 @@ int prepare_trace_t(b200rt_ctx *c, WaveLaunch *w) {
 
 int prepare_wave(b200rt_ctx *c, int trav, bool smem, bool stats, WaveLaunch *w) {
   int per_sm = 0;
-  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shade<false>, kShadeBlock, 0));
+  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shade<false, false>, kShadeBlock, 0));
   if (per_sm < 1) return fail(c, B200RT_ERR_CUDA, "k_shade does not fit on an SM");
   w->shade_grid = per_sm * c->sm_count;
   int key = trav * 4 + (smem ? 2 : 0) + (stats ? 1 : 0);
@@ -529,8 +533,53 @@ int check_frame_args(b200rt_ctx *c, const float *cam, int width, int height, int
   return 0;
 }
 
+constexpr int kAdaptBatch = 32;  // adaptive renders: wavefront iterations enqueued between two looks at the list length
+
+// The wavefront loop of an adaptive render: render_impl's launches, enqueued in batches of kAdaptBatch iterations rounded
+// up to a multiple of compact_every, so that every batch ends with a compaction and its last cnt word is the number of
+// live paths.  That word is copied to pinned memory behind an event; before batch k + 2 is enqueued the host waits for
+// batch k's and stops once it is 0.  One batch is always in flight, so the GPU does not wait for the host.  A k_shade
+// on an empty list does nothing, so stopping there leaves the image the full loop would make.
+int adaptive_wave(b200rt_ctx *c, const KernelArgs &A, const WaveLaunch &wl, int n_iter, bool nee, bool time_kernels) {
+  const int batch = (kAdaptBatch + A.compact_every - 1) / A.compact_every * A.compact_every;
+  int it = 0, n_shade = 0, n_trace = 0, n_compactions = 0;
+  for (int b = 0; it <= n_iter; ++b) {
+    if (b >= 2) {
+      CU(cudaEventSynchronize(c->ev_batch[b & 1]));
+      if (c->h_live[b & 1] == 0u) break;
+    }
+    const int end = std::min(it + batch, n_iter + 1);
+    for (; it < end; ++it) {
+      if (time_kernels) CU(cudaEventRecord(c->kev[c->kev_used++], c->stream));
+      if (nee) k_shade<true, true><<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
+      else k_shade<false, true><<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
+      ++n_shade;
+      if (it < n_iter && (it + 1) % A.compact_every == 0) {
+        k_compact<<<wl.shade_grid, kCompactBlock, 0, c->stream>>>(A.slots, A.cnt + it, 0u, A.part_count, A.list[(it + 1) & 1], A.cnt + it + 1);
+        ++n_compactions;
+      }
+      if (time_kernels) CU(cudaEventRecord(c->kev[c->kev_used++], c->stream));
+      if (it < n_iter) {
+        wl.trace<<<wl.trace_grid, kBlock, wl.trace_smem, c->stream>>>(A, it);
+        ++n_trace;
+      }
+    }
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(&c->h_live[b & 1], A.cnt + end, sizeof(unsigned int), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaEventRecord(c->ev_batch[b & 1], c->stream));
+  }
+  // k_count_parts + k_compact for the first list, then what the loop launched
+  c->stats.kernel_launches += 2 + n_shade + n_compactions + n_trace;
+  c->stats.wave_iterations = n_trace;
+  CU(cudaEventRecord(c->ev[2], c->stream));
+  c->stats_pending = true;
+  return 0;
+}
+
+// ad != NULL: adaptive sampling (b200rt_render_adaptive has validated ad and opts; the frame covers [0, spp) on one
+// stream).  The launch loop then runs in batches and stops once the path list is empty; it is synchronous.
 int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, int height, int spp, int max_bounce,
-                const b200rt_opts *opts, float *d_out) {
+                const b200rt_opts *opts, float *d_out, const b200rt_adaptive *ad = nullptr) {
   b200rt_opts o;
   if (opts) o = *opts; else b200rt_default_opts(&o);
   c->streams_used = 1;
@@ -579,12 +628,37 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   if (ensure(c, c->d_part_count, (size_t)wl.shade_grid * sizeof(unsigned int))) return B200RT_ERR_CUDA;
   A.part_count = static_cast<unsigned int *>(c->d_part_count.p);
   A.slots = static_cast<int *>(c->d_slots.p);
+  if (ad) {
+    if (ensure(c, c->d_welford, npix * sizeof(float2))) return B200RT_ERR_CUDA;
+    if (ensure(c, c->d_ad_spp, npix * sizeof(int))) return B200RT_ERR_CUDA;
+    if (ensure(c, c->d_ad_err, npix * sizeof(float))) return B200RT_ERR_CUDA;
+    A.ad.welford = static_cast<float2 *>(c->d_welford.p);
+    A.ad.spp_out = static_cast<int *>(c->d_ad_spp.p);
+    A.ad.err_out = static_cast<float *>(c->d_ad_err.p);
+    A.ad.min_spp = ad->min_spp;
+    A.ad.check_every = ad->check_every;
+    A.ad.rel_error = ad->rel_error;
+    A.ad.floor = ad->floor;
+    if (!c->h_live) CU(cudaMallocHost(&c->h_live, 2 * sizeof(unsigned int)));
+    for (int k = 0; k < 2; ++k)
+      if (!c->ev_batch[k]) CU(cudaEventCreateWithFlags(&c->ev_batch[k], cudaEventDisableTiming));
+  }
   c->stats.kernel_launches = 0;
   c->stats.sample_streams = 1;
   c->stats.scene_in_smem = smem ? 1 : 0;
   CU(cudaMemsetAsync(c->d_counters, 0, sizeof(DeviceCounters), c->stream));
   CU(cudaMemsetAsync(c->d_cnt.p, 0, cnt_bytes, c->stream));
+  if (ad) {  // pixels outside the rendered set read 0 in both maps
+    CU(cudaMemsetAsync(c->d_ad_spp.p, 0, npix * sizeof(int), c->stream));
+    CU(cudaMemsetAsync(c->d_ad_err.p, 0, npix * sizeof(float), c->stream));
+  }
   CU(cudaEventRecord(c->ev[0], c->stream));
+  if (ad) {
+    const int grid = (int)std::min<long long>(((long long)A.n_work + 255) / 256, (long long)c->sm_count * 8);
+    k_adaptive_init<<<grid, 256, 0, c->stream>>>(A);
+    CU(cudaGetLastError());
+    c->stats.kernel_launches++;
+  }
   rc = launch_primary(c, A, trav, smem, false, o.collect_stats != 0, nullptr, nullptr);
   if (rc) return rc;
   // the first path list: k_primary's live pixels in tile order
@@ -601,11 +675,12 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
       c->kev.push_back(e);
     }
   }
+  if (ad) return adaptive_wave(c, A, wl, n_iter, nee, o.time_kernels != 0);
   int n_compactions = 0;
   for (int it = 0; it <= n_iter; ++it) {
     if (o.time_kernels) CU(cudaEventRecord(c->kev[c->kev_used++], c->stream));
-    if (nee) k_shade<true><<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
-    else k_shade<false><<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
+    if (nee) k_shade<true, false><<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
+    else k_shade<false, false><<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
     if (it < n_iter && (it + 1) % A.compact_every == 0) {  // close the gaps the finished pixels left, order kept (timed with k_shade)
       k_compact<<<wl.shade_grid, kCompactBlock, 0, c->stream>>>(A.slots, A.cnt + it, 0u, A.part_count, A.list[(it + 1) & 1], A.cnt + it + 1);
       ++n_compactions;
@@ -841,9 +916,12 @@ void b200rt_destroy(b200rt_ctx *c) {
   DevBuf *bufs[] = {&c->d_nodes, &c->d_tris, &c->d_ctris, &c->d_normals, &c->d_tboxes, &c->d_frames, &c->d_mats, &c->d_bvh9, &c->d_leafcnt, &c->d_prim_dirk,
                     &c->d_prim_tri, &c->d_out, &c->d_misc, &c->d_tmp_a, &c->d_tmp_b, &c->d_pA, &c->d_pB, &c->d_pC,
                     &c->d_pHit, &c->d_list0, &c->d_list1, &c->d_cnt, &c->d_slots, &c->d_part_count, &c->d_light, &c->d_pS,
-                    &c->d_pL, &c->d_pR};
+                    &c->d_pL, &c->d_pR, &c->d_welford, &c->d_ad_spp, &c->d_ad_err};
   for (DevBuf *b : bufs)
     if (b->p && !b->borrowed) cudaFree(b->p);
+  if (c->h_live) cudaFreeHost(c->h_live);
+  for (cudaEvent_t e : c->ev_batch)
+    if (e) cudaEventDestroy(e);
   if (c->ibl_tex) cudaDestroyTextureObject(c->ibl_tex);
   if (c->ibl_array) cudaFreeArray(c->ibl_array);
   if (c->d_counters) cudaFree(c->d_counters);
@@ -1086,6 +1164,45 @@ int b200rt_render(b200rt_ctx *c, const float *cam, const float *env, int width, 
   int rc = render_frame(c, cam, env, width, height, spp, max_bounce, opts, static_cast<float *>(c->d_out.p));
   if (rc) return rc;
   CU(cudaMemcpyAsync(out, c->d_out.p, bytes, cudaMemcpyDeviceToHost, c->stream));  // blocking read-back, KernelLauncher.py:78
+  CU(cudaStreamSynchronize(c->stream));
+  return read_counters(c);
+}
+
+int b200rt_render_adaptive(b200rt_ctx *c, const float *cam, const float *env, int width, int height, int spp,
+                           int max_bounce, const b200rt_opts *opts, const b200rt_adaptive *ad, float *out,
+                           int32_t *out_spp, float *out_stderr) {
+  if (!c) return B200RT_ERR_INVALID;
+  if (!out) return fail(c, B200RT_ERR_INVALID, "out_rgb is NULL");
+  b200rt_opts o;
+  if (opts) o = *opts; else b200rt_default_opts(&o);
+  int rc = check_frame_args(c, cam, width, height, spp, max_bounce, o, true, env);
+  if (rc) return rc;
+  if (!ad) return fail(c, B200RT_ERR_INVALID, "adaptive parameters are NULL");
+  if (ad->min_spp < 2 || ad->min_spp > spp)
+    return fail(c, B200RT_ERR_INVALID, "adaptive min_spp %d outside [2, spp = %d]", ad->min_spp, spp);
+  if (ad->check_every < 1) return fail(c, B200RT_ERR_INVALID, "adaptive check_every %d must be >= 1", ad->check_every);
+  if (!std::isfinite(ad->rel_error) || !(ad->rel_error >= 0.0f))
+    return fail(c, B200RT_ERR_INVALID, "adaptive rel_error %g must be finite and >= 0", (double)ad->rel_error);
+  if (!std::isfinite(ad->floor) || !(ad->floor > 0.0f))
+    return fail(c, B200RT_ERR_INVALID, "adaptive floor %g must be finite and > 0", (double)ad->floor);
+  if (o.output != B200RT_OUT_FINAL) return fail(c, B200RT_ERR_INVALID, "adaptive sampling needs B200RT_OUT_FINAL");
+  if (o.sample_end > 0 && (o.sample_begin != 0 || o.sample_end != spp))
+    return fail(c, B200RT_ERR_INVALID, "adaptive sampling needs the whole sample range [0, spp)");
+  // the stopping rule needs the pixel's samples as one serial sequence; -1 (automatic) resolves to that one stream
+  if (o.sample_streams < -1 || o.sample_streams > 1)
+    return fail(c, B200RT_ERR_INVALID, "adaptive sampling runs one sample stream (sample_streams -1, 0 or 1, got %d)",
+                o.sample_streams);
+  o.sample_streams = 1;
+  const size_t npix = (size_t)width * height;
+  CU(cudaSetDevice(c->device));
+  if (ensure(c, c->d_out, npix * 3 * sizeof(float))) return B200RT_ERR_CUDA;
+  CU(cudaMemsetAsync(c->d_out.p, 0, npix * 3 * sizeof(float), c->stream));
+  c->frame_trace_cap = 0;
+  rc = render_impl(c, cam, env, width, height, spp, max_bounce, &o, static_cast<float *>(c->d_out.p), ad);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(out, c->d_out.p, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  if (out_spp) CU(cudaMemcpyAsync(out_spp, c->d_ad_spp.p, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+  if (out_stderr) CU(cudaMemcpyAsync(out_stderr, c->d_ad_err.p, npix * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
   CU(cudaStreamSynchronize(c->stream));
   return read_counters(c);
 }

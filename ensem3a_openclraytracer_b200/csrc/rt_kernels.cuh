@@ -13,6 +13,8 @@
 //               the warp together; a lane whose ray is done writes the hit and is refilled from the list, so
 //               the node loop stays full whatever the individual traversal lengths.
 //   k_finalize / k_reduce_finalize / k_img_processing   the accumulate / clamp / tonemap passes.
+// An adaptive frame (b200rt_render_adaptive) runs k_adaptive_init before k_primary and k_shade<NEE, true>, whose
+// end_sample block also applies the stopping rule (adaptive_end_sample); the host ends its loop once the list is empty.
 #pragma once
 #include "rt_shade.cuh"
 #include "rt_trace.cuh"
@@ -26,6 +28,15 @@ constexpr int kHitNeedsExactWalk = -2;  // pHit.x of a ray k_trace did not walk 
 
 struct DeviceCounters {
   unsigned long long rays, box_tests, tri_tests, mismatches, samples, revalidated, exact_walks, primary_rays;
+};
+
+// adaptive sampling (k_shade<NEE, true>, b200rt_render_adaptive): the stopping rule of b200rt.h's b200rt_adaptive
+struct AdaptArgs {
+  float2 *welford;        // per pixel (mean, m2) of the luminance of the samples taken so far; meaningful from sample 2 on
+  int *spp_out;           // per pixel: samples taken (k_adaptive_init writes spp for every rendered pixel)
+  float *err_out;         // per pixel: standard error of the mean luminance
+  int min_spp, check_every;
+  float rel_error, floor;
 };
 
 // path state, one entry per pixel:
@@ -65,6 +76,7 @@ struct KernelArgs {
   int refill_min;         // idle lanes pull new rays once this many are idle
   int tri_quorum;         // the leaf phase repeats while at least this many lanes hold a parked leaf
   int validate;           // 1: hits come from the conservative traversal and must pass validate_hit
+  AdaptArgs ad;           // k_shade<NEE, true> and k_adaptive_init only (last, so the other kernels' parameter offsets stay)
 };
 
 RT_DEV uint32_t meta_pack(int first, int sun, int type, int j, int s, int light = 0) {
@@ -144,6 +156,54 @@ RT_DEV void write_pixel(const KernelArgs &A, int i, v3 sum) {
     o[0] = clamp01(sum.x / n);
     o[1] = clamp01(sum.y / n);
     o[2] = clamp01(sum.z / n);
+  }
+}
+
+// ---- adaptive sampling --------------------------------------------------------------------------------------------
+// Called after the n-th sample of pixel i (n counted from 1; adaptive frames always cover [0, spp)) with that sample's
+// contribution c and the running sum: the Welford update of the mean luminance and the stopping rule, exactly as
+// b200rt.h states them (binary32, no contraction).  Returns true when the pixel stops here, before spp; its image,
+// sample count and standard error are then written.  A pixel that reaches spp gets its standard error here and its
+// image from write_pixel.
+RT_DEV bool adaptive_end_sample(const KernelArgs &A, int i, int n, v3 c, v3 sum) {
+  const AdaptArgs &ad = A.ad;
+  const float y = (0.2126f * c.x + 0.7152f * c.y) + 0.0722f * c.z;
+  float2 w = n > 1 ? ad.welford[i] : make_float2(0.0f, 0.0f);
+  const float delta = y - w.x;
+  w.x = w.x + delta / (float)n;
+  w.y = w.y + delta * (y - w.x);
+  bool stop = false;
+  if (n < A.F.spp) {
+    if (n >= ad.min_spp && (n - ad.min_spp) % ad.check_every == 0) {
+      const float v = (w.y / (float)(n - 1)) / (float)n;
+      const float e = ad.rel_error * fmaxf(fminf(w.x, 1.0f), ad.floor);
+      stop = v <= e * e;   // false for a NaN anywhere: such a pixel runs to spp
+    }
+    if (!stop) {
+      ad.welford[i] = w;
+      return false;
+    }
+  }
+  ad.err_out[i] = sqrtf((w.y / (float)(n - 1)) / (float)n);
+  if (stop) {
+    ad.spp_out[i] = n;
+    float *o = A.out + 3 * (size_t)i;
+    o[0] = clamp01(sum.x / (float)n);
+    o[1] = clamp01(sum.y / (float)n);
+    o[2] = clamp01(sum.z / (float)n);
+  }
+  return stop;
+}
+
+// spp / 0 into the sample-count / standard-error maps for every pixel of the rendered set, before k_primary (ray-free
+// pixels keep these; k_shade overwrites them for the others)
+__global__ void k_adaptive_init(const __grid_constant__ KernelArgs A) {
+  for (unsigned int w = blockIdx.x * blockDim.x + threadIdx.x; w < (unsigned)A.n_work; w += gridDim.x * blockDim.x) {
+    const int i = work_to_pixel(A, w);
+    if (i >= 0) {
+      A.ad.spp_out[i] = A.F.spp;
+      A.ad.err_out[i] = 0.0f;
+    }
   }
 }
 
@@ -303,8 +363,9 @@ __global__ void __launch_bounds__(kCompactBlock) k_compact(const int *__restrict
 // (bounce hit, or sample ended and the next one starts from the cached primary hit).
 // 8 CTAs per SM: the kernel is bound by the latency of its gathers; 5-7 (no spills) and 9-12 resident CTAs were all slower.
 // NEE = opt-in light sampling (b200rt_opts.sampling bit 1): a separate instantiation, so that the reference's
-// estimator runs exactly the code it ran before.
-template <bool NEE>
+// estimator runs exactly the code it ran before.  ADAPT = adaptive sampling (adaptive_end_sample at the end of every
+// sample), likewise a separate instantiation.
+template <bool NEE, bool ADAPT>
 __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant__ KernelArgs A, int iter) {
   const FrameParams &F = A.F;
   const SceneView &S = A.S;
@@ -452,8 +513,10 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
       sum = sum + acc;  // :207
       ++s;
       ++samples;
-      if (s >= F.s1) {
-        write_pixel(A, pix, sum);
+      bool finished = s >= F.s1;
+      if (ADAPT) finished = adaptive_end_sample(A, pix, s, acc, sum) || finished;
+      if (finished) {
+        if (!ADAPT || s >= F.s1) write_pixel(A, pix, sum);
         pixel_done = true;
       } else {
         acc_px[0] = sum.x; acc_px[1] = sum.y; acc_px[2] = sum.z;

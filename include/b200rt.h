@@ -139,6 +139,40 @@ int b200rt_set_ibl(b200rt_ctx *ctx, const uint8_t *rgba, int width, int height);
 int b200rt_render(b200rt_ctx *ctx, const float *cam, const float *env, int width, int height, int spp,
                   int max_bounce, const b200rt_opts *opts, float *out_rgb);
 
+/* ---- opt-in adaptive sampling: a pixel stops taking samples once its estimated error is below a tolerance ----------
+ * The rule, in binary32 with every operation rounded separately (no contraction), true division and a correctly
+ * rounded sqrtf:
+ *   - a sample's luminance is y = (0.2126f*r + 0.7152f*g) + 0.0722f*b of its final contribution (light-sampling term
+ *     included);
+ *   - per pixel (mean, m2) start at (0, 0); after the pixel's n-th sample (n counted from 1):
+ *       delta = y - mean;  mean = mean + delta / (float)n;  m2 = m2 + delta * (y - mean);
+ *   - after sample n with n >= min_spp, (n - min_spp) % check_every == 0 and n < spp:
+ *       v = (m2 / (float)(n - 1)) / (float)n;  e = rel_error * fmaxf(fminf(mean, 1.0f), floor);
+ *     the pixel stops iff v <= e * e (false for a NaN or Inf anywhere: such a pixel runs to spp);
+ *   - a pixel that stopped after n samples is clamp01(sum / (float)n) of the same running sum a fixed-spp render
+ *     keeps, i.e. the fixed-spp render of that pixel at spp = n; a pixel that reaches spp is what b200rt_render makes;
+ *   - its standard error is sqrtf((m2 / (float)(n - 1)) / (float)n) with its final n;
+ *   - pixels whose samples need no ray (primary miss or emitter) are not subject to the rule: they are rendered as
+ *     b200rt_render renders them and report spp samples and a standard error of 0.
+ * Stopping on a noisy estimate biases the image slightly (a pixel whose first samples happen to agree stops early);
+ * rel_error bounds the noise, not that bias. */
+typedef struct {
+  int32_t min_spp;      /* samples every pixel takes before the rule is first evaluated; 2 <= min_spp <= spp */
+  int32_t check_every;  /* evaluate after every check_every-th sample from min_spp on; >= 1 */
+  float rel_error;      /* target standard error of the pixel's mean luminance, relative to max(min(mean,1), floor); finite, >= 0 */
+  float floor;          /* finite, > 0: below this luminance the target is absolute (rel_error * floor) */
+} b200rt_adaptive;
+
+/* b200rt_render with a per-pixel sample count: spp is the maximum.  out_spp (int32 per pixel) and out_stderr
+ * (float per pixel) may be NULL; entries of pixels outside the rendered set (pixel range / tile rows) are 0.
+ * opts: output must be B200RT_OUT_FINAL over the whole sample range, sample_streams -1, 0 or 1 (the rule needs one
+ * serial sequence of samples per pixel; -1 resolves to one stream and stats.sample_streams says 1); pixel ranges,
+ * tile rows, both generators, every traversal and every sampling bit are allowed.  The launch loop stops once every
+ * pixel has stopped: stats.samples, wave_iterations and kernel_launches report the work actually done. */
+int b200rt_render_adaptive(b200rt_ctx *ctx, const float *cam, const float *env, int width, int height, int spp,
+                           int max_bounce, const b200rt_opts *opts, const b200rt_adaptive *ad,
+                           float *out_rgb, int32_t *out_spp, float *out_stderr);
+
 /* Render + the 8-bit conversion of FileManager.saveImg (FileManager.py:334-338: `(data*255).astype('uint8')`, float32
  * product truncated toward zero) on the device, so that only width*height*3 BYTES cross to the host.  out_rgb8:
  * width*height*3 bytes on the HOST, row-major RGB — what PIL's Image.fromarray(..., 'RGB') takes. */

@@ -1,0 +1,102 @@
+#!/usr/bin/env python3
+"""Adaptive sampling against fixed spp at equal error, on 1920x1080 fixture scenes (Philox).
+
+Truth: the mean of four long renders (OUT_SUMS / spp), clamped to [0, 1] like the images it is compared with.  Fixed
+baseline: spp = N with sample_streams = -1 (the best non-adaptive setting).  Adaptive: spp = 4N, the default min_spp /
+check_every / floor, a sweep of rel_error.  Per scene and N, one JSON line with every run and the pick: the fastest
+adaptive render whose RMSE against the truth is at most the fixed render's, with its time ratio, mean / max spp,
+stats.samples and the relative bias of its image mean against the truth's.  Call time = host clock around the
+synchronous call (best of `repeat`), device time = stats.total_ms of that call.
+
+usage: adaptive_probe.py [--out profiles/r03_adaptive.jsonl] [--truth-spp 8192] [--n 64,256] [--rel 0.005,...]
+                         [--scenes monkey_cfg2:preview,furnace_cfg3:grey,serre:8k]"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+import ensem3a_openclraytracer_b200 as rt  # noqa: E402
+from tests import fixtures  # noqa: E402
+
+W, H, BOUNCE = 1920, 1080, 4
+DEFAULTS = dict(min_spp=16, check_every=8, floor=0.05)
+
+
+def card():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
+                       capture_output=True, text=True, check=True).stdout.strip()
+    name, power = [x.strip() for x in q.split(",")]
+    return name, power
+
+
+def timed(fn, repeat):
+    best = None
+    for _ in range(repeat):
+        t0 = time.perf_counter()
+        r = fn()
+        ms = (time.perf_counter() - t0) * 1e3
+        if best is None or ms < best[0]:
+            best = (ms, r)
+    return best
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r03_adaptive.jsonl"))
+    ap.add_argument("--truth-spp", type=int, default=8192)
+    ap.add_argument("--n", default="64,256")
+    ap.add_argument("--rel", default="0.005,0.01,0.02,0.03,0.05,0.08,0.12")
+    ap.add_argument("--scenes", default="monkey_cfg2:preview,furnace_cfg3:grey,serre:8k")
+    ap.add_argument("--repeat", type=int, default=3)
+    a = ap.parse_args()
+    name, power = card()
+    ctx = rt.Context(0)
+    with open(a.out, "a") as f:
+        for entry in a.scenes.split(","):
+            scene, ibl_name = entry.split(":")
+            sc = fixtures.load_scene(scene)
+            fixtures.upload(ctx, sc, fixtures.load_ibl(ibl_name))
+            cam, env = fixtures.cam_env(sc["params"], W, H)
+            t0 = time.perf_counter()
+            acc = np.zeros(W * H * 3)
+            for seed in range(4):
+                o = rt.make_opts(rng_mode=rt.RNG_PHILOX, seed=1000 + seed, output=rt.OUT_SUMS, sample_streams=-1)
+                acc += ctx.render(cam, env, W, H, a.truth_spp, BOUNCE, opts=o).astype(np.float64) / a.truth_spp
+            truth = np.clip(acc / 4, 0.0, 1.0).reshape(H, W, 3)
+            truth_s = time.perf_counter() - t0
+            for n in (int(x) for x in a.n.split(",")):
+                o = rt.make_opts(rng_mode=rt.RNG_PHILOX, seed=1, sample_streams=-1)
+                ms, img = timed(lambda: ctx.render(cam, env, W, H, n, BOUNCE, opts=o), a.repeat)
+                st = ctx.stats()
+                fixed = dict(spp=n, call_ms=ms, device_ms=st["total_ms"], samples=st["samples"],
+                             rmse=float(np.sqrt(np.mean((img.reshape(H, W, 3) - truth) ** 2))))
+                runs = []
+                for rel in (float(x) for x in a.rel.split(",")):
+                    oa = rt.make_opts(rng_mode=rt.RNG_PHILOX, seed=1)
+                    ms, (img, spp_map, _) = timed(lambda: ctx.render_adaptive(cam, env, W, H, 4 * n, BOUNCE, rel_error=rel,
+                                                                                opts=oa, **DEFAULTS), a.repeat)
+                    st = ctx.stats()
+                    runs.append(dict(rel_error=rel, call_ms=ms, device_ms=st["total_ms"], samples=st["samples"],
+                                     wave_iterations=st["wave_iterations"], mean_spp=float(spp_map.mean()),
+                                     max_spp=int(spp_map.max()), rmse=float(np.sqrt(np.mean((img - truth) ** 2))),
+                                     rel_bias=float((img.mean() - truth.mean()) / truth.mean())))
+                ok = [r for r in runs if r["rmse"] <= fixed["rmse"]]
+                pick = min(ok, key=lambda r: r["call_ms"]) if ok else None
+                line = dict(tool="adaptive_probe", card=name, power_limit=power, scene=scene, ibl=ibl_name, width=W,
+                            height=H, max_bounce=BOUNCE, truth_spp=a.truth_spp, truth_renders=4, truth_seconds=truth_s,
+                            adaptive_defaults=DEFAULTS, fixed=fixed, adaptive_max_spp=4 * n, runs=runs, pick=pick,
+                            time_ratio=(pick["call_ms"] / fixed["call_ms"]) if pick else None)
+                print(json.dumps(line), flush=True)
+                f.write(json.dumps(line) + "\n")
+                f.flush()
+    ctx.close()
+
+
+if __name__ == "__main__":
+    main()
