@@ -116,22 +116,20 @@ def load_library():
     lib.b200rt_ipc_open.argtypes = [vp, vp, ctypes.POINTER(vp)]
     lib.b200rt_ipc_close.argtypes = [vp, vp]
     lib.b200rt_build_bvh.argtypes = [vp, i64, vp, i64, vp, i64, ctypes.POINTER(ctypes.c_int32)]
-    if "b200rt_repack_probe" in SYMBOLS:
-        lib.b200rt_repack_probe.argtypes = [vp, i64, vp, i64, vp, i64, i64, vp, i64, vp, i64, vp, vp]
-    if "b200rt_multi_create" in SYMBOLS:
-        lib.b200rt_multi_create.argtypes = [ctypes.POINTER(ctypes.c_int), i32, ctypes.POINTER(vp)]
-        lib.b200rt_multi_destroy.restype = None
-        lib.b200rt_multi_destroy.argtypes = [vp]
-        lib.b200rt_multi_last_error.restype = ctypes.c_char_p
-        lib.b200rt_multi_last_error.argtypes = [vp]
-        lib.b200rt_multi_device_count.argtypes = [vp]
-        lib.b200rt_multi_context.restype = vp
-        lib.b200rt_multi_context.argtypes = [vp, i32]
-        lib.b200rt_multi_set_scene.argtypes = [vp, vp, i64, vp, i64, vp, i64, vp, i64, vp, i64, vp, i64, vp, i64]
-        lib.b200rt_multi_set_ibl.argtypes = [vp, vp, i32, i32]
-        lib.b200rt_multi_invalidate.argtypes = [vp]
-        lib.b200rt_multi_render.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), vp]
-        lib.b200rt_multi_get_stats.argtypes = [vp, ctypes.POINTER(Stats)]
+    lib.b200rt_repack_probe.argtypes = [vp, i64, vp, i64, vp, i64, i64, vp, i64, vp, i64, vp, vp]
+    lib.b200rt_multi_create.argtypes = [ctypes.POINTER(ctypes.c_int), i32, ctypes.POINTER(vp)]
+    lib.b200rt_multi_destroy.restype = None
+    lib.b200rt_multi_destroy.argtypes = [vp]
+    lib.b200rt_multi_last_error.restype = ctypes.c_char_p
+    lib.b200rt_multi_last_error.argtypes = [vp]
+    lib.b200rt_multi_device_count.argtypes = [vp]
+    lib.b200rt_multi_context.restype = vp
+    lib.b200rt_multi_context.argtypes = [vp, i32]
+    lib.b200rt_multi_set_scene.argtypes = [vp, vp, i64, vp, i64, vp, i64, vp, i64, vp, i64, vp, i64, vp, i64]
+    lib.b200rt_multi_set_ibl.argtypes = [vp, vp, i32, i32]
+    lib.b200rt_multi_invalidate.argtypes = [vp]
+    lib.b200rt_multi_render.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), vp]
+    lib.b200rt_multi_get_stats.argtypes = [vp, ctypes.POINTER(Stats)]
     for name in SYMBOLS:
         fn = getattr(lib, name)
         if name not in ("b200rt_version", "b200rt_last_error", "b200rt_default_opts", "b200rt_destroy",
@@ -186,7 +184,7 @@ def build_bvh(face_data, vertex_p, return_depth=False):
 def device_count():
     """CUDA devices visible to the process."""
     lib = load_library()
-    return int(lib.b200rt_device_count()) if hasattr(lib, "b200rt_device_count") else 0
+    return int(lib.b200rt_device_count())
 
 
 def repack_probe(vertex_p, vertex_n, face_data, n_materials, bvh):
@@ -211,7 +209,73 @@ def repack_probe(vertex_p, vertex_n, face_data, n_materials, bvh):
     return nodes, d
 
 
-class Context:
+class _Handle:
+    """What Context and MultiContext share: the calls whose C symbols differ only in the prefix (`b200rt_` or
+    `b200rt_multi_`), and errors reported with the prefix's last-error getter."""
+
+    _prefix = "b200rt_"
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _check(self, rc, what):
+        if rc != 0:
+            err = getattr(self._lib, self._prefix + "last_error")(self._h).decode()
+            raise B200RTError(f"{what} failed ({rc}): {err}")
+
+    def _call(self, name, *args):
+        fn = self._prefix + name
+        self._check(getattr(self._lib, fn)(self._h, *args), fn)
+
+    # ---- uploads -----------------------------------------------------------------------------------
+    def set_scene(self, vertex_p, vertex_n, vertex_uv, face_data, material_data, light_data, bvh):
+        vp_, vn_, vuv_ = _f32(vertex_p), _f32(vertex_n), _f32(vertex_uv)
+        face, mat, bvh_ = _i32(face_data), _f32(material_data), _f32(bvh)
+        light = _i32(light_data) if light_data is not None and len(light_data) else None
+        self._call("set_scene", _ptr(vp_), vp_.size, _ptr(vn_), vn_.size, _ptr(vuv_), vuv_.size, _ptr(face), face.size,
+                   _ptr(mat), mat.size, _ptr(light), 0 if light is None else light.size, _ptr(bvh_), bvh_.size)
+
+    def set_ibl(self, rgba, width=None, height=None):
+        """rgba: (H, W, 4) uint8 array, or bytes with explicit width/height."""
+        if isinstance(rgba, (bytes, bytearray, memoryview)):
+            arr = np.frombuffer(rgba, dtype=np.uint8)
+        else:
+            arr = np.ascontiguousarray(rgba, dtype=np.uint8)
+            if width is None:
+                height, width = arr.shape[0], arr.shape[1]
+            arr = arr.reshape(-1)
+        if arr.size != int(width) * int(height) * 4:
+            raise B200RTError(f"environment map: {arr.size} bytes for {width}x{height} RGBA")
+        self._call("set_ibl", _ptr(arr), int(width), int(height))
+
+    def invalidate(self):
+        self._call("invalidate")
+
+    # ---- rendering ------------------------------------------------------------------------------------
+    def render(self, cam, env, width, height, spp, max_bounce, out=None, opts=None):
+        cam_, env_ = _f32(cam), _f32(env)
+        if cam_.size != 10 or env_.size != 5:
+            raise B200RTError("cam must hold 10 floats and envData 5 (main.py:59-61,72-73)")
+        n = int(width) * int(height) * 3
+        if out is None:
+            out = np.zeros(n, dtype=np.float32)
+        if out.dtype != np.float32 or not out.flags["C_CONTIGUOUS"] or out.size != n:
+            raise B200RTError(f"out must be a C-contiguous float32 array of {n} elements")
+        o = opts if opts is not None else make_opts()
+        self._call("render", _ptr(cam_), _ptr(env_), int(width), int(height), int(spp), int(max_bounce), ctypes.byref(o),
+                   _ptr(out))
+        return out
+
+    def stats(self):
+        s = Stats()
+        self._call("get_stats", ctypes.byref(s))
+        return s.as_dict()
+
+
+class Context(_Handle):
     """One GPU.  Thin, 1:1 over the C ABI; numpy in, numpy out."""
 
     def __init__(self, device=0, _borrowed=None):
@@ -234,58 +298,11 @@ class Context:
                 self._lib.b200rt_destroy(self._h)
             self._h = None
 
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def _check(self, rc, what):
-        if rc != 0:
-            raise B200RTError(f"{what} failed ({rc}): {self._lib.b200rt_last_error(self._h).decode()}")
-
-    # ---- uploads -----------------------------------------------------------------------------------
-    def set_scene(self, vertex_p, vertex_n, vertex_uv, face_data, material_data, light_data, bvh):
-        vp_, vn_, vuv_ = _f32(vertex_p), _f32(vertex_n), _f32(vertex_uv)
-        face, mat, bvh_ = _i32(face_data), _f32(material_data), _f32(bvh)
-        light = _i32(light_data) if light_data is not None and len(light_data) else None
-        self._check(self._lib.b200rt_set_scene(self._h, _ptr(vp_), vp_.size, _ptr(vn_), vn_.size, _ptr(vuv_), vuv_.size,
-                                               _ptr(face), face.size, _ptr(mat), mat.size, _ptr(light),
-                                               0 if light is None else light.size, _ptr(bvh_), bvh_.size),
-                    "b200rt_set_scene")
-
     def set_materials(self, material_data):
         mat = _f32(material_data)
         self._check(self._lib.b200rt_set_materials(self._h, _ptr(mat), mat.size), "b200rt_set_materials")
 
-    def set_ibl(self, rgba, width=None, height=None):
-        """rgba: (H, W, 4) uint8 array, or bytes with explicit width/height."""
-        if isinstance(rgba, (bytes, bytearray, memoryview)):
-            arr = np.frombuffer(rgba, dtype=np.uint8)
-        else:
-            arr = np.ascontiguousarray(rgba, dtype=np.uint8)
-            if width is None:
-                height, width = arr.shape[0], arr.shape[1]
-            arr = arr.reshape(-1)
-        if arr.size != int(width) * int(height) * 4:
-            raise B200RTError(f"environment map: {arr.size} bytes for {width}x{height} RGBA")
-        self._check(self._lib.b200rt_set_ibl(self._h, _ptr(arr), int(width), int(height)), "b200rt_set_ibl")
-
     # ---- rendering ------------------------------------------------------------------------------------
-    def render(self, cam, env, width, height, spp, max_bounce, out=None, opts=None):
-        cam_, env_ = _f32(cam), _f32(env)
-        if cam_.size != 10 or env_.size != 5:
-            raise B200RTError("cam must hold 10 floats and envData 5 (main.py:59-61,72-73)")
-        n = int(width) * int(height) * 3
-        if out is None:
-            out = np.zeros(n, dtype=np.float32)
-        if out.dtype != np.float32 or not out.flags["C_CONTIGUOUS"] or out.size != n:
-            raise B200RTError(f"out must be a C-contiguous float32 array of {n} elements")
-        o = opts if opts is not None else make_opts()
-        self._check(self._lib.b200rt_render(self._h, _ptr(cam_), _ptr(env_), int(width), int(height), int(spp),
-                                            int(max_bounce), ctypes.byref(o), _ptr(out)), "b200rt_render")
-        return out
-
     def render_adaptive(self, cam, env, width, height, spp, max_bounce, rel_error, min_spp=16, check_every=8, floor=0.05,
                         opts=None):
         """Adaptive sampling (b200rt_render_adaptive): every pixel takes at least min_spp and at most spp samples and
@@ -345,9 +362,6 @@ class Context:
             h = ctypes.c_void_p(int(cuda_stream) or 1)
         self._check(self._lib.b200rt_set_stream(self._h, h), "b200rt_set_stream")
 
-    def invalidate(self):
-        self._check(self._lib.b200rt_invalidate(self._h), "b200rt_invalidate")
-
     def primary_hits(self, cam, width, height, opts=None):
         cam_ = _f32(cam)
         n = int(width) * int(height)
@@ -377,11 +391,6 @@ class Context:
             raise B200RTError("src/dst smaller than the global size")
         self._check(self._lib.b200rt_img_processing(self._h, _ptr(src_), _ptr(dst), int(n), g), "b200rt_img_processing")
         return dst
-
-    def stats(self):
-        s = Stats()
-        self._check(self._lib.b200rt_get_stats(self._h, ctypes.byref(s)), "b200rt_get_stats")
-        return s.as_dict()
 
     # ---- probes ---------------------------------------------------------------------------------------------
     def math_probe(self, fn, a, b=None):
@@ -423,9 +432,11 @@ class Context:
         self._check(self._lib.b200rt_ipc_close(self._h, ctypes.c_void_p(int(d_ptr))), "b200rt_ipc_close")
 
 
-class MultiContext:
+class MultiContext(_Handle):
     """Several GPUs of one box behind one handle (b200rt_multi_*): same set_scene / set_ibl / render / stats surface as
     Context, the frame divided among the GPUs inside the library.  `contexts[i]` are the per-GPU contexts (lent)."""
+
+    _prefix = "b200rt_multi_"
 
     def __init__(self, devices):
         self._lib = load_library()
@@ -446,59 +457,6 @@ class MultiContext:
                 c.close()
             self._lib.b200rt_multi_destroy(self._h)
             self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def _check(self, rc, what):
-        if rc != 0:
-            raise B200RTError(f"{what} failed ({rc}): {self._lib.b200rt_multi_last_error(self._h).decode()}")
-
-    def set_scene(self, vertex_p, vertex_n, vertex_uv, face_data, material_data, light_data, bvh):
-        vp_, vn_, vuv_ = _f32(vertex_p), _f32(vertex_n), _f32(vertex_uv)
-        face, mat, bvh_ = _i32(face_data), _f32(material_data), _f32(bvh)
-        light = _i32(light_data) if light_data is not None and len(light_data) else None
-        self._check(self._lib.b200rt_multi_set_scene(self._h, _ptr(vp_), vp_.size, _ptr(vn_), vn_.size, _ptr(vuv_), vuv_.size,
-                                                     _ptr(face), face.size, _ptr(mat), mat.size, _ptr(light),
-                                                     0 if light is None else light.size, _ptr(bvh_), bvh_.size),
-                    "b200rt_multi_set_scene")
-
-    def set_ibl(self, rgba, width=None, height=None):
-        if isinstance(rgba, (bytes, bytearray, memoryview)):
-            arr = np.frombuffer(rgba, dtype=np.uint8)
-        else:
-            arr = np.ascontiguousarray(rgba, dtype=np.uint8)
-            if width is None:
-                height, width = arr.shape[0], arr.shape[1]
-            arr = arr.reshape(-1)
-        if arr.size != int(width) * int(height) * 4:
-            raise B200RTError(f"environment map: {arr.size} bytes for {width}x{height} RGBA")
-        self._check(self._lib.b200rt_multi_set_ibl(self._h, _ptr(arr), int(width), int(height)), "b200rt_multi_set_ibl")
-
-    def invalidate(self):
-        self._check(self._lib.b200rt_multi_invalidate(self._h), "b200rt_multi_invalidate")
-
-    def render(self, cam, env, width, height, spp, max_bounce, out=None, opts=None):
-        cam_, env_ = _f32(cam), _f32(env)
-        if cam_.size != 10 or env_.size != 5:
-            raise B200RTError("cam must hold 10 floats and envData 5 (main.py:59-61,72-73)")
-        n = int(width) * int(height) * 3
-        if out is None:
-            out = np.zeros(n, dtype=np.float32)
-        if out.dtype != np.float32 or not out.flags["C_CONTIGUOUS"] or out.size != n:
-            raise B200RTError(f"out must be a C-contiguous float32 array of {n} elements")
-        o = opts if opts is not None else make_opts()
-        self._check(self._lib.b200rt_multi_render(self._h, _ptr(cam_), _ptr(env_), int(width), int(height), int(spp),
-                                                  int(max_bounce), ctypes.byref(o), _ptr(out)), "b200rt_multi_render")
-        return out
-
-    def stats(self):
-        s = Stats()
-        self._check(self._lib.b200rt_multi_get_stats(self._h, ctypes.byref(s)), "b200rt_multi_get_stats")
-        return s.as_dict()
 
     def img_processing(self, src, dst, n, global_size=None):
         return self.contexts[0].img_processing(src, dst, n, global_size)

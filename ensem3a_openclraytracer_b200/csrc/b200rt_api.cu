@@ -11,6 +11,7 @@
 #include <cstring>
 #include <chrono>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/b200rt.h"
@@ -29,6 +30,18 @@ struct DevBuf {
   bool borrowed = false;  // a helper context's view of its parent's scene buffer: never freed or resized here
 };
 
+// the scene's device buffers, which sample-stream helpers borrow as a set
+enum SceneBuf { kNodes, kTris, kCtris, kNormals, kTboxes, kFrames, kMats, kBvh9, kLeafcnt, kLight, kSceneBufs };
+
+// k_trace's lane scheduling (KernelArgs::quorum, refill_min, tri_quorum) and the wavefront iterations between two
+// compactions of the path list
+constexpr int kQuorum = 12, kRefillMin = 8, kTriQuorum = 2;
+constexpr int kCompactEvery = 4;
+// Resident k_trace CTAs per SM while three or more sample streams share the GPU.  A k_trace that fills every SM's
+// register file leaves the other streams' kernels nothing but its tail to run in; capped, one stream's shading and
+// another's tracing are resident side by side (bench scene -4 %, Cornell 1080p -12 %, measured with 3 streams).
+constexpr int kStreamTraceCtas = 4;
+
 }  // namespace
 
 struct b200rt_ctx {
@@ -46,27 +59,12 @@ struct b200rt_ctx {
   bool have_scene = false;
   bool have_scene_cached = false;  // scene_hash / ibl_hash are valid
   uint64_t scene_hash = 0, mat_hash = 0;
-  DevBuf d_nodes, d_tris, d_ctris, d_normals, d_tboxes, d_frames, d_mats, d_bvh9, d_leafcnt;
-  int n_nodes9 = 0, n_inner = 0, n_tris = 0, n_mats = 0;
-  int depth = 0, ref_stack_need = 0;
-  int cull_depth = 0;      // depth of the tree the node records hold (the culling tree, scene_repack.h)
-  bool canonical = true;
-  int root_ref = 0;
-  int node_f4 = 2;
-  float grid_base[3] = {0, 0, 0}, grid_pitch[3] = {1, 1, 1};
-  uint32_t root_w[3] = {0x7fff0000u, 0x7fff0000u, 0x7fff0000u};
-  float cull_abs = 0.0f, cmax = 0.0f;
-  int fast_ok = 1;
-  // k_trace tuning knobs (B200RT_QUORUM / B200RT_REFILL_MIN / B200RT_TRI_QUORUM / B200RT_STEPS override)
-  int quorum = 12, refill_min = 8, tri_quorum = 2;
-  int carveout = -1;       // B200RT_CARVEOUT: k_trace's shared-memory carve-out (-1 driver's choice, 0 computed, else per cent)
-  int max_trace_ctas = 0;  // B200RT_MAX_TRACE_CTAS: cap on resident k_trace CTAs per SM (0 = what fits)
-  int stream_trace_ctas = 4;  // B200RT_STREAM_TRACE_CTAS: the cap while three or more sample streams share the GPU (0 = none)
-  int frame_trace_cap = 0; // the cap of the frame being enqueued (set by render_frame)
-  int compact_every = 4;   // B200RT_COMPACT_EVERY: wavefront iterations between two compactions of the path list
-  std::vector<int32_t> tri_mat;  // for re-validating material edits
-  DevBuf d_light;                // triangles whose material is emissive, ascending (opt-in light sampling)
+  DevBuf d_scene[kSceneBufs];  // kLight: triangles whose material is emissive, ascending (opt-in light sampling)
+  SceneDesc scene;
+  int n_mats = 0;
   int n_light = 0;
+  int frame_trace_cap = 0; // resident k_trace CTAs per SM in the frame being enqueued (0 = what fits; set by render_frame)
+  std::vector<int32_t> tri_mat;  // for re-validating material edits
   DevBuf d_pS, d_pL, d_pR;       // light sampling: three more float4 of path state
 
   // environment map
@@ -207,13 +205,13 @@ void frame_setup(const b200rt_ctx *c, const float *cam, const float *env, int wi
   F->sampling = o.sampling;
 }
 
-size_t scene_smem_bytes(const b200rt_ctx *c) { return (size_t)c->n_inner * 48 + (size_t)c->n_tris * 48; }
+size_t scene_smem_bytes(const b200rt_ctx *c) { return (size_t)c->scene.n_inner * 48 + (size_t)c->scene.n_tris * 48; }
 
-bool use_smem_scene(const b200rt_ctx *c) { return c->node_f4 == 3; }
+bool use_smem_scene(const b200rt_ctx *c) { return c->scene.node_f4 == 3; }
 
 // entries of the per-lane shared-memory traversal stack: the near-first walk holds at most one entry per level;
 // trees walked in reference order keep their stack in thread-local memory instead
-int stack_entries(const b200rt_ctx *c) { return c->canonical ? c->cull_depth + 2 : 2; }
+int stack_entries(const b200rt_ctx *c) { return c->scene.canonical ? c->scene.cull_depth + 2 : 2; }
 
 size_t smem_bytes(const b200rt_ctx *c, bool smem_scene) {
   return lane_smem_bytes(stack_entries(c)) + (smem_scene ? scene_smem_bytes(c) : 0);
@@ -223,35 +221,37 @@ int effective_stack_cap(const b200rt_ctx *c, const b200rt_opts &o);
 
 void fill_args(b200rt_ctx *c, const FrameParams &F, const b200rt_opts &o, float *d_out, KernelArgs *A) {
   A->F = F;
+  const SceneDesc &D = c->scene;
+  const DevBuf *B = c->d_scene;
   SceneView &S = A->S;
-  S.nodes = static_cast<const uint4 *>(c->d_nodes.p);
-  S.node_f4 = c->node_f4;
-  S.tris = static_cast<const float4 *>(c->d_tris.p);
-  S.ctris = static_cast<const float4 *>(c->d_ctris.p);
-  S.normals = static_cast<const float4 *>(c->d_normals.p);
-  S.tboxes = static_cast<const float4 *>(c->d_tboxes.p);
-  S.frames = static_cast<const float4 *>(c->d_frames.p);
-  S.mats = static_cast<const float *>(c->d_mats.p);
-  S.bvh9 = static_cast<const float *>(c->d_bvh9.p);
-  S.leafcnt = static_cast<const int *>(c->d_leafcnt.p);
-  S.root_ref = c->root_ref;
+  S.nodes = static_cast<const uint4 *>(B[kNodes].p);
+  S.node_f4 = D.node_f4;
+  S.tris = static_cast<const float4 *>(B[kTris].p);
+  S.ctris = static_cast<const float4 *>(B[kCtris].p);
+  S.normals = static_cast<const float4 *>(B[kNormals].p);
+  S.tboxes = static_cast<const float4 *>(B[kTboxes].p);
+  S.frames = static_cast<const float4 *>(B[kFrames].p);
+  S.mats = static_cast<const float *>(B[kMats].p);
+  S.bvh9 = static_cast<const float *>(B[kBvh9].p);
+  S.leafcnt = static_cast<const int *>(B[kLeafcnt].p);
+  S.root_ref = D.root_ref;
   for (int i = 0; i < 3; ++i) {
-    S.grid_base[i] = c->grid_base[i];
-    S.grid_pitch[i] = c->grid_pitch[i];
-    S.root_w[i] = c->root_w[i];
+    S.grid_base[i] = D.grid_base[i];
+    S.grid_pitch[i] = D.grid_pitch[i];
+    S.root_w[i] = D.root_w[i];
   }
-  S.cull_abs = c->cull_abs;
-  S.cmax = c->cmax;
+  S.cull_abs = D.cull_abs;
+  S.cmax = D.cmax;
   {
     // traversal-stack entry layout (rt_trace.cuh, LaneStack): 2^E above every culling limit, refs in the low bits
-    const int E = std::ilogb((1001.0f + c->cull_abs) * 1.01f) + 1;
+    const int E = std::ilogb((1001.0f + D.cull_abs) * 1.01f) + 1;
     S.st_bias = (uint32_t)(E - 32 + 127) << 23;
     unsigned long long m = 1;
-    while (m < (unsigned long long)std::max(1, c->n_inner) * (unsigned long long)std::max(1, c->node_f4)) m <<= 1;
+    while (m < (unsigned long long)std::max(1, D.n_inner) * (unsigned long long)std::max(1, D.node_f4)) m <<= 1;
     S.st_rmask = (uint32_t)(m - 1ull);
   }
   S.stack_cap = effective_stack_cap(c, o);
-  S.fast_ok = c->fast_ok;
+  S.fast_ok = D.fast_ok;
   A->ibl = c->ibl_tex;
   A->prim_dirk = static_cast<float4 *>(c->d_prim_dirk.p);
   A->prim_tri = static_cast<int *>(c->d_prim_tri.p);
@@ -260,7 +260,7 @@ void fill_args(b200rt_ctx *c, const FrameParams &F, const b200rt_opts &o, float 
   A->pB = static_cast<float4 *>(c->d_pB.p);
   A->pC = static_cast<float4 *>(c->d_pC.p);
   A->pHit = static_cast<int2 *>(c->d_pHit.p);
-  A->light = static_cast<const int *>(c->d_light.p);
+  A->light = static_cast<const int *>(B[kLight].p);
   A->n_light = c->n_light;
   A->pS = static_cast<float4 *>(c->d_pS.p);
   A->pL = static_cast<float4 *>(c->d_pL.p);
@@ -271,17 +271,17 @@ void fill_args(b200rt_ctx *c, const FrameParams &F, const b200rt_opts &o, float 
   A->slots = static_cast<int *>(c->d_slots.p);
   A->part_count = static_cast<unsigned int *>(c->d_part_count.p);
   A->wc = nullptr;
-  A->compact_every = c->compact_every;
+  A->compact_every = kCompactEvery;
   A->counters = c->d_counters;
-  A->n_nodes = c->n_inner;
-  A->n_tris = c->n_tris;
+  A->n_nodes = D.n_inner;
+  A->n_tris = D.n_tris;
   A->stack_depth = stack_entries(c);
   A->tiles_x = (F.width + 7) / 8;
   int tiles_y = (F.height + 3) / 4;
   A->n_work = A->tiles_x * tiles_y * 32;
-  A->quorum = c->quorum;
-  A->refill_min = c->refill_min;
-  A->tri_quorum = c->tri_quorum;
+  A->quorum = kQuorum;
+  A->refill_min = kRefillMin;
+  A->tri_quorum = kTriQuorum;
   A->validate = 0;
   A->ad = AdaptArgs();
 }
@@ -290,12 +290,12 @@ void fill_args(b200rt_ctx *c, const FrameParams &F, const b200rt_opts &o, float 
 // the caller asked for FAST (a walk that never drops a push) the substitute keeps that promise as far as its
 // thread-local stack reaches: it runs with the largest cap instead of the reference's 20.
 int effective_traversal(const b200rt_ctx *c, const b200rt_opts &o) {
-  if (!c->canonical) return B200RT_TRAVERSAL_REFERENCE;
+  if (!c->scene.canonical) return B200RT_TRAVERSAL_REFERENCE;
   return o.traversal;
 }
 
 int effective_stack_cap(const b200rt_ctx *c, const b200rt_opts &o) {
-  if (!c->canonical && o.traversal == B200RT_TRAVERSAL_FAST) return kRefStack;
+  if (!c->scene.canonical && o.traversal == B200RT_TRAVERSAL_FAST) return kRefStack;
   return o.stack_cap <= 0 ? 20 : (o.stack_cap > kRefStack ? kRefStack : o.stack_cap);
 }
 
@@ -314,6 +314,28 @@ int persistent_grid(b200rt_ctx *c, K kernel, size_t smem, int *grid) {
   return 0;
 }
 
+// Calls f(trav, smem, stats) with the three as std::integral_constant, so that f can name the kernel instance.  VERIFY
+// has no STATS instance: asked for stats, it runs the one without.
+template <int TRAV, bool SMEM, class F>
+int with_stats(bool stats, F &f) {
+  using T = std::integral_constant<int, TRAV>;
+  using S = std::bool_constant<SMEM>;
+  if constexpr (TRAV != B200RT_TRAVERSAL_VERIFY) {
+    if (stats) return f(T{}, S{}, std::true_type{});
+  }
+  return f(T{}, S{}, std::false_type{});
+}
+
+template <class F>
+int with_variant(b200rt_ctx *c, int trav, bool smem, bool stats, F &&f) {
+  switch (trav) {
+    case 0: return smem ? with_stats<0, true>(stats, f) : with_stats<0, false>(stats, f);
+    case 1: return smem ? with_stats<1, true>(stats, f) : with_stats<1, false>(stats, f);
+    case 2: return smem ? with_stats<2, true>(stats, f) : with_stats<2, false>(stats, f);
+  }
+  return fail(c, B200RT_ERR_INVALID, "bad traversal mode %d", trav);
+}
+
 template <int TRAV, bool SMEM, bool PARITY, bool STATS>
 int launch_primary_t(b200rt_ctx *c, const KernelArgs &A, int *tri_out, float *k_out) {
   auto k = k_primary<TRAV, SMEM, PARITY, STATS>;
@@ -329,30 +351,19 @@ int launch_primary_t(b200rt_ctx *c, const KernelArgs &A, int *tri_out, float *k_
   return 0;
 }
 
-template <int TRAV, bool SMEM>
-int launch_primary_ts(b200rt_ctx *c, const KernelArgs &A, bool parity, bool stats, int *tri_out, float *k_out) {
-  if (TRAV == 2) stats = false;
-  if (parity) return stats ? launch_primary_t<TRAV, SMEM, true, (TRAV != 2)>(c, A, tri_out, k_out)
-                           : launch_primary_t<TRAV, SMEM, true, false>(c, A, tri_out, k_out);
-  return stats ? launch_primary_t<TRAV, SMEM, false, (TRAV != 2)>(c, A, tri_out, k_out)
-               : launch_primary_t<TRAV, SMEM, false, false>(c, A, tri_out, k_out);
-}
-
 int launch_primary(b200rt_ctx *c, const KernelArgs &A, int trav, bool smem, bool parity, bool stats, int *tri_out,
                    float *k_out) {
-  switch (trav * 2 + (smem ? 1 : 0)) {
-    case 0: return launch_primary_ts<0, false>(c, A, parity, stats, tri_out, k_out);
-    case 1: return launch_primary_ts<0, true>(c, A, parity, stats, tri_out, k_out);
-    case 2: return launch_primary_ts<1, false>(c, A, parity, stats, tri_out, k_out);
-    case 3: return launch_primary_ts<1, true>(c, A, parity, stats, tri_out, k_out);
-    case 4: return launch_primary_ts<2, false>(c, A, parity, stats, tri_out, k_out);
-    case 5: return launch_primary_ts<2, true>(c, A, parity, stats, tri_out, k_out);
-  }
-  return fail(c, B200RT_ERR_INVALID, "bad traversal mode %d", trav);
+  return with_variant(c, trav, smem, stats, [&](auto t, auto s, auto st) {
+    constexpr int T = decltype(t)::value;
+    constexpr bool S = decltype(s)::value, ST = decltype(st)::value;
+    return parity ? launch_primary_t<T, S, true, ST>(c, A, tri_out, k_out)
+                  : launch_primary_t<T, S, false, ST>(c, A, tri_out, k_out);
+  });
 }
 
 // Launch geometry of the wavefront kernels, resolved once per frame (the occupancy queries are host calls)
 struct WaveLaunch {
+  void (*shade)(const KernelArgs, int) = nullptr;
   void (*trace)(const KernelArgs, int) = nullptr;
   int trace_grid = 0;
   size_t trace_smem = 0;
@@ -365,45 +376,22 @@ int prepare_trace_t(b200rt_ctx *c, WaveLaunch *w) {
   w->trace_smem = smem_bytes(c, SMEM);
   if (set_smem_attr(c, k, w->trace_smem)) return B200RT_ERR_CUDA;
   if (persistent_grid(c, k, w->trace_smem, &w->trace_grid)) return B200RT_ERR_CUDA;
-  if (c->carveout >= 0) {
-    // shared memory is carved out of the SM's L1: ask for what the resident CTAs need (+1 KB each, the system's share)
-    // and no more, so that the rest keeps caching nodes and triangles
-    int pct = c->carveout;
-    if (pct == 0) {
-      const size_t need = (size_t)(w->trace_grid / c->sm_count) * (w->trace_smem + 1024);
-      pct = (int)((need * 100 + 228 * 1024 - 1) / (228 * 1024));
-    }
-    if (pct > 100) pct = 100;
-    CU(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
-  }
-  // With several sample streams on the GPU a k_trace that fills every SM's register file leaves the other streams'
-  // kernels nothing but its tail to run in; capped, one stream's shading and another's tracing are resident side by side
-  // (bench scene -4 %, Cornell 1080p -12 %, measured with 3 streams and 4 CTAs per SM).
-  const int cap = c->max_trace_ctas > 0 ? c->max_trace_ctas : c->frame_trace_cap;
+  const int cap = c->frame_trace_cap;
   if (cap > 0 && w->trace_grid > cap * c->sm_count) w->trace_grid = cap * c->sm_count;
   w->trace = k;
   return 0;
 }
 
-int prepare_wave(b200rt_ctx *c, int trav, bool smem, bool stats, WaveLaunch *w) {
+int prepare_wave(b200rt_ctx *c, int trav, bool smem, bool stats, bool nee, bool adaptive, WaveLaunch *w) {
   int per_sm = 0;
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shade<false, false>, kShadeBlock, 0));
   if (per_sm < 1) return fail(c, B200RT_ERR_CUDA, "k_shade does not fit on an SM");
   w->shade_grid = per_sm * c->sm_count;
-  int key = trav * 4 + (smem ? 2 : 0) + (stats ? 1 : 0);
-  switch (key) {
-    case 0: return prepare_trace_t<0, false, false>(c, w);
-    case 1: return prepare_trace_t<0, false, true>(c, w);
-    case 2: return prepare_trace_t<0, true, false>(c, w);
-    case 3: return prepare_trace_t<0, true, true>(c, w);
-    case 4: return prepare_trace_t<1, false, false>(c, w);
-    case 5: return prepare_trace_t<1, false, true>(c, w);
-    case 6: return prepare_trace_t<1, true, false>(c, w);
-    case 7: return prepare_trace_t<1, true, true>(c, w);
-    case 8: case 9: return prepare_trace_t<2, false, false>(c, w);
-    case 10: case 11: return prepare_trace_t<2, true, false>(c, w);
-  }
-  return fail(c, B200RT_ERR_INVALID, "bad traversal mode %d", trav);
+  if (nee) w->shade = adaptive ? k_shade<true, true> : k_shade<true, false>;
+  else w->shade = adaptive ? k_shade<false, true> : k_shade<false, false>;
+  return with_variant(c, trav, smem, stats, [&](auto t, auto s, auto st) {
+    return prepare_trace_t<decltype(t)::value, decltype(s)::value, decltype(st)::value>(c, w);
+  });
 }
 
 template <int TRAV, bool SMEM, bool STATS>
@@ -440,28 +428,24 @@ int read_counters_one(b200rt_ctx *c) {
   if (cudaEventElapsedTime(&ms, c->ev[0], c->ev[2]) == cudaSuccess) c->stats.total_ms = ms;
   c->stats.shade_kernel_ms = 0.0f;
   c->stats.trace_kernel_ms = 0.0f;
-  // B200RT_DUMP_WAVE=<file> (development): one line per wavefront iteration — live paths, k_shade ms, k_trace ms
-  FILE *dump = nullptr;
-  std::vector<unsigned int> live;
-  if (c->kev_used > 1)
-    if (const char *path = getenv("B200RT_DUMP_WAVE")) {
-      dump = fopen(path, "w");
-      live.resize((size_t)c->kev_used / 2 + 2, 0u);
-      if (cudaMemcpy(live.data(), c->d_cnt.p, live.size() * sizeof(unsigned int), cudaMemcpyDeviceToHost) != cudaSuccess) live.assign(live.size(), 0u);
-    }
-  float shade_ms = 0.0f;
   for (int i = 0; i + 1 < c->kev_used; ++i)  // event i sits before launch i; launches alternate shade, trace, shade, ...
-    if (cudaEventElapsedTime(&ms, c->kev[i], c->kev[i + 1]) == cudaSuccess) {
+    if (cudaEventElapsedTime(&ms, c->kev[i], c->kev[i + 1]) == cudaSuccess)
       ((i & 1) ? c->stats.trace_kernel_ms : c->stats.shade_kernel_ms) += ms;
-      if (dump) {
-        if (i & 1) fprintf(dump, "%d %u %.4f %.4f\n", i / 2, live[(size_t)i / 2], shade_ms, ms);
-        else shade_ms = ms;
-      }
-    }
-  if (dump) fclose(dump);
   c->kev_used = 0;
   c->stats_pending = false;
   return 0;
+}
+
+// the additive work counters of one render; times, scene facts and primary_rays are each caller's own rule
+void add_work(b200rt_stats &dst, const b200rt_stats &src) {
+  dst.rays += src.rays;
+  dst.box_tests += src.box_tests;
+  dst.tri_tests += src.tri_tests;
+  dst.mismatches += src.mismatches;
+  dst.samples += src.samples;
+  dst.revalidated += src.revalidated;
+  dst.exact_walks += src.exact_walks;
+  dst.kernel_launches += src.kernel_launches;
 }
 
 // Counters and timings of the last render.  A frame cut into sample streams sums the work of its helper contexts
@@ -473,14 +457,8 @@ int read_counters(b200rt_ctx *c) {
     b200rt_ctx *h = c->helpers[(size_t)k - 1];
     rc = read_counters_one(h);
     if (rc) return fail(c, rc, "sample stream %d: %s", k, h->err.c_str());
-    c->stats.rays += h->stats.rays - h->stats.primary_rays;
-    c->stats.box_tests += h->stats.box_tests;
-    c->stats.tri_tests += h->stats.tri_tests;
-    c->stats.mismatches += h->stats.mismatches;
-    c->stats.samples += h->stats.samples;
-    c->stats.revalidated += h->stats.revalidated;
-    c->stats.exact_walks += h->stats.exact_walks;
-    c->stats.kernel_launches += h->stats.kernel_launches;
+    add_work(c->stats, h->stats);
+    c->stats.rays -= h->stats.primary_rays;
     c->stats.shade_kernel_ms += h->stats.shade_kernel_ms;   // kernels of different streams overlap: these are sums of
     c->stats.trace_kernel_ms += h->stats.trace_kernel_ms;   // durations, not a partition of total_ms
     c->stats.primary_ms = std::max(c->stats.primary_ms, h->stats.primary_ms);
@@ -535,51 +513,10 @@ int check_frame_args(b200rt_ctx *c, const float *cam, int width, int height, int
 
 constexpr int kAdaptBatch = 32;  // adaptive renders: wavefront iterations enqueued between two looks at the list length
 
-// The wavefront loop of an adaptive render: render_impl's launches, enqueued in batches of kAdaptBatch iterations rounded
-// up to a multiple of compact_every, so that every batch ends with a compaction and its last cnt word is the number of
-// live paths.  That word is copied to pinned memory behind an event; before batch k + 2 is enqueued the host waits for
-// batch k's and stops once it is 0.  One batch is always in flight, so the GPU does not wait for the host.  A k_shade
-// on an empty list does nothing, so stopping there leaves the image the full loop would make.
-int adaptive_wave(b200rt_ctx *c, const KernelArgs &A, const WaveLaunch &wl, int n_iter, bool nee, bool time_kernels) {
-  const int batch = (kAdaptBatch + A.compact_every - 1) / A.compact_every * A.compact_every;
-  int it = 0, n_shade = 0, n_trace = 0, n_compactions = 0;
-  for (int b = 0; it <= n_iter; ++b) {
-    if (b >= 2) {
-      CU(cudaEventSynchronize(c->ev_batch[b & 1]));
-      if (c->h_live[b & 1] == 0u) break;
-    }
-    const int end = std::min(it + batch, n_iter + 1);
-    for (; it < end; ++it) {
-      if (time_kernels) CU(cudaEventRecord(c->kev[c->kev_used++], c->stream));
-      if (nee) k_shade<true, true><<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
-      else k_shade<false, true><<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
-      ++n_shade;
-      if (it < n_iter && (it + 1) % A.compact_every == 0) {
-        k_compact<<<wl.shade_grid, kCompactBlock, 0, c->stream>>>(A.slots, A.cnt + it, 0u, A.part_count, A.list[(it + 1) & 1], A.cnt + it + 1);
-        ++n_compactions;
-      }
-      if (time_kernels) CU(cudaEventRecord(c->kev[c->kev_used++], c->stream));
-      if (it < n_iter) {
-        wl.trace<<<wl.trace_grid, kBlock, wl.trace_smem, c->stream>>>(A, it);
-        ++n_trace;
-      }
-    }
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(&c->h_live[b & 1], A.cnt + end, sizeof(unsigned int), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaEventRecord(c->ev_batch[b & 1], c->stream));
-  }
-  // k_count_parts + k_compact for the first list, then what the loop launched
-  c->stats.kernel_launches += 2 + n_shade + n_compactions + n_trace;
-  c->stats.wave_iterations = n_trace;
-  CU(cudaEventRecord(c->ev[2], c->stream));
-  c->stats_pending = true;
-  return 0;
-}
-
 // ad != NULL: adaptive sampling (b200rt_render_adaptive has validated ad and opts; the frame covers [0, spp) on one
 // stream).  The launch loop then runs in batches and stops once the path list is empty; it is synchronous.
 int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, int height, int spp, int max_bounce,
-                const b200rt_opts *opts, float *d_out, const b200rt_adaptive *ad = nullptr) {
+                const b200rt_opts *opts, float *d_out, const b200rt_adaptive *ad) {
   b200rt_opts o;
   if (opts) o = *opts; else b200rt_default_opts(&o);
   c->streams_used = 1;
@@ -623,11 +560,17 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   A.validate = (trav == B200RT_TRAVERSAL_FAST) ? 1 : 0;
   const bool smem = use_smem_scene(c);
   WaveLaunch wl;
-  rc = prepare_wave(c, trav, smem, o.collect_stats != 0, &wl);
+  rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, &wl);
   if (rc) return rc;
   if (ensure(c, c->d_part_count, (size_t)wl.shade_grid * sizeof(unsigned int))) return B200RT_ERR_CUDA;
   A.part_count = static_cast<unsigned int *>(c->d_part_count.p);
   A.slots = static_cast<int *>(c->d_slots.p);
+  c->stats.kernel_launches = 0;
+  c->stats.sample_streams = 1;
+  c->stats.scene_in_smem = smem ? 1 : 0;
+  CU(cudaMemsetAsync(c->d_counters, 0, sizeof(DeviceCounters), c->stream));
+  CU(cudaMemsetAsync(c->d_cnt.p, 0, cnt_bytes, c->stream));
+  CU(cudaEventRecord(c->ev[0], c->stream));
   if (ad) {
     if (ensure(c, c->d_welford, npix * sizeof(float2))) return B200RT_ERR_CUDA;
     if (ensure(c, c->d_ad_spp, npix * sizeof(int))) return B200RT_ERR_CUDA;
@@ -642,18 +585,9 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
     if (!c->h_live) CU(cudaMallocHost(&c->h_live, 2 * sizeof(unsigned int)));
     for (int k = 0; k < 2; ++k)
       if (!c->ev_batch[k]) CU(cudaEventCreateWithFlags(&c->ev_batch[k], cudaEventDisableTiming));
-  }
-  c->stats.kernel_launches = 0;
-  c->stats.sample_streams = 1;
-  c->stats.scene_in_smem = smem ? 1 : 0;
-  CU(cudaMemsetAsync(c->d_counters, 0, sizeof(DeviceCounters), c->stream));
-  CU(cudaMemsetAsync(c->d_cnt.p, 0, cnt_bytes, c->stream));
-  if (ad) {  // pixels outside the rendered set read 0 in both maps
+    // pixels outside the rendered set read 0 in both maps
     CU(cudaMemsetAsync(c->d_ad_spp.p, 0, npix * sizeof(int), c->stream));
     CU(cudaMemsetAsync(c->d_ad_err.p, 0, npix * sizeof(float), c->stream));
-  }
-  CU(cudaEventRecord(c->ev[0], c->stream));
-  if (ad) {
     const int grid = (int)std::min<long long>(((long long)A.n_work + 255) / 256, (long long)c->sm_count * 8);
     k_adaptive_init<<<grid, 256, 0, c->stream>>>(A);
     CU(cudaGetLastError());
@@ -675,23 +609,43 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
       c->kev.push_back(e);
     }
   }
-  if (ad) return adaptive_wave(c, A, wl, n_iter, nee, o.time_kernels != 0);
-  int n_compactions = 0;
-  for (int it = 0; it <= n_iter; ++it) {
-    if (o.time_kernels) CU(cudaEventRecord(c->kev[c->kev_used++], c->stream));
-    if (nee) k_shade<true, false><<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
-    else k_shade<false, false><<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
-    if (it < n_iter && (it + 1) % A.compact_every == 0) {  // close the gaps the finished pixels left, order kept (timed with k_shade)
-      k_compact<<<wl.shade_grid, kCompactBlock, 0, c->stream>>>(A.slots, A.cnt + it, 0u, A.part_count, A.list[(it + 1) & 1], A.cnt + it + 1);
-      ++n_compactions;
+  // A fixed-spp frame is one batch of every iteration, enqueued without a look back.  An adaptive frame runs batches of
+  // kAdaptBatch iterations rounded up to a multiple of compact_every, so that every batch ends with a compaction and its
+  // last cnt word is the number of live paths.  That word is copied to pinned memory behind an event; before batch k + 2
+  // is enqueued the host waits for batch k's and stops once it is 0.  One batch is always in flight, so the GPU does not
+  // wait for the host.  A k_shade on an empty list does nothing, so stopping there leaves the image the full loop would
+  // make.
+  const int batch = ad ? (kAdaptBatch + A.compact_every - 1) / A.compact_every * A.compact_every : n_iter + 1;
+  int it = 0, n_shade = 0, n_trace = 0, n_compactions = 0;
+  for (int b = 0; it <= n_iter; ++b) {
+    if (ad && b >= 2) {
+      CU(cudaEventSynchronize(c->ev_batch[b & 1]));
+      if (c->h_live[b & 1] == 0u) break;
     }
-    if (o.time_kernels) CU(cudaEventRecord(c->kev[c->kev_used++], c->stream));
-    if (it < n_iter) wl.trace<<<wl.trace_grid, kBlock, wl.trace_smem, c->stream>>>(A, it);
+    const int end = std::min(it + batch, n_iter + 1);
+    for (; it < end; ++it) {
+      if (o.time_kernels) CU(cudaEventRecord(c->kev[c->kev_used++], c->stream));
+      wl.shade<<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
+      ++n_shade;
+      if (it < n_iter && (it + 1) % A.compact_every == 0) {  // close the gaps the finished pixels left, order kept (timed with k_shade)
+        k_compact<<<wl.shade_grid, kCompactBlock, 0, c->stream>>>(A.slots, A.cnt + it, 0u, A.part_count, A.list[(it + 1) & 1], A.cnt + it + 1);
+        ++n_compactions;
+      }
+      if (o.time_kernels) CU(cudaEventRecord(c->kev[c->kev_used++], c->stream));
+      if (it < n_iter) {
+        wl.trace<<<wl.trace_grid, kBlock, wl.trace_smem, c->stream>>>(A, it);
+        ++n_trace;
+      }
+    }
+    CU(cudaGetLastError());
+    if (ad) {
+      CU(cudaMemcpyAsync(&c->h_live[b & 1], A.cnt + end, sizeof(unsigned int), cudaMemcpyDeviceToHost, c->stream));
+      CU(cudaEventRecord(c->ev_batch[b & 1], c->stream));
+    }
   }
-  CU(cudaGetLastError());
-  // k_count_parts + k_compact for the first list; k_shade + k_trace per iteration; the compactions; the closing k_shade
-  c->stats.kernel_launches += 2 + 2 * n_iter + n_compactions + 1;
-  c->stats.wave_iterations = n_iter;
+  // k_count_parts + k_compact for the first list, then what the loop launched
+  c->stats.kernel_launches += 2 + n_shade + n_compactions + n_trace;
+  c->stats.wave_iterations = n_trace;
   CU(cudaEventRecord(c->ev[2], c->stream));
   c->stats_pending = true;
   return 0;
@@ -705,24 +659,42 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
 // holds N samples of a pixel at once: small frames fill it, and on large frames one part's shading overlaps another
 // part's tracing (the two kernels are bound by different units).
 void borrow_scene(b200rt_ctx *p, b200rt_ctx *h) {
-  auto lend = [](DevBuf &dst, const DevBuf &src) { dst.p = src.p; dst.cap = src.cap; dst.borrowed = true; };
-  lend(h->d_nodes, p->d_nodes); lend(h->d_tris, p->d_tris); lend(h->d_ctris, p->d_ctris); lend(h->d_normals, p->d_normals); lend(h->d_tboxes, p->d_tboxes);
-  lend(h->d_frames, p->d_frames); lend(h->d_mats, p->d_mats); lend(h->d_bvh9, p->d_bvh9); lend(h->d_leafcnt, p->d_leafcnt);
-  lend(h->d_light, p->d_light);
-  h->n_light = p->n_light;
-  h->n_nodes9 = p->n_nodes9; h->n_inner = p->n_inner; h->n_tris = p->n_tris; h->n_mats = p->n_mats;
-  h->node_f4 = p->node_f4; h->depth = p->depth; h->cull_depth = p->cull_depth; h->ref_stack_need = p->ref_stack_need; h->canonical = p->canonical;
-  h->root_ref = p->root_ref;
-  for (int k = 0; k < 3; ++k) {
-    h->grid_base[k] = p->grid_base[k]; h->grid_pitch[k] = p->grid_pitch[k];
-    h->root_w[k] = p->root_w[k];
+  for (int i = 0; i < kSceneBufs; ++i) {
+    h->d_scene[i] = p->d_scene[i];
+    h->d_scene[i].borrowed = true;
   }
-  h->cull_abs = p->cull_abs; h->cmax = p->cmax; h->fast_ok = p->fast_ok;
-  h->quorum = p->quorum; h->refill_min = p->refill_min; h->tri_quorum = p->tri_quorum;
-  h->max_trace_ctas = p->max_trace_ctas; h->compact_every = p->compact_every; h->carveout = p->carveout;
+  h->scene = p->scene;
+  h->n_light = p->n_light;
   h->have_scene = p->have_scene;
   h->ibl_tex = p->ibl_tex; h->ibl_w = p->ibl_w; h->ibl_h = p->ibl_h; h->have_ibl = p->have_ibl;
   h->shared_epoch = p->scene_epoch;
+}
+
+// Runs fn(k) for every part k in [0, n) on a host thread of its own: a frame is thousands of small launches, and one
+// thread feeding several streams or GPUs would be the bottleneck.  Returns 0, or the code of the first part that
+// failed with its index in *failed.
+template <class F>
+int run_parts(int n, int *failed, F &&fn) {
+  std::vector<int> rcs((size_t)n, 0);
+#pragma omp parallel for num_threads(n) schedule(static, 1)
+  for (int k = 0; k < n; ++k) rcs[(size_t)k] = fn(k);
+  for (int k = 0; k < n; ++k)
+    if (rcs[(size_t)k]) {
+      *failed = k;
+      return rcs[(size_t)k];
+    }
+  return 0;
+}
+
+// One k_reduce_finalize on c's stream: out[0, n) = the parts' sums in part order, divided by spp and clamped, or left as
+// sums when spp is 0.  It reads float4s when every pointer is 16-byte aligned.
+int launch_reduce(b200rt_ctx *c, const PartList &parts, float *out, long long n, float spp) {
+  bool aligned = reinterpret_cast<uintptr_t>(out) % 16 == 0;
+  for (int i = 0; i < parts.n; ++i) aligned = aligned && reinterpret_cast<uintptr_t>(parts.p[i]) % 16 == 0;
+  const int grid = (int)std::min<long long>((n / 4 + 255) / 256 + 1, (long long)c->sm_count * 8);
+  k_reduce_finalize<<<grid, 256, 0, c->stream>>>(parts, out, aligned ? n / 4 : 0, n, spp);
+  CU(cudaGetLastError());
+  return 0;
 }
 
 int resolve_streams(const b200rt_opts &o, int width, int height, int s0, int s1) {
@@ -737,17 +709,18 @@ int resolve_streams(const b200rt_opts &o, int width, int height, int s0, int s1)
   return n < 1 ? 1 : n;
 }
 
+// ad != NULL: an adaptive frame, which runs on one stream (b200rt_render_adaptive has validated ad and opts)
 int render_frame(b200rt_ctx *c, const float *cam, const float *env, int width, int height, int spp, int max_bounce,
-                 const b200rt_opts *opts, float *d_out) {
+                 const b200rt_opts *opts, float *d_out, const b200rt_adaptive *ad = nullptr) {
   b200rt_opts o;
   if (opts) o = *opts; else b200rt_default_opts(&o);
   if (o.sample_streams < -1 || o.sample_streams > 16)
     return fail(c, B200RT_ERR_INVALID, "bad sample_streams %d (-1 automatic, 0 / 1 off, up to 16)", o.sample_streams);
   int s0 = o.sample_begin, s1 = o.sample_end;
   if (s1 <= 0) { s0 = 0; s1 = spp; }
-  const int n = (width > 0 && height > 0 && spp > 0) ? resolve_streams(o, width, height, s0, s1) : 1;
+  const int n = (!ad && width > 0 && height > 0 && spp > 0) ? resolve_streams(o, width, height, s0, s1) : 1;
   if (!c->is_helper) c->frame_trace_cap = 0;
-  if (n <= 1 || c->is_helper) return render_impl(c, cam, env, width, height, spp, max_bounce, &o, d_out);
+  if (n <= 1 || c->is_helper) return render_impl(c, cam, env, width, height, spp, max_bounce, &o, d_out, ad);
   int rc = check_frame_args(c, cam, width, height, spp, max_bounce, o, true, env);
   if (rc) return rc;
   if (!c->have_ibl) return fail(c, B200RT_ERR_NO_SCENE, "no environment map: call b200rt_set_ibl first");
@@ -759,8 +732,6 @@ int render_frame(b200rt_ctx *c, const float *cam, const float *env, int width, i
     h->is_helper = true;
     c->helpers.push_back(h);
   }
-  c->frame_trace_cap = n >= 3 ? c->stream_trace_ctas : 0;
-  for (int k = 1; k < n; ++k) c->helpers[(size_t)k - 1]->frame_trace_cap = c->frame_trace_cap;
   if (!c->ev_fork) {
     CU(cudaEventCreate(&c->ev_fork));
     CU(cudaEventCreate(&c->ev_done));
@@ -768,10 +739,9 @@ int render_frame(b200rt_ctx *c, const float *cam, const float *env, int width, i
   const size_t bytes = (size_t)width * height * 3 * sizeof(float);
   if (ensure(c, c->d_part, bytes)) return B200RT_ERR_CUDA;
   CU(cudaEventRecord(c->ev_fork, c->stream));   // the parts start after whatever the caller enqueued before this frame
-  std::vector<int> rcs((size_t)n, 0);
   const int total = s1 - s0, base = total / n, extra = total % n;
-#pragma omp parallel for num_threads(n) schedule(static, 1)
-  for (int k = 0; k < n; ++k) {
+  int bad = 0;
+  rc = run_parts(n, &bad, [&](int k) {
     b200rt_ctx *h = k == 0 ? c : c->helpers[(size_t)k - 1];
     b200rt_opts ok = o;
     ok.sample_streams = 1;
@@ -791,17 +761,16 @@ int render_frame(b200rt_ctx *c, const float *cam, const float *env, int width, i
       part = static_cast<float *>(c->d_part.p);
     }
     if (!r && cudaMemsetAsync(part, 0, bytes, h->stream) != cudaSuccess) r = B200RT_ERR_CUDA;
-    if (!r) r = render_impl(h, cam, env, width, height, spp, max_bounce, &ok, part);
+    h->frame_trace_cap = n >= 3 ? kStreamTraceCtas : 0;
+    if (!r) r = render_impl(h, cam, env, width, height, spp, max_bounce, &ok, part, nullptr);
     if (!r && k > 0 && cudaEventRecord(h->ev_join, h->stream) != cudaSuccess) r = B200RT_ERR_CUDA;
     if (r == B200RT_ERR_CUDA && h->err.empty()) h->err = "CUDA call failed while enqueueing a sample stream";
-    rcs[(size_t)k] = r;
+    return r;
+  });
+  if (rc) {
+    const std::string msg = (bad == 0 ? c : c->helpers[(size_t)bad - 1])->err;
+    return fail(c, rc, "sample stream %d: %s", bad, msg.c_str());
   }
-  for (int k = 0; k < n; ++k)
-    if (rcs[(size_t)k]) {
-      b200rt_ctx *h = k == 0 ? c : c->helpers[(size_t)k - 1];
-      const std::string msg = h->err;
-      return fail(c, rcs[(size_t)k], "sample stream %d: %s", k, msg.c_str());
-    }
   // join on this context's stream, add the parts in order; a whole frame is finalised, a partial range stays sums
   PartList pl;
   pl.n = n;
@@ -810,11 +779,8 @@ int render_frame(b200rt_ctx *c, const float *cam, const float *env, int width, i
     CU(cudaStreamWaitEvent(c->stream, c->helpers[(size_t)k - 1]->ev_join, 0));
     pl.p[k] = static_cast<const float *>(c->helpers[(size_t)k - 1]->d_part.p);
   }
-  const long long nn = (long long)width * height * 3;
-  const bool aligned = (reinterpret_cast<uintptr_t>(d_out) % 16) == 0;
-  const int grid = (int)std::min<long long>((nn / 4 + 255) / 256 + 1, (long long)c->sm_count * 8);
-  k_reduce_finalize<<<grid, 256, 0, c->stream>>>(pl, d_out, aligned ? nn / 4 : 0, nn, o.output == B200RT_OUT_FINAL ? (float)spp : 0.0f);
-  CU(cudaGetLastError());
+  rc = launch_reduce(c, pl, d_out, (long long)width * height * 3, o.output == B200RT_OUT_FINAL ? (float)spp : 0.0f);
+  if (rc) return rc;
   CU(cudaEventRecord(c->ev_done, c->stream));
   c->streams_used = n;
   c->stats.sample_streams = n;
@@ -871,19 +837,6 @@ int b200rt_create(int device, b200rt_ctx **out) {
   c->sm_count = prop.multiProcessorCount;
   c->smem_optin = prop.sharedMemPerBlockOptin;
   memset(&c->stats, 0, sizeof c->stats);
-  auto env_int = [](const char *name, int lo, int hi, int *dst) {
-    if (const char *q = getenv(name)) {
-      int v = atoi(q);
-      if (v >= lo && v <= hi) *dst = v;
-    }
-  };
-  env_int("B200RT_QUORUM", 1, 32, &c->quorum);
-  env_int("B200RT_REFILL_MIN", 1, 32, &c->refill_min);
-  env_int("B200RT_TRI_QUORUM", 1, 32, &c->tri_quorum);
-  env_int("B200RT_MAX_TRACE_CTAS", 1, 32, &c->max_trace_ctas);
-  env_int("B200RT_STREAM_TRACE_CTAS", 0, 32, &c->stream_trace_ctas);
-  env_int("B200RT_CARVEOUT", -1, 100, &c->carveout);
-  env_int("B200RT_COMPACT_EVERY", 1, 1 << 20, &c->compact_every);
   auto bail = [&](const char *what, cudaError_t err) {
     fail(nullptr, B200RT_ERR_CUDA, "%s: %s", what, cudaGetErrorString(err));
     delete c;
@@ -913,12 +866,13 @@ void b200rt_destroy(b200rt_ctx *c) {
     c->ibl_tex = 0;
     c->ibl_array = nullptr;
   }
-  DevBuf *bufs[] = {&c->d_nodes, &c->d_tris, &c->d_ctris, &c->d_normals, &c->d_tboxes, &c->d_frames, &c->d_mats, &c->d_bvh9, &c->d_leafcnt, &c->d_prim_dirk,
-                    &c->d_prim_tri, &c->d_out, &c->d_misc, &c->d_tmp_a, &c->d_tmp_b, &c->d_pA, &c->d_pB, &c->d_pC,
-                    &c->d_pHit, &c->d_list0, &c->d_list1, &c->d_cnt, &c->d_slots, &c->d_part_count, &c->d_light, &c->d_pS,
+  for (DevBuf &b : c->d_scene)
+    if (b.p && !b.borrowed) cudaFree(b.p);
+  DevBuf *bufs[] = {&c->d_prim_dirk, &c->d_prim_tri, &c->d_out, &c->d_misc, &c->d_tmp_a, &c->d_tmp_b, &c->d_pA, &c->d_pB,
+                    &c->d_pC, &c->d_pHit, &c->d_list0, &c->d_list1, &c->d_cnt, &c->d_slots, &c->d_part_count, &c->d_pS,
                     &c->d_pL, &c->d_pR, &c->d_welford, &c->d_ad_spp, &c->d_ad_err};
   for (DevBuf *b : bufs)
-    if (b->p && !b->borrowed) cudaFree(b->p);
+    if (b->p) cudaFree(b->p);
   if (c->h_live) cudaFreeHost(c->h_live);
   for (cudaEvent_t e : c->ev_batch)
     if (e) cudaEventDestroy(e);
@@ -945,9 +899,10 @@ int b200rt_set_materials(b200rt_ctx *c, const float *mat, int64_t n_mat) {
     if (m < 0 || m >= nm) return fail(c, B200RT_ERR_INVALID, "a triangle uses material %d but only %d materials were given", m, nm);
   CU(cudaSetDevice(c->device));
   uint64_t h = hash_bytes(mat, (size_t)n_mat * 4, 0x6d617473ull);
-  if (c->n_mats == nm && c->mat_hash != 0 && h == c->mat_hash && c->d_mats.p) return 0;
-  if (ensure(c, c->d_mats, (size_t)n_mat * 4)) return B200RT_ERR_CUDA;
-  CU(cudaMemcpyAsync(c->d_mats.p, mat, (size_t)n_mat * 4, cudaMemcpyHostToDevice, c->stream));
+  DevBuf &d_mats = c->d_scene[kMats], &d_light = c->d_scene[kLight];
+  if (c->n_mats == nm && c->mat_hash != 0 && h == c->mat_hash && d_mats.p) return 0;
+  if (ensure(c, d_mats, (size_t)n_mat * 4)) return B200RT_ERR_CUDA;
+  CU(cudaMemcpyAsync(d_mats.p, mat, (size_t)n_mat * 4, cudaMemcpyHostToDevice, c->stream));
   // The emitter list of the opt-in light sampling: what FileManager.py:235-240 builds as lightData — the triangles
   // whose material is emissive, in triangle order — derived here from the materials just given, so that it can never
   // be stale after a material edit (the reference's kernel receives lightData and never reads it, Raytracing.cl:163).
@@ -957,8 +912,8 @@ int b200rt_set_materials(b200rt_ctx *c, const float *mat, int64_t n_mat) {
       if ((int)mat[6 * (size_t)c->tri_mat[t]] == 0) lights.push_back((int32_t)t);
     c->n_light = (int)lights.size();
     if (!lights.empty()) {
-      if (ensure(c, c->d_light, lights.size() * sizeof(int32_t))) return B200RT_ERR_CUDA;
-      CU(cudaMemcpy(c->d_light.p, lights.data(), lights.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+      if (ensure(c, d_light, lights.size() * sizeof(int32_t))) return B200RT_ERR_CUDA;
+      CU(cudaMemcpy(d_light.p, lights.data(), lights.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
     }
   }
   CU(cudaStreamSynchronize(c->stream));
@@ -1012,44 +967,29 @@ int upload_scene(b200rt_ctx *c, const Repacked &R, const SceneArgs &a, uint64_t 
   c->have_scene_cached = false;
   c->scene_hash = 0;
   const int n_tris = R.n_tris;
+  DevBuf *B = c->d_scene;
   CU(cudaSetDevice(c->device));
-  if (ensure(c, c->d_tris, R.tris.size() * sizeof(float4))) return B200RT_ERR_CUDA;
-  if (ensure(c, c->d_ctris, R.ctris.size() * sizeof(float4))) return B200RT_ERR_CUDA;
-  if (ensure(c, c->d_normals, R.normals.size() * sizeof(float4))) return B200RT_ERR_CUDA;
-  if (ensure(c, c->d_tboxes, R.tboxes.size() * sizeof(float4))) return B200RT_ERR_CUDA;
-  if (ensure(c, c->d_frames, (size_t)n_tris * kFrameVec * sizeof(float4))) return B200RT_ERR_CUDA;
-  if (ensure(c, c->d_nodes, R.nodes.size() * sizeof(uint4))) return B200RT_ERR_CUDA;
-  if (ensure(c, c->d_bvh9, (size_t)a.n_bvh * 4)) return B200RT_ERR_CUDA;
-  if (ensure(c, c->d_leafcnt, R.leaf_count.size() * sizeof(int32_t))) return B200RT_ERR_CUDA;
-  CU(cudaMemcpyAsync(c->d_leafcnt.p, R.leaf_count.data(), R.leaf_count.size() * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-  CU(cudaMemcpyAsync(c->d_tris.p, R.tris.data(), R.tris.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
-  CU(cudaMemcpyAsync(c->d_ctris.p, R.ctris.data(), R.ctris.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
-  CU(cudaMemcpyAsync(c->d_normals.p, R.normals.data(), R.normals.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
-  CU(cudaMemcpyAsync(c->d_tboxes.p, R.tboxes.data(), R.tboxes.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+  if (ensure(c, B[kTris], R.tris.size() * sizeof(float4))) return B200RT_ERR_CUDA;
+  if (ensure(c, B[kCtris], R.ctris.size() * sizeof(float4))) return B200RT_ERR_CUDA;
+  if (ensure(c, B[kNormals], R.normals.size() * sizeof(float4))) return B200RT_ERR_CUDA;
+  if (ensure(c, B[kTboxes], R.tboxes.size() * sizeof(float4))) return B200RT_ERR_CUDA;
+  if (ensure(c, B[kFrames], (size_t)n_tris * kFrameVec * sizeof(float4))) return B200RT_ERR_CUDA;
+  if (ensure(c, B[kNodes], R.nodes.size() * sizeof(uint4))) return B200RT_ERR_CUDA;
+  if (ensure(c, B[kBvh9], (size_t)a.n_bvh * 4)) return B200RT_ERR_CUDA;
+  if (ensure(c, B[kLeafcnt], R.leaf_count.size() * sizeof(int32_t))) return B200RT_ERR_CUDA;
+  CU(cudaMemcpyAsync(B[kLeafcnt].p, R.leaf_count.data(), R.leaf_count.size() * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(B[kTris].p, R.tris.data(), R.tris.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(B[kCtris].p, R.ctris.data(), R.ctris.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(B[kNormals].p, R.normals.data(), R.normals.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(B[kTboxes].p, R.tboxes.data(), R.tboxes.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
   if (!R.nodes.empty())
-    CU(cudaMemcpyAsync(c->d_nodes.p, R.nodes.data(), R.nodes.size() * sizeof(uint4), cudaMemcpyHostToDevice, c->stream));
-  CU(cudaMemcpyAsync(c->d_bvh9.p, a.bvh, (size_t)a.n_bvh * 4, cudaMemcpyHostToDevice, c->stream));
-  k_tri_frames<<<(n_tris + 127) / 128, 128, 0, c->stream>>>(static_cast<const float4 *>(c->d_normals.p), n_tris,
-                                                           static_cast<float4 *>(c->d_frames.p));
+    CU(cudaMemcpyAsync(B[kNodes].p, R.nodes.data(), R.nodes.size() * sizeof(uint4), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(B[kBvh9].p, a.bvh, (size_t)a.n_bvh * 4, cudaMemcpyHostToDevice, c->stream));
+  k_tri_frames<<<(n_tris + 127) / 128, 128, 0, c->stream>>>(static_cast<const float4 *>(B[kNormals].p), n_tris,
+                                                           static_cast<float4 *>(B[kFrames].p));
   CU(cudaGetLastError());
   CU(cudaStreamSynchronize(c->stream));
-  c->n_nodes9 = R.n_nodes9;
-  c->n_inner = R.n_inner;
-  c->n_tris = n_tris;
-  c->node_f4 = R.node_f4;
-  c->depth = R.depth;
-  c->cull_depth = R.cull_depth;
-  c->ref_stack_need = R.ref_stack_need;
-  c->canonical = R.canonical;
-  c->root_ref = R.root_ref;
-  for (int k = 0; k < 3; ++k) {
-    c->grid_base[k] = R.grid_base[k];
-    c->grid_pitch[k] = R.grid_pitch[k];
-    c->root_w[k] = R.root_w[k];
-  }
-  c->cull_abs = R.cull_abs;
-  c->cmax = R.cmax;
-  c->fast_ok = R.fast_ok;
+  c->scene = R;
   c->tri_mat = R.tri_mat;
   c->mat_hash = 0;
   c->n_mats = 0;
@@ -1060,11 +1000,27 @@ int upload_scene(b200rt_ctx *c, const Repacked &R, const SceneArgs &a, uint64_t 
   c->scene_hash = h;
   ++c->scene_epoch;
   c->stats.repack_ms = (float)(R.ms_tris + R.ms_walk + R.ms_nodes);
-  c->stats.ref_stack_need = c->ref_stack_need;
+  c->stats.ref_stack_need = R.ref_stack_need;
   c->stats.nodes = R.n_nodes9;
   c->stats.triangles = n_tris;
-  c->stats.bvh_depth = c->depth;
+  c->stats.bvh_depth = R.depth;
   return 0;
+}
+
+// What every host-output render does: render into the zeroed d_out on the context's stream, enqueue `read_back` (the
+// copies to the caller's memory), wait for them and read the counters.
+template <class ReadBack>
+int render_to_host(b200rt_ctx *c, const float *cam, const float *env, int width, int height, int spp, int max_bounce,
+                   const b200rt_opts *opts, const b200rt_adaptive *ad, ReadBack &&read_back) {
+  const size_t bytes = (size_t)width * height * 3 * sizeof(float);
+  CU(cudaSetDevice(c->device));
+  if (ensure(c, c->d_out, bytes)) return B200RT_ERR_CUDA;
+  CU(cudaMemsetAsync(c->d_out.p, 0, bytes, c->stream));
+  int rc = render_frame(c, cam, env, width, height, spp, max_bounce, opts, static_cast<float *>(c->d_out.p), ad);
+  if (!rc) rc = read_back();
+  if (rc) return rc;
+  CU(cudaStreamSynchronize(c->stream));
+  return read_counters(c);
 }
 
 }  // namespace
@@ -1157,15 +1113,10 @@ int b200rt_render(b200rt_ctx *c, const float *cam, const float *env, int width, 
   if (!c) return B200RT_ERR_INVALID;
   if (!out) return fail(c, B200RT_ERR_INVALID, "out_rgb is NULL");
   if (width <= 0 || height <= 0) return fail(c, B200RT_ERR_INVALID, "bad frame size %d x %d", width, height);
-  const size_t bytes = (size_t)width * height * 3 * sizeof(float);
-  CU(cudaSetDevice(c->device));
-  if (ensure(c, c->d_out, bytes)) return B200RT_ERR_CUDA;
-  CU(cudaMemsetAsync(c->d_out.p, 0, bytes, c->stream));
-  int rc = render_frame(c, cam, env, width, height, spp, max_bounce, opts, static_cast<float *>(c->d_out.p));
-  if (rc) return rc;
-  CU(cudaMemcpyAsync(out, c->d_out.p, bytes, cudaMemcpyDeviceToHost, c->stream));  // blocking read-back, KernelLauncher.py:78
-  CU(cudaStreamSynchronize(c->stream));
-  return read_counters(c);
+  return render_to_host(c, cam, env, width, height, spp, max_bounce, opts, nullptr, [&] {
+    CU(cudaMemcpyAsync(out, c->d_out.p, (size_t)width * height * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));  // blocking read-back, KernelLauncher.py:78
+    return 0;
+  });
 }
 
 int b200rt_render_adaptive(b200rt_ctx *c, const float *cam, const float *env, int width, int height, int spp,
@@ -1192,19 +1143,13 @@ int b200rt_render_adaptive(b200rt_ctx *c, const float *cam, const float *env, in
   if (o.sample_streams < -1 || o.sample_streams > 1)
     return fail(c, B200RT_ERR_INVALID, "adaptive sampling runs one sample stream (sample_streams -1, 0 or 1, got %d)",
                 o.sample_streams);
-  o.sample_streams = 1;
   const size_t npix = (size_t)width * height;
-  CU(cudaSetDevice(c->device));
-  if (ensure(c, c->d_out, npix * 3 * sizeof(float))) return B200RT_ERR_CUDA;
-  CU(cudaMemsetAsync(c->d_out.p, 0, npix * 3 * sizeof(float), c->stream));
-  c->frame_trace_cap = 0;
-  rc = render_impl(c, cam, env, width, height, spp, max_bounce, &o, static_cast<float *>(c->d_out.p), ad);
-  if (rc) return rc;
-  CU(cudaMemcpyAsync(out, c->d_out.p, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-  if (out_spp) CU(cudaMemcpyAsync(out_spp, c->d_ad_spp.p, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-  if (out_stderr) CU(cudaMemcpyAsync(out_stderr, c->d_ad_err.p, npix * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-  CU(cudaStreamSynchronize(c->stream));
-  return read_counters(c);
+  return render_to_host(c, cam, env, width, height, spp, max_bounce, &o, ad, [&] {
+    CU(cudaMemcpyAsync(out, c->d_out.p, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    if (out_spp) CU(cudaMemcpyAsync(out_spp, c->d_ad_spp.p, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    if (out_stderr) CU(cudaMemcpyAsync(out_stderr, c->d_ad_err.p, npix * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    return 0;
+  });
 }
 
 int b200rt_render_rgb8(b200rt_ctx *c, const float *cam, const float *env, int width, int height, int spp, int max_bounce,
@@ -1215,18 +1160,15 @@ int b200rt_render_rgb8(b200rt_ctx *c, const float *cam, const float *env, int wi
   if (opts && opts->output != B200RT_OUT_FINAL) return fail(c, B200RT_ERR_INVALID, "8-bit output needs B200RT_OUT_FINAL");
   const size_t n = (size_t)width * height * 3;
   CU(cudaSetDevice(c->device));
-  if (ensure(c, c->d_out, n * sizeof(float))) return B200RT_ERR_CUDA;
   if (ensure(c, c->d_tmp_a, n)) return B200RT_ERR_CUDA;
-  CU(cudaMemsetAsync(c->d_out.p, 0, n * sizeof(float), c->stream));
-  int rc = render_frame(c, cam, env, width, height, spp, max_bounce, opts, static_cast<float *>(c->d_out.p));
-  if (rc) return rc;
-  int grid = (int)std::min<long long>(((long long)n + 255) / 256, (long long)c->sm_count * 16);
-  k_quantize8<<<grid, 256, 0, c->stream>>>(static_cast<const float *>(c->d_out.p), static_cast<uint8_t *>(c->d_tmp_a.p), (long long)n);
-  CU(cudaGetLastError());
-  c->stats.kernel_launches++;
-  CU(cudaMemcpyAsync(out, c->d_tmp_a.p, n, cudaMemcpyDeviceToHost, c->stream));
-  CU(cudaStreamSynchronize(c->stream));
-  return read_counters(c);
+  return render_to_host(c, cam, env, width, height, spp, max_bounce, opts, nullptr, [&] {
+    int grid = (int)std::min<long long>(((long long)n + 255) / 256, (long long)c->sm_count * 16);
+    k_quantize8<<<grid, 256, 0, c->stream>>>(static_cast<const float *>(c->d_out.p), static_cast<uint8_t *>(c->d_tmp_a.p), (long long)n);
+    CU(cudaGetLastError());
+    c->stats.kernel_launches++;
+    CU(cudaMemcpyAsync(out, c->d_tmp_a.p, n, cudaMemcpyDeviceToHost, c->stream));
+    return 0;
+  });
 }
 
 int b200rt_sync(b200rt_ctx *c) {
@@ -1274,18 +1216,11 @@ int b200rt_reduce_finalize_device(b200rt_ctx *c, const float *const *d_parts, in
   CU(cudaSetDevice(c->device));
   PartList pl;
   pl.n = n_parts;
-  bool aligned = (reinterpret_cast<uintptr_t>(d_out) % 16) == 0;
   for (int i = 0; i < n_parts; ++i) {
     if (!d_parts[i]) return fail(c, B200RT_ERR_INVALID, "part %d is NULL", i);
     pl.p[i] = d_parts[i];
-    aligned = aligned && (reinterpret_cast<uintptr_t>(d_parts[i]) % 16) == 0;
   }
-  long long n = (long long)n_pixels * 3;
-  long long n4 = aligned ? n / 4 : 0;
-  int grid = (int)std::min<long long>((n / 4 + 255) / 256 + 1, (long long)c->sm_count * 8);
-  k_reduce_finalize<<<grid, 256, 0, c->stream>>>(pl, d_out, n4, n, (float)spp);
-  CU(cudaGetLastError());
-  return 0;
+  return launch_reduce(c, pl, d_out, (long long)n_pixels * 3, (float)spp);
 }
 
 int b200rt_primary_hits(b200rt_ctx *c, const float *cam, int width, int height, const b200rt_opts *opts,
@@ -1343,14 +1278,9 @@ int b200rt_trace_rays(b200rt_ctx *c, const float *rays, int64_t n, const b200rt_
   float *dk = static_cast<float *>(c->d_tmp_b.p);
   CU(cudaEventRecord(c->ev[0], c->stream));
   CU(cudaEventRecord(c->ev[1], c->stream));
-  int rc;
-  const bool smem = use_smem_scene(c), st = o.collect_stats != 0;
-  const int trav = effective_traversal(c, o);
-  if (trav == 0) rc = smem ? (st ? launch_trace_t<0, true, true>(c, A, dr, n, dt, dk) : launch_trace_t<0, true, false>(c, A, dr, n, dt, dk))
-                           : (st ? launch_trace_t<0, false, true>(c, A, dr, n, dt, dk) : launch_trace_t<0, false, false>(c, A, dr, n, dt, dk));
-  else if (trav == 1) rc = smem ? (st ? launch_trace_t<1, true, true>(c, A, dr, n, dt, dk) : launch_trace_t<1, true, false>(c, A, dr, n, dt, dk))
-                                : (st ? launch_trace_t<1, false, true>(c, A, dr, n, dt, dk) : launch_trace_t<1, false, false>(c, A, dr, n, dt, dk));
-  else rc = smem ? launch_trace_t<2, true, false>(c, A, dr, n, dt, dk) : launch_trace_t<2, false, false>(c, A, dr, n, dt, dk);
+  int rc = with_variant(c, effective_traversal(c, o), use_smem_scene(c), o.collect_stats != 0, [&](auto t, auto s, auto st) {
+    return launch_trace_t<decltype(t)::value, decltype(s)::value, decltype(st)::value>(c, A, dr, n, dt, dk);
+  });
   if (rc) return rc;
   CU(cudaEventRecord(c->ev[2], c->stream));
   CU(cudaMemcpyAsync(tri_out, dt, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
@@ -1623,15 +1553,12 @@ int b200rt_multi_set_scene(b200rt_multi *m, const float *vp, int64_t n_vp, const
       return mfail(m, rc, "%s", msg.c_str());
     }
   }
-  const int n = (int)m->ctx.size();
-  std::vector<int> rcs((size_t)n, 0);
-#pragma omp parallel for num_threads(n) schedule(static, 1)
-  for (int i = 0; i < n; ++i) {
+  int bad = 0;
+  rc = run_parts((int)m->ctx.size(), &bad, [&](int i) {
     b200rt_ctx *c = m->ctx[i];
-    rcs[i] = scene_is_cached(c, h) ? b200rt_set_materials(c, mat, n_mat) : upload_scene(c, R, a, h);
-  }
-  for (int i = 0; i < n; ++i)
-    if (rcs[i]) return mfail(m, rcs[i], "GPU %d: %s", m->ctx[i]->device, m->ctx[i]->err.c_str());
+    return scene_is_cached(c, h) ? b200rt_set_materials(c, mat, n_mat) : upload_scene(c, R, a, h);
+  });
+  if (rc) return mfail(m, rc, "GPU %d: %s", m->ctx[bad]->device, m->ctx[bad]->err.c_str());
   m->stats.upload_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
   m->stats.nodes = m->ctx[0]->stats.nodes;
   m->stats.triangles = m->ctx[0]->stats.triangles;
@@ -1643,12 +1570,9 @@ int b200rt_multi_set_scene(b200rt_multi *m, const float *vp, int64_t n_vp, const
 
 int b200rt_multi_set_ibl(b200rt_multi *m, const uint8_t *rgba, int width, int height) {
   if (!m) return B200RT_ERR_INVALID;
-  const int n = (int)m->ctx.size();
-  std::vector<int> rcs((size_t)n, 0);
-#pragma omp parallel for num_threads(n) schedule(static, 1)
-  for (int i = 0; i < n; ++i) rcs[i] = b200rt_set_ibl(m->ctx[i], rgba, width, height);
-  for (int i = 0; i < n; ++i)
-    if (rcs[i]) return mfail(m, rcs[i], "GPU %d: %s", m->ctx[i]->device, m->ctx[i]->err.c_str());
+  int bad = 0;
+  const int rc = run_parts((int)m->ctx.size(), &bad, [&](int i) { return b200rt_set_ibl(m->ctx[i], rgba, width, height); });
+  if (rc) return mfail(m, rc, "GPU %d: %s", m->ctx[bad]->device, m->ctx[bad]->err.c_str());
   return 0;
 }
 
@@ -1678,26 +1602,24 @@ int b200rt_multi_render(b200rt_multi *m, const float *cam, const float *env, int
     m->d_final.cap = bytes;
   }
   // ---- every GPU renders its share into its own buffer; one host thread per GPU issues the launches ------------
-  std::vector<int> rcs((size_t)n, 0);
   const int tile_rows = (height + 3) / 4;
-#pragma omp parallel for num_threads(n) schedule(static, 1)
-  for (int i = 0; i < n; ++i) {
+  int bad = 0;
+  int rc = run_parts(n, &bad, [&](int i) {
     b200rt_ctx *c = m->ctx[i];
     b200rt_opts oi = o;
     multi_share(i, n, spp, o.rng_mode, &oi);
-    int rc = 0;
-    if (cudaSetDevice(c->device) != cudaSuccess) rc = B200RT_ERR_CUDA;
-    if (!rc) rc = ensure(c, c->d_out, bytes);
-    if (!rc && cudaMemsetAsync(c->d_out.p, 0, bytes, c->stream) != cudaSuccess) rc = B200RT_ERR_CUDA;
+    int r = 0;
+    if (cudaSetDevice(c->device) != cudaSuccess) r = B200RT_ERR_CUDA;
+    if (!r) r = ensure(c, c->d_out, bytes);
+    if (!r && cudaMemsetAsync(c->d_out.p, 0, bytes, c->stream) != cudaSuccess) r = B200RT_ERR_CUDA;
     const bool empty = (oi.sample_begin == oi.sample_end) || (oi.tile_row_mod > 1 && oi.tile_row_rem >= tile_rows);
     c->stats.rays = 0; c->stats.samples = 0; c->stats.total_ms = 0; c->stats.kernel_launches = 0;
-    if (!rc && !empty) rc = render_frame(c, cam, env, width, height, spp, max_bounce, &oi, static_cast<float *>(c->d_out.p));
-    if (!rc && cudaEventRecord(m->done[i], c->stream) != cudaSuccess) rc = B200RT_ERR_CUDA;
-    if (rc == B200RT_ERR_CUDA && c->err.empty()) c->err = "CUDA call failed while enqueueing the frame";
-    rcs[i] = rc;
-  }
-  for (int i = 0; i < n; ++i)
-    if (rcs[i]) return mfail(m, rcs[i], "GPU %d: %s", m->ctx[i]->device, m->ctx[i]->err.c_str());
+    if (!r && !empty) r = render_frame(c, cam, env, width, height, spp, max_bounce, &oi, static_cast<float *>(c->d_out.p));
+    if (!r && cudaEventRecord(m->done[i], c->stream) != cudaSuccess) r = B200RT_ERR_CUDA;
+    if (r == B200RT_ERR_CUDA && c->err.empty()) c->err = "CUDA call failed while enqueueing the frame";
+    return r;
+  });
+  if (rc) return mfail(m, rc, "GPU %d: %s", m->ctx[bad]->device, m->ctx[bad]->err.c_str());
   // ---- GPU 0: wait for the peers (device-side), then one kernel reads every partial buffer and finalises ----------
   MCU(cudaSetDevice(c0->device));
   MCU(cudaEventRecord(m->ev_begin, c0->stream));
@@ -1719,10 +1641,8 @@ int b200rt_multi_render(b200rt_multi *m, const float *cam, const float *env, int
     }
     pl.p[i] = src;
   }
-  const long long nn = (long long)npix * 3;
-  const int grid = (int)std::min<long long>((nn / 4 + 255) / 256 + 1, (long long)c0->sm_count * 8);
-  k_reduce_finalize<<<grid, 256, 0, c0->stream>>>(pl, static_cast<float *>(m->d_final.p), nn / 4, nn, (float)spp);
-  MCU(cudaGetLastError());
+  rc = launch_reduce(c0, pl, static_cast<float *>(m->d_final.p), (long long)npix * 3, (float)spp);
+  if (rc) return mfail(m, rc, "%s", c0->err.c_str());
   MCU(cudaEventRecord(m->ev_end, c0->stream));
   MCU(cudaMemcpyAsync(out, m->d_final.p, bytes, cudaMemcpyDeviceToHost, c0->stream));
   MCU(cudaStreamSynchronize(c0->stream));
@@ -1736,17 +1656,10 @@ int b200rt_multi_render(b200rt_multi *m, const float *cam, const float *env, int
     b200rt_ctx *c = m->ctx[i];
     if (c->stats_pending) {
       MCU(cudaSetDevice(c->device));
-      int rc = read_counters(c);
+      rc = read_counters(c);
       if (rc) return mfail(m, rc, "GPU %d: %s", c->device, c->err.c_str());
     }
-    agg.rays += c->stats.rays;
-    agg.box_tests += c->stats.box_tests;
-    agg.tri_tests += c->stats.tri_tests;
-    agg.mismatches += c->stats.mismatches;
-    agg.samples += c->stats.samples;
-    agg.kernel_launches += c->stats.kernel_launches;
-    agg.revalidated += c->stats.revalidated;
-    agg.exact_walks += c->stats.exact_walks;
+    add_work(agg, c->stats);
     slowest = std::max(slowest, c->stats.total_ms);
     agg.primary_ms = std::max(agg.primary_ms, c->stats.primary_ms);
     agg.trace_ms = std::max(agg.trace_ms, c->stats.trace_ms);

@@ -13,7 +13,6 @@
 #include <algorithm>
 #include <atomic>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 #include "scene_repack.h"
@@ -22,7 +21,7 @@ namespace b200rt {
 
 namespace {
 
-constexpr int kBins = 64;             // capacity; the number in use is Builder::bins
+constexpr int kBins = 32;             // SAH bins per axis
 constexpr int kSahLevels = 64;        // below this level ranges are halved by index: bounds the depth at 64 + log2(n)
 constexpr int kTaskMin = 256;         // sub-trees smaller than this are built by the task that reached them
 constexpr int kParallelBin = 1 << 18; // ranges larger than this are binned by several tasks
@@ -75,7 +74,6 @@ struct Builder {
 
   static float centre(const Prim &p, int a) { return 0.5f * p.mn[a] + 0.5f * p.mx[a]; }
 
-  int bins = 32;
   static int bin_of(float c, float c0, float scale, int nb) {
     int b = (int)((c - c0) * scale);
     return b < 0 ? 0 : (b >= nb ? nb - 1 : b);
@@ -110,7 +108,7 @@ struct Builder {
           c1[a] = std::max(c1[a], c);
         }
       // a range of a few triangles does not need (and should not pay for clearing and sweeping) all the bins
-      const int nb = std::min(bins, std::max(4, 2 * n));
+      const int nb = std::min(kBins, std::max(4, 2 * n));
       float scale[3];
       bool any = false;
       for (int a = 0; a < 3; ++a) {
@@ -231,10 +229,6 @@ void build_cull_tree(const Repacked::f4 *tboxes, int n_tris, std::vector<CullNod
   Builder B;
   B.prim = prim.data();
   B.nodes = tmp.data();
-  if (const char *q = getenv("B200RT_CULL_BINS")) {   // development knob
-    const int v = atoi(q);
-    if (v >= 2 && v <= kBins) B.bins = v;
-  }
   Box root;
 #pragma omp parallel
 #pragma omp single
@@ -244,9 +238,8 @@ void build_cull_tree(const Repacked::f4 *tboxes, int n_tris, std::vector<CullNod
 
   // ---- tree rotations: a child changes places with a grandchild on the other side where that shrinks the box in between
   // (bottom-up sweeps until nothing improves; the root's box and every leaf box stay what they were)
-  int passes = n_tris > 1000000 ? 1 : 2;   // the sweeps are serial: one is most of the gain
-  if (const char *q = getenv("B200RT_CULL_ROTATE")) passes = atoi(q);   // development knob
-  if (passes > 0) {
+  const int passes = n_tris > 1000000 ? 1 : 2;   // the sweeps are serial: one is most of the gain
+  {
     auto area6 = [](const float *b) {
       const double dx = (double)b[3] - b[0], dy = (double)b[4] - b[1], dz = (double)b[5] - b[2];
       return dx * dy + dy * dz + dz * dx;

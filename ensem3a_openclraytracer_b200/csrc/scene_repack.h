@@ -22,7 +22,22 @@ struct raw_alloc : std::allocator<T> {
 };
 template <class T> using raw_vector = std::vector<T, raw_alloc<T>>;
 
-struct Repacked {
+// The scalar description of a repacked scene: what the kernels' launch geometry, margins and stacks derive from.  A
+// context commits it in one assignment once the scene's buffers are on its GPU.
+struct SceneDesc {
+  int n_nodes9 = 0, n_inner = 0, n_tris = 0;
+  int node_f4 = 2;              // 2 in global memory, 3 when nodes + triangles fit the shared-memory staging area
+  int depth = 0, ref_stack_need = 0;   // of the caller's tree
+  int cull_depth = 0;           // level of the deepest leaf of the tree `nodes` holds (sizes the traversal stacks)
+  bool canonical = true;        // strict two-child tree with nested boxes: the fast traversal applies
+  int root_ref = 0;
+  float grid_base[3] = {0, 0, 0}, grid_pitch[3] = {1, 1, 1};
+  uint32_t root_w[3] = {0x7fff0000u, 0x7fff0000u, 0x7fff0000u};  // the root box as node-record words (max plane << 16 | min plane)
+  float cull_abs = 0.0f, cmax = 0.0f;
+  int fast_ok = 0;
+};
+
+struct Repacked : SceneDesc {
   struct f4 { float x, y, z, w; };
   struct u4 { uint32_t x, y, z, w; };
   raw_vector<u4> nodes;         // node_f4 x 16 bytes per interior node (rt_trace.cuh "repacked scene")
@@ -31,17 +46,7 @@ struct Repacked {
                                 // third vector = the triangle's id
   std::vector<int32_t> tri_mat;
   raw_vector<int32_t> leaf_count;  // per node of the as-is array: leaves in its sub-tree (validate_chain, rt_trace.cuh)
-  int n_nodes9 = 0, n_inner = 0, n_tris = 0;
-  int node_f4 = 2;              // 2 in global memory, 3 when nodes + triangles fit the shared-memory staging area
-  int depth = 0, ref_stack_need = 0;   // of the caller's tree
-  int cull_depth = 0;           // level of the deepest leaf of the tree `nodes` holds (sizes the traversal stacks)
   int cull_tree = 0;            // 0: `nodes` has the caller's topology, 1: the tree of cull_tree.cpp
-  bool canonical = true;        // strict two-child tree with nested boxes: the fast traversal applies
-  int root_ref = 0;
-  float grid_base[3] = {0, 0, 0}, grid_pitch[3] = {1, 1, 1};
-  uint32_t root_w[3] = {0x7fff0000u, 0x7fff0000u, 0x7fff0000u};  // the root box as node-record words (max plane << 16 | min plane)
-  float cull_abs = 0.0f, cmax = 0.0f;
-  int fast_ok = 0;
   double ms_tris = 0, ms_walk = 0, ms_nodes = 0;  // host time of the three stages
 };
 

@@ -77,7 +77,7 @@ typedef struct {
                              parts that run concurrently on N CUDA streams of the same GPU (each with its own path state) and
                              whose per-pixel sums are added in part order by the reduce kernel — several samples of a pixel in
                              flight, which fills the GPU on small frames and overlaps shading with tracing on large ones.
-                             -1: chosen from the frame size (2 from 1 Mpixel, 4 from 0.2 Mpixel, else 8).  The image equals
+                             -1: chosen from the frame size (3 from 1 Mpixel, 4 from 0.2 Mpixel, else 8).  The image equals
                              the one-stream image up to the order of N float additions per pixel. */
   int32_t sampling;       /* bit mask of B200RT_SAMPLING_*; 0 = the reference's estimator (default) */
 } b200rt_opts;
