@@ -33,10 +33,6 @@ struct DevBuf {
 // the scene's device buffers, which sample-stream helpers borrow as a set
 enum SceneBuf { kNodes, kTris, kCtris, kNormals, kTboxes, kFrames, kMats, kBvh9, kLeafcnt, kLight, kSceneBufs };
 
-// k_trace's lane scheduling (KernelArgs::quorum, refill_min, tri_quorum) and the wavefront iterations between two
-// compactions of the path list
-constexpr int kQuorum = 12, kRefillMin = 8, kTriQuorum = 2;
-constexpr int kCompactEvery = 4;
 // Resident k_trace CTAs per SM while three or more sample streams share the GPU.  A k_trace that fills every SM's
 // register file leaves the other streams' kernels nothing but its tail to run in; capped, one stream's shading and
 // another's tracing are resident side by side (bench scene -4 %, Cornell 1080p -12 %, measured with 3 streams).
@@ -271,7 +267,6 @@ void fill_args(b200rt_ctx *c, const FrameParams &F, const b200rt_opts &o, float 
   A->slots = static_cast<int *>(c->d_slots.p);
   A->part_count = static_cast<unsigned int *>(c->d_part_count.p);
   A->wc = nullptr;
-  A->compact_every = kCompactEvery;
   A->counters = c->d_counters;
   A->n_nodes = D.n_inner;
   A->n_tris = D.n_tris;
@@ -279,9 +274,6 @@ void fill_args(b200rt_ctx *c, const FrameParams &F, const b200rt_opts &o, float 
   A->tiles_x = (F.width + 7) / 8;
   int tiles_y = (F.height + 3) / 4;
   A->n_work = A->tiles_x * tiles_y * 32;
-  A->quorum = kQuorum;
-  A->refill_min = kRefillMin;
-  A->tri_quorum = kTriQuorum;
   A->validate = 0;
   A->ad = AdaptArgs();
 }
@@ -610,12 +602,12 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
     }
   }
   // A fixed-spp frame is one batch of every iteration, enqueued without a look back.  An adaptive frame runs batches of
-  // kAdaptBatch iterations rounded up to a multiple of compact_every, so that every batch ends with a compaction and its
+  // kAdaptBatch iterations rounded up to a multiple of kCompactEvery, so that every batch ends with a compaction and its
   // last cnt word is the number of live paths.  That word is copied to pinned memory behind an event; before batch k + 2
   // is enqueued the host waits for batch k's and stops once it is 0.  One batch is always in flight, so the GPU does not
   // wait for the host.  A k_shade on an empty list does nothing, so stopping there leaves the image the full loop would
   // make.
-  const int batch = ad ? (kAdaptBatch + A.compact_every - 1) / A.compact_every * A.compact_every : n_iter + 1;
+  const int batch = ad ? (kAdaptBatch + kCompactEvery - 1) / kCompactEvery * kCompactEvery : n_iter + 1;
   int it = 0, n_shade = 0, n_trace = 0, n_compactions = 0;
   for (int b = 0; it <= n_iter; ++b) {
     if (ad && b >= 2) {
@@ -627,7 +619,7 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
       if (o.time_kernels) CU(cudaEventRecord(c->kev[c->kev_used++], c->stream));
       wl.shade<<<wl.shade_grid, kShadeBlock, 0, c->stream>>>(A, it);
       ++n_shade;
-      if (it < n_iter && (it + 1) % A.compact_every == 0) {  // close the gaps the finished pixels left, order kept (timed with k_shade)
+      if (it < n_iter && (it + 1) % kCompactEvery == 0) {  // close the gaps the finished pixels left, order kept (timed with k_shade)
         k_compact<<<wl.shade_grid, kCompactBlock, 0, c->stream>>>(A.slots, A.cnt + it, 0u, A.part_count, A.list[(it + 1) & 1], A.cnt + it + 1);
         ++n_compactions;
       }
@@ -1201,11 +1193,10 @@ int b200rt_finalize_device(b200rt_ctx *c, const float *d_sums, float *d_out, int
   if (!c) return B200RT_ERR_INVALID;
   if (!d_sums || !d_out || n_pixels <= 0 || spp <= 0) return fail(c, B200RT_ERR_INVALID, "bad finalize arguments");
   CU(cudaSetDevice(c->device));
-  long long n = (long long)n_pixels * 3;
-  int grid = (int)std::min<long long>((n + 255) / 256, (long long)c->sm_count * 8);
-  k_finalize<<<grid, 256, 0, c->stream>>>(d_sums, d_out, n, (float)spp);
-  CU(cudaGetLastError());
-  return 0;
+  PartList pl;
+  pl.n = 1;
+  pl.p[0] = d_sums;
+  return launch_reduce(c, pl, d_out, (long long)n_pixels * 3, (float)spp);
 }
 
 int b200rt_reduce_finalize_device(b200rt_ctx *c, const float *const *d_parts, int n_parts, float *d_out,

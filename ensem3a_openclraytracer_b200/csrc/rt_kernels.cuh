@@ -12,7 +12,7 @@
 //               registers and advance them one node per turn; leaves are parked in shared memory and tested by
 //               the warp together; a lane whose ray is done writes the hit and is refilled from the list, so
 //               the node loop stays full whatever the individual traversal lengths.
-//   k_finalize / k_reduce_finalize / k_img_processing   the accumulate / clamp / tonemap passes.
+//   k_reduce_finalize / k_img_processing   the accumulate / clamp / tonemap passes.
 // An adaptive frame (b200rt_render_adaptive) runs k_adaptive_init before k_primary and k_shade<NEE, true>, whose
 // end_sample block also applies the stopping rule (adaptive_end_sample); the host ends its loop once the list is empty.
 #pragma once
@@ -24,6 +24,10 @@ namespace b200rt {
 constexpr int kBlock = 128;        // k_primary, k_trace, k_trace_rays
 constexpr int kShadeBlock = 128;
 constexpr unsigned kChunk = 32;    // rays a warp claims from the list per atomic (64 / 128 lose to the longer tails)
+// k_trace's lane scheduling: the node phase ends when fewer than kQuorum lanes can step; idle lanes pull new rays once
+// kRefillMin are idle; the leaf phase repeats while at least kTriQuorum lanes hold a parked leaf
+constexpr int kQuorum = 12, kRefillMin = 8, kTriQuorum = 2;
+constexpr int kCompactEvery = 4;   // k_shade(i) hands its output to k_compact when (i + 1) % kCompactEvery == 0
 constexpr int kHitNeedsExactWalk = -2;  // pHit.x of a ray k_trace did not walk (see k_trace); k_shade walks it exactly
 
 struct DeviceCounters {
@@ -39,12 +43,6 @@ struct AdaptArgs {
   float rel_error, floor;
 };
 
-// path state, one entry per pixel:
-//   pA = origin.xyz, dir.x     pB = dir.y, dir.z, meta, rng     pC = throughput.rgb, -     pHit = triangle, distance
-// origin / dir describe the ray in flight (for a sun ray `dir` keeps the escaped direction for the environment
-// lookup and the ray itself points along FrameParams::sun_dir).
-// meta: bit 0 first iteration (no ray traced yet), bit 1 light ray (opt-in light sampling), bit 3 sun ray, bits 4-7
-// material type of the surface the ray left, bits 8-15 bounce j, bits 16-31 sample index
 struct KernelArgs {
   FrameParams F;
   SceneView S;            // global-memory view (the SMEM variant rebuilds node / triangle pointers)
@@ -52,7 +50,7 @@ struct KernelArgs {
   float4 *prim_dirk;      // per pixel: primary direction xyz, hit distance
   int *prim_tri;          // per pixel: primary triangle
   float *out;             // width*height*3: running sums, then the image
-  float4 *pA, *pB, *pC;   // pC.w: density with which the surface the ray left drew its direction (light sampling only)
+  float4 *pA, *pB, *pC;   // path state (below); pC.w: density with which the surface the ray left drew its direction (light sampling only)
   int2 *pHit;
   // opt-in light sampling (k_shade<true>): the emitter triangles, and three more float4 of path state
   const int *light;       // triangles whose material is emissive, ascending (what FileManager.py:235-240 lists)
@@ -64,7 +62,6 @@ struct KernelArgs {
                           // left the wavefront since the last compaction (k_shade and k_trace skip such entries)
   int *slots;             // k_primary's / k_shade's output on the iterations that are followed by a compaction
   unsigned int *part_count;  // survivors per contiguous part of `slots` (one part per producer CTA)
-  int compact_every;      // k_shade(i) hands its output to k_compact when (i + 1) % compact_every == 0
   unsigned int *cnt;      // cnt[i] = entries of the list consumed by shade iteration i
   unsigned int *wc;       // wc[i]  = rays of trace iteration i handed out so far
   DeviceCounters *counters;
@@ -72,15 +69,54 @@ struct KernelArgs {
   int stack_depth;        // entries per lane
   int n_work;             // work items (32-pixel tiles x 32)
   int tiles_x;
-  int quorum;             // k_trace: the node phase ends when fewer lanes than this can step
-  int refill_min;         // idle lanes pull new rays once this many are idle
-  int tri_quorum;         // the leaf phase repeats while at least this many lanes hold a parked leaf
   int validate;           // 1: hits come from the conservative traversal and must pass validate_hit
-  AdaptArgs ad;           // k_shade<NEE, true> and k_adaptive_init only (last, so the other kernels' parameter offsets stay)
+  AdaptArgs ad;           // k_shade<NEE, true> and k_adaptive_init only
+};
+
+// path state, one entry per pixel:
+//   pA = origin.xyz, dir.x     pB = dir.y, dir.z, meta, rng     pC = throughput.rgb, -     pHit = triangle, distance
+// origin / dir describe the ray in flight (for a sun ray `dir` keeps the escaped direction for the environment
+// lookup and the ray itself points along FrameParams::sun_dir: trace_dir).
+// meta: bit 0 first iteration (no ray traced yet), bit 1 light ray (opt-in light sampling), bit 3 sun ray, bits 4-7
+// material type of the surface the ray left, bits 8-15 bounce j, bits 16-31 sample index
+struct PathMeta {
+  int first, light, sun, type, j, s;
 };
 
 RT_DEV uint32_t meta_pack(int first, int sun, int type, int j, int s, int light = 0) {
   return (uint32_t)first | ((uint32_t)light << 1) | ((uint32_t)sun << 3) | ((uint32_t)(type & 15) << 4) | ((uint32_t)(j & 255) << 8) | ((uint32_t)s << 16);
+}
+
+RT_DEV PathMeta meta_unpack(uint32_t m) {
+  return {(int)(m & 1u), (int)((m >> 1) & 1u), (int)((m >> 3) & 1u), (int)((m >> 4) & 15u), (int)((m >> 8) & 255u), (int)(m >> 16)};
+}
+
+// direction of the ray a path traces, from its stored direction d
+RT_DEV v3 trace_dir(const FrameParams &F, v3 d, int sun) { return sun ? F.sun_dir : d; }
+
+// ---- counters -------------------------------------------------------------------------------------------------------
+// the sum of v over the warp, in lane 0 (every lane calls it)
+template <class T>
+RT_DEV T warp_sum(T v) {
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+  return v;
+}
+
+// adds a warp's sum (warp_sum) to a device counter: one atomic from lane 0, none for 0
+template <class T>
+RT_DEV void flush(unsigned long long *dst, T warp_total) {
+  if ((threadIdx.x & 31u) == 0u && warp_total) atomicAdd(dst, (unsigned long long)warp_total);
+}
+
+// part_count[blockIdx.x] = the sum of v over the CTA (every thread calls it)
+RT_DEV void cta_count(unsigned int *part_count, unsigned int v) {
+  __shared__ unsigned int total;
+  if (threadIdx.x == 0) total = 0u;
+  __syncthreads();
+  v = warp_sum(v);
+  if ((threadIdx.x & 31u) == 0u && v) atomicAdd(&total, v);
+  __syncthreads();
+  if (threadIdx.x == 0) part_count[blockIdx.x] = total;
 }
 
 // ---- shared-memory staging of a small scene with the bulk-copy engine (TMA 1-D) ------------------------
@@ -147,15 +183,19 @@ RT_DEV int work_to_pixel(const KernelArgs &A, unsigned int w) {
   return i;
 }
 
+// a pixel's image from the sum of its n samples (Raytracing.cl:211-219)
+RT_DEV void write_mean(float *o, v3 sum, float n) {
+  o[0] = clamp01(sum.x / n);
+  o[1] = clamp01(sum.y / n);
+  o[2] = clamp01(sum.z / n);
+}
+
 RT_DEV void write_pixel(const KernelArgs &A, int i, v3 sum) {
   float *o = A.out + 3 * (size_t)i;
   if (A.F.out_mode == 1) {
     o[0] = sum.x; o[1] = sum.y; o[2] = sum.z;
-  } else {  // Raytracing.cl:211-219
-    float n = (float)A.F.spp;
-    o[0] = clamp01(sum.x / n);
-    o[1] = clamp01(sum.y / n);
-    o[2] = clamp01(sum.z / n);
+  } else {
+    write_mean(o, sum, (float)A.F.spp);
   }
 }
 
@@ -187,10 +227,7 @@ RT_DEV bool adaptive_end_sample(const KernelArgs &A, int i, int n, v3 c, v3 sum)
   ad.err_out[i] = sqrtf((w.y / (float)(n - 1)) / (float)n);
   if (stop) {
     ad.spp_out[i] = n;
-    float *o = A.out + 3 * (size_t)i;
-    o[0] = clamp01(sum.x / (float)n);
-    o[1] = clamp01(sum.y / (float)n);
-    o[2] = clamp01(sum.z / (float)n);
+    write_mean(A.out + 3 * (size_t)i, sum, (float)n);
   }
   return stop;
 }
@@ -218,7 +255,6 @@ __global__ void __launch_bounds__(kBlock) k_primary(const __grid_constant__ Kern
   st.base = reinterpret_cast<uint32_t *>(smem + used) + threadIdx.x;
   st.stride = kBlock;
   uint32_t *parks = reinterpret_cast<uint32_t *>(smem + used + (size_t)kBlock * A.stack_depth * sizeof(uint32_t)) + threadIdx.x;
-  const unsigned int lane = threadIdx.x & 31u;
   TraceCounters tc;
   tc.box_tests = 0; tc.tri_tests = 0;
   unsigned int mism = 0;
@@ -238,8 +274,7 @@ __global__ void __launch_bounds__(kBlock) k_primary(const __grid_constant__ Kern
         int mat_type = -1;
         float emit = 0.0f;
         if (h.tri >= 0) {
-          int mat = __float_as_int(__ldg(S.tris + 3 * (size_t)h.tri + 2).y);
-          Material m = load_material(S.mats, mat);
+          Material m = load_material(S.mats, tri_material(S, h.tri));
           mat_type = m.type;
           emit = m.roughness;
         }
@@ -267,19 +302,13 @@ __global__ void __launch_bounds__(kBlock) k_primary(const __grid_constant__ Kern
     }
     if (!PARITY) A.slots[w] = live ? i : -1;   // work items are in tile order; k_count_parts + k_compact make the first list
   }
-  // one atomic per warp
-  for (int o = 16; o > 0; o >>= 1) {
-    rays += __shfl_down_sync(0xffffffffu, rays, o);
-    mism += __shfl_down_sync(0xffffffffu, mism, o);
-  }
-  if (lane == 0) {
-    if (rays) atomicAdd(&A.counters->rays, rays);
-    if (rays) atomicAdd(&A.counters->primary_rays, rays);
-    if (mism) atomicAdd(&A.counters->mismatches, (unsigned long long)mism);
-  }
+  rays = warp_sum(rays);
+  flush(&A.counters->rays, rays);
+  flush(&A.counters->primary_rays, rays);
+  flush(&A.counters->mismatches, warp_sum(mism));
   if (STATS) {
-    if (tc.box_tests) atomicAdd(&A.counters->box_tests, tc.box_tests);
-    if (tc.tri_tests) atomicAdd(&A.counters->tri_tests, tc.tri_tests);
+    flush(&A.counters->box_tests, warp_sum(tc.box_tests));
+    flush(&A.counters->tri_tests, warp_sum(tc.tri_tests));
   }
 }
 
@@ -300,13 +329,7 @@ __global__ void __launch_bounds__(kCompactBlock) k_count_parts(const int *__rest
   const unsigned int end = min(n, (blockIdx.x + 1u) * part);
   unsigned int c = 0;
   for (unsigned int t = blockIdx.x * part + threadIdx.x; t < end; t += kCompactBlock) c += slots[t] >= 0 ? 1u : 0u;
-  __shared__ unsigned int total;
-  if (threadIdx.x == 0) total = 0u;
-  __syncthreads();
-  for (int o = 16; o > 0; o >>= 1) c += __shfl_down_sync(0xffffffffu, c, o);
-  if ((threadIdx.x & 31) == 0 && c) atomicAdd(&total, c);
-  __syncthreads();
-  if (threadIdx.x == 0) part_count[blockIdx.x] = total;
+  cta_count(part_count, c);
 }
 
 // list_out = the non-negative entries of slots[0 .. n), order kept; *n_out = their number.  One CTA per part (same
@@ -328,10 +351,8 @@ __global__ void __launch_bounds__(kCompactBlock) k_compact(const int *__restrict
   if (threadIdx.x == 0) s_base = 0u;
   if (threadIdx.x < kCompactBlock / 32) s_warp[threadIdx.x] = 0u;
   __syncthreads();
-  for (int o = 16; o > 0; o >>= 1) {
-    before += __shfl_down_sync(0xffffffffu, before, o);
-    all += __shfl_down_sync(0xffffffffu, all, o);
-  }
+  before = warp_sum(before);
+  all = warp_sum(all);
   if (lane == 0) {
     if (before) atomicAdd(&s_base, before);
     if (all) atomicAdd(&s_warp[0], all);
@@ -375,13 +396,13 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
   unsigned long long samples = 0;
   unsigned int reval = 0, exact = 0, survivors = 0;
   // Every CTA shades one contiguous part of the list and leaves, entry for entry, the path or -1 in the next list;
-  // every compact_every iterations k_compact closes the gaps without changing the order (paths leave the wavefront
+  // every kCompactEvery iterations k_compact closes the gaps without changing the order (paths leave the wavefront
   // only when their pixel is finished, so gaps accumulate slowly).  The list therefore stays sorted by tile for the whole
   // frame: the 32 paths of a warp — here and in k_trace — belong to neighbouring pixels, so the rays that restart
   // from the cached primary hits leave from neighbouring points.  (An atomically appended list is a random
   // permutation of the pixels after a few hundred iterations; on the 5 M-triangle scene that cost a third of the
   // traversal speed.)
-  const bool compacting = ((iter + 1) % A.compact_every) == 0;
+  const bool compacting = ((iter + 1) % kCompactEvery) == 0;
   int *out = compacting ? A.slots : A.list[(iter + 1) & 1];
   const unsigned int part = part_size(n_in, gridDim.x);
   const unsigned int part_end = min(n_in, (blockIdx.x + 1u) * part);
@@ -414,19 +435,19 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
         hk = __int_as_float(hh.y);
       }
     }
-    const bool first = (meta & 1u) != 0u;
-    int sun_ray = (int)((meta >> 3) & 1u), seg_type = (int)((meta >> 4) & 15u);
-    int j = (int)((meta >> 8) & 255u), s = (int)(meta >> 16);
-    const bool light_ray = NEE && ((meta >> 1) & 1u) != 0u;
+    const PathMeta pm = meta_unpack(meta);
+    const bool first = pm.first != 0;
+    int sun_ray = pm.sun, seg_type = pm.type, j = pm.j, s = pm.s;
+    const bool light_ray = NEE && pm.light != 0;
     bool pixel_done = false, start = valid && first, shade = false, end_sample = false, sun_done = false;
     bool want_light = false, light_done = false, from_light = false;
 
     // ---- phase 1: the winner of the conservative walk must pass the exact leaf-box test ---------------------------------
     if (valid && !first && A.validate && htri != -1) {
-      const v3 dray = sun_ray ? F.sun_dir : d;   // a light ray's direction sits in d
+      const v3 dray = trace_dir(F, d, sun_ray);   // a light ray's direction sits in d
       if (htri == kHitNeedsExactWalk ||
-          !validate_winner(S, o, dray, htri, __float_as_int(__ldg(S.tris + 3 * (size_t)htri + 2).z))) {  // out-of-range or grazing ray: re-trace exactly
-        const Hit h = closest_hit_nodrop<false>(S, o, dray);
+          !validate_winner(S, o, dray, htri, tri_rank(S, htri))) {  // out-of-range or grazing ray: re-trace exactly
+        const Hit h = closest_hit_nodrop(S, o, dray);
         if (htri != kHitNeedsExactWalk) ++reval; else ++exact;
         htri = h.tri;
         hk = h.k;
@@ -440,8 +461,7 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
         light_done = true;
       } else if (!sun_ray) {
         if (htri >= 0) {  // the bounce ray becomes the current segment (:91-93)
-          const int mat = __float_as_int(__ldg(S.tris + 3 * (size_t)htri + 2).y);
-          const Material mb = load_material(S.mats, mat);
+          const Material mb = load_material(S.mats, tri_material(S, htri));
           if (mb.type != 0) {
             if (j == F.max_bounce) {  // :99-103
               acc = mk3(0.0f, 0.0f, 0.0f);
@@ -454,9 +474,8 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
             acc = acc * mb.roughness;
             if (NEE && seg_type != 3) {
               // the light sample at the surface this ray left could have made the same connection: balance heuristic
-              const float4 t0 = __ldg(S.tris + 3 * (size_t)htri), t1 = __ldg(S.tris + 3 * (size_t)htri + 1);
-              const float4 t2 = __ldg(S.tris + 3 * (size_t)htri + 2);
-              const float pl = light_pdf(mk3(t0.w, t1.x, t1.y), mk3(t1.z, t1.w, t2.x), A.n_light, unit(d), (hk * hk) * dot(d, d));
+              const Tri t = load_tri(S.tris, htri);
+              const float pl = light_pdf(t.e1, t.e2, A.n_light, unit(d), (hk * hk) * dot(d, d));
               const float den = pb_ray + pl;
               acc = acc * (den > 0.0f ? pb_ray / den : 0.0f);
             }
@@ -475,8 +494,7 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
       if (htri < 0) {
         if (seg_type != 3) sun = mk3(F.sun_power, F.sun_power, F.sun_power);
       } else {
-        const int mat = __float_as_int(__ldg(S.tris + 3 * (size_t)htri + 2).y);
-        const Material ms = load_material(S.mats, mat);
+        const Material ms = load_material(S.mats, tri_material(S, htri));
         if (ms.type == 3) sun = ms.color * F.sun_power;
       }
       v3 envl;
@@ -534,8 +552,7 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
       j = 0;
       if (NEE) {
         A.pR[pix] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-        const int mat0 = __float_as_int(__ldg(S.tris + 3 * (size_t)htri + 2).y);
-        if ((int)__ldg(S.mats + 6 * mat0) != 3) want_light = true; else shade = true;
+        if ((int)__ldg(S.mats + 6 * tri_material(S, htri)) != 3) want_light = true; else shade = true;
       } else {
         shade = true;
       }
@@ -544,10 +561,9 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
 
     // ---- phase 3b (light sampling only): one emitter point seen from the surface, and the shadow ray towards it --------------
     if (NEE && want_light) {
-      const float4 t2 = __ldg(S.tris + 3 * (size_t)htri + 2);
       const float4 nn = __ldg(S.normals + htri);
       const v3 n = mk3(nn.x, nn.y, nn.z);
-      const Material m = load_material(S.mats, __float_as_int(t2.y));
+      const Material m = load_material(S.mats, tri_material(S, htri));
       const v3 un = unit(n);
       float ul, ua, ub;
       if (F.rng_mode == 0) draw3_light<0>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, F.key0, F.key1, &ul, &ua, &ub);
@@ -555,13 +571,12 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
       int idx = (int)(ul * (float)A.n_light);
       if (idx > A.n_light - 1) idx = A.n_light - 1;
       const int lt = __ldg(A.light + idx);
-      const float4 l0 = __ldg(S.tris + 3 * (size_t)lt), l1 = __ldg(S.tris + 3 * (size_t)lt + 1), l2 = __ldg(S.tris + 3 * (size_t)lt + 2);
-      const Material ml = load_material(S.mats, __float_as_int(l2.y));
+      const Tri l = load_tri(S.tris, lt);
+      const Material ml = load_material(S.mats, l.mat);
       const float Le = ml.type == 0 ? ml.roughness : 0.0f;
       const v3 x = o + unit(d) * hk;
       v3 w;
-      const v3 direct = sample_light(m, F.sampling, n, un, x, d, acc, mk3(l0.x, l0.y, l0.z), mk3(l0.w, l1.x, l1.y),
-                                     mk3(l1.z, l1.w, l2.x), Le, A.n_light, ua, ub, &w);
+      const v3 direct = sample_light(m, F.sampling, n, un, x, d, acc, l.A, l.e1, l.e2, Le, A.n_light, ua, ub, &w);
       A.pS[pix] = make_float4(d.x, d.y, d.z, __int_as_float(htri));
       A.pL[pix] = make_float4(direct.x, direct.y, direct.z, __int_as_float(lt));
       o = x;
@@ -572,10 +587,9 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
 
     // ---- phase 4: next direction, BRDF * cos / pdf (:51-87); segment = (o, d, hk, htri) ------------------------------------------
     if (shade) {
-      const float4 t2 = __ldg(S.tris + 3 * (size_t)htri + 2);
       const float4 nn = __ldg(S.normals + htri);
       const v3 n = mk3(nn.x, nn.y, nn.z);
-      const Material m = load_material(S.mats, __float_as_int(t2.y));
+      const Material m = load_material(S.mats, tri_material(S, htri));
       const TriFrame tf = load_tri_frame(S.frames, htri, m.type == 3 ? 0 : (m.type == 1 ? 1 : 2));
       v3 nd, brdf;
       float inv_pdf;
@@ -620,24 +634,11 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
   if (!compacting) {  // the next list has this one's length
     if (blockIdx.x == 0 && threadIdx.x == 0) A.cnt[iter + 1] = n_in;
   } else {  // survivors of this CTA's part, for k_compact
-    __shared__ unsigned int cta_survivors;
-    if (threadIdx.x == 0) cta_survivors = 0u;
-    __syncthreads();
-    for (int o = 16; o > 0; o >>= 1) survivors += __shfl_down_sync(0xffffffffu, survivors, o);
-    if (lane == 0 && survivors) atomicAdd(&cta_survivors, survivors);
-    __syncthreads();
-    if (threadIdx.x == 0) A.part_count[blockIdx.x] = cta_survivors;
+    cta_count(A.part_count, survivors);
   }
-  for (int o = 16; o > 0; o >>= 1) {
-    samples += __shfl_down_sync(0xffffffffu, samples, o);
-    reval += __shfl_down_sync(0xffffffffu, reval, o);
-    exact += __shfl_down_sync(0xffffffffu, exact, o);
-  }
-  if (lane == 0) {
-    if (samples) atomicAdd(&A.counters->samples, samples);
-    if (reval) atomicAdd(&A.counters->revalidated, (unsigned long long)reval);
-    if (exact) atomicAdd(&A.counters->exact_walks, (unsigned long long)exact);
-  }
+  flush(&A.counters->samples, warp_sum(samples));
+  flush(&A.counters->revalidated, warp_sum(reval));
+  flush(&A.counters->exact_walks, warp_sum(exact));
 }
 
 // per-triangle sampling frames, once per scene upload
@@ -682,7 +683,7 @@ __global__ void __launch_bounds__(kBlock) k_trace(const __grid_constant__ Kernel
   TraceCounters tc;
   tc.box_tests = 0; tc.tri_tests = 0;
 
-  int thresh = A.quorum;  // the node phase runs while at least this many lanes can step
+  int thresh = kQuorum;  // the node phase runs while at least this many lanes can step
   for (;;) {
     // ---- node phase: one node per lane per turn -----------------------------------------------------------------------------
     for (;;) {
@@ -698,7 +699,7 @@ __global__ void __launch_bounds__(kBlock) k_trace(const __grid_constant__ Kernel
         test_parked<SMEM>(S, T, parks[pn * kBlock], T.o, T.d);
       }
       pm = __ballot_sync(0xffffffffu, pn > 0);
-      if (__popc(pm) < A.tri_quorum) break;
+      if (__popc(pm) < kTriQuorum) break;
     }
     // ---- finished rays are handed back; idle lanes pull the next rays together ---------------------------------------------------
     const bool finished = (path >= 0) && !trav_active(T) && pn == 0;
@@ -713,8 +714,8 @@ __global__ void __launch_bounds__(kBlock) k_trace(const __grid_constant__ Kernel
     }
     const int n_idle = __popc(idle);
     if (n_idle == 0) continue;
-    if (n_idle < A.refill_min &&
-        __popc(__ballot_sync(0xffffffffu, trav_active(T) && pn <= kParkCap - 2)) >= A.quorum)
+    if (n_idle < kRefillMin &&
+        __popc(__ballot_sync(0xffffffffu, trav_active(T) && pn <= kParkCap - 2)) >= kQuorum)
       continue;  // enough lanes can still step: let more finish before paying for a refill
     {
       int need = n_idle;
@@ -736,7 +737,7 @@ __global__ void __launch_bounds__(kBlock) k_trace(const __grid_constant__ Kernel
           if (path >= 0) {   // -1: the path left the wavefront since the last compaction; the lane waits for the next refill
             const float4 sa = ld_stream(A.pA + path), sb = ld_stream(A.pB + path);
             const v3 o = mk3(sa.x, sa.y, sa.z);
-            const v3 d = ((__float_as_uint(sb.z) >> 3) & 1u) ? A.F.sun_dir : mk3(sa.w, sb.x, sb.y);
+            const v3 d = trace_dir(A.F, mk3(sa.w, sb.x, sb.y), meta_unpack(__float_as_uint(sb.z)).sun);
             rays++;
             if (TRAV == 0) {
               if (ray_is_fast(S, o)) {
@@ -762,21 +763,11 @@ __global__ void __launch_bounds__(kBlock) k_trace(const __grid_constant__ Kernel
     }
   }
 
-  for (int o = 16; o > 0; o >>= 1) {
-    rays += __shfl_down_sync(0xffffffffu, rays, o);
-    mism += __shfl_down_sync(0xffffffffu, mism, o);
-    if (STATS) {
-      tc.box_tests += __shfl_down_sync(0xffffffffu, tc.box_tests, o);
-      tc.tri_tests += __shfl_down_sync(0xffffffffu, tc.tri_tests, o);
-    }
-  }
-  if (lane == 0) {
-    atomicAdd(&A.counters->rays, (unsigned long long)rays);
-    if (mism) atomicAdd(&A.counters->mismatches, (unsigned long long)mism);
-    if (STATS) {
-      atomicAdd(&A.counters->box_tests, tc.box_tests);
-      atomicAdd(&A.counters->tri_tests, tc.tri_tests);
-    }
+  flush(&A.counters->rays, warp_sum(rays));
+  flush(&A.counters->mismatches, warp_sum(mism));
+  if (STATS) {
+    flush(&A.counters->box_tests, warp_sum(tc.box_tests));
+    flush(&A.counters->tri_tests, warp_sum(tc.tri_tests));
   }
 }
 
@@ -800,22 +791,16 @@ __global__ void __launch_bounds__(kBlock) k_trace_rays(const __grid_constant__ K
     tri_out[i] = h.tri;
     k_out[i] = h.k;
   }
+  flush(&A.counters->mismatches, warp_sum(mism));
   if (STATS) {
-    atomicAdd(&A.counters->box_tests, tc.box_tests);
-    atomicAdd(&A.counters->tri_tests, tc.tri_tests);
+    flush(&A.counters->box_tests, warp_sum(tc.box_tests));
+    flush(&A.counters->tri_tests, warp_sum(tc.tri_tests));
   }
-  if (mism) atomicAdd(&A.counters->mismatches, (unsigned long long)mism);
 }
 
 // ---- accumulate / clamp / tonemap ---------------------------------------------------------------------------------------------
-// out = clamp(sum / spp)   (Raytracing.cl:211-219), float4-vectorised when aligned
-__global__ void k_finalize(const float *__restrict__ sums, float *__restrict__ out, long long n, float spp) {
-  long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-  long long stride = (long long)gridDim.x * blockDim.x;
-  for (; i < n; i += stride) out[i] = clamp01(sums[i] / spp);
-}
-
-// fused multi-GPU reduce + finalize: parts[] may live on peer GPUs (NVLink P2P loads); summed in rank order
+// out = clamp(sum of the parts / spp)   (Raytracing.cl:211-219), float4-vectorised when aligned; parts[] may live on peer
+// GPUs (NVLink P2P loads) and are summed in rank order
 struct PartList {
   const float *p[16];
   int n;

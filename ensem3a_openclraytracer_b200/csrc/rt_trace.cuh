@@ -94,12 +94,6 @@ struct Hit {
 
 // Path state is read once per kernel and streams through the SM: these loads do not allocate a line in L1, which is
 // left to the nodes and triangles the lanes come back to.
-#ifdef B200RT_NO_STREAM   // development A/B
-RT_DEV float4 ld_stream(const float4 *p) { return *p; }
-RT_DEV int2 ld_stream(const int2 *p) { return *p; }
-RT_DEV int ld_stream(const int *p) { return *p; }
-RT_DEV float ld_stream(const float *p) { return *p; }
-#else
 RT_DEV float4 ld_stream(const float4 *p) {
   float4 v;
   asm volatile("ld.global.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
@@ -120,13 +114,29 @@ RT_DEV float ld_stream(const float *p) {
   asm volatile("ld.global.L1::no_allocate.f32 %0, [%1];" : "=f"(v) : "l"(p));
   return v;
 }
-#endif
 
 template <bool SMEM>
 RT_DEV float4 ld4(const float4 *p) {
   if (SMEM) return *p;
   return __ldg(p);
 }
+
+// triangle record `t` of `tris` or `ctris` (format above), decoded; SMEM: the copy staged in shared memory
+struct Tri {
+  v3 A, e1, e2;
+  int mat, rank, id;   // id: ctris records only
+};
+template <bool SMEM = false>
+RT_DEV Tri load_tri(const float4 *tris, int t) {
+  const float4 *p = tris + 3 * (size_t)t;
+  const float4 t0 = ld4<SMEM>(p), t1 = ld4<SMEM>(p + 1), t2 = ld4<SMEM>(p + 2);
+  return {mk3(t0.x, t0.y, t0.z), mk3(t0.w, t1.x, t1.y), mk3(t1.z, t1.w, t2.x), __float_as_int(t2.y), __float_as_int(t2.z),
+          __float_as_int(t2.w)};
+}
+
+// material id / visiting rank of triangle `tri`: the record's third float4 alone
+RT_DEV int tri_material(const SceneView &S, int tri) { return __float_as_int(__ldg(S.tris + 3 * (size_t)tri + 2).y); }
+RT_DEV int tri_rank(const SceneView &S, int tri) { return __float_as_int(__ldg(S.tris + 3 * (size_t)tri + 2).z); }
 
 // One node = 32 contiguous bytes: one 256-bit load from global memory (LDG.E.256, sm_100+), two 128-bit loads from
 // shared memory.  Lanes of a warp sit at unrelated nodes, so the L1 cost of a node visit is one wavefront per lane
@@ -292,15 +302,13 @@ RT_DEV bool tri_hit(v3 o, v3 d, v3 A, v3 e1, v3 e2, float *k_out) {
 
 template <bool SMEM>
 RT_DEV void test_triangle(const SceneView &S, int leaf, v3 o, v3 d, Hit &best, int &best_rank) {
-  const float4 *p = S.ctris + 3 * (size_t)leaf;
-  float4 t0 = ld4<SMEM>(p), t1 = ld4<SMEM>(p + 1), t2 = ld4<SMEM>(p + 2);
+  const Tri t = load_tri<SMEM>(S.ctris, leaf);
   float k;
-  if (tri_hit(o, d, mk3(t0.x, t0.y, t0.z), mk3(t0.w, t1.x, t1.y), mk3(t1.z, t1.w, t2.x), &k) && k > 0.0001f) {
-    int rank = __float_as_int(t2.z);
-    if (k < best.k || (k == best.k && best.tri >= 0 && rank < best_rank)) {
+  if (tri_hit(o, d, t.A, t.e1, t.e2, &k) && k > 0.0001f) {
+    if (k < best.k || (k == best.k && best.tri >= 0 && t.rank < best_rank)) {
       best.k = k;
-      best.tri = __float_as_int(t2.w);
-      best_rank = rank;
+      best.tri = t.id;
+      best_rank = t.rank;
     }
   }
 }
@@ -347,7 +355,7 @@ RT_DEV bool validate_winner(const SceneView &S, v3 o, v3 d, int tri, int rank) {
 // ---- reference-order traversal ---------------------------------------------------------------------------
 constexpr int kRefStack = 64;   // b200rt_set_scene routes trees that need more to REFERENCE mode with the caller's cap
 
-template <bool SMEM, bool STATS>
+template <bool STATS>
 RT_DEV Hit closest_hit_reference_cap(const SceneView &S, v3 o, v3 d, TraceCounters *cnt, const int cap) {
   Hit best;
   best.tri = -1;
@@ -365,11 +373,9 @@ RT_DEV Hit closest_hit_reference_cap(const SceneView &S, v3 o, v3 d, TraceCounte
     int t = (int)__ldg(n + 8);
     if (t != -1) {
       if (STATS) cnt->tri_tests++;
-      const float4 *p = S.tris + 3 * (size_t)t;
-      float4 t0 = __ldg(p), t1 = __ldg(p + 1), t2 = __ldg(p + 2);
+      const Tri tr = load_tri(S.tris, t);
       float k;
-      if (tri_hit(o, d, mk3(t0.x, t0.y, t0.z), mk3(t0.w, t1.x, t1.y), mk3(t1.z, t1.w, t2.x), &k) && k < best.k &&
-          k > 0.0001f) {
+      if (tri_hit(o, d, tr.A, tr.e1, tr.e2, &k) && k < best.k && k > 0.0001f) {
         best.k = k;
         best.tri = t;
       }
@@ -381,18 +387,17 @@ RT_DEV Hit closest_hit_reference_cap(const SceneView &S, v3 o, v3 d, TraceCounte
   return best;
 }
 
-template <bool SMEM, bool STATS>
+template <bool STATS>
 RT_DEV Hit closest_hit_reference(const SceneView &S, v3 o, v3 d, TraceCounters *cnt) {
-  return closest_hit_reference_cap<SMEM, STATS>(S, o, d, cnt, S.stack_cap);
+  return closest_hit_reference_cap<STATS>(S, o, d, cnt, S.stack_cap);
 }
 
 // The reference's walk with a stack that cannot drop: what the fast path computes, obtained the slow way.  Out of
 // line: reached only by rays with a zero / denormal / huge direction component and by the (very rare) rays whose
 // fast-path winner fails validate_hit.
-template <bool SMEM>
 __device__ __noinline__ Hit closest_hit_nodrop(const SceneView &S, v3 o, v3 d) {
   TraceCounters dummy;
-  return closest_hit_reference_cap<SMEM, false>(S, o, d, &dummy, kRefStack);
+  return closest_hit_reference_cap<false>(S, o, d, &dummy, kRefStack);
 }
 
 // ---- fast traversal ---------------------------------------------------------------------------------------------
@@ -434,10 +439,7 @@ RT_DEV float cull_limit(const SceneView &S, const Trav &T) { return __fmaf_rn(T.
 // Leaves whose box passes the conservative test are not tested on the spot (only a few lanes of a warp reach a
 // leaf in the same turn) but parked, at most kParkCap per lane (entry e of lane l at parks[e * stride]); the
 // warp tests parked triangles together.  Last in, first out; of a pair of leaves the farther is parked first.
-#ifndef B200RT_PARK_CAP
-#define B200RT_PARK_CAP 6
-#endif
-constexpr int kParkCap = B200RT_PARK_CAP;
+constexpr int kParkCap = 6;
 
 // starts a traversal of a ray for which ray_is_fast() holds
 template <bool SMEM, bool STATS>
@@ -516,7 +518,7 @@ RT_DEV void test_parked(const SceneView &S, Trav &T, uint32_t ref, v3 o, v3 d) {
 template <bool SMEM, bool STATS>
 RT_DEV Hit closest_hit_fast(const SceneView &S, v3 o, v3 d, LaneStack st, uint32_t *parks, int pstride,
                             TraceCounters *cnt) {
-  if (!ray_is_fast(S, o)) return closest_hit_nodrop<SMEM>(S, o, d);
+  if (!ray_is_fast(S, o)) return closest_hit_nodrop(S, o, d);
   Trav T;
   int pn = 0;
   trav_begin<SMEM, STATS>(S, T, o, d, pn, parks, cnt);
@@ -529,7 +531,7 @@ RT_DEV Hit closest_hit_fast(const SceneView &S, v3 o, v3 d, LaneStack st, uint32
       trav_step<SMEM, STATS>(S, T, pn, parks, pstride, st, cnt);
     }
   }
-  if (T.best.tri >= 0 && !validate_winner(S, o, d, T.best.tri, T.best_rank)) return closest_hit_nodrop<SMEM>(S, o, d);
+  if (T.best.tri >= 0 && !validate_winner(S, o, d, T.best.tri, T.best_rank)) return closest_hit_nodrop(S, o, d);
   return T.best;
 }
 
@@ -538,8 +540,8 @@ template <int TRAV, bool SMEM, bool STATS>
 RT_DEV Hit closest_hit(const SceneView &S, v3 o, v3 d, LaneStack st, uint32_t *parks, int pstride, TraceCounters *cnt,
                        unsigned int *mismatch) {
   if (TRAV == 0) return closest_hit_fast<SMEM, STATS>(S, o, d, st, parks, pstride, cnt);
-  if (TRAV == 1) return closest_hit_reference<SMEM, STATS>(S, o, d, cnt);
-  Hit a = closest_hit_reference<SMEM, STATS>(S, o, d, cnt);
+  if (TRAV == 1) return closest_hit_reference<STATS>(S, o, d, cnt);
+  Hit a = closest_hit_reference<STATS>(S, o, d, cnt);
   TraceCounters dummy;
   dummy.box_tests = 0; dummy.tri_tests = 0;
   Hit b = closest_hit_fast<SMEM, false>(S, o, d, st, parks, pstride, &dummy);
