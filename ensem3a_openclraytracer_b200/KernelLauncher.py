@@ -27,7 +27,12 @@ Differences a caller can observe (all documented in INTEGRATION.md):
   * `adaptive = dict(rel_error=..., min_spp=16, check_every=8, floor=0.05)` (the keys of Context.render_adaptive) lets
     each pixel stop sampling once its estimated error is below the tolerance, with the caller's spp as the maximum;
     `last_spp` then holds the (height, width) map of samples taken.  B200RT_ADAPTIVE=rel_error[,min_spp[,check_every]]
-    in the environment sets it for callers that never touch the attribute.  One GPU only.
+    in the environment sets it for callers that never touch the attribute.  One GPU only;
+  * `denoise = dict(passes=5, sigma_color=0.5, sigma_normal=0.2, sigma_position=0)` (the keywords of
+    Context.render_denoised; missing keys take DENOISE_DEFAULTS) runs the edge-avoiding à-trous filter of include/b200rt.h
+    over every frame, on one GPU or on `cuda_devices`.  B200RT_DENOISE=1 (the defaults) or
+    B200RT_DENOISE=passes[,sigma_color[,sigma_normal[,sigma_position]]] sets it for callers that never touch the
+    attribute.  It cannot be combined with `adaptive`.
 """
 import math
 import os
@@ -60,6 +65,31 @@ def adaptive_from_env(text):
     return ad
 
 
+def denoise_from_env(text):
+    """The `denoise` dict that B200RT_DENOISE=1 or =passes[,sigma_color[,sigma_normal[,sigma_position]]] stands for
+    ("1" is the defaults); ValueError if malformed."""
+    usage = (f"B200RT_DENOISE={text!r}: expected 1 (defaults) or passes[,sigma_color[,sigma_normal[,sigma_position]]], "
+             "e.g. 5,0.5,0.2 (sigma_position <= 0: automatic)")
+    parts = [p.strip() for p in str(text).split(",")]
+    if not 1 <= len(parts) <= 4 or "" in parts:
+        raise ValueError(usage)
+    try:
+        passes = int(parts[0])
+        sigmas = [float(p) for p in parts[1:]]
+    except ValueError:
+        raise ValueError(usage) from None
+    if not 1 <= passes <= 8:
+        raise ValueError(usage + " (passes must be 1..8)")
+    if not all(math.isfinite(x) for x in sigmas) or any(x <= 0 for x in sigmas[:2]):
+        raise ValueError(usage + " (sigma_color and sigma_normal must be finite and > 0, sigma_position finite)")
+    dn = dict(_capi.DENOISE_DEFAULTS)
+    if parts == ["1"]:   # the switch, not a one-pass filter
+        return dn
+    dn["passes"] = passes
+    dn.update(zip(("sigma_color", "sigma_normal", "sigma_position"), sigmas))
+    return dn
+
+
 class KernelLauncher(object):
 
     def __init__(self, context=None, platform=None, device=None, queue=None, cuda_device=0, cuda_devices=None):
@@ -86,6 +116,8 @@ class KernelLauncher(object):
         self.collect_stats = False
         # None: every pixel takes spp samples (the reference's image); a dict: adaptive sampling (module docstring)
         self.adaptive = adaptive_from_env(os.environ["B200RT_ADAPTIVE"]) if os.environ.get("B200RT_ADAPTIVE") else None
+        # None: the render as it comes; a dict: denoised (module docstring)
+        self.denoise = denoise_from_env(os.environ["B200RT_DENOISE"]) if os.environ.get("B200RT_DENOISE") else None
         self.last_spp = None
         self.last_stats = None
         self._warned_deep = False
@@ -93,6 +125,9 @@ class KernelLauncher(object):
     # reference KernelLauncher.py:33
     def launch_Raytracing(self, h_img_out, h_vertex_p, h_vertex_n, h_vertex_uv, h_face_data, h_material_data,
                           h_light_data, h_BVH, h_cam, h_envData, imgDim, spp, maxBounce, h_IBL):
+        if self.adaptive is not None and self.denoise is not None:
+            raise ValueError("adaptive sampling and denoising cannot be combined: set launcher.adaptive = None or "
+                             "launcher.denoise = None")
         if self.adaptive is not None and isinstance(self._ctx, _capi.MultiContext):
             raise ValueError("adaptive sampling renders on one GPU: its stopping rule needs each pixel's samples in one "
                              f"sequence, which a split over cuda_devices={self._ctx.devices} would cut apart; set "
@@ -135,6 +170,10 @@ class KernelLauncher(object):
         if self.adaptive is not None:
             img, self.last_spp, _ = self._ctx.render_adaptive(cam[:10], h_envData, width, height, int(spp), int(maxBounce),
                                                               opts=opts, **self.adaptive)
+            out[:] = img.reshape(-1)
+        elif self.denoise is not None:
+            img = self._ctx.render_denoised(cam[:10], h_envData, width, height, int(spp), int(maxBounce), opts=opts,
+                                            **self.denoise)
             out[:] = img.reshape(-1)
         else:
             self._ctx.render(cam[:10], h_envData, width, height, int(spp), int(maxBounce), out=out, opts=opts)

@@ -51,17 +51,32 @@ class Adaptive(ctypes.Structure):
                 ("floor", ctypes.c_float)]
 
 
+class Denoise(ctypes.Structure):
+    """b200rt_denoise_params: the edge-avoiding à-trous filter's parameters (include/b200rt.h)."""
+    _fields_ = [("passes", ctypes.c_int32), ("sigma_color", ctypes.c_float), ("sigma_normal", ctypes.c_float),
+                ("sigma_position", ctypes.c_float)]
+
+
+# B200RT_DENOISE_* of include/b200rt.h; sigma_position 0 = automatic (1 % of the scene's BVH root-box diagonal)
+DENOISE_DEFAULTS = dict(passes=5, sigma_color=0.5, sigma_normal=0.2, sigma_position=0.0)
+
+
+def _denoise_params(passes=DENOISE_DEFAULTS["passes"], sigma_color=DENOISE_DEFAULTS["sigma_color"],
+                    sigma_normal=DENOISE_DEFAULTS["sigma_normal"], sigma_position=DENOISE_DEFAULTS["sigma_position"]):
+    return Denoise(int(passes), float(sigma_color), float(sigma_normal), float(sigma_position))
+
+
 # every symbol include/b200rt.h declares (tests/test_abi.py checks the header against this list)
 SYMBOLS = [
     "b200rt_default_opts", "b200rt_create", "b200rt_destroy", "b200rt_last_error", "b200rt_set_scene",
-    "b200rt_set_materials", "b200rt_set_ibl", "b200rt_render", "b200rt_render_adaptive", "b200rt_render_rgb8", "b200rt_render_device", "b200rt_finalize_device",
+    "b200rt_set_materials", "b200rt_set_ibl", "b200rt_render", "b200rt_render_adaptive", "b200rt_gbuffer", "b200rt_denoise", "b200rt_render_denoised", "b200rt_render_rgb8", "b200rt_render_device", "b200rt_finalize_device",
     "b200rt_reduce_finalize_device", "b200rt_sync", "b200rt_set_stream", "b200rt_invalidate", "b200rt_primary_hits", "b200rt_trace_rays",
     "b200rt_img_processing", "b200rt_get_stats", "b200rt_math_probe", "b200rt_philox_probe", "b200rt_alloc",
     "b200rt_free", "b200rt_ipc_export",
     "b200rt_ipc_open", "b200rt_ipc_close", "b200rt_build_bvh", "b200rt_repack_probe", "b200rt_version", "b200rt_device_count",
     "b200rt_multi_create", "b200rt_multi_destroy", "b200rt_multi_last_error", "b200rt_multi_device_count",
     "b200rt_multi_context", "b200rt_multi_set_scene", "b200rt_multi_set_ibl", "b200rt_multi_invalidate",
-    "b200rt_multi_render", "b200rt_multi_get_stats",
+    "b200rt_multi_render", "b200rt_multi_render_denoised", "b200rt_multi_get_stats",
 ]
 
 _lib = None
@@ -97,6 +112,11 @@ def load_library():
     lib.b200rt_render.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), vp]
     lib.b200rt_render_adaptive.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), ctypes.POINTER(Adaptive),
                                            vp, vp, vp]
+    lib.b200rt_gbuffer.argtypes = [vp, vp, i32, i32, ctypes.POINTER(Opts), vp, vp, vp, vp]
+    lib.b200rt_denoise.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, ctypes.POINTER(Denoise), vp]
+    lib.b200rt_render_denoised.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), ctypes.POINTER(Denoise),
+                                           vp, vp]
+    lib.b200rt_multi_render_denoised.argtypes = lib.b200rt_render_denoised.argtypes
     lib.b200rt_render_device.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), vp]
     lib.b200rt_render_rgb8.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), vp]
     lib.b200rt_finalize_device.argtypes = [vp, vp, vp, i64, i32]
@@ -269,6 +289,22 @@ class _Handle:
                    _ptr(out))
         return out
 
+    def render_denoised(self, cam, env, width, height, spp, max_bounce, opts=None, return_noisy=False, **denoise):
+        """A render followed by the edge-avoiding à-trous filter of include/b200rt.h on the device (b200rt_render_denoised,
+        or b200rt_multi_render_denoised).  denoise: passes, sigma_color, sigma_normal, sigma_position (0 = automatic),
+        defaults DENOISE_DEFAULTS.  Returns the (H, W, 3) float32 image, and the undenoised one with return_noisy."""
+        cam_, env_ = _f32(cam), _f32(env)
+        if cam_.size != 10 or env_.size != 5:
+            raise B200RTError("cam must hold 10 floats and envData 5 (main.py:59-61,72-73)")
+        h, w = int(height), int(width)
+        img = np.zeros((h, w, 3), dtype=np.float32)
+        noisy = np.zeros((h, w, 3), dtype=np.float32) if return_noisy else None
+        dn = _denoise_params(**denoise)
+        o = opts if opts is not None else make_opts()
+        self._call("render_denoised", _ptr(cam_), _ptr(env_), w, h, int(spp), int(max_bounce), ctypes.byref(o),
+                   ctypes.byref(dn), _ptr(img), _ptr(noisy))
+        return (img, noisy) if return_noisy else img
+
     def stats(self):
         s = Stats()
         self._call("get_stats", ctypes.byref(s))
@@ -321,6 +357,33 @@ class Context(_Handle):
                                                      ctypes.byref(o), ctypes.byref(ad), _ptr(img), _ptr(spp_map),
                                                      _ptr(err_map)), "b200rt_render_adaptive")
         return img, spp_map, err_map
+
+    def gbuffer(self, cam, width, height, opts=None):
+        """The denoiser's G-buffer of the frame's primary hits (b200rt_gbuffer): a dict of albedo / normal / position
+        (H, W, 3) float32 and kind (H, W) int32 (-1 miss, 0 emitter, 1 surface)."""
+        cam_ = _f32(cam)
+        h, w = int(height), int(width)
+        gb = {k: np.zeros((h, w, 3), np.float32) for k in ("albedo", "normal", "position")}
+        gb["kind"] = np.zeros((h, w), np.int32)
+        o = opts if opts is not None else make_opts()
+        self._check(self._lib.b200rt_gbuffer(self._h, _ptr(cam_), w, h, ctypes.byref(o), _ptr(gb["albedo"]),
+                                             _ptr(gb["normal"]), _ptr(gb["position"]), _ptr(gb["kind"])), "b200rt_gbuffer")
+        return gb
+
+    def denoise(self, img, gb, **denoise):
+        """The filter on its own (b200rt_denoise) over an (H, W, 3) image and a G-buffer as gbuffer() returns it;
+        denoise as for render_denoised.  Returns a new (H, W, 3) float32 image."""
+        kind = np.ascontiguousarray(gb["kind"], np.int32)
+        h, w = kind.shape
+        n = h * w * 3
+        arrs = [_f32(a) for a in (img, gb["albedo"], gb["normal"], gb["position"])]
+        if any(a.size != n for a in arrs):
+            raise B200RTError(f"image and G-buffer must hold {n} floats each for a {w}x{h} kind map")
+        out = np.zeros((h, w, 3), np.float32)
+        dn = _denoise_params(**denoise)
+        self._check(self._lib.b200rt_denoise(self._h, *[_ptr(a) for a in arrs], _ptr(kind), w, h, ctypes.byref(dn),
+                                             _ptr(out)), "b200rt_denoise")
+        return out
 
     def render_rgb8(self, cam, env, width, height, spp, max_bounce, opts=None):
         """(height, width, 3) uint8 image, quantised on the device like FileManager.saveImg does on the host."""

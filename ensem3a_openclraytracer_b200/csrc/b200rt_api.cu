@@ -15,7 +15,7 @@
 #include <vector>
 
 #include "../../include/b200rt.h"
-#include "rt_kernels.cuh"
+#include "rt_denoise.cuh"
 #include "scene_repack.h"
 
 using namespace b200rt;
@@ -75,6 +75,7 @@ struct b200rt_ctx {
   DevBuf d_pA, d_pB, d_pC, d_pHit, d_list0, d_list1, d_cnt;  // wavefront path state (rt_kernels.cuh)
   DevBuf d_slots, d_part_count;                               // order-preserving list compaction
   DevBuf d_welford, d_ad_spp, d_ad_err;                       // adaptive sampling (AdaptArgs)
+  DevBuf d_dn_tri, d_dn_k, d_gb[3], d_dn_col[2];              // denoising: primary hits, G-buffer (GBufferView), colour
   unsigned int *h_live = nullptr;   // adaptive sampling: pinned, the path-list length after each of the two batches in flight
   cudaEvent_t ev_batch[2] = {nullptr, nullptr};
   DeviceCounters *d_counters = nullptr;
@@ -862,7 +863,8 @@ void b200rt_destroy(b200rt_ctx *c) {
     if (b.p && !b.borrowed) cudaFree(b.p);
   DevBuf *bufs[] = {&c->d_prim_dirk, &c->d_prim_tri, &c->d_out, &c->d_misc, &c->d_tmp_a, &c->d_tmp_b, &c->d_pA, &c->d_pB,
                     &c->d_pC, &c->d_pHit, &c->d_list0, &c->d_list1, &c->d_cnt, &c->d_slots, &c->d_part_count, &c->d_pS,
-                    &c->d_pL, &c->d_pR, &c->d_welford, &c->d_ad_spp, &c->d_ad_err};
+                    &c->d_pL, &c->d_pR, &c->d_welford, &c->d_ad_spp, &c->d_ad_err, &c->d_dn_tri, &c->d_dn_k,
+                    &c->d_gb[0], &c->d_gb[1], &c->d_gb[2], &c->d_dn_col[0], &c->d_dn_col[1]};
   for (DevBuf *b : bufs)
     if (b->p) cudaFree(b->p);
   if (c->h_live) cudaFreeHost(c->h_live);
@@ -1015,6 +1017,115 @@ int render_to_host(b200rt_ctx *c, const float *cam, const float *env, int width,
   return read_counters(c);
 }
 
+// ---- denoising (rt_denoise.cuh) --------------------------------------------------------------------------------------
+// Validates the filter's parameters and resolves sigma_position to the scale s_x = sigma_position^2 (b200rt.h).
+int check_denoise(b200rt_ctx *c, const b200rt_denoise_params *dn, float *s_x) {
+  if (!dn) return fail(c, B200RT_ERR_INVALID, "denoise parameters are NULL");
+  if (dn->passes < 1 || dn->passes > kDnMaxPasses)
+    return fail(c, B200RT_ERR_INVALID, "denoise passes %d outside [1, %d]", dn->passes, kDnMaxPasses);
+  if (!std::isfinite(dn->sigma_color) || !(dn->sigma_color > 0.0f))
+    return fail(c, B200RT_ERR_INVALID, "denoise sigma_color %g must be finite and > 0", (double)dn->sigma_color);
+  if (!std::isfinite(dn->sigma_normal) || !(dn->sigma_normal > 0.0f))
+    return fail(c, B200RT_ERR_INVALID, "denoise sigma_normal %g must be finite and > 0", (double)dn->sigma_normal);
+  if (!std::isfinite(dn->sigma_position))
+    return fail(c, B200RT_ERR_INVALID, "denoise sigma_position %g must be finite (<= 0: automatic)", (double)dn->sigma_position);
+  float sp = dn->sigma_position;
+  if (!(sp > 0.0f)) {
+    if (!c->have_scene) return fail(c, B200RT_ERR_NO_SCENE, "an automatic sigma_position needs a scene: call b200rt_set_scene first");
+    const float *b = c->scene.root_box;
+    const float dx = b[3] - b[0], dy = b[4] - b[1], dz = b[5] - b[2];
+    sp = 0.01f * std::sqrt((dx * dx + dy * dy) + dz * dz);
+    if (!(sp > 0.0f) || !std::isfinite(sp))
+      return fail(c, B200RT_ERR_INVALID, "automatic sigma_position is %g (degenerate BVH root box): give one", (double)sp);
+  }
+  *s_x = sp * sp;
+  return 0;
+}
+
+// the filter needs the whole finalised frame
+int check_denoise_frame(b200rt_ctx *c, const b200rt_opts &o, int spp) {
+  if (o.output != B200RT_OUT_FINAL) return fail(c, B200RT_ERR_INVALID, "denoising needs B200RT_OUT_FINAL");
+  if (o.sample_end > 0 && (o.sample_begin != 0 || o.sample_end != spp))
+    return fail(c, B200RT_ERR_INVALID, "denoising needs the whole sample range [0, spp)");
+  if (o.pixel_end > 0) return fail(c, B200RT_ERR_INVALID, "denoising needs the whole frame: no pixel range");
+  if (o.tile_row_mod > 1) return fail(c, B200RT_ERR_INVALID, "denoising needs the whole frame: no tile rows");
+  return 0;
+}
+
+int ensure_denoise_bufs(b200rt_ctx *c, size_t npix) {
+  for (DevBuf &b : c->d_gb)
+    if (ensure(c, b, npix * sizeof(float4))) return B200RT_ERR_CUDA;
+  for (DevBuf &b : c->d_dn_col)
+    if (ensure(c, b, npix * sizeof(float4))) return B200RT_ERR_CUDA;
+  return 0;
+}
+
+GBufferView gbuffer_view(b200rt_ctx *c) {
+  return GBufferView{static_cast<float4 *>(c->d_gb[0].p), static_cast<float4 *>(c->d_gb[1].p), static_cast<float4 *>(c->d_gb[2].p)};
+}
+
+// k_primary (PARITY: the hit the render's k_primary finds, same traversal and stack cap) + k_gbuffer over the whole frame,
+// on c's stream.  d_rgb (may be NULL): the frame's image on the device, packed into d_dn_col[0] for the passes.
+int launch_gbuffer(b200rt_ctx *c, const float *cam, int width, int height, const b200rt_opts &o, const float *d_rgb) {
+  const size_t npix = (size_t)width * height;
+  if (ensure(c, c->d_dn_tri, npix * sizeof(int))) return B200RT_ERR_CUDA;
+  if (ensure(c, c->d_dn_k, npix * sizeof(float))) return B200RT_ERR_CUDA;
+  if (ensure_denoise_bufs(c, npix)) return B200RT_ERR_CUDA;
+  b200rt_opts og = o;
+  og.sample_begin = og.sample_end = 0;
+  og.pixel_begin = og.pixel_end = 0;
+  og.tile_row_mod = og.tile_row_rem = 0;
+  FrameParams F;
+  frame_setup(c, cam, nullptr, width, height, 1, 0, og, &F);
+  KernelArgs A;
+  fill_args(c, F, og, nullptr, &A);
+  int *tri = static_cast<int *>(c->d_dn_tri.p);
+  float *k = static_cast<float *>(c->d_dn_k.p);
+  int rc = launch_primary(c, A, effective_traversal(c, og), use_smem_scene(c), true, og.collect_stats != 0, tri, k);
+  if (rc) return rc;
+  k_gbuffer<<<(unsigned)((npix + kBlock - 1) / kBlock), kBlock, 0, c->stream>>>(A, tri, k, gbuffer_view(c), d_rgb,
+                                                                                 static_cast<float4 *>(c->d_dn_col[0].p));
+  CU(cudaGetLastError());
+  c->stats.kernel_launches++;
+  return 0;
+}
+
+// The passes over the G-buffer and input colour (d_dn_col[0]) already on the device; the image goes to d_out.
+int launch_atrous(b200rt_ctx *c, int width, int height, const b200rt_denoise_params &dn, float s_x, float *d_out) {
+  const dim3 block(kDnBlockX, kDnBlockY);
+  const dim3 grid((unsigned)((width + kDnBlockX - 1) / kDnBlockX), (unsigned)((height + kDnBlockY - 1) / kDnBlockY));
+  if (grid.y > 65535u) return fail(c, B200RT_ERR_UNSUPPORTED, "denoising a frame of %d rows: at most %d", height, 65535 * kDnBlockY);
+  const GBufferView G = gbuffer_view(c);
+  float4 *col[2] = {static_cast<float4 *>(c->d_dn_col[0].p), static_cast<float4 *>(c->d_dn_col[1].p)};
+  AtrousArgs P;
+  P.gn = G.gn; P.gx = G.gx; P.ga = G.ga;
+  P.out = d_out;
+  P.width = width;
+  P.height = height;
+  P.s_n = dn.sigma_normal * dn.sigma_normal;
+  P.s_x = s_x;
+  for (int l = 0; l < dn.passes; ++l) {
+    P.cin = col[l & 1];
+    P.cout = col[(l + 1) & 1];
+    P.step = 1 << l;
+    P.s_c = (dn.sigma_color * dn.sigma_color) * std::ldexp(1.0f, -2 * l);   // sigma_color halves every pass
+    const bool first = l == 0, last = l == dn.passes - 1;
+    auto k = first ? (last ? k_atrous<true, true> : k_atrous<true, false>) : (last ? k_atrous<false, true> : k_atrous<false, false>);
+    k<<<grid, block, 0, c->stream>>>(P);
+    CU(cudaGetLastError());
+    c->stats.kernel_launches++;
+  }
+  return 0;
+}
+
+// G-buffer + passes over the image d_img (3 floats per pixel, on c's GPU), in place, on c's stream
+int denoise_frame(b200rt_ctx *c, const float *cam, int width, int height, const b200rt_opts &o, const b200rt_denoise_params &dn,
+                  float s_x, float *d_img) {
+  int rc = launch_gbuffer(c, cam, width, height, o, d_img);
+  if (rc) return rc;
+  return launch_atrous(c, width, height, dn, s_x, d_img);
+}
+
 }  // namespace
 
 extern "C" {
@@ -1142,6 +1253,97 @@ int b200rt_render_adaptive(b200rt_ctx *c, const float *cam, const float *env, in
     if (out_stderr) CU(cudaMemcpyAsync(out_stderr, c->d_ad_err.p, npix * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     return 0;
   });
+}
+
+int b200rt_render_denoised(b200rt_ctx *c, const float *cam, const float *env, int width, int height, int spp,
+                           int max_bounce, const b200rt_opts *opts, const b200rt_denoise_params *dn, float *out,
+                           float *out_noisy) {
+  if (!c) return B200RT_ERR_INVALID;
+  if (!out) return fail(c, B200RT_ERR_INVALID, "out_rgb is NULL");
+  b200rt_opts o;
+  if (opts) o = *opts; else b200rt_default_opts(&o);
+  int rc = check_frame_args(c, cam, width, height, spp, max_bounce, o, true, env);
+  if (!rc) rc = check_denoise_frame(c, o, spp);
+  float s_x = 0.0f;
+  if (!rc) rc = check_denoise(c, dn, &s_x);
+  if (rc) return rc;
+  const size_t bytes = (size_t)width * height * 3 * sizeof(float);
+  return render_to_host(c, cam, env, width, height, spp, max_bounce, &o, nullptr, [&] {
+    float *img = static_cast<float *>(c->d_out.p);
+    if (out_noisy) CU(cudaMemcpyAsync(out_noisy, img, bytes, cudaMemcpyDeviceToHost, c->stream));
+    const int r = denoise_frame(c, cam, width, height, o, *dn, s_x, img);
+    if (r) return r;
+    CU(cudaMemcpyAsync(out, img, bytes, cudaMemcpyDeviceToHost, c->stream));
+    return 0;
+  });
+}
+
+int b200rt_gbuffer(b200rt_ctx *c, const float *cam, int width, int height, const b200rt_opts *opts, float *albedo,
+                   float *normal, float *position, int32_t *kind) {
+  if (!c) return B200RT_ERR_INVALID;
+  b200rt_opts o;
+  if (opts) o = *opts; else b200rt_default_opts(&o);
+  int rc = check_frame_args(c, cam, width, height, 1, 0, o, false, nullptr);
+  if (!rc && (o.pixel_end > 0 || o.tile_row_mod > 1))
+    rc = fail(c, B200RT_ERR_INVALID, "the G-buffer covers the whole frame: no pixel range or tile rows");
+  if (rc) return rc;
+  CU(cudaSetDevice(c->device));
+  const size_t npix = (size_t)width * height;
+  c->stats.kernel_launches = 0;
+  c->streams_used = 1;
+  CU(cudaMemsetAsync(c->d_counters, 0, sizeof(DeviceCounters), c->stream));
+  CU(cudaEventRecord(c->ev[0], c->stream));
+  rc = launch_gbuffer(c, cam, width, height, o, nullptr);
+  if (rc) return rc;
+  CU(cudaEventRecord(c->ev[1], c->stream));
+  CU(cudaEventRecord(c->ev[2], c->stream));
+  // float4 records -> 3 floats per pixel (a strided copy); kind travels as the float .w of the normal record
+  float *dst[3] = {normal, position, albedo};
+  for (int r = 0; r < 3; ++r)
+    if (dst[r]) CU(cudaMemcpy2DAsync(dst[r], 3 * sizeof(float), c->d_gb[r].p, sizeof(float4), 3 * sizeof(float), npix,
+                                     cudaMemcpyDeviceToHost, c->stream));
+  std::vector<float> kind_f(kind ? npix : 0);
+  if (kind) CU(cudaMemcpy2DAsync(kind_f.data(), sizeof(float), static_cast<const float *>(c->d_gb[0].p) + 3, sizeof(float4),
+                                 sizeof(float), npix, cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  for (size_t i = 0; i < kind_f.size(); ++i) kind[i] = (int32_t)kind_f[i];
+  return read_counters(c);
+}
+
+int b200rt_denoise(b200rt_ctx *c, const float *rgb, const float *albedo, const float *normal, const float *position,
+                   const int32_t *kind, int width, int height, const b200rt_denoise_params *dn, float *out) {
+  if (!c) return B200RT_ERR_INVALID;
+  if (!rgb || !albedo || !normal || !position || !kind || !out) return fail(c, B200RT_ERR_INVALID, "NULL denoise buffer");
+  if (width <= 0 || height <= 0 || (long long)width * height > 0x7fffffffLL / 4)
+    return fail(c, B200RT_ERR_INVALID, "bad frame size %d x %d", width, height);
+  float s_x = 0.0f;
+  int rc = check_denoise(c, dn, &s_x);
+  if (rc) return rc;
+  const size_t npix = (size_t)width * height;
+  for (size_t i = 0; i < npix; ++i)
+    if (kind[i] < -1 || kind[i] > 1) return fail(c, B200RT_ERR_INVALID, "kind[%zu] = %d is not -1, 0 or 1", i, (int)kind[i]);
+  // host records in the layout of GBufferView and the passes' colour buffer
+  std::vector<float4> rec[4];
+  for (auto &r : rec) r.resize(npix);
+  for (size_t i = 0; i < npix; ++i) {
+    const size_t e = 3 * i;
+    rec[0][i] = make_float4(normal[e], normal[e + 1], normal[e + 2], (float)kind[i]);
+    rec[1][i] = make_float4(position[e], position[e + 1], position[e + 2], 0.0f);
+    rec[2][i] = make_float4(albedo[e], albedo[e + 1], albedo[e + 2], 0.0f);
+    rec[3][i] = make_float4(rgb[e], rgb[e + 1], rgb[e + 2], 0.0f);
+  }
+  CU(cudaSetDevice(c->device));
+  if (ensure_denoise_bufs(c, npix)) return B200RT_ERR_CUDA;
+  if (ensure(c, c->d_misc, npix * 3 * sizeof(float))) return B200RT_ERR_CUDA;
+  for (int r = 0; r < 3; ++r)
+    CU(cudaMemcpyAsync(c->d_gb[r].p, rec[r].data(), npix * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(c->d_dn_col[0].p, rec[3].data(), npix * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+  c->stats.kernel_launches = 0;
+  rc = launch_atrous(c, width, height, *dn, s_x, static_cast<float *>(c->d_misc.p));
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(out, c->d_misc.p, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return 0;
 }
 
 int b200rt_render_rgb8(b200rt_ctx *c, const float *cam, const float *env, int width, int height, int spp, int max_bounce,
@@ -1573,8 +1775,13 @@ int b200rt_multi_invalidate(b200rt_multi *m) {
   return 0;
 }
 
-int b200rt_multi_render(b200rt_multi *m, const float *cam, const float *env, int width, int height, int spp, int max_bounce,
-                        const b200rt_opts *opts, float *out) {
+}  // extern "C"
+
+namespace {
+
+// b200rt_multi_render; dn != NULL: then b200rt_render_denoised's G-buffer and passes on GPU 0 after the reduce
+int multi_render(b200rt_multi *m, const float *cam, const float *env, int width, int height, int spp, int max_bounce,
+                 const b200rt_opts *opts, const b200rt_denoise_params *dn, float *out, float *out_noisy) {
   if (!m) return B200RT_ERR_INVALID;
   if (!out) return mfail(m, B200RT_ERR_INVALID, "out_rgb is NULL");
   if (width <= 0 || height <= 0) return mfail(m, B200RT_ERR_INVALID, "bad frame size %d x %d", width, height);
@@ -1585,6 +1792,12 @@ int b200rt_multi_render(b200rt_multi *m, const float *cam, const float *env, int
   const int n = (int)m->ctx.size();
   const size_t npix = (size_t)width * height, bytes = npix * 3 * sizeof(float);
   b200rt_ctx *c0 = m->ctx[0];
+  float s_x = 0.0f;
+  if (dn) {
+    int rc = check_denoise_frame(c0, o, spp);
+    if (!rc) rc = check_denoise(c0, dn, &s_x);
+    if (rc) return mfail(m, rc, "%s", c0->err.c_str());
+  }
   MCU(cudaSetDevice(c0->device));
   if (m->d_final.cap < bytes) {
     if (m->d_final.p) cudaFree(m->d_final.p);
@@ -1635,6 +1848,12 @@ int b200rt_multi_render(b200rt_multi *m, const float *cam, const float *env, int
   rc = launch_reduce(c0, pl, static_cast<float *>(m->d_final.p), (long long)npix * 3, (float)spp);
   if (rc) return mfail(m, rc, "%s", c0->err.c_str());
   MCU(cudaEventRecord(m->ev_end, c0->stream));
+  if (dn) {
+    float *img = static_cast<float *>(m->d_final.p);
+    if (out_noisy) MCU(cudaMemcpyAsync(out_noisy, img, bytes, cudaMemcpyDeviceToHost, c0->stream));
+    rc = denoise_frame(c0, cam, width, height, o, *dn, s_x, img);   // its launches and rays count in GPU 0's stats
+    if (rc) return mfail(m, rc, "GPU %d: %s", c0->device, c0->err.c_str());
+  }
   MCU(cudaMemcpyAsync(out, m->d_final.p, bytes, cudaMemcpyDeviceToHost, c0->stream));
   MCU(cudaStreamSynchronize(c0->stream));
   // ---- statistics: work summed over the GPUs, device time = the slowest GPU + the reduce ---------------------------
@@ -1668,6 +1887,22 @@ int b200rt_multi_render(b200rt_multi *m, const float *cam, const float *env, int
   agg.ref_stack_need = c0->stats.ref_stack_need;
   m->stats = agg;
   return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int b200rt_multi_render(b200rt_multi *m, const float *cam, const float *env, int width, int height, int spp, int max_bounce,
+                        const b200rt_opts *opts, float *out) {
+  return multi_render(m, cam, env, width, height, spp, max_bounce, opts, nullptr, out, nullptr);
+}
+
+int b200rt_multi_render_denoised(b200rt_multi *m, const float *cam, const float *env, int width, int height, int spp,
+                                 int max_bounce, const b200rt_opts *opts, const b200rt_denoise_params *dn, float *out,
+                                 float *out_noisy) {
+  if (m && !dn) return mfail(m, B200RT_ERR_INVALID, "denoise parameters are NULL");
+  return multi_render(m, cam, env, width, height, spp, max_bounce, opts, dn, out, out_noisy);
 }
 
 int b200rt_multi_get_stats(const b200rt_multi *m, b200rt_stats *s) {

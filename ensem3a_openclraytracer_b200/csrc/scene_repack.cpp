@@ -389,6 +389,7 @@ int repack_scene(const float *vp, int64_t n_vp, const float *vn, int64_t n_vn, c
     }
     const float dx = bvh[5] - bvh[2], dy = bvh[6] - bvh[3], dz = bvh[7] - bvh[4];
     R.cull_abs = 1e-3f * std::sqrt(dx * dx + dy * dy + dz * dz);
+    for (int k = 0; k < 6; ++k) R.root_box[k] = bvh[2 + k];
   }
   R.cmax = cmax;
   // range the conservative slab test's error margin is proven for (rt_trace.cuh); outside it every ray takes

@@ -35,6 +35,7 @@ struct SceneDesc {
   uint32_t root_w[3] = {0x7fff0000u, 0x7fff0000u, 0x7fff0000u};  // the root box as node-record words (max plane << 16 | min plane)
   float cull_abs = 0.0f, cmax = 0.0f;
   int fast_ok = 0;
+  float root_box[6] = {0, 0, 0, 0, 0, 0};  // the caller's root box, bvh[2..7] (min.xyz, max.xyz): the denoiser's scale
 };
 
 struct Repacked : SceneDesc {

@@ -173,6 +173,63 @@ int b200rt_render_adaptive(b200rt_ctx *ctx, const float *cam, const float *env, 
                            int max_bounce, const b200rt_opts *opts, const b200rt_adaptive *ad,
                            float *out_rgb, int32_t *out_spp, float *out_stderr);
 
+/* ---- opt-in denoising: an edge-avoiding à-trous filter guided by a G-buffer of the primary hits --------------------
+ * The G-buffer, per pixel i, from the primary hit of the render's own traversal mode and stack cap (so that `kind`
+ * marks exactly the pixels whose samples need no ray, which the render finishes without tracing):
+ *   - kind = -1 for a primary miss, 0 for an emissive material (type 0), 1 otherwise;
+ *   - albedo = the material colour (material_data[6m + 1 .. 3]) for kind 1, (1, 1, 1) otherwise;
+ *   - normal = normalize(first-vertex normal of the hit triangle) = n / sqrtf((n.x*n.x + n.y*n.y) + n.z*n.z): the
+ *     reference's flat, unflipped normal; (0, 0, 0) if a component of it is not finite, and for a miss;
+ *   - position = cam_pos + d * k per component (no FMA), d the camera direction of pixel i, k the hit distance;
+ *     (0, 0, 0) for a miss.
+ * The filter, in binary32 with every operation rounded separately (no contraction), true division, and no
+ * transcendental function (so that a restatement can reproduce every bit of the ~10^9 weights of a 1080p frame):
+ *   - a pixel with kind != 1 is output unchanged, bit for bit, and is never a tap of another pixel;
+ *   - demodulate: c = I / fmaxf(a, 0.01f) per channel (I the input colour, a the albedo);
+ *   - for pass l = 0 .. passes-1 with step h = 2^l:  c'_p = (sum_q w_pq * c_q) / (sum_q w_pq) per channel, over the
+ *     taps q = p + h*(i, j) with j = -2..2 (rows, outer loop) and i = -2..2 (inner); every sum starts at 0.0f and adds
+ *     in that order; a tap outside the frame or with kind_q != 1 is skipped;
+ *   - weights, with k1 = {1/16, 1/4, 3/8, 1/4, 1/16} and f(d2, s) = 1.0f / (1.0f + d2 / s):
+ *       the centre tap weighs exactly k1[2] * k1[2] (so the denominator is never 0);
+ *       any other tap weighs w = (((k1[j+2] * k1[i+2]) * f(dc2, s_c)) * f(dn2, s_n)) * f(dx2, s_x), where
+ *       d2 of a vector difference D = q - p is (D.x*D.x + D.y*D.y) + D.z*D.z, dc2 uses the current pass's c,
+ *       s_c = (sigma_color * sigma_color) * 2^(-2l) (sigma_color halves every pass), s_n = sigma_normal * sigma_normal and
+ *       s_x = sigma_position * sigma_position; a tap whose w is not > 0 (NaN, or 0 through underflow or an infinite
+ *       distance) is skipped, so a NaN or infinite colour never reaches another pixel through a zero weight;
+ *   - remodulate: out = clamp01(c' * fmaxf(a, 0.01f)), clamp01 being the reference's fmax(fmin(x, 1), 0) with NaN -> 1.
+ * Known limits: a primary hit on pass-through glass describes the glass, not what is seen through it; reflections on
+ * smooth glossy surfaces are blurred like texture.  The filter keeps the expectation of flat regions but not of
+ * every pixel: it trades noise for a little blur. */
+#define B200RT_DENOISE_PASSES 5
+#define B200RT_DENOISE_SIGMA_COLOR 0.5f
+#define B200RT_DENOISE_SIGMA_NORMAL 0.2f
+typedef struct {
+  int32_t passes;        /* 1..8; default B200RT_DENOISE_PASSES */
+  float sigma_color;     /* finite, > 0: colour-distance scale of the first pass (demodulated units) */
+  float sigma_normal;    /* finite, > 0: normal-distance scale */
+  float sigma_position;  /* finite: > 0 world-distance scale; <= 0 automatic = 0.01f * the binary32 diagonal
+                            sqrtf((dx*dx + dy*dy) + dz*dz) of the context's BVH root box (bvh[2..4] min, bvh[5..7] max) */
+} b200rt_denoise_params;
+
+/* The G-buffer of a frame: host outputs, 3 floats per pixel for albedo / normal / position and one int32 for kind; each
+ * may be NULL.  opts: traversal and stack cap as for b200rt_render; pixel ranges and tile rows are refused. */
+int b200rt_gbuffer(b200rt_ctx *ctx, const float *cam, int width, int height, const b200rt_opts *opts, float *albedo,
+                   float *normal, float *position, int32_t *kind);
+
+/* The filter on its own: host inputs (rgb / albedo / normal / position 3 floats per pixel, kind one int32 in {-1, 0, 1}),
+ * host output, synchronous; out may be rgb.  An automatic sigma_position needs the context's scene. */
+int b200rt_denoise(b200rt_ctx *ctx, const float *rgb, const float *albedo, const float *normal, const float *position,
+                   const int32_t *kind, int width, int height, const b200rt_denoise_params *dn, float *out);
+
+/* b200rt_render, then the G-buffer and the filter's passes on the device, then one read-back.  out_noisy (may be NULL)
+ * receives the image b200rt_render makes.  opts: both generators, every traversal, every sampling bit and any
+ * sample_streams; the filter needs the whole finalised frame, so B200RT_OUT_SUMS, a partial sample range, pixel ranges
+ * and tile rows are refused.  stats: as b200rt_render, plus 2 + passes kernel launches and width*height camera rays in
+ * rays and primary_rays (the G-buffer's); total_ms covers the render only. */
+int b200rt_render_denoised(b200rt_ctx *ctx, const float *cam, const float *env, int width, int height, int spp,
+                           int max_bounce, const b200rt_opts *opts, const b200rt_denoise_params *dn, float *out_rgb,
+                           float *out_noisy);
+
 /* Render + the 8-bit conversion of FileManager.saveImg (FileManager.py:334-338: `(data*255).astype('uint8')`, float32
  * product truncated toward zero) on the device, so that only width*height*3 BYTES cross to the host.  out_rgb8:
  * width*height*3 bytes on the HOST, row-major RGB — what PIL's Image.fromarray(..., 'RGB') takes. */
@@ -269,6 +326,11 @@ int b200rt_multi_set_ibl(b200rt_multi *m, const uint8_t *rgba, int width, int he
 int b200rt_multi_invalidate(b200rt_multi *m);
 int b200rt_multi_render(b200rt_multi *m, const float *cam, const float *env, int width, int height, int spp,
                         int max_bounce, const b200rt_opts *opts, float *out_rgb);
+/* b200rt_multi_render, then b200rt_render_denoised's G-buffer (whole frame) and passes on the first GPU after the
+ * reduce; same arguments and refusals as b200rt_multi_render, dn and out_noisy as b200rt_render_denoised. */
+int b200rt_multi_render_denoised(b200rt_multi *m, const float *cam, const float *env, int width, int height, int spp,
+                                 int max_bounce, const b200rt_opts *opts, const b200rt_denoise_params *dn, float *out_rgb,
+                                 float *out_noisy);
 /* rays / samples / launches summed over the GPUs (every GPU traces the frame's primary rays once); total_ms = the
  * slowest GPU, reduce included */
 int b200rt_multi_get_stats(const b200rt_multi *m, b200rt_stats *stats);

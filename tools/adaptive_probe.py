@@ -46,6 +46,15 @@ def timed(fn, repeat):
     return best
 
 
+def truth_image(ctx, cam, env, truth_spp, renders=4):
+    """(H, W, 3) float64: the mean of `renders` long Philox renders (OUT_SUMS / spp), clamped to [0, 1]"""
+    acc = np.zeros(W * H * 3)
+    for seed in range(renders):
+        o = rt.make_opts(rng_mode=rt.RNG_PHILOX, seed=1000 + seed, output=rt.OUT_SUMS, sample_streams=-1)
+        acc += ctx.render(cam, env, W, H, truth_spp, BOUNCE, opts=o).astype(np.float64) / truth_spp
+    return np.clip(acc / renders, 0.0, 1.0).reshape(H, W, 3)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r03_adaptive.jsonl"))
@@ -64,11 +73,7 @@ def main():
             fixtures.upload(ctx, sc, fixtures.load_ibl(ibl_name))
             cam, env = fixtures.cam_env(sc["params"], W, H)
             t0 = time.perf_counter()
-            acc = np.zeros(W * H * 3)
-            for seed in range(4):
-                o = rt.make_opts(rng_mode=rt.RNG_PHILOX, seed=1000 + seed, output=rt.OUT_SUMS, sample_streams=-1)
-                acc += ctx.render(cam, env, W, H, a.truth_spp, BOUNCE, opts=o).astype(np.float64) / a.truth_spp
-            truth = np.clip(acc / 4, 0.0, 1.0).reshape(H, W, 3)
+            truth = truth_image(ctx, cam, env, a.truth_spp)
             truth_s = time.perf_counter() - t0
             for n in (int(x) for x in a.n.split(",")):
                 o = rt.make_opts(rng_mode=rt.RNG_PHILOX, seed=1, sample_streams=-1)
