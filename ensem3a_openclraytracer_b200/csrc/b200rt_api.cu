@@ -38,16 +38,20 @@ enum SceneBuf { kNodes, kTris, kCtris, kNormals, kTboxes, kFrames, kMats, kBvh9,
 // another's tracing are resident side by side (bench scene -4 %, Cornell 1080p -12 %, measured with 3 streams).
 constexpr int kStreamTraceCtas = 4;
 
+// what both handle types (b200rt_ctx, b200rt_multi) keep for b200rt_last_error / b200rt_multi_last_error
+struct Handle {
+  std::string err;
+};
+
 }  // namespace
 
-struct b200rt_ctx {
+struct b200rt_ctx : Handle {
   int device = 0;
   cudaStream_t stream = nullptr;      // stream in use
   cudaStream_t own_stream = nullptr;  // created by b200rt_create
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
   std::vector<cudaEvent_t> kev;  // per-launch events of the last time_kernels render
   int kev_used = 0;
-  std::string err;
   int sm_count = 0;
   size_t smem_optin = 0;
 
@@ -101,13 +105,14 @@ bool own_cull_tree() {
   return !(q && q[0] == '0');
 }
 
-int fail(b200rt_ctx *c, int code, const char *fmt, ...) {
+// the message goes to the handle, or to the create-error slot while there is none
+int fail(Handle *h, int code, const char *fmt, ...) {
   char buf[512];
   va_list ap;
   va_start(ap, fmt);
   vsnprintf(buf, sizeof buf, fmt, ap);
   va_end(ap);
-  if (c) c->err = buf; else g_create_error = buf;
+  if (h) h->err = buf; else g_create_error = buf;
   return code;
 }
 
@@ -441,6 +446,15 @@ void add_work(b200rt_stats &dst, const b200rt_stats &src) {
   dst.kernel_launches += src.kernel_launches;
 }
 
+// the statistics that describe the uploaded scene rather than a render
+void copy_scene_facts(b200rt_stats &dst, const b200rt_stats &src) {
+  dst.nodes = src.nodes;
+  dst.triangles = src.triangles;
+  dst.bvh_depth = src.bvh_depth;
+  dst.repack_ms = src.repack_ms;
+  dst.ref_stack_need = src.ref_stack_need;
+}
+
 // Counters and timings of the last render.  A frame cut into sample streams sums the work of its helper contexts
 // (the primary rays, which every stream traces for itself, count once) and is timed from the fork to the reduce.
 int read_counters(b200rt_ctx *c) {
@@ -506,16 +520,12 @@ int check_frame_args(b200rt_ctx *c, const float *cam, int width, int height, int
 
 constexpr int kAdaptBatch = 32;  // adaptive renders: wavefront iterations enqueued between two looks at the list length
 
-// ad != NULL: adaptive sampling (b200rt_render_adaptive has validated ad and opts; the frame covers [0, spp) on one
-// stream).  The launch loop then runs in batches and stops once the path list is empty; it is synchronous.
+// One render on c's stream; render_frame has checked the frame.  ad != NULL: adaptive sampling (b200rt_render_adaptive
+// has validated ad and opts; the frame covers [0, spp) on one stream).  The launch loop then runs in batches and stops
+// once the path list is empty; it is synchronous.
 int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, int height, int spp, int max_bounce,
-                const b200rt_opts *opts, float *d_out, const b200rt_adaptive *ad) {
-  b200rt_opts o;
-  if (opts) o = *opts; else b200rt_default_opts(&o);
+                const b200rt_opts &o, float *d_out, const b200rt_adaptive *ad) {
   c->streams_used = 1;
-  int rc = check_frame_args(c, cam, width, height, spp, max_bounce, o, true, env);
-  if (rc) return rc;
-  if (!c->have_ibl) return fail(c, B200RT_ERR_NO_SCENE, "no environment map: call b200rt_set_ibl first");
   CU(cudaSetDevice(c->device));
   const size_t npix = (size_t)width * height;
   FrameParams F;
@@ -553,7 +563,7 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   A.validate = (trav == B200RT_TRAVERSAL_FAST) ? 1 : 0;
   const bool smem = use_smem_scene(c);
   WaveLaunch wl;
-  rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, &wl);
+  int rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, &wl);
   if (rc) return rc;
   if (ensure(c, c->d_part_count, (size_t)wl.shade_grid * sizeof(unsigned int))) return B200RT_ERR_CUDA;
   A.part_count = static_cast<unsigned int *>(c->d_part_count.p);
@@ -644,24 +654,10 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   return 0;
 }
 
-// ---- sample streams ------------------------------------------------------------------------------------------------
-// One path per pixel is in flight inside a render (a pixel's samples run in order).  With the counter-based
-// generator a frame's sample range can be cut into N contiguous parts that do not depend on each other; each part is
-// an ordinary render into its own partial-sum buffer, issued on its own CUDA stream by a helper context that borrows
-// this context's scene, and one k_reduce_finalize on this context's stream adds the parts in order.  The GPU then
-// holds N samples of a pixel at once: small frames fill it, and on large frames one part's shading overlaps another
-// part's tracing (the two kernels are bound by different units).
-void borrow_scene(b200rt_ctx *p, b200rt_ctx *h) {
-  for (int i = 0; i < kSceneBufs; ++i) {
-    h->d_scene[i] = p->d_scene[i];
-    h->d_scene[i].borrowed = true;
-  }
-  h->scene = p->scene;
-  h->n_light = p->n_light;
-  h->have_scene = p->have_scene;
-  h->ibl_tex = p->ibl_tex; h->ibl_w = p->ibl_w; h->ibl_h = p->ibl_h; h->have_ibl = p->have_ibl;
-  h->shared_epoch = p->scene_epoch;
-}
+// ---- partitioned frames --------------------------------------------------------------------------------------------
+// Sample streams (render_frame) and the multi-GPU handle (multi_render) cut a frame into parts the same way: every
+// part is an OUT_SUMS render into a buffer of its own, and one k_reduce_finalize on the home context's stream adds
+// the parts in part order (render_parts).
 
 // Runs fn(k) for every part k in [0, n) on a host thread of its own: a frame is thousands of small launches, and one
 // thread feeding several streams or GPUs would be the bottleneck.  Returns 0, or the code of the first part that
@@ -690,6 +686,97 @@ int launch_reduce(b200rt_ctx *c, const PartList &parts, float *out, long long n,
   return 0;
 }
 
+// Part k of n of the sample range [s0, s1): contiguous, sizes differing by at most one, the longer parts first
+// (multigpu.py::split_range is the same rule).
+void sample_share(int k, int n, int s0, int s1, b200rt_opts *o) {
+  const int base = (s1 - s0) / n, extra = (s1 - s0) % n;
+  o->sample_begin = s0 + k * base + std::min(k, extra);
+  o->sample_end = o->sample_begin + base + (k < extra ? 1 : 0);
+}
+
+// The statistics of a context that renders nothing in this frame: no work and no time; the scene facts stay.
+void clear_frame_stats(b200rt_ctx *c) {
+  const b200rt_stats s = c->stats;
+  memset(&c->stats, 0, sizeof c->stats);
+  copy_scene_facts(c->stats, s);
+  c->stats_pending = false;
+}
+
+struct Part {
+  b200rt_ctx *c;       // renders the part on its stream
+  b200rt_opts o;       // OUT_SUMS, with the part's sample range or tile rows
+  DevBuf *sums;        // on c's GPU, never the buffer the reduce writes
+  cudaEvent_t join;    // recorded on c's stream once the sums are complete (parts k > 0)
+  DevBuf *staging;     // on the home GPU when it cannot read `sums` directly, else NULL
+};
+
+// Renders one frame as parts, parts[0].c being the home context, and adds them up into out (on the home GPU), divided
+// by spp or left as sums when spp is 0.  `fork` and `done` bracket the frame on home's stream.  Each part zeroes its
+// sums and calls render(c, opts, sums) on a host thread of its own; a part whose share is empty renders nothing and
+// reports no work and no time.  On failure the message is in the context of part *failed, or in home's (-1).
+template <class Render>
+int render_parts(const std::vector<Part> &parts, int width, int height, float spp, cudaEvent_t fork, cudaEvent_t done,
+                 float *out, int *failed, Render &&render) {
+  b200rt_ctx *c = parts[0].c;
+  const int n = (int)parts.size(), tile_rows = (height + 3) / 4;
+  const size_t bytes = (size_t)width * height * 3 * sizeof(float);
+  *failed = -1;
+  CU(cudaSetDevice(c->device));
+  CU(cudaEventRecord(fork, c->stream));   // the parts start after whatever the caller enqueued before this frame
+  // from this thread, before the parts run: a part that cuts its share into streams re-records its own fork event
+  for (int k = 1; k < n; ++k) CU(cudaStreamWaitEvent(parts[(size_t)k].c->stream, fork, 0));
+  int rc = run_parts(n, failed, [&](int k) {
+    const Part &p = parts[(size_t)k];
+    b200rt_ctx *h = p.c;
+    const bool idle = p.o.sample_begin == p.o.sample_end || (p.o.tile_row_mod > 1 && p.o.tile_row_rem >= tile_rows);
+    int r = cudaSetDevice(h->device) == cudaSuccess ? ensure(h, *p.sums, bytes) : B200RT_ERR_CUDA;
+    if (!r && cudaMemsetAsync(p.sums->p, 0, bytes, h->stream) != cudaSuccess) r = B200RT_ERR_CUDA;
+    if (!r && idle) clear_frame_stats(h);
+    else if (!r) r = render(h, p.o, static_cast<float *>(p.sums->p));
+    if (!r && k > 0 && cudaEventRecord(p.join, h->stream) != cudaSuccess) r = B200RT_ERR_CUDA;
+    if (r == B200RT_ERR_CUDA && h->err.empty()) h->err = "CUDA call failed while enqueueing a part of the frame";
+    return r;
+  });
+  if (rc) return rc;
+  // join on home's stream and add the parts in part order
+  CU(cudaSetDevice(c->device));
+  PartList pl;
+  pl.n = n;
+  for (int k = 0; k < n; ++k) {
+    const Part &p = parts[(size_t)k];
+    if (k > 0) CU(cudaStreamWaitEvent(c->stream, p.join, 0));
+    pl.p[k] = static_cast<const float *>(p.sums->p);
+    if (p.staging) {
+      if (ensure(c, *p.staging, bytes)) return B200RT_ERR_CUDA;
+      CU(cudaMemcpyPeerAsync(p.staging->p, c->device, pl.p[k], p.c->device, bytes, c->stream));
+      pl.p[k] = static_cast<const float *>(p.staging->p);
+    }
+  }
+  rc = launch_reduce(c, pl, out, (long long)width * height * 3, spp);
+  if (rc) return rc;
+  CU(cudaEventRecord(done, c->stream));
+  return 0;
+}
+
+// ---- sample streams ------------------------------------------------------------------------------------------------
+// One path per pixel is in flight inside a render (a pixel's samples run in order).  With the counter-based
+// generator a frame's sample range can be cut into N contiguous parts that do not depend on each other; each part is
+// an ordinary render into its own partial-sum buffer, issued on its own CUDA stream by a helper context that borrows
+// this context's scene, and render_parts adds them on this context's stream.  The GPU then holds N samples of a pixel
+// at once: small frames fill it, and on large frames one part's shading overlaps another part's tracing (the two
+// kernels are bound by different units).
+void borrow_scene(b200rt_ctx *p, b200rt_ctx *h) {
+  for (int i = 0; i < kSceneBufs; ++i) {
+    h->d_scene[i] = p->d_scene[i];
+    h->d_scene[i].borrowed = true;
+  }
+  h->scene = p->scene;
+  h->n_light = p->n_light;
+  h->have_scene = p->have_scene;
+  h->ibl_tex = p->ibl_tex; h->ibl_w = p->ibl_w; h->ibl_h = p->ibl_h; h->have_ibl = p->have_ibl;
+  h->shared_epoch = p->scene_epoch;
+}
+
 int resolve_streams(const b200rt_opts &o, int width, int height, int s0, int s1) {
   if (o.rng_mode != B200RT_RNG_PHILOX) return 1;   // the reference generator is one serial stream per pixel
   int n = o.sample_streams;
@@ -709,14 +796,14 @@ int render_frame(b200rt_ctx *c, const float *cam, const float *env, int width, i
   if (opts) o = *opts; else b200rt_default_opts(&o);
   if (o.sample_streams < -1 || o.sample_streams > 16)
     return fail(c, B200RT_ERR_INVALID, "bad sample_streams %d (-1 automatic, 0 / 1 off, up to 16)", o.sample_streams);
-  int s0 = o.sample_begin, s1 = o.sample_end;
-  if (s1 <= 0) { s0 = 0; s1 = spp; }
-  const int n = (!ad && width > 0 && height > 0 && spp > 0) ? resolve_streams(o, width, height, s0, s1) : 1;
-  if (!c->is_helper) c->frame_trace_cap = 0;
-  if (n <= 1 || c->is_helper) return render_impl(c, cam, env, width, height, spp, max_bounce, &o, d_out, ad);
   int rc = check_frame_args(c, cam, width, height, spp, max_bounce, o, true, env);
   if (rc) return rc;
   if (!c->have_ibl) return fail(c, B200RT_ERR_NO_SCENE, "no environment map: call b200rt_set_ibl first");
+  int s0 = o.sample_begin, s1 = o.sample_end;
+  if (s1 <= 0) { s0 = 0; s1 = spp; }
+  const int n = ad ? 1 : resolve_streams(o, width, height, s0, s1);
+  c->frame_trace_cap = 0;
+  if (n <= 1) return render_impl(c, cam, env, width, height, spp, max_bounce, o, d_out, ad);
   CU(cudaSetDevice(c->device));
   while ((int)c->helpers.size() < n - 1) {
     b200rt_ctx *h = nullptr;
@@ -729,52 +816,29 @@ int render_frame(b200rt_ctx *c, const float *cam, const float *env, int width, i
     CU(cudaEventCreate(&c->ev_fork));
     CU(cudaEventCreate(&c->ev_done));
   }
-  const size_t bytes = (size_t)width * height * 3 * sizeof(float);
-  if (ensure(c, c->d_part, bytes)) return B200RT_ERR_CUDA;
-  CU(cudaEventRecord(c->ev_fork, c->stream));   // the parts start after whatever the caller enqueued before this frame
-  const int total = s1 - s0, base = total / n, extra = total % n;
-  int bad = 0;
-  rc = run_parts(n, &bad, [&](int k) {
+  std::vector<Part> parts((size_t)n);
+  for (int k = 0; k < n; ++k) {
     b200rt_ctx *h = k == 0 ? c : c->helpers[(size_t)k - 1];
-    b200rt_opts ok = o;
+    if (k > 0) {
+      if (h->shared_epoch != c->scene_epoch) borrow_scene(c, h);
+      if (!h->ev_join) CU(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
+    }
+    parts[(size_t)k] = Part{h, o, &h->d_part, h->ev_join, nullptr};
+    b200rt_opts &ok = parts[(size_t)k].o;
     ok.sample_streams = 1;
     ok.output = B200RT_OUT_SUMS;
-    ok.sample_begin = s0 + k * base + (k < extra ? k : extra);
-    ok.sample_end = ok.sample_begin + base + (k < extra ? 1 : 0);
-    int r = 0;
-    if (cudaSetDevice(c->device) != cudaSuccess) r = B200RT_ERR_CUDA;
-    float *part = nullptr;
-    if (!r && k > 0) {
-      if (h->shared_epoch != c->scene_epoch) borrow_scene(c, h);
-      if (!h->ev_join && cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming) != cudaSuccess) r = B200RT_ERR_CUDA;
-      if (!r && cudaStreamWaitEvent(h->stream, c->ev_fork, 0) != cudaSuccess) r = B200RT_ERR_CUDA;
-      if (!r) r = ensure(h, h->d_part, bytes);
-      part = static_cast<float *>(h->d_part.p);
-    } else if (!r) {
-      part = static_cast<float *>(c->d_part.p);
-    }
-    if (!r && cudaMemsetAsync(part, 0, bytes, h->stream) != cudaSuccess) r = B200RT_ERR_CUDA;
-    h->frame_trace_cap = n >= 3 ? kStreamTraceCtas : 0;
-    if (!r) r = render_impl(h, cam, env, width, height, spp, max_bounce, &ok, part, nullptr);
-    if (!r && k > 0 && cudaEventRecord(h->ev_join, h->stream) != cudaSuccess) r = B200RT_ERR_CUDA;
-    if (r == B200RT_ERR_CUDA && h->err.empty()) h->err = "CUDA call failed while enqueueing a sample stream";
-    return r;
-  });
-  if (rc) {
-    const std::string msg = (bad == 0 ? c : c->helpers[(size_t)bad - 1])->err;
-    return fail(c, rc, "sample stream %d: %s", bad, msg.c_str());
+    sample_share(k, n, s0, s1, &ok);
   }
-  // join on this context's stream, add the parts in order; a whole frame is finalised, a partial range stays sums
-  PartList pl;
-  pl.n = n;
-  pl.p[0] = static_cast<const float *>(c->d_part.p);
-  for (int k = 1; k < n; ++k) {
-    CU(cudaStreamWaitEvent(c->stream, c->helpers[(size_t)k - 1]->ev_join, 0));
-    pl.p[k] = static_cast<const float *>(c->helpers[(size_t)k - 1]->d_part.p);
-  }
-  rc = launch_reduce(c, pl, d_out, (long long)width * height * 3, o.output == B200RT_OUT_FINAL ? (float)spp : 0.0f);
+  // a whole frame is finalised, a partial range stays sums
+  const float div = o.output == B200RT_OUT_FINAL ? (float)spp : 0.0f;
+  int bad = -1;
+  rc = render_parts(parts, width, height, div, c->ev_fork, c->ev_done, d_out, &bad,
+                    [&](b200rt_ctx *h, const b200rt_opts &ok, float *sums) {
+                      h->frame_trace_cap = n >= 3 ? kStreamTraceCtas : 0;
+                      return render_impl(h, cam, env, width, height, spp, max_bounce, ok, sums, nullptr);
+                    });
+  if (rc && bad >= 0) return fail(c, rc, "sample stream %d: %s", bad, parts[(size_t)bad].c->err.c_str());
   if (rc) return rc;
-  CU(cudaEventRecord(c->ev_done, c->stream));
   c->streams_used = n;
   c->stats.sample_streams = n;
   c->stats_pending = true;
@@ -1602,54 +1666,15 @@ int b200rt_ipc_close(b200rt_ctx *c, void *d_ptr) {
 // peer mappings (NVLink loads), sums in GPU order, divides by spp and clamps (k_reduce_finalize).  Kernel launches
 // are issued by one host thread per GPU: a frame is thousands of small launches, and a single thread feeding eight
 // GPUs would be the bottleneck.
-struct b200rt_multi {
+struct b200rt_multi : Handle {
   std::vector<b200rt_ctx *> ctx;
   std::vector<cudaEvent_t> done;   // per GPU: its partial sums are complete
   std::vector<int> peer_ok;        // GPU 0 can read GPU i's memory directly
   std::vector<DevBuf> staging;     // on GPU 0, for GPUs it cannot read directly
   DevBuf d_final;                  // on GPU 0
-  cudaEvent_t ev_begin = nullptr, ev_end = nullptr;  // on GPU 0's stream, around wait + reduce
-  std::string err;
+  cudaEvent_t ev_fork = nullptr, ev_done = nullptr;  // on GPU 0's stream: the frame's start and the end of its reduce
   b200rt_stats stats;
 };
-
-namespace {
-
-int mfail(b200rt_multi *m, int code, const char *fmt, ...) {
-  char buf[512];
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(buf, sizeof buf, fmt, ap);
-  va_end(ap);
-  if (m) m->err = buf; else g_create_error = buf;
-  return code;
-}
-
-#define MCU(call)                                                                                    \
-  do {                                                                                               \
-    cudaError_t e_ = (call);                                                                         \
-    if (e_ != cudaSuccess) return mfail(m, B200RT_ERR_CUDA, "%s: %s", #call, cudaGetErrorString(e_)); \
-  } while (0)
-
-// what GPU `r` of `n` renders (ensem3a_openclraytracer_b200/multigpu.py::rank_work is the same rule)
-void multi_share(int r, int n, int spp, int rng_mode, b200rt_opts *o) {
-  o->output = B200RT_OUT_SUMS;
-  if (rng_mode == B200RT_RNG_PHILOX) {
-    const int base = spp / n, extra = spp % n;
-    const int s0 = r * base + (r < extra ? r : extra);
-    o->sample_begin = s0;
-    o->sample_end = s0 + base + (r < extra ? 1 : 0);
-    o->tile_row_mod = 0;
-    o->tile_row_rem = 0;
-  } else {
-    o->sample_begin = 0;
-    o->sample_end = spp;
-    o->tile_row_mod = n > 1 ? n : 0;
-    o->tile_row_rem = n > 1 ? r : 0;
-  }
-}
-
-}  // namespace
 
 extern "C" {
 
@@ -1663,8 +1688,8 @@ void b200rt_multi_destroy(b200rt_multi *m) {
     for (DevBuf &b : m->staging)
       if (b.p) cudaFree(b.p);
     if (m->d_final.p) cudaFree(m->d_final.p);
-    if (m->ev_begin) cudaEventDestroy(m->ev_begin);
-    if (m->ev_end) cudaEventDestroy(m->ev_end);
+    if (m->ev_fork) cudaEventDestroy(m->ev_fork);
+    if (m->ev_done) cudaEventDestroy(m->ev_done);
   }
   for (size_t i = 0; i < m->ctx.size(); ++i) {
     if (!m->ctx[i]) continue;
@@ -1679,9 +1704,9 @@ void b200rt_multi_destroy(b200rt_multi *m) {
 
 int b200rt_multi_create(const int *devices, int n_devices, b200rt_multi **out) {
   b200rt_multi *m = nullptr;
-  if (!out) return mfail(nullptr, B200RT_ERR_INVALID, "out is NULL");
+  if (!out) return fail(nullptr, B200RT_ERR_INVALID, "out is NULL");
   *out = nullptr;
-  if (!devices || n_devices < 1 || n_devices > 16) return mfail(nullptr, B200RT_ERR_INVALID, "1..16 devices expected (got %d)", n_devices);
+  if (!devices || n_devices < 1 || n_devices > 16) return fail(nullptr, B200RT_ERR_INVALID, "1..16 devices expected (got %d)", n_devices);
   // A device may be listed several times: every entry gets its own context, buffers and stream, so a frame too small
   // to fill one GPU (one path per pixel in flight) runs as several concurrent sample-range renders on it.
   m = new b200rt_multi();
@@ -1694,7 +1719,7 @@ int b200rt_multi_create(const int *devices, int n_devices, b200rt_multi **out) {
     int rc = b200rt_create(devices[i], &m->ctx[i]);   // leaves its message in the create-error slot
     if (rc) { b200rt_multi_destroy(m); return rc; }
     cudaError_t e = cudaEventCreateWithFlags(&m->done[i], cudaEventDisableTiming);
-    if (e != cudaSuccess) { mfail(nullptr, B200RT_ERR_CUDA, "cudaEventCreate: %s", cudaGetErrorString(e)); b200rt_multi_destroy(m); return B200RT_ERR_CUDA; }
+    if (e != cudaSuccess) { fail(nullptr, B200RT_ERR_CUDA, "cudaEventCreate: %s", cudaGetErrorString(e)); b200rt_multi_destroy(m); return B200RT_ERR_CUDA; }
   }
   cudaSetDevice(devices[0]);
   for (int i = 1; i < n_devices; ++i) {
@@ -1709,8 +1734,8 @@ int b200rt_multi_create(const int *devices, int n_devices, b200rt_multi **out) {
     }
     m->peer_ok[i] = can;
   }
-  if (cudaEventCreate(&m->ev_begin) != cudaSuccess || cudaEventCreate(&m->ev_end) != cudaSuccess) {
-    mfail(nullptr, B200RT_ERR_CUDA, "cudaEventCreate failed");
+  if (cudaEventCreate(&m->ev_fork) != cudaSuccess || cudaEventCreate(&m->ev_done) != cudaSuccess) {
+    fail(nullptr, B200RT_ERR_CUDA, "cudaEventCreate failed");
     b200rt_multi_destroy(m);
     return B200RT_ERR_CUDA;
   }
@@ -1743,7 +1768,7 @@ int b200rt_multi_set_scene(b200rt_multi *m, const float *vp, int64_t n_vp, const
     rc = repack_scene(vp, n_vp, vn, n_vn, face, n_face, n_mat / 6, bvh, n_bvh, &R, &msg, own_cull_tree());
     if (rc) {
       for (b200rt_ctx *c : m->ctx) { c->have_scene = false; c->have_scene_cached = false; c->scene_hash = 0; }
-      return mfail(m, rc, "%s", msg.c_str());
+      return fail(m, rc, "%s", msg.c_str());
     }
   }
   int bad = 0;
@@ -1751,13 +1776,9 @@ int b200rt_multi_set_scene(b200rt_multi *m, const float *vp, int64_t n_vp, const
     b200rt_ctx *c = m->ctx[i];
     return scene_is_cached(c, h) ? b200rt_set_materials(c, mat, n_mat) : upload_scene(c, R, a, h);
   });
-  if (rc) return mfail(m, rc, "GPU %d: %s", m->ctx[bad]->device, m->ctx[bad]->err.c_str());
+  if (rc) return fail(m, rc, "GPU %d: %s", m->ctx[bad]->device, m->ctx[bad]->err.c_str());
   m->stats.upload_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
-  m->stats.nodes = m->ctx[0]->stats.nodes;
-  m->stats.triangles = m->ctx[0]->stats.triangles;
-  m->stats.bvh_depth = m->ctx[0]->stats.bvh_depth;
-  m->stats.repack_ms = m->ctx[0]->stats.repack_ms;
-  m->stats.ref_stack_need = m->ctx[0]->stats.ref_stack_need;
+  copy_scene_facts(m->stats, m->ctx[0]->stats);
   return 0;
 }
 
@@ -1765,7 +1786,7 @@ int b200rt_multi_set_ibl(b200rt_multi *m, const uint8_t *rgba, int width, int he
   if (!m) return B200RT_ERR_INVALID;
   int bad = 0;
   const int rc = run_parts((int)m->ctx.size(), &bad, [&](int i) { return b200rt_set_ibl(m->ctx[i], rgba, width, height); });
-  if (rc) return mfail(m, rc, "GPU %d: %s", m->ctx[bad]->device, m->ctx[bad]->err.c_str());
+  if (rc) return fail(m, rc, "GPU %d: %s", m->ctx[bad]->device, m->ctx[bad]->err.c_str());
   return 0;
 }
 
@@ -1783,108 +1804,73 @@ namespace {
 int multi_render(b200rt_multi *m, const float *cam, const float *env, int width, int height, int spp, int max_bounce,
                  const b200rt_opts *opts, const b200rt_denoise_params *dn, float *out, float *out_noisy) {
   if (!m) return B200RT_ERR_INVALID;
-  if (!out) return mfail(m, B200RT_ERR_INVALID, "out_rgb is NULL");
-  if (width <= 0 || height <= 0) return mfail(m, B200RT_ERR_INVALID, "bad frame size %d x %d", width, height);
+  if (!out) return fail(m, B200RT_ERR_INVALID, "out_rgb is NULL");
+  if (width <= 0 || height <= 0) return fail(m, B200RT_ERR_INVALID, "bad frame size %d x %d", width, height);
   b200rt_opts o;
   if (opts) o = *opts; else b200rt_default_opts(&o);
   if (o.output != B200RT_OUT_FINAL || o.sample_end > 0 || o.tile_row_mod > 1)
-    return mfail(m, B200RT_ERR_INVALID, "the multi-GPU handle divides the frame itself: leave output / sample range / tile rows at their defaults");
+    return fail(m, B200RT_ERR_INVALID, "the multi-GPU handle divides the frame itself: leave output / sample range / tile rows at their defaults");
   const int n = (int)m->ctx.size();
-  const size_t npix = (size_t)width * height, bytes = npix * 3 * sizeof(float);
-  b200rt_ctx *c0 = m->ctx[0];
+  const size_t bytes = (size_t)width * height * 3 * sizeof(float);
+  b200rt_ctx *c = m->ctx[0];   // GPU 0: the reduce, the denoiser and the read-back
   float s_x = 0.0f;
   if (dn) {
-    int rc = check_denoise_frame(c0, o, spp);
-    if (!rc) rc = check_denoise(c0, dn, &s_x);
-    if (rc) return mfail(m, rc, "%s", c0->err.c_str());
+    int rc = check_denoise_frame(c, o, spp);
+    if (!rc) rc = check_denoise(c, dn, &s_x);
+    if (rc) return fail(m, rc, "%s", c->err.c_str());
   }
-  MCU(cudaSetDevice(c0->device));
-  if (m->d_final.cap < bytes) {
-    if (m->d_final.p) cudaFree(m->d_final.p);
-    m->d_final.p = nullptr; m->d_final.cap = 0;
-    MCU(cudaMalloc(&m->d_final.p, bytes));
-    m->d_final.cap = bytes;
-  }
-  // ---- every GPU renders its share into its own buffer; one host thread per GPU issues the launches ------------
-  const int tile_rows = (height + 3) / 4;
-  int bad = 0;
-  int rc = run_parts(n, &bad, [&](int i) {
-    b200rt_ctx *c = m->ctx[i];
-    b200rt_opts oi = o;
-    multi_share(i, n, spp, o.rng_mode, &oi);
-    int r = 0;
-    if (cudaSetDevice(c->device) != cudaSuccess) r = B200RT_ERR_CUDA;
-    if (!r) r = ensure(c, c->d_out, bytes);
-    if (!r && cudaMemsetAsync(c->d_out.p, 0, bytes, c->stream) != cudaSuccess) r = B200RT_ERR_CUDA;
-    const bool empty = (oi.sample_begin == oi.sample_end) || (oi.tile_row_mod > 1 && oi.tile_row_rem >= tile_rows);
-    c->stats.rays = 0; c->stats.samples = 0; c->stats.total_ms = 0; c->stats.kernel_launches = 0;
-    if (!r && !empty) r = render_frame(c, cam, env, width, height, spp, max_bounce, &oi, static_cast<float *>(c->d_out.p));
-    if (!r && cudaEventRecord(m->done[i], c->stream) != cudaSuccess) r = B200RT_ERR_CUDA;
-    if (r == B200RT_ERR_CUDA && c->err.empty()) c->err = "CUDA call failed while enqueueing the frame";
-    return r;
-  });
-  if (rc) return mfail(m, rc, "GPU %d: %s", m->ctx[bad]->device, m->ctx[bad]->err.c_str());
-  // ---- GPU 0: wait for the peers (device-side), then one kernel reads every partial buffer and finalises ----------
-  MCU(cudaSetDevice(c0->device));
-  MCU(cudaEventRecord(m->ev_begin, c0->stream));
-  PartList pl;
-  pl.n = n;
+  // every GPU renders its share into its own d_out: a contiguous sample range with the counter-based generator, the
+  // tile rows r mod n with the reference's serial per-pixel generator
+  const bool philox = o.rng_mode == B200RT_RNG_PHILOX;
+  std::vector<Part> parts((size_t)n);
   for (int i = 0; i < n; ++i) {
-    if (i > 0) MCU(cudaStreamWaitEvent(c0->stream, m->done[i], 0));
-    const float *src = static_cast<const float *>(m->ctx[i]->d_out.p);
-    if (i > 0 && !m->peer_ok[i]) {  // no direct mapping: stage the partial sums on GPU 0
-      DevBuf &sb = m->staging[i];
-      if (sb.cap < bytes) {
-        if (sb.p) cudaFree(sb.p);
-        sb.p = nullptr; sb.cap = 0;
-        MCU(cudaMalloc(&sb.p, bytes));
-        sb.cap = bytes;
-      }
-      MCU(cudaMemcpyPeerAsync(sb.p, c0->device, src, m->ctx[i]->device, bytes, c0->stream));
-      src = static_cast<const float *>(sb.p);
-    }
-    pl.p[i] = src;
+    b200rt_ctx *ci = m->ctx[(size_t)i];
+    parts[(size_t)i] = Part{ci, o, &ci->d_out, m->done[(size_t)i], m->peer_ok[(size_t)i] ? nullptr : &m->staging[(size_t)i]};
+    b200rt_opts &oi = parts[(size_t)i].o;
+    oi.output = B200RT_OUT_SUMS;
+    sample_share(philox ? i : 0, philox ? n : 1, 0, spp, &oi);
+    if (!philox && n > 1) { oi.tile_row_mod = n; oi.tile_row_rem = i; }
   }
-  rc = launch_reduce(c0, pl, static_cast<float *>(m->d_final.p), (long long)npix * 3, (float)spp);
-  if (rc) return mfail(m, rc, "%s", c0->err.c_str());
-  MCU(cudaEventRecord(m->ev_end, c0->stream));
-  if (dn) {
+  int bad = -1;
+  int rc = [&]() -> int {   // GPU 0's work; a failure leaves its message in GPU 0's context or in part bad's
+    CU(cudaSetDevice(c->device));
+    if (ensure(c, m->d_final, bytes)) return B200RT_ERR_CUDA;
     float *img = static_cast<float *>(m->d_final.p);
-    if (out_noisy) MCU(cudaMemcpyAsync(out_noisy, img, bytes, cudaMemcpyDeviceToHost, c0->stream));
-    rc = denoise_frame(c0, cam, width, height, o, *dn, s_x, img);   // its launches and rays count in GPU 0's stats
-    if (rc) return mfail(m, rc, "GPU %d: %s", c0->device, c0->err.c_str());
-  }
-  MCU(cudaMemcpyAsync(out, m->d_final.p, bytes, cudaMemcpyDeviceToHost, c0->stream));
-  MCU(cudaStreamSynchronize(c0->stream));
-  // ---- statistics: work summed over the GPUs, device time = the slowest GPU + the reduce ---------------------------
-  b200rt_stats agg = m->stats;
-  const float upload_ms = agg.upload_ms;
-  memset(&agg, 0, sizeof agg);
-  agg.upload_ms = upload_ms;
-  float slowest = 0.0f;
-  for (int i = 0; i < n; ++i) {
-    b200rt_ctx *c = m->ctx[i];
-    if (c->stats_pending) {
-      MCU(cudaSetDevice(c->device));
-      rc = read_counters(c);
-      if (rc) return mfail(m, rc, "GPU %d: %s", c->device, c->err.c_str());
+    int r = render_parts(parts, width, height, (float)spp, m->ev_fork, m->ev_done, img, &bad,
+                         [&](b200rt_ctx *ci, const b200rt_opts &oi, float *sums) {
+                           return render_frame(ci, cam, env, width, height, spp, max_bounce, &oi, sums);
+                         });
+    if (r) return r;
+    if (dn) {
+      if (out_noisy) CU(cudaMemcpyAsync(out_noisy, img, bytes, cudaMemcpyDeviceToHost, c->stream));
+      r = denoise_frame(c, cam, width, height, o, *dn, s_x, img);   // its launches and rays count in GPU 0's stats
+      if (r) return r;
     }
-    add_work(agg, c->stats);
-    slowest = std::max(slowest, c->stats.total_ms);
-    agg.primary_ms = std::max(agg.primary_ms, c->stats.primary_ms);
-    agg.trace_ms = std::max(agg.trace_ms, c->stats.trace_ms);
+    CU(cudaMemcpyAsync(out, img, bytes, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
+  }();
+  if (rc) {
+    const b200rt_ctx *e = bad >= 0 ? parts[(size_t)bad].c : c;
+    return fail(m, rc, "GPU %d: %s", e->device, e->err.c_str());
   }
-  float red = 0.0f;
-  MCU(cudaSetDevice(c0->device));
-  cudaEventElapsedTime(&red, m->ev_begin, m->ev_end);  // includes waiting for the slowest peer after GPU 0 finished
-  agg.total_ms = std::max(slowest, c0->stats.total_ms + red);
-  agg.kernel_launches += 1;
-  agg.nodes = c0->stats.nodes;
-  agg.triangles = c0->stats.triangles;
-  agg.bvh_depth = c0->stats.bvh_depth;
-  agg.scene_in_smem = c0->stats.scene_in_smem;
-  agg.repack_ms = c0->stats.repack_ms;
-  agg.ref_stack_need = c0->stats.ref_stack_need;
+  // ---- statistics: work summed over the GPUs, device time from the fork to the end of the reduce (the slowest GPU) --
+  b200rt_stats agg;
+  memset(&agg, 0, sizeof agg);
+  agg.upload_ms = m->stats.upload_ms;
+  cudaEventElapsedTime(&agg.total_ms, m->ev_fork, m->ev_done);
+  for (b200rt_ctx *ci : m->ctx) {
+    if (ci->stats_pending) {
+      rc = read_counters(ci);
+      if (rc) return fail(m, rc, "GPU %d: %s", ci->device, ci->err.c_str());
+    }
+    add_work(agg, ci->stats);
+    agg.primary_ms = std::max(agg.primary_ms, ci->stats.primary_ms);
+    agg.trace_ms = std::max(agg.trace_ms, ci->stats.trace_ms);
+  }
+  agg.kernel_launches += 1;   // the reduce
+  copy_scene_facts(agg, c->stats);
+  agg.scene_in_smem = c->stats.scene_in_smem;
   m->stats = agg;
   return 0;
 }
@@ -1901,7 +1887,7 @@ int b200rt_multi_render(b200rt_multi *m, const float *cam, const float *env, int
 int b200rt_multi_render_denoised(b200rt_multi *m, const float *cam, const float *env, int width, int height, int spp,
                                  int max_bounce, const b200rt_opts *opts, const b200rt_denoise_params *dn, float *out,
                                  float *out_noisy) {
-  if (m && !dn) return mfail(m, B200RT_ERR_INVALID, "denoise parameters are NULL");
+  if (m && !dn) return fail(m, B200RT_ERR_INVALID, "denoise parameters are NULL");
   return multi_render(m, cam, env, width, height, spp, max_bounce, opts, dn, out, out_noisy);
 }
 

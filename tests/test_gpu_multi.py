@@ -98,6 +98,38 @@ def test_n_devices_philox_sample_ranges(gpu_ctx, n):
         m.close()
 
 
+WORK = ("rays", "samples", "box_tests", "tri_tests", "mismatches", "revalidated", "exact_walks", "kernel_launches")
+
+
+@pytest.mark.parametrize("rng,spp,height", [(rt.RNG_PHILOX, 2, 32), (rt.RNG_REFERENCE, 3, 8)])
+def test_idle_entry_reports_no_work_of_an_earlier_frame(gpu_ctx, rng, spp, height):
+    """A frame in which an entry has nothing to render (Philox with spp below the entry count; two tile rows for three
+    entries) reports the statistics it reports on a fresh handle: the idle entry adds nothing from the frame before."""
+    sc, ibl = fixtures.load_scene("cornell"), fixtures.load_ibl()
+    width = 32
+    o = dict(rng_mode=rng, traversal=rt.TRAVERSAL_REFERENCE, collect_stats=True, seed=7)
+    cam_a, env_a = fixtures.cam_env(sc["params"], width, 32)
+    cam_b, env_b = fixtures.cam_env(sc["params"], width, height)
+
+    def frame_b(m):
+        img = m.render(cam_b, env_b, width, height, spp, 4, opts=rt.make_opts(**o))
+        return img, {k: m.stats()[k] for k in WORK}
+
+    used, fresh = rt.MultiContext([0, 0, 0]), rt.MultiContext([0, 0, 0])
+    try:
+        fixtures.upload(used, sc, ibl)
+        fixtures.upload(fresh, sc, ibl)
+        used.render(cam_a, env_a, width, 32, 6, 4, opts=rt.make_opts(**o))
+        assert used.stats()["box_tests"] > 0
+        got_img, got = frame_b(used)
+        want_img, want = frame_b(fresh)
+        assert got == want
+        assert np.array_equal(bits(got_img), bits(want_img))
+    finally:
+        used.close()
+        fresh.close()
+
+
 def test_launcher_drives_two_gpus_through_the_reference_call():
     """KernelLauncher(cuda_devices=[0, 1]).launch_Raytracing — the call main.py makes (main.py:84-86) — on two GPUs."""
     devs = devices(2)
