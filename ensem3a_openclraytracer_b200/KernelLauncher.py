@@ -32,7 +32,11 @@ Differences a caller can observe (all documented in INTEGRATION.md):
     Context.render_denoised; missing keys take DENOISE_DEFAULTS) runs the edge-avoiding à-trous filter of include/b200rt.h
     over every frame, on one GPU or on `cuda_devices`.  B200RT_DENOISE=1 (the defaults) or
     B200RT_DENOISE=passes[,sigma_color[,sigma_normal[,sigma_position]]] sets it for callers that never touch the
-    attribute.  It cannot be combined with `adaptive`.
+    attribute.  It cannot be combined with `adaptive`;
+  * `pixel_jitter = True` anti-aliases: every sample traces its own camera ray through a jittered point of its pixel
+    (B200RT_SAMPLING_PIXEL_JITTER), so the image converges to the pixel-area average instead of the reference's one
+    point per pixel.  B200RT_PIXEL_JITTER=1 (or 0) sets it for callers that never touch the attribute.  It cannot be
+    combined with `adaptive`.
 """
 import math
 import os
@@ -90,6 +94,14 @@ def denoise_from_env(text):
     return dn
 
 
+def pixel_jitter_from_env(text):
+    """The `pixel_jitter` flag that B200RT_PIXEL_JITTER=0 or =1 stands for; ValueError otherwise."""
+    t = str(text).strip()
+    if t not in ("0", "1"):
+        raise ValueError(f"B200RT_PIXEL_JITTER={text!r}: expected 0 or 1")
+    return t == "1"
+
+
 class KernelLauncher(object):
 
     def __init__(self, context=None, platform=None, device=None, queue=None, cuda_device=0, cuda_devices=None):
@@ -118,6 +130,9 @@ class KernelLauncher(object):
         self.adaptive = adaptive_from_env(os.environ["B200RT_ADAPTIVE"]) if os.environ.get("B200RT_ADAPTIVE") else None
         # None: the render as it comes; a dict: denoised (module docstring)
         self.denoise = denoise_from_env(os.environ["B200RT_DENOISE"]) if os.environ.get("B200RT_DENOISE") else None
+        # False: one camera ray per pixel (the reference's image); True: anti-aliasing (module docstring)
+        self.pixel_jitter = (pixel_jitter_from_env(os.environ["B200RT_PIXEL_JITTER"])
+                             if os.environ.get("B200RT_PIXEL_JITTER") else False)
         self.last_spp = None
         self.last_stats = None
         self._warned_deep = False
@@ -128,6 +143,9 @@ class KernelLauncher(object):
         if self.adaptive is not None and self.denoise is not None:
             raise ValueError("adaptive sampling and denoising cannot be combined: set launcher.adaptive = None or "
                              "launcher.denoise = None")
+        if self.adaptive is not None and self.pixel_jitter:
+            raise ValueError("adaptive sampling and pixel jitter cannot be combined: set launcher.adaptive = None or "
+                             "launcher.pixel_jitter = False")
         if self.adaptive is not None and isinstance(self._ctx, _capi.MultiContext):
             raise ValueError("adaptive sampling renders on one GPU: its stopping rule needs each pixel's samples in one "
                              f"sequence, which a split over cuda_devices={self._ctx.devices} would cut apart; set "
@@ -165,7 +183,8 @@ class KernelLauncher(object):
                               RuntimeWarning, stacklevel=2)
                 self._warned_deep = True
         opts = _capi.make_opts(rng_mode=self.rng_mode, traversal=traversal, stack_cap=self.stack_cap,
-                               seed=self.seed, collect_stats=self.collect_stats, sample_streams=self.sample_streams)
+                               seed=self.seed, collect_stats=self.collect_stats, sample_streams=self.sample_streams,
+                               sampling=_capi.SAMPLING_PIXEL_JITTER if self.pixel_jitter else _capi.SAMPLING_REFERENCE)
         out = h_img_out.reshape(-1)[:imgDim * 3]
         if self.adaptive is not None:
             img, self.last_spp, _ = self._ctx.render_adaptive(cam[:10], h_envData, width, height, int(spp), int(maxBounce),

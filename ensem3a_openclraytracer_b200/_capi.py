@@ -17,6 +17,7 @@ RNG_REFERENCE, RNG_PHILOX = 0, 1
 TRAVERSAL_FAST, TRAVERSAL_REFERENCE, TRAVERSAL_VERIFY = 0, 1, 2
 OUT_FINAL, OUT_SUMS = 0, 1
 SAMPLING_REFERENCE, SAMPLING_IMPORTANCE, SAMPLING_LIGHTS = 0, 1, 2
+SAMPLING_PIXEL_JITTER = 8   # anti-aliasing: changes the integrand to the pixel's area (include/b200rt.h)
 
 
 class B200RTError(RuntimeError):

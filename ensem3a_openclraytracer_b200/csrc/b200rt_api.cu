@@ -380,12 +380,14 @@ int prepare_trace_t(b200rt_ctx *c, WaveLaunch *w) {
   return 0;
 }
 
-int prepare_wave(b200rt_ctx *c, int trav, bool smem, bool stats, bool nee, bool adaptive, WaveLaunch *w) {
+// jitter and adaptive are never both set (b200rt_render_adaptive refuses the jitter bit)
+int prepare_wave(b200rt_ctx *c, int trav, bool smem, bool stats, bool nee, bool adaptive, bool jitter, WaveLaunch *w) {
   int per_sm = 0;
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shade<false, false>, kShadeBlock, 0));
   if (per_sm < 1) return fail(c, B200RT_ERR_CUDA, "k_shade does not fit on an SM");
   w->shade_grid = per_sm * c->sm_count;
-  if (nee) w->shade = adaptive ? k_shade<true, true> : k_shade<true, false>;
+  if (jitter) w->shade = nee ? k_shade<true, false, true> : k_shade<false, false, true>;
+  else if (nee) w->shade = adaptive ? k_shade<true, true> : k_shade<true, false>;
   else w->shade = adaptive ? k_shade<false, true> : k_shade<false, false>;
   return with_variant(c, trav, smem, stats, [&](auto t, auto s, auto st) {
     return prepare_trace_t<decltype(t)::value, decltype(s)::value, decltype(st)::value>(c, w);
@@ -497,7 +499,8 @@ int check_frame_args(b200rt_ctx *c, const float *cam, int width, int height, int
   if (o.rng_mode != B200RT_RNG_REFERENCE && o.rng_mode != B200RT_RNG_PHILOX)
     return fail(c, B200RT_ERR_INVALID, "bad rng_mode %d", o.rng_mode);
   if (o.traversal < 0 || o.traversal > 2) return fail(c, B200RT_ERR_INVALID, "bad traversal %d", o.traversal);
-  if (o.sampling < 0 || o.sampling > (B200RT_SAMPLING_IMPORTANCE | B200RT_SAMPLING_LIGHTS))
+  if (o.sampling < 0 ||
+      (o.sampling & ~(B200RT_SAMPLING_IMPORTANCE | B200RT_SAMPLING_LIGHTS | B200RT_SAMPLING_PIXEL_JITTER)) != 0)
     return fail(c, B200RT_ERR_INVALID, "bad sampling mode %d", o.sampling);
   if (o.output != B200RT_OUT_FINAL && o.output != B200RT_OUT_SUMS)
     return fail(c, B200RT_ERR_INVALID, "bad output mode %d", o.output);
@@ -533,13 +536,17 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   // every live path traces exactly one ray per iteration and a sample needs at most max_bounce + 1 bounce rays
   // plus one sun ray (Raytracing.cl:46-137)
   // with light sampling every surface that scatters adds one shadow ray towards an emitter: up to 2 (max_bounce + 1) + 1
+  // with pixel jitter every sample also traces its own camera ray: one more
   const bool nee = (o.sampling & B200RT_SAMPLING_LIGHTS) != 0 && c->n_light > 0;
-  const long long per_sample = nee ? 2 * ((long long)max_bounce + 1) + 1 : (long long)max_bounce + 2;
+  const bool jitter = (o.sampling & B200RT_SAMPLING_PIXEL_JITTER) != 0;
+  const long long per_sample = (nee ? 2 * ((long long)max_bounce + 1) + 1 : (long long)max_bounce + 2) + (jitter ? 1 : 0);
   const long long n_iter_ll = (long long)(F.s1 - F.s0) * per_sample;
   if (n_iter_ll > (1 << 22)) return fail(c, B200RT_ERR_UNSUPPORTED, "%lld wavefront iterations exceed 2^22", n_iter_ll);
   const int n_iter = (int)n_iter_ll;
-  if (ensure(c, c->d_prim_dirk, npix * sizeof(float4))) return B200RT_ERR_CUDA;
-  if (ensure(c, c->d_prim_tri, npix * sizeof(int))) return B200RT_ERR_CUDA;
+  if (!jitter) {  // the cached primary hits; a jittered sample traces its own camera ray
+    if (ensure(c, c->d_prim_dirk, npix * sizeof(float4))) return B200RT_ERR_CUDA;
+    if (ensure(c, c->d_prim_tri, npix * sizeof(int))) return B200RT_ERR_CUDA;
+  }
   if (ensure(c, c->d_pA, npix * sizeof(float4))) return B200RT_ERR_CUDA;
   if (ensure(c, c->d_pB, npix * sizeof(float4))) return B200RT_ERR_CUDA;
   if (ensure(c, c->d_pC, npix * sizeof(float4))) return B200RT_ERR_CUDA;
@@ -563,7 +570,7 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   A.validate = (trav == B200RT_TRAVERSAL_FAST) ? 1 : 0;
   const bool smem = use_smem_scene(c);
   WaveLaunch wl;
-  int rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, &wl);
+  int rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, jitter, &wl);
   if (rc) return rc;
   if (ensure(c, c->d_part_count, (size_t)wl.shade_grid * sizeof(unsigned int))) return B200RT_ERR_CUDA;
   A.part_count = static_cast<unsigned int *>(c->d_part_count.p);
@@ -596,9 +603,16 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
     CU(cudaGetLastError());
     c->stats.kernel_launches++;
   }
-  rc = launch_primary(c, A, trav, smem, false, o.collect_stats != 0, nullptr, nullptr);
-  if (rc) return rc;
-  // the first path list: k_primary's live pixels in tile order
+  if (jitter) {  // no primary-hit kernel: every pixel of the rendered set starts with a camera ray in k_shade
+    const int grid = (int)std::min<long long>(((long long)A.n_work + 255) / 256, (long long)c->sm_count * 8);
+    k_jitter_init<<<grid, 256, 0, c->stream>>>(A);
+    CU(cudaGetLastError());
+    c->stats.kernel_launches++;
+  } else {
+    rc = launch_primary(c, A, trav, smem, false, o.collect_stats != 0, nullptr, nullptr);
+    if (rc) return rc;
+  }
+  // the first path list: k_primary's live pixels (k_jitter_init's pixels) in tile order
   k_count_parts<<<wl.shade_grid, kCompactBlock, 0, c->stream>>>(A.slots, (unsigned)A.n_work, A.part_count);
   k_compact<<<wl.shade_grid, kCompactBlock, 0, c->stream>>>(A.slots, nullptr, (unsigned)A.n_work, A.part_count, A.list[0], A.cnt);
   CU(cudaGetLastError());
@@ -1304,6 +1318,8 @@ int b200rt_render_adaptive(b200rt_ctx *c, const float *cam, const float *env, in
   if (!std::isfinite(ad->floor) || !(ad->floor > 0.0f))
     return fail(c, B200RT_ERR_INVALID, "adaptive floor %g must be finite and > 0", (double)ad->floor);
   if (o.output != B200RT_OUT_FINAL) return fail(c, B200RT_ERR_INVALID, "adaptive sampling needs B200RT_OUT_FINAL");
+  if (o.sampling & B200RT_SAMPLING_PIXEL_JITTER)
+    return fail(c, B200RT_ERR_INVALID, "adaptive sampling cannot be combined with B200RT_SAMPLING_PIXEL_JITTER");
   if (o.sample_end > 0 && (o.sample_begin != 0 || o.sample_end != spp))
     return fail(c, B200RT_ERR_INVALID, "adaptive sampling needs the whole sample range [0, spp)");
   // the stopping rule needs the pixel's samples as one serial sequence; -1 (automatic) resolves to that one stream

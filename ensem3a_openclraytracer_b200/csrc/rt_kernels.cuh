@@ -15,6 +15,8 @@
 //   k_reduce_finalize / k_img_processing   the accumulate / clamp / tonemap passes.
 // An adaptive frame (b200rt_render_adaptive) runs k_adaptive_init before k_primary and k_shade<NEE, true>, whose
 // end_sample block also applies the stopping rule (adaptive_end_sample); the host ends its loop once the list is empty.
+// A jittered frame (opt-in pixel jitter) runs k_jitter_init instead of k_primary and k_shade<NEE, false, true>, in
+// which every sample traces its own camera ray: one more wavefront iteration per sample.
 #pragma once
 #include "rt_shade.cuh"
 #include "rt_trace.cuh"
@@ -77,18 +79,20 @@ struct KernelArgs {
 //   pA = origin.xyz, dir.x     pB = dir.y, dir.z, meta, rng     pC = throughput.rgb, -     pHit = triangle, distance
 // origin / dir describe the ray in flight (for a sun ray `dir` keeps the escaped direction for the environment
 // lookup and the ray itself points along FrameParams::sun_dir: trace_dir).
-// meta: bit 0 first iteration (no ray traced yet), bit 1 light ray (opt-in light sampling), bit 3 sun ray, bits 4-7
-// material type of the surface the ray left, bits 8-15 bounce j, bits 16-31 sample index
+// meta: bit 0 first iteration (no ray traced yet), bit 1 light ray (opt-in light sampling), bit 2 camera ray (opt-in
+// pixel jitter: the ray leaves cam_pos and the sample has not hit anything yet), bit 3 sun ray, bits 4-7 material type
+// of the surface the ray left, bits 8-15 bounce j, bits 16-31 sample index
 struct PathMeta {
-  int first, light, sun, type, j, s;
+  int first, light, sun, type, j, s, cam;
 };
 
-RT_DEV uint32_t meta_pack(int first, int sun, int type, int j, int s, int light = 0) {
-  return (uint32_t)first | ((uint32_t)light << 1) | ((uint32_t)sun << 3) | ((uint32_t)(type & 15) << 4) | ((uint32_t)(j & 255) << 8) | ((uint32_t)s << 16);
+RT_DEV uint32_t meta_pack(int first, int sun, int type, int j, int s, int light = 0, int cam = 0) {
+  return (uint32_t)first | ((uint32_t)light << 1) | ((uint32_t)cam << 2) | ((uint32_t)sun << 3) | ((uint32_t)(type & 15) << 4) | ((uint32_t)(j & 255) << 8) | ((uint32_t)s << 16);
 }
 
 RT_DEV PathMeta meta_unpack(uint32_t m) {
-  return {(int)(m & 1u), (int)((m >> 1) & 1u), (int)((m >> 3) & 1u), (int)((m >> 4) & 15u), (int)((m >> 8) & 255u), (int)(m >> 16)};
+  return {(int)(m & 1u), (int)((m >> 1) & 1u), (int)((m >> 3) & 1u), (int)((m >> 4) & 15u), (int)((m >> 8) & 255u), (int)(m >> 16),
+          (int)((m >> 2) & 1u)};
 }
 
 // direction of the ray a path traces, from its stored direction d
@@ -244,6 +248,22 @@ __global__ void k_adaptive_init(const __grid_constant__ KernelArgs A) {
   }
 }
 
+// ---- jittered frames: the first path list without a primary-hit kernel -------------------------------------------
+// Every pixel of the rendered set starts its first sample (s0) with a camera ray of its own in k_shade<NEE, false,
+// true>, so no pixel is ray-free: pB (first iteration, s0, generator word i as Raytracing.cl:171 seeds it), a zero
+// running sum, and the pixel into slots for k_count_parts + k_compact (-1 outside the rendered set).
+__global__ void k_jitter_init(const __grid_constant__ KernelArgs A) {
+  for (unsigned int w = blockIdx.x * blockDim.x + threadIdx.x; w < (unsigned)A.n_work; w += gridDim.x * blockDim.x) {
+    const int i = work_to_pixel(A, w);
+    if (i >= 0) {
+      A.pB[i] = make_float4(0.0f, 0.0f, __uint_as_float(meta_pack(1, 0, 0, 0, A.F.s0)), __uint_as_float((uint32_t)i));
+      float *acc_px = A.out + 3 * (size_t)i;
+      acc_px[0] = 0.0f; acc_px[1] = 0.0f; acc_px[2] = 0.0f;
+    }
+    A.slots[w] = i;
+  }
+}
+
 // ---- primary hits ---------------------------------------------------------------------------------------
 // PARITY: write tri / k for every pixel of [pixel_begin,pixel_end) and nothing else.
 template <int TRAV, bool SMEM, bool PARITY, bool STATS>
@@ -385,8 +405,10 @@ __global__ void __launch_bounds__(kCompactBlock) k_compact(const int *__restrict
 // 8 CTAs per SM: the kernel is bound by the latency of its gathers; 5-7 (no spills) and 9-12 resident CTAs were all slower.
 // NEE = opt-in light sampling (b200rt_opts.sampling bit 1): a separate instantiation, so that the reference's
 // estimator runs exactly the code it ran before.  ADAPT = adaptive sampling (adaptive_end_sample at the end of every
-// sample), likewise a separate instantiation.
-template <bool NEE, bool ADAPT>
+// sample), likewise a separate instantiation.  JITTER = opt-in pixel jitter (sampling bit B200RT_SAMPLING_PIXEL_JITTER):
+// a sample starts with a camera ray through a jittered point of its pixel (phase 3), which phase 2 resolves the way
+// k_primary resolves the cached primary ray, instead of from the cached primary hit.
+template <bool NEE, bool ADAPT, bool JITTER = false>
 __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant__ KernelArgs A, int iter) {
   const FrameParams &F = A.F;
   const SceneView &S = A.S;
@@ -439,8 +461,9 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
     const bool first = pm.first != 0;
     int sun_ray = pm.sun, seg_type = pm.type, j = pm.j, s = pm.s;
     const bool light_ray = NEE && pm.light != 0;
+    const bool cam_ray = JITTER && pm.cam != 0;
     bool pixel_done = false, start = valid && first, shade = false, end_sample = false, sun_done = false;
-    bool want_light = false, light_done = false, from_light = false;
+    bool want_light = false, light_done = false, from_light = false, cam_out = false;
 
     // ---- phase 1: the winner of the conservative walk must pass the exact leaf-box test ---------------------------------
     if (valid && !first && A.validate && htri != -1) {
@@ -457,7 +480,21 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
 
     // ---- phase 2: resolve the traced ray (Raytracing.cl:91-137) ------------------------------------------------------------
     if (valid && !first) {
-      if (light_ray) {
+      if (cam_ray) {  // the sample's camera ray, as k_primary resolves the primary ray
+        if (htri < 0) {  // :146-150
+          acc = (mk3(1.0f, 1.0f, 1.0f) * ibl_lookup(F, A.ibl, d)) * F.ibl_power;
+          end_sample = true;
+        } else {
+          const Material mc = load_material(S.mats, tri_material(S, htri));
+          if (mc.type == 0) {  // :140-144
+            acc = mk3(1.0f, 1.0f, 1.0f) * mc.roughness;
+            end_sample = true;
+          } else {  // the hit starts the path, as the cached primary hit does in phase 3
+            j = 0;
+            if (NEE && mc.type != 3) want_light = true; else shade = true;
+          }
+        }
+      } else if (light_ray) {
         light_done = true;
       } else if (!sun_ray) {
         if (htri >= 0) {  // the bounce ray becomes the current segment (:91-93)
@@ -541,8 +578,19 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
         start = true;
       }
     }
-    // ---- phase 3: a new sample starts from the cached primary hit (Raytracing.cl:195-201) --------------------------------------
-    if (start) {
+    // ---- phase 3: a new sample starts from the cached primary hit (Raytracing.cl:195-201), or with a jittered camera ray -------
+    if (JITTER && start) {
+      float ux, uy;
+      if (F.rng_mode == 0) draw2_jitter<0>(g, (uint32_t)pix, (uint32_t)s, F.key0, F.key1, &ux, &uy);
+      else draw2_jitter<1>(g, (uint32_t)pix, (uint32_t)s, F.key0, F.key1, &ux, &uy);
+      o = F.cam_pos;
+      d = camera_dir_jittered(F, pix, ux, uy);
+      acc = mk3(1.0f, 1.0f, 1.0f);
+      j = 0;
+      sun_ray = 0;
+      if (NEE) A.pR[pix] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+      cam_out = true;
+    } else if (start) {
       const float4 dk = ld_stream(A.prim_dirk + pix);
       o = F.cam_pos;
       d = mk3(dk.x, dk.y, dk.z);
@@ -624,7 +672,8 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
     const bool alive = valid && !pixel_done;
     if (alive) {
       A.pA[pix] = make_float4(o.x, o.y, o.z, d.x);
-      A.pB[pix] = make_float4(d.y, d.z, __uint_as_float(meta_pack(0, sun_ray, seg_type, j, s, (NEE && want_light) ? 1 : 0)),
+      A.pB[pix] = make_float4(d.y, d.z, __uint_as_float(meta_pack(0, sun_ray, seg_type, j, s, (NEE && want_light) ? 1 : 0,
+                                                                  (JITTER && cam_out) ? 1 : 0)),
                               __uint_as_float(g.a));
       A.pC[pix] = make_float4(acc.x, acc.y, acc.z, NEE ? pb_ray : 0.0f);
     }

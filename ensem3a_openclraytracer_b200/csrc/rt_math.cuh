@@ -216,4 +216,18 @@ RT_DEV void draw3_light(rng_state &g, uint32_t pixel, uint32_t sample, uint32_t 
   }
 }
 
+// The two uniforms of a sample's jittered camera ray (opt-in pixel jitter), drawn when the sample starts: the
+// generator's next two values in reference mode, words 0 and 1 of the Philox block (pixel, sample, 0, 2) otherwise.
+template <int RNG>
+RT_DEV void draw2_jitter(rng_state &g, uint32_t pixel, uint32_t sample, uint32_t k0, uint32_t k1, float *ux, float *uy) {
+  if (RNG == 0) {
+    draw2<0>(g, pixel, sample, 0u, k0, k1, ux, uy);
+  } else {
+    uint32_t o[4];
+    philox4x32_10(pixel, sample, 0u, 2u, k0, k1, o);
+    *ux = bits_to_unit(o[0]);
+    *uy = bits_to_unit(o[1]);
+  }
+}
+
 }  // namespace b200rt

@@ -44,17 +44,30 @@ RT_DEV Material load_material(const float *mats, int idx) {  // Raytracing.cl:5-
   return r;
 }
 
-// Raytracing.cl:18-37
-RT_DEV v3 camera_dir(const FrameParams &F, int i) {
-  int col = (i + 1) % F.width;
-  int row = (i - col) / F.width;
+// Raytracing.cl:18-37: the camera direction through image-plane point (fx, fz), in pixels (column, row)
+RT_DEV v3 camera_dir_at(const FrameParams &F, float fx, float fz) {
   v3 focal = mk3(F.cam_pos.x, F.cam_pos.y - F.focal_off, F.cam_pos.z);
-  v3 pix = mk3((float)col * F.step - 0.5f, 0.0f, 0.5f - (float)row * F.step);
+  v3 pix = mk3(fx * F.step - 0.5f, 0.0f, 0.5f - fz * F.step);
   v3 d = unit((F.cam_pos + pix) - focal);
   d = apply_rotor(F.cam_rx, d);
   d = apply_rotor(F.cam_ry, d);
   d = apply_rotor(F.cam_rz, d);
   return d;
+}
+
+// the reference's camera ray of work-item i (column (i + 1) % width, its off-by-one included, Raytracing.cl:21-22)
+RT_DEV v3 camera_dir(const FrameParams &F, int i) {
+  int col = (i + 1) % F.width;
+  int row = (i - col) / F.width;
+  return camera_dir_at(F, (float)col, (float)row);
+}
+
+// opt-in pixel jitter (b200rt_opts.sampling bit 3): the ray through (col + ux - 0.5, row + uy - 0.5), a point of the
+// one-pixel footprint centred on the reference's ray; (ux, uy) uniform in [0, 1)
+RT_DEV v3 camera_dir_jittered(const FrameParams &F, int i, float ux, float uy) {
+  int col = (i + 1) % F.width;
+  int row = (i - col) / F.width;
+  return camera_dir_at(F, (float)col + (ux - 0.5f), (float)row + (uy - 0.5f));
 }
 
 // uv * extent -> integer texel, exactly the reference's chain of binary32 roundings (MathLib.cl:78-80,87):

@@ -10,6 +10,8 @@ instead of sample by sample): relative difference ~1e-7 per addition, far inside
 `denoise` (a dict of Context.denoise's keywords, {} for the defaults) passes every preview and image() through the
 edge-avoiding à-trous filter of include/b200rt.h, with the G-buffer computed once, on the first slice.  The saved state
 (`sums`, `done`) stays undenoised, so a resumed render denoises the same way.
+
+`sampling` (a mask of the SAMPLING_* bits, e.g. SAMPLING_PIXEL_JITTER) goes into every slice's options.
 """
 import numpy as np
 
@@ -26,7 +28,7 @@ class ProgressiveRender:
     """Iterate to refine:  for preview in ProgressiveRender(ctx, cam, env, w, h, spp, bounce, slice_spp=16): ..."""
 
     def __init__(self, ctx, cam, env, width, height, spp, max_bounce, slice_spp=16, seed=0, sums=None, done=0,
-                 denoise=None):
+                 denoise=None, sampling=0):
         if slice_spp <= 0 or spp <= 0:
             raise ValueError("spp and slice_spp must be positive")
         self.ctx, self.cam, self.env = ctx, cam, env
@@ -36,6 +38,7 @@ class ProgressiveRender:
         self.sums = np.zeros(n, np.float32) if sums is None else np.ascontiguousarray(sums, np.float32).reshape(n).copy()
         self.done = int(done)          # samples accumulated so far — (sums, done) is the checkpoint
         self.denoise = denoise
+        self.sampling = int(sampling)
         self._gb = None
 
     def _view(self, img):
@@ -53,7 +56,7 @@ class ProgressiveRender:
             raise StopIteration
         s0, s1 = self.done, min(self.done + self.slice_spp, self.spp)
         opts = _capi.make_opts(rng_mode=_capi.RNG_PHILOX, seed=self.seed, output=_capi.OUT_SUMS, sample_begin=s0,
-                               sample_end=s1)
+                               sample_end=s1, sampling=self.sampling)
         part = self.ctx.render(self.cam, self.env, self.width, self.height, self.spp, self.max_bounce, opts=opts)
         self.sums += part
         self.done = s1

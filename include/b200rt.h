@@ -52,6 +52,26 @@ typedef enum {
                                         intent: the dead sampleLight, MathLib.cl:404-454) at every surface that scatters,
                                         combined with the surface's own sample by the balance heuristic; one more ray per
                                         such surface, three more float4 of path state */
+#define B200RT_SAMPLING_PIXEL_JITTER 8
+/* Anti-aliasing: every sample traces its own camera ray through a jittered point of its pixel.  Unlike bits 0 and 1
+ * this bit CHANGES THE INTEGRAND: the image converges to the box-filtered (pixel-area) image, no longer to the
+ * reference's, whose pixel is one point (one camera ray per pixel, whose hit every sample restarts from,
+ * Raytracing.cl:184-187).  Its value is 8: 4 is not assigned and is refused, as is anything above 15.  The rule, in
+ * binary32 with every operation rounded separately (no contraction):
+ *   - (ux, uy) are two uniforms in [0, 1): with B200RT_RNG_PHILOX words 0 and 1 of the block at counter (i, s, 0, 2) for
+ *     sample s of work-item i (direction sampling uses n = 0, light sampling n = 1); with B200RT_RNG_REFERENCE the pixel
+ *     generator's next two values (ux first), drawn when the sample starts, before any other draw of that sample;
+ *   - col = (i + 1) % width, row = (i - col) / width (the reference's mapping, Raytracing.cl:21-22);
+ *     fx = (float)col + (ux - 0.5f), fz = (float)row + (uy - 0.5f);
+ *     pix = (fx * step - 0.5f, 0, 0.5f - fz * step); the rest of Raytracing.cl:18-37 is unchanged (normalise
+ *     (cam + pix) - focal, then the three rotations).  The footprint is one pixel wide, centred on the reference's ray;
+ *   - the sample then goes on as the reference's sample from its primary hit: a miss contributes env x IBL power, an
+ *     emitter its power, anything else scatters from the hit (Raytracing.cl:140-150, :51-137).
+ * b200rt_primary_hits, b200rt_gbuffer and b200rt_trace_rays ignore the bit (the denoiser's G-buffer stays the unjittered
+ * primary hit); b200rt_render_adaptive refuses it.  Statistics of a jittered render: `rays` counts one camera ray per
+ * sample; `primary_rays` is 0 (no primary-hit kernel runs); `samples` = rendered pixels x (sample_end - sample_begin),
+ * since no pixel is ray-free; wave_iterations = (sample_end - sample_begin) x (max_bounce + 3), or
+ * x (2 (max_bounce + 1) + 2) with light sampling; kernel_launches = 3 + the shading, compaction and tracing launches. */
 
 /* output modes */
 #define B200RT_OUT_FINAL 0 /* mean over spp, clamped to [0,1]  (Raytracing.cl:211-219) */
@@ -167,7 +187,8 @@ typedef struct {
  * (float per pixel) may be NULL; entries of pixels outside the rendered set (pixel range / tile rows) are 0.
  * opts: output must be B200RT_OUT_FINAL over the whole sample range, sample_streams -1, 0 or 1 (the rule needs one
  * serial sequence of samples per pixel; -1 resolves to one stream and stats.sample_streams says 1); pixel ranges,
- * tile rows, both generators, every traversal and every sampling bit are allowed.  The launch loop stops once every
+ * tile rows, both generators, every traversal and sampling bits 0 and 1 are allowed (B200RT_SAMPLING_PIXEL_JITTER is
+ * refused: the stopping rule is stated for the reference's pixel).  The launch loop stops once every
  * pixel has stopped: stats.samples, wave_iterations and kernel_launches report the work actually done. */
 int b200rt_render_adaptive(b200rt_ctx *ctx, const float *cam, const float *env, int width, int height, int spp,
                            int max_bounce, const b200rt_opts *opts, const b200rt_adaptive *ad,
