@@ -72,7 +72,7 @@ SYMBOLS = [
     "b200rt_default_opts", "b200rt_create", "b200rt_destroy", "b200rt_last_error", "b200rt_set_scene",
     "b200rt_set_materials", "b200rt_set_ibl", "b200rt_render", "b200rt_render_adaptive", "b200rt_gbuffer", "b200rt_denoise", "b200rt_render_denoised", "b200rt_render_rgb8", "b200rt_render_device", "b200rt_finalize_device",
     "b200rt_reduce_finalize_device", "b200rt_sync", "b200rt_set_stream", "b200rt_invalidate", "b200rt_primary_hits", "b200rt_trace_rays",
-    "b200rt_img_processing", "b200rt_get_stats", "b200rt_math_probe", "b200rt_philox_probe", "b200rt_alloc",
+    "b200rt_img_processing", "b200rt_get_stats", "b200rt_math_probe", "b200rt_texel_probe", "b200rt_philox_probe", "b200rt_alloc",
     "b200rt_free", "b200rt_ipc_export",
     "b200rt_ipc_open", "b200rt_ipc_close", "b200rt_build_bvh", "b200rt_repack_probe", "b200rt_version", "b200rt_device_count",
     "b200rt_multi_create", "b200rt_multi_destroy", "b200rt_multi_last_error", "b200rt_multi_device_count",
@@ -130,6 +130,7 @@ def load_library():
     lib.b200rt_img_processing.argtypes = [vp, vp, vp, i64, i64]
     lib.b200rt_get_stats.argtypes = [vp, ctypes.POINTER(Stats)]
     lib.b200rt_math_probe.argtypes = [vp, i32, vp, vp, i64, vp]
+    lib.b200rt_texel_probe.argtypes = [vp, i32, vp, vp, i64, i32, vp]
     lib.b200rt_philox_probe.argtypes = [vp, ctypes.POINTER(u32 * 4), u32, u32, ctypes.POINTER(u32 * 4)]
     lib.b200rt_alloc.argtypes = [vp, i64, ctypes.POINTER(vp)]
     lib.b200rt_free.argtypes = [vp, vp]
@@ -457,12 +458,17 @@ class Context(_Handle):
         return dst
 
     # ---- probes ---------------------------------------------------------------------------------------------
-    def math_probe(self, fn, a, b=None):
+    def math_probe(self, fn, a, b=None, extent=None):
+        """extent: environment-map width (fn 11/12) or height (fn 13/14); None = 8192 / 4096"""
         a_ = _f32(a)
         b_ = None if b is None else _f32(b)
         out = np.zeros_like(a_)
-        self._check(self._lib.b200rt_math_probe(self._h, int(fn), _ptr(a_), _ptr(b_), a_.size, _ptr(out)),
-                    "b200rt_math_probe")
+        if extent is None:
+            self._check(self._lib.b200rt_math_probe(self._h, int(fn), _ptr(a_), _ptr(b_), a_.size, _ptr(out)),
+                        "b200rt_math_probe")
+        else:
+            self._check(self._lib.b200rt_texel_probe(self._h, int(fn), _ptr(a_), _ptr(b_), a_.size, int(extent),
+                                                     _ptr(out)), "b200rt_texel_probe")
         return out
 
     def philox_probe(self, ctr, key0, key1):

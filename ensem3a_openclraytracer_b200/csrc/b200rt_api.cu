@@ -1594,9 +1594,7 @@ int b200rt_get_stats(const b200rt_ctx *c, b200rt_stats *s) {
   return 0;
 }
 
-int b200rt_math_probe(b200rt_ctx *c, int fn, const float *a, const float *b, int64_t n, float *out) {
-  if (!c) return B200RT_ERR_INVALID;
-  if (!a || !out || n <= 0 || fn < 0 || fn > 16) return fail(c, B200RT_ERR_INVALID, "bad math_probe arguments");
+static int math_probe(b200rt_ctx *c, int fn, const float *a, const float *b, int64_t n, int extent, float *out) {
   CU(cudaSetDevice(c->device));
   size_t bytes = (size_t)n * sizeof(float);
   if (ensure(c, c->d_tmp_a, bytes)) return B200RT_ERR_CUDA;
@@ -1607,11 +1605,23 @@ int b200rt_math_probe(b200rt_ctx *c, int fn, const float *a, const float *b, int
   else CU(cudaMemsetAsync(c->d_tmp_b.p, 0, bytes, c->stream));
   k_math_probe<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(fn, static_cast<const float *>(c->d_tmp_a.p),
                                                                     static_cast<const float *>(c->d_tmp_b.p), (long long)n,
-                                                                    static_cast<float *>(c->d_misc.p));
+                                                                    extent, static_cast<float *>(c->d_misc.p));
   CU(cudaGetLastError());
   CU(cudaMemcpyAsync(out, c->d_misc.p, bytes, cudaMemcpyDeviceToHost, c->stream));
   CU(cudaStreamSynchronize(c->stream));
   return 0;
+}
+
+int b200rt_math_probe(b200rt_ctx *c, int fn, const float *a, const float *b, int64_t n, float *out) {
+  if (!c) return B200RT_ERR_INVALID;
+  if (!a || !out || n <= 0 || fn < 0 || fn > 17) return fail(c, B200RT_ERR_INVALID, "bad math_probe arguments");
+  return math_probe(c, fn, a, b, n, (fn == 13 || fn == 14) ? 4096 : 8192, out);
+}
+
+int b200rt_texel_probe(b200rt_ctx *c, int fn, const float *a, const float *b, int64_t n, int extent, float *out) {
+  if (!c) return B200RT_ERR_INVALID;
+  if (!a || !out || n <= 0 || fn < 11 || fn > 14 || extent < 1) return fail(c, B200RT_ERR_INVALID, "bad texel_probe arguments");
+  return math_probe(c, fn, a, b, n, extent, out);
 }
 
 int b200rt_philox_probe(b200rt_ctx *c, const uint32_t ctr[4], uint32_t key0, uint32_t key1, uint32_t out[4]) {

@@ -903,7 +903,8 @@ __global__ void k_img_processing(const float *__restrict__ in, float *__restrict
 }
 
 // ---- probes -----------------------------------------------------------------------------------------------------------------------
-__global__ void k_math_probe(int fn, const float *a, const float *b, long long n, float *out) {
+// extent: the environment map's width (fn 11/12) or height (fn 13/14)
+__global__ void k_math_probe(int fn, const float *a, const float *b, long long n, int extent, float *out) {
   long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (i >= n) return;
   float x = a[i], y = b[i], r = 0.0f;
@@ -919,13 +920,14 @@ __global__ void k_math_probe(int fn, const float *a, const float *b, long long n
     case 8: r = sqrtf(x); break;
     case 9: { float s, c; cr_sincos(x, &s, &c); r = s; break; }
     case 10: { float s, c; cr_sincos(x, &s, &c); r = c; break; }
-    case 11: r = (float)ibl_texel_u(x, y, 8192); break;                       // fast path with its fallback
-    case 12: r = (float)texel_coord(cr_atan2(x, y), 0.1591f, 8192); break;    // correctly rounded angle only
-    case 13: r = (float)ibl_texel_v(x, 4096); break;
-    case 14: r = (float)texel_coord(cr_asin(x), 0.3183f, 4096); break;
+    case 11: r = (float)ibl_texel_u(x, y, extent); break;                       // fast path with its fallback
+    case 12: r = (float)texel_coord(cr_atan2(x, y), 0.1591f, extent); break;    // correctly rounded angle only
+    case 13: r = (float)ibl_texel_v(x, extent); break;
+    case 14: r = (float)texel_coord(cr_asin(x), 0.3183f, extent); break;
     case 15: { const float a = atan2f(x, y), del = fabsf(a) * 4.76837158203125e-07f;   // 1 = the column needs the exact angle (600 wide)
                r = texel_coord(a - del, 0.1591f, 600) != texel_coord(a + del, 0.1591f, 600) ? 1.0f : 0.0f; break; }
     case 16: r = atan2f(x, y); break;
+    case 17: r = asinf(x); break;
   }
   out[i] = r;
 }

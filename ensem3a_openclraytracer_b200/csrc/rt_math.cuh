@@ -10,6 +10,7 @@
 // independent of any vendor's float libm.
 #pragma once
 #include <cuda_runtime.h>
+#include <limits.h>
 #include <stdint.h>
 
 namespace b200rt {
@@ -50,9 +51,61 @@ RT_DEV float clamp01(float x) {
 }
 
 // ---- correctly-rounded binary32 transcendentals (binary64 evaluation, one rounding) ----
+// A binary64 value within e ulps of the true value, rounded once, is the correctly rounded binary32 unless the true value
+// lies within e binary64 ulps of a binary32 rounding boundary.  CUDA's binary64 acos / asin / pow are within 2 ulp, and on
+// the domains the kernels reach (every float with |x| <= 1 for acos / asin, 0 < p <= 1 for pow(p, 2.2f)) every input
+// where that matters is known: tests/golden/make_cr_hard_cases.py lists each float whose binary64 value lies within 64
+// binary64 ulps of a boundary, with its correctly rounded result (cr_hard_cases.inc: 84 acos, 68 asin, 122 pow).  These
+// routines take their value from that table whenever their own binary64 result lies within kCrTieGuard ulps of a boundary,
+// so they are correctly rounded on all of those domains; without it, acos was wrong on 2 of its 2.13e9 inputs.
+// tests/test_gpu_arith_exhaustive.py compares every input of the domains with the oracle.  Elsewhere (exponents other
+// than 2.2f, tan, atan2, the probes' cr_sin / cr_cos, cr_sincos beyond |a| <= 8) the once-rounded binary64 value is
+// returned, correctly rounded except within ~2 binary64 ulps of a boundary; those inputs are only sampled.
+#include "cr_hard_cases.inc"
+constexpr long long kCrTieGuard = 16;  // binary64 ulps; the oracle's CR_TIE_GUARD (oracle/cr_tie.h)
+
+// distance of |r| from the nearer binary32 rounding boundary around it, in binary64 ulps (the boundary is the mean of
+// two neighbouring floats, exact in binary64, so the one below a power of two is found at a quarter ulp)
+RT_DEV long long cr_tie_dist(double r) {
+  const double a = fabs(r);
+  if (!(a <= 3.4028234663852886e38)) return LLONG_MAX;
+  const float f = __double2float_rn(a);
+  const unsigned fb = __float_as_uint(f);
+  const long long ab = __double_as_longlong(a);
+  long long d = __double_as_longlong(0.5 * ((double)f + (double)__uint_as_float(fb + 1u))) - ab;
+  if (fb != 0u) d = min(d, ab - __double_as_longlong(0.5 * ((double)f + (double)__uint_as_float(fb - 1u))));
+  return d;
+}
+
+// The correctly rounded binary32 value of the binary64 result r of a routine at input x: the once-rounded r, or the table
+// entry of x where r lies within kCrTieGuard binary64 ulps of a rounding boundary.  Where |r| is in the normal binary32
+// range the boundaries inside its binade are where the 29 low mantissa bits read 2^28 (the one just below the next power
+// of two included), so integer operations on the low word filter; the rare rest (and anything below 2^-126) goes out of
+// line to cr_tie_dist and the table, sorted by input bits, in which x is looked up (r rounded once if x is not listed).
+#define RT_NOINLINE __device__ __noinline__
+RT_NOINLINE float cr_hard_case(const uint32_t (*t)[2], int n, float x, double r) {
+  if (cr_tie_dist(r) <= kCrTieGuard) {
+    const uint32_t k = __float_as_uint(x);
+    int lo = 0, hi = n - 1;
+    while (lo <= hi) {
+      const int m = (lo + hi) >> 1;
+      const uint32_t v = t[m][0];
+      if (v == k) return __uint_as_float(t[m][1]);
+      if (v < k) lo = m + 1;
+      else hi = m - 1;
+    }
+  }
+  return __double2float_rn(r);
+}
+RT_DEV float cr_round(const uint32_t (*t)[2], int n, float x, double r) {
+  const unsigned lo = (unsigned)__double2loint(r) & 0x1fffffffu;
+  const bool tiny = (__double2hiint(r) & 0x7fffffff) < 0x38100000;  // |r| < 2^-126
+  if (tiny || lo - (0x10000000u - (unsigned)kCrTieGuard) <= 2u * (unsigned)kCrTieGuard) return cr_hard_case(t, n, x, r);
+  return __double2float_rn(r);
+}
+
 // The binary64 routines are large; they are kept out of line so that the shading code holds one copy of each
 // and stays resident in the instruction cache next to the traversal loop.
-#define RT_NOINLINE __device__ __noinline__
 RT_NOINLINE float cr_sin(float a) { return __double2float_rn(sin((double)a)); }
 RT_NOINLINE float cr_cos(float a) { return __double2float_rn(cos((double)a)); }
 RT_NOINLINE float2 cr_sincos2(float a) {  // (sin, cos), any argument
@@ -62,10 +115,11 @@ RT_NOINLINE float2 cr_sincos2(float a) {  // (sin, cos), any argument
 }
 // The samplers only take sines and cosines of angles in [0, 2·3.14] (MathLib.cl:316,344-345).  For |a| <= 8 the
 // binary64 evaluation is done here directly: Cody–Waite reduction by pi/2 in two parts (exact for |k| <= 6),
-// then the classic minimax kernels on [-pi/4, pi/4] (error < 1 ulp of binary64, i.e. the same class as the
-// library routine: the binary32 rounding of the result is the correctly rounded one unless the true value lies
-// within ~2^-52 relative of a rounding boundary).  A third of the instructions of the general routine and no
-// branches, which matters in a kernel whose lanes are already scattered over material types.
+// then the classic minimax kernels on [-pi/4, pi/4] (error < 1 ulp of binary64).  Its arithmetic is fixed, so its
+// correct rounding is a fact about these 2.18e9 inputs, not an estimate: tests/test_gpu_arith_exhaustive.py compares
+// every one of them with the oracle (0 disagreements; the 120 inputs of the hard-case list are all correctly rounded),
+// and it needs no table.  A third of the instructions of the general routine and no branches, which matters in a kernel
+// whose lanes are already scattered over material types.
 RT_DEV void cr_sincos(float a, float *s, float *c) {
   if (!(fabsf(a) <= 8.0f)) {
     float2 r = cr_sincos2(a);
@@ -97,10 +151,13 @@ RT_DEV void cr_sincos(float a, float *s, float *c) {
   *c = __double2float_rn(((n + 1) & 2) ? -cv : cv);
 }
 RT_NOINLINE float cr_tan(float a) { return __double2float_rn(tan((double)a)); }
-RT_NOINLINE float cr_acos(float a) { return __double2float_rn(acos((double)a)); }
-RT_NOINLINE float cr_asin(float a) { return __double2float_rn(asin((double)a)); }
+RT_NOINLINE float cr_acos(float a) { return cr_round(cr_hard_acos, CR_HARD_ACOS_N, a, acos((double)a)); }
+RT_NOINLINE float cr_asin(float a) { return cr_round(cr_hard_asin, CR_HARD_ASIN_N, a, asin((double)a)); }
 RT_NOINLINE float cr_atan2(float y, float x) { return __double2float_rn(atan2((double)y, (double)x)); }
-RT_NOINLINE float cr_pow(float a, float b) { return __double2float_rn(pow((double)a, (double)b)); }
+RT_NOINLINE float cr_pow(float a, float b) {  // the table holds the exponent 2.2f (the tonemap's) only
+  const double r = pow((double)a, (double)b);
+  return b == 2.2f ? cr_round(cr_hard_pow, CR_HARD_POW_N, a, r) : __double2float_rn(r);
+}
 
 // ---- quaternion rotation, MathLib.cl:51-65 ------------------------------------------------
 RT_HD quat qmul(quat q, quat p) {

@@ -78,13 +78,15 @@ RT_DEV int texel_coord(float a, float inv, int extent) {
   return max(0, min(p, extent - 1));
 }
 
-// The environment lookup needs atan2 / asin only to pick a texel.  The binary32 library routines are within
-// 2 ulp of the true value, so the correctly rounded angle lies within 4 ulp of theirs; texel_coord is monotone,
-// so if both ends of that interval land in the same texel the texel is decided — otherwise (a lookup within
-// ~1e-6 of a texel boundary) the correctly rounded binary64 path is taken.
+// The environment lookup needs atan2 / asin only to pick a texel.  CUDA documents the binary32 atan2f at 3 ulp and asinf
+// at 2 ulp of the true value (measured around every texel boundary of 1x1 .. 8192x4096 maps, and within a few ulp of
+// +-2^k: at most 2 and 1 ulp from the correctly rounded angle, tests/test_gpu_arith_exhaustive.py).  del = |a| 2^-21 is
+// at least 4 ulp of a, so [a - del, a + del] holds the correctly rounded angle; texel_coord is monotone, so if both
+// ends of that interval land in the same texel the texel is decided — otherwise (a lookup within ~1e-6 of a texel
+// boundary) the correctly rounded binary64 path is taken.
 RT_DEV int ibl_texel_u(float z, float x, int w) {
   const float a = atan2f(z, x);
-  const float del = fabsf(a) * 4.76837158203125e-07f;  // 2^-21 >= 4 ulp
+  const float del = fabsf(a) * 4.76837158203125e-07f;  // 2^-21 >= 4 ulp of a
   int p = texel_coord(a - del, 0.1591f, w);
   if (p != texel_coord(a + del, 0.1591f, w)) p = texel_coord(cr_atan2(z, x), 0.1591f, w);
   return p;

@@ -299,8 +299,12 @@ int b200rt_get_stats(const b200rt_ctx *ctx, b200rt_stats *stats);
 /* Device math used by the kernels, exposed so tests can compare it value by value with the oracle:
  * fn 0 sin, 1 cos, 2 acos, 3 asin, 4 atan2(a,b), 5 tan, 6 pow(a,b), 7 a/b, 8 sqrt, 9/10 the samplers' sincos,
  * 11/12 environment-map column of atan2(a,b) by the fast path / by the correctly rounded angle (8192 wide),
- * 13/14 the same for the row of asin(a) (4096 high). */
+ * 13/14 the same for the row of asin(a) (4096 high), 15 whether the column of atan2f(a,b) needs the exact angle (600
+ * wide), 16/17 the binary32 atan2f(a,b) / asinf(a) the fast paths of 11/13 start from. */
 int b200rt_math_probe(b200rt_ctx *ctx, int fn, const float *a, const float *b, int64_t n, float *out);
+
+/* fn 11-14 of b200rt_math_probe for an environment map of any size: `extent` is its width (11/12) or height (13/14). */
+int b200rt_texel_probe(b200rt_ctx *ctx, int fn, const float *a, const float *b, int64_t n, int extent, float *out);
 
 /* Philox4x32-10 block of the device implementation (known-answer tests). */
 int b200rt_philox_probe(b200rt_ctx *ctx, const uint32_t ctr[4], uint32_t key0, uint32_t key1, uint32_t out[4]);

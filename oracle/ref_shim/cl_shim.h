@@ -13,11 +13,18 @@
 //   normalize(v)           v / sqrt(dot(v,v))   (true divisions)
 //   cos sin tan acos asin atan2 powr
 //                          CORRECTLY ROUNDED binary32: evaluated by the host
-//                          libm in binary64 and rounded once to binary32.
-//                          (glibc's binary64 functions are < 1 ulp, so the
-//                          single rounding is the correctly-rounded float
-//                          except when the double lies within ~1e-16
-//                          relative of a float rounding boundary, p ~ 2^-28.)
+//                          libm in binary64 and rounded once to binary32;
+//                          where that value lies within CR_TIE_GUARD binary64
+//                          ulps of a binary32 rounding boundary (../cr_tie.h)
+//                          cos / sin (|x| <= 8), acos, asin and powr(x, 2.2f)
+//                          are evaluated again in x87 extended precision and
+//                          that is rounded.  Checked against mpmath on every
+//                          float of those domains (tests/test_cr_hard_cases.py;
+//                          the once-rounded binary64 value alone was wrong on
+//                          2 of 2.13e9 acos inputs, 0 elsewhere).  tan and
+//                          atan2 are the once-rounded binary64 value, wrong
+//                          only within ~1 binary64 ulp of a boundary; sampled.
+//                          Same rule as oracle/rt_oracle.c.
 //                          Correct rounding is the one definition every
 //                          conforming implementation — CPU or GPU — can meet
 //                          independently, which is what makes a bit-exact
@@ -34,6 +41,8 @@
 #include <cmath>
 #include <cstdint>
 #include <cstring>
+
+#include "../cr_tie.h"
 
 namespace clref {
 
@@ -71,13 +80,28 @@ static inline float asin(float x) { return ::asinf(x); }
 static inline float atan2(float y, float x) { return ::atan2f(y, x); }
 static inline float powr(float x, float y) { return ::powf(x, y); }
 #else
-static inline float cos(float x) { return (float)::cos((double)x); }
-static inline float sin(float x) { return (float)::sin((double)x); }
+static inline float cos(float x) {
+  const double r = ::cos((double)x);
+  return (::fabsf(x) <= 8.0f && cr_tie_dist(r) <= CR_TIE_GUARD) ? (float)::cosl((long double)x) : (float)r;
+}
+static inline float sin(float x) {
+  const double r = ::sin((double)x);
+  return (::fabsf(x) <= 8.0f && cr_tie_dist(r) <= CR_TIE_GUARD) ? (float)::sinl((long double)x) : (float)r;
+}
 static inline float tan(float x) { return (float)::tan((double)x); }
-static inline float acos(float x) { return (float)::acos((double)x); }
-static inline float asin(float x) { return (float)::asin((double)x); }
+static inline float acos(float x) {
+  const double r = ::acos((double)x);
+  return cr_tie_dist(r) <= CR_TIE_GUARD ? (float)::acosl((long double)x) : (float)r;
+}
+static inline float asin(float x) {
+  const double r = ::asin((double)x);
+  return cr_tie_dist(r) <= CR_TIE_GUARD ? (float)::asinl((long double)x) : (float)r;
+}
 static inline float atan2(float y, float x) { return (float)::atan2((double)y, (double)x); }
-static inline float powr(float x, float y) { return (float)::pow((double)x, (double)y); }
+static inline float powr(float x, float y) {
+  const double r = ::pow((double)x, (double)y);
+  return (y == 2.2f && cr_tie_dist(r) <= CR_TIE_GUARD) ? (float)::powl((long double)x, (long double)y) : (float)r;
+}
 #endif
 static inline float sqrt(float x) { return ::sqrtf(x); }
 static inline float fabs(float x) { return ::fabsf(x); }

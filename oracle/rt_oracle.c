@@ -34,6 +34,8 @@
 #include <stdint.h>
 #include <stdlib.h>
 #include <string.h>
+
+#include "cr_tie.h"
 #ifdef _OPENMP
 #include <omp.h>
 #endif
@@ -42,13 +44,33 @@ typedef struct { float x, y, z; } v3;
 typedef struct { float w, x, y, z; } quat;
 
 /* ---- correctly-rounded binary32 transcendentals ------------------------------------ */
-static inline float cr_cos(float a) { return (float)cos((double)a); }
-static inline float cr_sin(float a) { return (float)sin((double)a); }
+/* glibc's binary64 value rounded once; where it lies within CR_TIE_GUARD binary64 ulps of a binary32 rounding boundary
+ * (cr_tie.h) it is evaluated again in x87 extended precision and that is rounded instead.  Done on the domains on which
+ * the kernels are correctly rounded (every float with |a| <= 8 for sin / cos, all of acos / asin, pow with the exponent
+ * 2.2f; tests/test_cr_hard_cases.py checks every input the guard catches against mpmath); elsewhere the once-rounded
+ * binary64 value, as on the GPU.  ref_shim/cl_shim.h states the same rule. */
+static inline float cr_cos(float a) {
+  const double r = cos((double)a);
+  return (fabsf(a) <= 8.0f && cr_tie_dist(r) <= CR_TIE_GUARD) ? (float)cosl((long double)a) : (float)r;
+}
+static inline float cr_sin(float a) {
+  const double r = sin((double)a);
+  return (fabsf(a) <= 8.0f && cr_tie_dist(r) <= CR_TIE_GUARD) ? (float)sinl((long double)a) : (float)r;
+}
 static inline float cr_tan(float a) { return (float)tan((double)a); }
-static inline float cr_acos(float a) { return (float)acos((double)a); }
-static inline float cr_asin(float a) { return (float)asin((double)a); }
+static inline float cr_acos(float a) {
+  const double r = acos((double)a);
+  return cr_tie_dist(r) <= CR_TIE_GUARD ? (float)acosl((long double)a) : (float)r;
+}
+static inline float cr_asin(float a) {
+  const double r = asin((double)a);
+  return cr_tie_dist(r) <= CR_TIE_GUARD ? (float)asinl((long double)a) : (float)r;
+}
 static inline float cr_atan2(float y, float x) { return (float)atan2((double)y, (double)x); }
-static inline float cr_pow(float a, float b) { return (float)pow((double)a, (double)b); }
+static inline float cr_pow(float a, float b) {
+  const double r = pow((double)a, (double)b);
+  return (b == 2.2f && cr_tie_dist(r) <= CR_TIE_GUARD) ? (float)powl((long double)a, (long double)b) : (float)r;
+}
 
 /* ---- small vector algebra (every product and sum rounded separately) ---------------- */
 static inline v3 V(float x, float y, float z) { v3 r = {x, y, z}; return r; }
