@@ -36,7 +36,11 @@ Differences a caller can observe (all documented in INTEGRATION.md):
   * `pixel_jitter = True` anti-aliases: every sample traces its own camera ray through a jittered point of its pixel
     (B200RT_SAMPLING_PIXEL_JITTER), so the image converges to the pixel-area average instead of the reference's one
     point per pixel.  B200RT_PIXEL_JITTER=1 (or 0) sets it for callers that never touch the attribute.  It cannot be
-    combined with `adaptive`.
+    combined with `adaptive`;
+  * `smooth_normals = True` shades every hit with the interpolation of its triangle's three vertex normals instead of
+    the first vertex's (B200RT_SAMPLING_SMOOTH_NORMALS), so smooth meshes no longer render as facets.
+    B200RT_SMOOTH_NORMALS=1 (or 0) sets it for callers that never touch the attribute.  It combines with `adaptive`,
+    `denoise`, `pixel_jitter` and `cuda_devices`.
 """
 import math
 import os
@@ -102,6 +106,14 @@ def pixel_jitter_from_env(text):
     return t == "1"
 
 
+def smooth_normals_from_env(text):
+    """The `smooth_normals` flag that B200RT_SMOOTH_NORMALS=0 or =1 stands for; ValueError otherwise."""
+    t = str(text).strip()
+    if t not in ("0", "1"):
+        raise ValueError(f"B200RT_SMOOTH_NORMALS={text!r}: expected 0 or 1")
+    return t == "1"
+
+
 class KernelLauncher(object):
 
     def __init__(self, context=None, platform=None, device=None, queue=None, cuda_device=0, cuda_devices=None):
@@ -133,6 +145,9 @@ class KernelLauncher(object):
         # False: one camera ray per pixel (the reference's image); True: anti-aliasing (module docstring)
         self.pixel_jitter = (pixel_jitter_from_env(os.environ["B200RT_PIXEL_JITTER"])
                              if os.environ.get("B200RT_PIXEL_JITTER") else False)
+        # False: the first vertex's normal (the reference's faceted shading); True: smooth shading (module docstring)
+        self.smooth_normals = (smooth_normals_from_env(os.environ["B200RT_SMOOTH_NORMALS"])
+                               if os.environ.get("B200RT_SMOOTH_NORMALS") else False)
         self.last_spp = None
         self.last_stats = None
         self._warned_deep = False
@@ -184,7 +199,8 @@ class KernelLauncher(object):
                 self._warned_deep = True
         opts = _capi.make_opts(rng_mode=self.rng_mode, traversal=traversal, stack_cap=self.stack_cap,
                                seed=self.seed, collect_stats=self.collect_stats, sample_streams=self.sample_streams,
-                               sampling=_capi.SAMPLING_PIXEL_JITTER if self.pixel_jitter else _capi.SAMPLING_REFERENCE)
+                               sampling=((_capi.SAMPLING_PIXEL_JITTER if self.pixel_jitter else 0) |
+                                         (_capi.SAMPLING_SMOOTH_NORMALS if self.smooth_normals else 0)))
         out = h_img_out.reshape(-1)[:imgDim * 3]
         if self.adaptive is not None:
             img, self.last_spp, _ = self._ctx.render_adaptive(cam[:10], h_envData, width, height, int(spp), int(maxBounce),

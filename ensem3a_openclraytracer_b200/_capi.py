@@ -18,6 +18,7 @@ TRAVERSAL_FAST, TRAVERSAL_REFERENCE, TRAVERSAL_VERIFY = 0, 1, 2
 OUT_FINAL, OUT_SUMS = 0, 1
 SAMPLING_REFERENCE, SAMPLING_IMPORTANCE, SAMPLING_LIGHTS = 0, 1, 2
 SAMPLING_PIXEL_JITTER = 8   # anti-aliasing: changes the integrand to the pixel's area (include/b200rt.h)
+SAMPLING_SMOOTH_NORMALS = 32   # smooth shading: the interpolated vertex normal at the hit (include/b200rt.h)
 
 
 class B200RTError(RuntimeError):

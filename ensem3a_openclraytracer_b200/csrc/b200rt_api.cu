@@ -381,14 +381,21 @@ int prepare_trace_t(b200rt_ctx *c, WaveLaunch *w) {
 }
 
 // jitter and adaptive are never both set (b200rt_render_adaptive refuses the jitter bit)
-int prepare_wave(b200rt_ctx *c, int trav, bool smem, bool stats, bool nee, bool adaptive, bool jitter, WaveLaunch *w) {
+template <bool SMOOTH>
+void pick_shade(bool nee, bool adaptive, bool jitter, WaveLaunch *w) {
+  if (jitter) w->shade = nee ? k_shade<true, false, true, SMOOTH> : k_shade<false, false, true, SMOOTH>;
+  else if (nee) w->shade = adaptive ? k_shade<true, true, false, SMOOTH> : k_shade<true, false, false, SMOOTH>;
+  else w->shade = adaptive ? k_shade<false, true, false, SMOOTH> : k_shade<false, false, false, SMOOTH>;
+}
+
+int prepare_wave(b200rt_ctx *c, int trav, bool smem, bool stats, bool nee, bool adaptive, bool jitter, bool smooth,
+                 WaveLaunch *w) {
   int per_sm = 0;
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shade<false, false>, kShadeBlock, 0));
   if (per_sm < 1) return fail(c, B200RT_ERR_CUDA, "k_shade does not fit on an SM");
   w->shade_grid = per_sm * c->sm_count;
-  if (jitter) w->shade = nee ? k_shade<true, false, true> : k_shade<false, false, true>;
-  else if (nee) w->shade = adaptive ? k_shade<true, true> : k_shade<true, false>;
-  else w->shade = adaptive ? k_shade<false, true> : k_shade<false, false>;
+  if (!smooth) pick_shade<false>(nee, adaptive, jitter, w);
+  else pick_shade<true>(nee, adaptive, jitter, w);
   return with_variant(c, trav, smem, stats, [&](auto t, auto s, auto st) {
     return prepare_trace_t<decltype(t)::value, decltype(s)::value, decltype(st)::value>(c, w);
   });
@@ -500,7 +507,8 @@ int check_frame_args(b200rt_ctx *c, const float *cam, int width, int height, int
     return fail(c, B200RT_ERR_INVALID, "bad rng_mode %d", o.rng_mode);
   if (o.traversal < 0 || o.traversal > 2) return fail(c, B200RT_ERR_INVALID, "bad traversal %d", o.traversal);
   if (o.sampling < 0 ||
-      (o.sampling & ~(B200RT_SAMPLING_IMPORTANCE | B200RT_SAMPLING_LIGHTS | B200RT_SAMPLING_PIXEL_JITTER)) != 0)
+      (o.sampling & ~(B200RT_SAMPLING_IMPORTANCE | B200RT_SAMPLING_LIGHTS | B200RT_SAMPLING_PIXEL_JITTER |
+                      B200RT_SAMPLING_SMOOTH_NORMALS)) != 0)
     return fail(c, B200RT_ERR_INVALID, "bad sampling mode %d", o.sampling);
   if (o.output != B200RT_OUT_FINAL && o.output != B200RT_OUT_SUMS)
     return fail(c, B200RT_ERR_INVALID, "bad output mode %d", o.output);
@@ -518,6 +526,16 @@ int check_frame_args(b200rt_ctx *c, const float *cam, int width, int height, int
     return fail(c, B200RT_ERR_INVALID, "bad tile row split %d mod %d", o.tile_row_rem, o.tile_row_mod);
   if (o.pixel_end > 0 && (o.pixel_begin < 0 || o.pixel_begin >= o.pixel_end || o.pixel_end > width * height))
     return fail(c, B200RT_ERR_INVALID, "bad pixel range [%d,%d)", o.pixel_begin, o.pixel_end);
+  return 0;
+}
+
+// Smooth shading reads all three vertex normals, of which b200rt_set_scene validates the first only: a frame with the bit
+// refuses a scene that has an out-of-range n1 / n2 index.
+int check_smooth_scene(b200rt_ctx *c, const b200rt_opts &o) {
+  if ((o.sampling & B200RT_SAMPLING_SMOOTH_NORMALS) && c->scene.smooth_bad >= 0)
+    return fail(c, B200RT_ERR_INVALID,
+                "B200RT_SAMPLING_SMOOTH_NORMALS: triangle %d has a vertex-normal index (faceData[10t+5 .. 10t+6]) out of "
+                "range", c->scene.smooth_bad);
   return 0;
 }
 
@@ -539,6 +557,7 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   // with pixel jitter every sample also traces its own camera ray: one more
   const bool nee = (o.sampling & B200RT_SAMPLING_LIGHTS) != 0 && c->n_light > 0;
   const bool jitter = (o.sampling & B200RT_SAMPLING_PIXEL_JITTER) != 0;
+  const bool smooth = (o.sampling & B200RT_SAMPLING_SMOOTH_NORMALS) != 0;
   const long long per_sample = (nee ? 2 * ((long long)max_bounce + 1) + 1 : (long long)max_bounce + 2) + (jitter ? 1 : 0);
   const long long n_iter_ll = (long long)(F.s1 - F.s0) * per_sample;
   if (n_iter_ll > (1 << 22)) return fail(c, B200RT_ERR_UNSUPPORTED, "%lld wavefront iterations exceed 2^22", n_iter_ll);
@@ -570,7 +589,7 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   A.validate = (trav == B200RT_TRAVERSAL_FAST) ? 1 : 0;
   const bool smem = use_smem_scene(c);
   WaveLaunch wl;
-  int rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, jitter, &wl);
+  int rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, jitter, smooth, &wl);
   if (rc) return rc;
   if (ensure(c, c->d_part_count, (size_t)wl.shade_grid * sizeof(unsigned int))) return B200RT_ERR_CUDA;
   A.part_count = static_cast<unsigned int *>(c->d_part_count.p);
@@ -811,6 +830,7 @@ int render_frame(b200rt_ctx *c, const float *cam, const float *env, int width, i
   if (o.sample_streams < -1 || o.sample_streams > 16)
     return fail(c, B200RT_ERR_INVALID, "bad sample_streams %d (-1 automatic, 0 / 1 off, up to 16)", o.sample_streams);
   int rc = check_frame_args(c, cam, width, height, spp, max_bounce, o, true, env);
+  if (!rc) rc = check_smooth_scene(c, o);
   if (rc) return rc;
   if (!c->have_ibl) return fail(c, B200RT_ERR_NO_SCENE, "no environment map: call b200rt_set_ibl first");
   int s0 = o.sample_begin, s1 = o.sample_end;
@@ -1043,7 +1063,8 @@ int upload_scene(b200rt_ctx *c, const Repacked &R, const SceneArgs &a, uint64_t 
   CU(cudaSetDevice(c->device));
   if (ensure(c, B[kTris], R.tris.size() * sizeof(float4))) return B200RT_ERR_CUDA;
   if (ensure(c, B[kCtris], R.ctris.size() * sizeof(float4))) return B200RT_ERR_CUDA;
-  if (ensure(c, B[kNormals], R.normals.size() * sizeof(float4))) return B200RT_ERR_CUDA;
+  // the first-vertex normals, then the other two vertex normals of opt-in smooth shading (rt_trace.cuh)
+  if (ensure(c, B[kNormals], (R.normals.size() + R.nsmooth.size()) * sizeof(float4))) return B200RT_ERR_CUDA;
   if (ensure(c, B[kTboxes], R.tboxes.size() * sizeof(float4))) return B200RT_ERR_CUDA;
   if (ensure(c, B[kFrames], (size_t)n_tris * kFrameVec * sizeof(float4))) return B200RT_ERR_CUDA;
   if (ensure(c, B[kNodes], R.nodes.size() * sizeof(uint4))) return B200RT_ERR_CUDA;
@@ -1053,6 +1074,8 @@ int upload_scene(b200rt_ctx *c, const Repacked &R, const SceneArgs &a, uint64_t 
   CU(cudaMemcpyAsync(B[kTris].p, R.tris.data(), R.tris.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
   CU(cudaMemcpyAsync(B[kCtris].p, R.ctris.data(), R.ctris.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
   CU(cudaMemcpyAsync(B[kNormals].p, R.normals.data(), R.normals.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(static_cast<float4 *>(B[kNormals].p) + R.normals.size(), R.nsmooth.data(), R.nsmooth.size() * sizeof(float4),
+                     cudaMemcpyHostToDevice, c->stream));
   CU(cudaMemcpyAsync(B[kTboxes].p, R.tboxes.data(), R.tboxes.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
   if (!R.nodes.empty())
     CU(cudaMemcpyAsync(B[kNodes].p, R.nodes.data(), R.nodes.size() * sizeof(uint4), cudaMemcpyHostToDevice, c->stream));
@@ -1161,8 +1184,9 @@ int launch_gbuffer(b200rt_ctx *c, const float *cam, int width, int height, const
   float *k = static_cast<float *>(c->d_dn_k.p);
   int rc = launch_primary(c, A, effective_traversal(c, og), use_smem_scene(c), true, og.collect_stats != 0, tri, k);
   if (rc) return rc;
-  k_gbuffer<<<(unsigned)((npix + kBlock - 1) / kBlock), kBlock, 0, c->stream>>>(A, tri, k, gbuffer_view(c), d_rgb,
-                                                                                 static_cast<float4 *>(c->d_dn_col[0].p));
+  auto kg = (o.sampling & B200RT_SAMPLING_SMOOTH_NORMALS) ? k_gbuffer<true> : k_gbuffer<false>;
+  kg<<<(unsigned)((npix + kBlock - 1) / kBlock), kBlock, 0, c->stream>>>(A, tri, k, gbuffer_view(c), d_rgb,
+                                                                          static_cast<float4 *>(c->d_dn_col[0].p));
   CU(cudaGetLastError());
   c->stats.kernel_launches++;
   return 0;
@@ -1366,6 +1390,7 @@ int b200rt_gbuffer(b200rt_ctx *c, const float *cam, int width, int height, const
   int rc = check_frame_args(c, cam, width, height, 1, 0, o, false, nullptr);
   if (!rc && (o.pixel_end > 0 || o.tile_row_mod > 1))
     rc = fail(c, B200RT_ERR_INVALID, "the G-buffer covers the whole frame: no pixel range or tile rows");
+  if (!rc) rc = check_smooth_scene(c, o);
   if (rc) return rc;
   CU(cudaSetDevice(c->device));
   const size_t npix = (size_t)width * height;

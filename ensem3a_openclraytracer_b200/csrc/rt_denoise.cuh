@@ -21,6 +21,9 @@ struct GBufferView {
   float4 *gn, *gx, *ga;
 };
 
+// SMOOTH (B200RT_SAMPLING_SMOOTH_NORMALS): the normal of a hit on a curved triangle is the normalised shading normal at
+// the render's point cam_pos + unit(d) * k
+template <bool SMOOTH>
 __global__ void __launch_bounds__(kBlock) k_gbuffer(const __grid_constant__ KernelArgs A, const int *__restrict__ tri,
                                                     const float *__restrict__ k, GBufferView G,
                                                     const float *__restrict__ rgb, float4 *__restrict__ col) {
@@ -38,6 +41,15 @@ __global__ void __launch_bounds__(kBlock) k_gbuffer(const __grid_constant__ Kern
     const float4 f0 = __ldg(S.frames + (size_t)kFrameVec * t);   // normalize(first-vertex normal), k_tri_frames
     if (isfinite(f0.x) && isfinite(f0.y) && isfinite(f0.z)) nrm = mk3(f0.x, f0.y, f0.z);
     const v3 d = camera_dir(A.F, i);
+    if (SMOOTH) {
+      const float4 nn = __ldg(S.normals + t);
+      bool curved;
+      const v3 n = shading_normal<true>(S, A.n_tris, t, mk3(nn.x, nn.y, nn.z), A.F.cam_pos + unit(d) * __ldg(k + i), &curved);
+      if (curved) {
+        const v3 un = unit(n);
+        nrm = (isfinite(un.x) && isfinite(un.y) && isfinite(un.z)) ? un : mk3(0.0f, 0.0f, 0.0f);
+      }
+    }
     pos = A.F.cam_pos + d * __ldg(k + i);
   }
   G.gn[i] = make_float4(nrm.x, nrm.y, nrm.z, kind);

@@ -398,6 +398,34 @@ __global__ void __launch_bounds__(kCompactBlock) k_compact(const int *__restrict
   }
 }
 
+// ---- opt-in smooth shading (b200rt_opts.sampling bit B200RT_SAMPLING_SMOOTH_NORMALS) ---------------------------------
+// The shading normal of a hit on triangle `tri` at point x, by the rule b200rt.h states: n0 (the normals record) for a
+// flat triangle, else the normalised barycentric interpolation of n0, n1, n2, or n0 when that is not a usable direction.  The
+// normals buffer holds n_tris first-vertex normals, then 2 float4 per triangle: (n1.xyz, flat / curved flag), (n2.xyz, -)
+// (scene_repack.h).  *curved: the triangle is not flat, so its precomputed frame does not apply and tri_frame_at builds
+// one.
+template <bool SMOOTH>
+RT_DEV v3 shading_normal(const SceneView &S, int n_tris, int tri, v3 n0, v3 x, bool *curved) {
+  *curved = false;
+  if (!SMOOTH) return n0;
+  const float4 *nsmooth = S.normals + n_tris;
+  const float4 c1 = __ldg(nsmooth + 2 * (size_t)tri);
+  if (!(c1.w > 0.0f)) return n0;   // flat (scene_repack.h kSmoothFlat; kSmoothBadIndex never reaches a render)
+  *curved = true;
+  const float4 c2 = __ldg(nsmooth + 2 * (size_t)tri + 1);
+  const Tri t = load_tri(S.tris, tri);
+  const v3 p = x - t.A;
+  const float d00 = dot(t.e1, t.e1), d01 = dot(t.e1, t.e2), d11 = dot(t.e2, t.e2);
+  const float d20 = dot(p, t.e1), d21 = dot(p, t.e2);
+  const float den = d00 * d11 - d01 * d01;
+  const float b1 = (d11 * d20 - d01 * d21) / den;
+  const float b2 = (d00 * d21 - d01 * d20) / den;
+  const float b0 = (1.0f - b1) - b2;
+  const v3 n = unit(((n0 * b0) + (mk3(c1.x, c1.y, c1.z) * b1)) + (mk3(c2.x, c2.y, c2.z) * b2));
+  if (!isfinite(n.x) || !isfinite(n.y) || !isfinite(n.z) || !(dot(n, n) > 0.0f)) return n0;
+  return n;
+}
+
 // ---- shading ----------------------------------------------------------------------------------------------------
 // The per-path state machine is written as a sequence of phases with the warp re-converged between them, so that
 // e.g. the direction sampling runs once per warp for every lane that needs it, whichever way the lane got there
@@ -407,8 +435,10 @@ __global__ void __launch_bounds__(kCompactBlock) k_compact(const int *__restrict
 // estimator runs exactly the code it ran before.  ADAPT = adaptive sampling (adaptive_end_sample at the end of every
 // sample), likewise a separate instantiation.  JITTER = opt-in pixel jitter (sampling bit B200RT_SAMPLING_PIXEL_JITTER):
 // a sample starts with a camera ray through a jittered point of its pixel (phase 3), which phase 2 resolves the way
-// k_primary resolves the cached primary ray, instead of from the cached primary hit.
-template <bool NEE, bool ADAPT, bool JITTER = false>
+// k_primary resolves the cached primary ray, instead of from the cached primary hit.  SMOOTH = opt-in smooth shading
+// (B200RT_SAMPLING_SMOOTH_NORMALS): a hit on a curved triangle is shaded with the interpolated normal and a frame built
+// in registers (shading_normal, tri_frame_at); a flat one keeps its precomputed frame.
+template <bool NEE, bool ADAPT, bool JITTER = false, bool SMOOTH = false>
 __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant__ KernelArgs A, int iter) {
   const FrameParams &F = A.F;
   const SceneView &S = A.S;
@@ -610,9 +640,9 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
     // ---- phase 3b (light sampling only): one emitter point seen from the surface, and the shadow ray towards it --------------
     if (NEE && want_light) {
       const float4 nn = __ldg(S.normals + htri);
-      const v3 n = mk3(nn.x, nn.y, nn.z);
+      v3 n = mk3(nn.x, nn.y, nn.z);
       const Material m = load_material(S.mats, tri_material(S, htri));
-      const v3 un = unit(n);
+      v3 un = unit(n);
       float ul, ua, ub;
       if (F.rng_mode == 0) draw3_light<0>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, F.key0, F.key1, &ul, &ua, &ub);
       else draw3_light<1>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, F.key0, F.key1, &ul, &ua, &ub);
@@ -623,6 +653,11 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
       const Material ml = load_material(S.mats, l.mat);
       const float Le = ml.type == 0 ? ml.roughness : 0.0f;
       const v3 x = o + unit(d) * hk;
+      if (SMOOTH) {
+        bool curved;
+        n = shading_normal<true>(S, A.n_tris, htri, n, x, &curved);
+        un = unit(n);
+      }
       v3 w;
       const v3 direct = sample_light(m, F.sampling, n, un, x, d, acc, l.A, l.e1, l.e2, Le, A.n_light, ua, ub, &w);
       A.pS[pix] = make_float4(d.x, d.y, d.z, __int_as_float(htri));
@@ -636,9 +671,11 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
     // ---- phase 4: next direction, BRDF * cos / pdf (:51-87); segment = (o, d, hk, htri) ------------------------------------------
     if (shade) {
       const float4 nn = __ldg(S.normals + htri);
-      const v3 n = mk3(nn.x, nn.y, nn.z);
+      bool curved;   // the surface point: o itself when the light ray is back at it (phase 3b moved o there)
+      const v3 n = shading_normal<SMOOTH>(S, A.n_tris, htri, mk3(nn.x, nn.y, nn.z), (NEE && from_light) ? o : o + unit(d) * hk, &curved);
       const Material m = load_material(S.mats, tri_material(S, htri));
-      const TriFrame tf = load_tri_frame(S.frames, htri, m.type == 3 ? 0 : (m.type == 1 ? 1 : 2));
+      const int which = m.type == 3 ? 0 : (m.type == 1 ? 1 : 2);
+      const TriFrame tf = curved ? tri_frame_at(n, which) : load_tri_frame(S.frames, htri, which);
       v3 nd, brdf;
       float inv_pdf;
       if (m.type == 3) {

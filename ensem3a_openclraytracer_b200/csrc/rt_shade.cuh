@@ -156,6 +156,25 @@ RT_DEV TriFrame load_tri_frame(const float4 *frames, int tri, int which) {
   return T;
 }
 
+// opt-in smooth shading (B200RT_SAMPLING_SMOOTH_NORMALS): load_tri_frame's result for a normal known only at the hit,
+// make_tri_frame's statements in registers.  Glass (which 0) needs the unit normal alone.
+RT_DEV TriFrame tri_frame_at(v3 n, int which) {
+  TriFrame T;
+  if (which == 0) {
+    T.un = unit(n);
+    T.zal = false;
+    return T;
+  }
+  float4 f[kFrameVec];
+  make_tri_frame(n, f);
+  T.un = mk3(f[0].x, f[0].y, f[0].z);
+  T.zal = f[0].w != 0.0f;
+  const float4 a = which == 1 ? f[1] : f[3], b = which == 1 ? f[2] : f[4];
+  T.rot.q.w = a.x; T.rot.q.x = a.y; T.rot.q.y = a.z; T.rot.q.z = a.w;
+  T.rot.qi.w = b.x; T.rot.qi.x = b.y; T.rot.qi.y = b.z; T.rot.qi.z = b.w;
+  return T;
+}
+
 // MathLib.cl:313-339
 RT_DEV v3 sample_cosine(v3 n, const TriFrame &T, float u, float u2, float *inv_pdf) {
   float theta = u2 * 2.0f * 3.14f;

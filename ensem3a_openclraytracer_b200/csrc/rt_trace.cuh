@@ -56,7 +56,8 @@ namespace b200rt {
 // triangle (48 B, 3 x float4):
 //   t0 = A.x A.y A.z e1.x     t1 = e1.y e1.z e2.x e2.y     t2 = e2.z mat rank -   (mat, rank int bits)
 //   with e1 = B - A, e2 = C - A rounded exactly as MathLib.cl:129-130 rounds them.
-// normal (16 B): first-vertex normal of the triangle (MathLib.cl:151), w unused.
+// normal (16 B): first-vertex normal of the triangle (MathLib.cl:151), w unused.  The normals buffer continues with 2 x
+// float4 per triangle, read by smooth-shaded renders only: n1.xyz flag   n2.xyz -   (scene_repack.h kSmooth*).
 // leaf box (32 B, 2 x float4): min.xyz -, max.xyz -   of the leaf that holds the triangle (validate_hit).
 struct SceneView {
   const uint4 *nodes;

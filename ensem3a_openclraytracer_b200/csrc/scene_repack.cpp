@@ -105,13 +105,15 @@ int repack_scene(const float *vp, int64_t n_vp, const float *vn, int64_t n_vn, c
   // ---- triangles: validate indices, precompute edges exactly as MathLib.cl:129-130 rounds them ------------------
   R.tris.resize((size_t)n_tris * 3);
   R.normals.resize((size_t)n_tris);
+  R.nsmooth.resize((size_t)n_tris * 2);
   R.tboxes.resize((size_t)n_tris * 2);
   R.tri_mat.resize((size_t)n_tris);
   float cmax = 0.0f;
   int first_bad = n_tris;   // first triangle with an out-of-range index
+  int smooth_bad = n_tris;  // first triangle with an out-of-range n1 / n2 index (refused by smooth-shaded renders only)
   int nonfinite = 0;
   const float unranked = as_float(0x7fffffffu);
-#pragma omp parallel for schedule(static) reduction(max : cmax) reduction(min : first_bad) reduction(| : nonfinite)
+#pragma omp parallel for schedule(static) reduction(max : cmax) reduction(min : first_bad, smooth_bad) reduction(| : nonfinite)
   for (int t = 0; t < n_tris; ++t) {
     const int32_t *f = face + 10 * (size_t)t;
     bool ok = f[4] >= 0 && f[4] < nvn && f[0] >= 0 && f[0] < nm;
@@ -128,6 +130,17 @@ int repack_scene(const float *vp, int64_t n_vp, const float *vn, int64_t n_vn, c
     R.tris[3 * (size_t)t + 2] = Repacked::f4{e2z, as_float((uint32_t)f[0]), unranked, 0.0f};
     const float *n0 = vn + 3 * (size_t)f[4];
     R.normals[t] = Repacked::f4{n0[0], n0[1], n0[2], 0.0f};
+    // opt-in smooth shading: the other two vertex normals and whether the triangle is curved (b200rt.h)
+    if (f[5] >= 0 && f[5] < nvn && f[6] >= 0 && f[6] < nvn) {
+      const float *n1 = vn + 3 * (size_t)f[5], *n2 = vn + 3 * (size_t)f[6];
+      const bool flat = memcmp(n0, n1, 3 * sizeof(float)) == 0 && memcmp(n0, n2, 3 * sizeof(float)) == 0;
+      R.nsmooth[2 * (size_t)t] = Repacked::f4{n1[0], n1[1], n1[2], flat ? kSmoothFlat : kSmoothCurved};
+      R.nsmooth[2 * (size_t)t + 1] = Repacked::f4{n2[0], n2[1], n2[2], 0.0f};
+    } else {
+      R.nsmooth[2 * (size_t)t] = Repacked::f4{0.0f, 0.0f, 0.0f, kSmoothBadIndex};
+      R.nsmooth[2 * (size_t)t + 1] = Repacked::f4{0.0f, 0.0f, 0.0f, 0.0f};
+      if (t < smooth_bad) smooth_bad = t;
+    }
     R.tboxes[2 * (size_t)t] = Repacked::f4{0, 0, 0, 0};   // stays empty if no leaf holds the triangle
     R.tboxes[2 * (size_t)t + 1] = Repacked::f4{0, 0, 0, 0};
     R.tri_mat[t] = f[0];
@@ -152,6 +165,7 @@ int repack_scene(const float *vp, int64_t n_vp, const float *vn, int64_t n_vn, c
     *err = fmt("triangle %lld: material %lld out of range [0,%lld)", first_bad, f[0], nm);
     return B200RT_ERR_INVALID;
   }
+  R.smooth_bad = smooth_bad < n_tris ? smooth_bad : -1;
   double t1 = now_ms();
   R.ms_tris = t1 - t0;
 

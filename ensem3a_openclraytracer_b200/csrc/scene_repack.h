@@ -36,13 +36,20 @@ struct SceneDesc {
   float cull_abs = 0.0f, cmax = 0.0f;
   int fast_ok = 0;
   float root_box[6] = {0, 0, 0, 0, 0, 0};  // the caller's root box, bvh[2..7] (min.xyz, max.xyz): the denoiser's scale
+  int smooth_bad = -1;          // first triangle whose n1 or n2 index is out of range: smooth-shaded renders refuse it
 };
+
+// .w of the first `nsmooth` record of a triangle (opt-in smooth shading, b200rt.h B200RT_SAMPLING_SMOOTH_NORMALS)
+constexpr float kSmoothFlat = 0.0f;       // n0 = n1 = n2 bit for bit: shaded with n0 and its precomputed frame
+constexpr float kSmoothCurved = 1.0f;     // the interpolated normal, its frame built at the hit
+constexpr float kSmoothBadIndex = -1.0f;  // n1 or n2 index out of range (SceneDesc::smooth_bad)
 
 struct Repacked : SceneDesc {
   struct f4 { float x, y, z, w; };
   struct u4 { uint32_t x, y, z, w; };
   raw_vector<u4> nodes;         // node_f4 x 16 bytes per interior node (rt_trace.cuh "repacked scene")
   raw_vector<f4> tris, normals, tboxes;
+  raw_vector<f4> nsmooth;       // 2 per triangle: (n1.xyz, kSmooth* flag), (n2.xyz, 0)
   raw_vector<f4> ctris;         // the triangle records in the order of the culling tree's leaves (what leaf refs index); .w of the
                                 // third vector = the triangle's id
   std::vector<int32_t> tri_mat;

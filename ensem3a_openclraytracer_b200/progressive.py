@@ -11,7 +11,8 @@ instead of sample by sample): relative difference ~1e-7 per addition, far inside
 edge-avoiding à-trous filter of include/b200rt.h, with the G-buffer computed once, on the first slice.  The saved state
 (`sums`, `done`) stays undenoised, so a resumed render denoises the same way.
 
-`sampling` (a mask of the SAMPLING_* bits, e.g. SAMPLING_PIXEL_JITTER) goes into every slice's options.
+`sampling` (a mask of the SAMPLING_* bits, e.g. SAMPLING_PIXEL_JITTER) goes into every slice's options and into the
+denoiser's G-buffer (with SAMPLING_SMOOTH_NORMALS its normal is the interpolated one).
 """
 import numpy as np
 
@@ -45,7 +46,7 @@ class ProgressiveRender:
         if self.denoise is None:
             return img
         if self._gb is None:
-            self._gb = self.ctx.gbuffer(self.cam, self.width, self.height)
+            self._gb = self.ctx.gbuffer(self.cam, self.width, self.height, opts=_capi.make_opts(sampling=self.sampling))
         return self.ctx.denoise(img, self._gb, **self.denoise).reshape(-1)
 
     def __iter__(self):

@@ -56,7 +56,7 @@ typedef enum {
 /* Anti-aliasing: every sample traces its own camera ray through a jittered point of its pixel.  Unlike bits 0 and 1
  * this bit CHANGES THE INTEGRAND: the image converges to the box-filtered (pixel-area) image, no longer to the
  * reference's, whose pixel is one point (one camera ray per pixel, whose hit every sample restarts from,
- * Raytracing.cl:184-187).  Its value is 8: 4 is not assigned and is refused, as is anything above 15.  The rule, in
+ * Raytracing.cl:184-187).  Its value is 8: 4 and 16 are not assigned and are refused, as is any bit above 32.  The rule, in
  * binary32 with every operation rounded separately (no contraction):
  *   - (ux, uy) are two uniforms in [0, 1): with B200RT_RNG_PHILOX words 0 and 1 of the block at counter (i, s, 0, 2) for
  *     sample s of work-item i (direction sampling uses n = 0, light sampling n = 1); with B200RT_RNG_REFERENCE the pixel
@@ -72,6 +72,37 @@ typedef enum {
  * sample; `primary_rays` is 0 (no primary-hit kernel runs); `samples` = rendered pixels x (sample_end - sample_begin),
  * since no pixel is ray-free; wave_iterations = (sample_end - sample_begin) x (max_bounce + 3), or
  * x (2 (max_bounce + 1) + 2) with light sampling; kernel_launches = 3 + the shading, compaction and tracing launches. */
+#define B200RT_SAMPLING_SMOOTH_NORMALS 32
+/* Smooth shading: every scattering surface is shaded with the barycentric interpolation of its triangle's three vertex
+ * normals at the hit point, instead of the first vertex's normal (MathLib.cl:151), so that a smooth mesh no longer
+ * renders as facets.  This bit CHANGES THE INTEGRAND.  The rule, in binary32 with every operation rounded separately
+ * (no contraction), true division, and dot(a, b) = (a.x*b.x + a.y*b.y) + a.z*b.z, for a hit on triangle t at distance
+ * k of the ray (o, d):
+ *   - x = o + unit(d) * k, the point the path continues from (Raytracing.cl:79; the cached primary hit has o = cam_pos
+ *     and d the camera direction); light sampling uses the same x;
+ *   - A, e1 = B - A, e2 = C - A are the triangle record's (rounded as MathLib.cl:129-130); n0, n1, n2 =
+ *     V_n[faceData[10t+4 .. 10t+6]] as given, not renormalised;
+ *   - flat triangle: if the nine components of n0, n1, n2 are equal as binary32 bit patterns, n = n0 (the reference's
+ *     normal, so a triangle that carries one normal renders bit for bit as without the bit);
+ *   - otherwise p = x - A; d00 = dot(e1,e1), d01 = dot(e1,e2), d11 = dot(e2,e2), d20 = dot(p,e1), d21 = dot(p,e2);
+ *     den = d00*d11 - d01*d01; b1 = (d11*d20 - d01*d21) / den; b2 = (d00*d21 - d01*d20) / den; b0 = (1 - b1) - b2;
+ *     m = (n0*b0 + n1*b1) + n2*b2 per component, the weights unclamped; n = m / sqrtf(dot(m, m)) per component; if a
+ *     component of n is not finite or dot(n, n) is not > 0, n = n0.  The normalisation is needed: the samplers rotate
+ *     +Z onto n by the angle acos(n.z), which is n's direction only for a unit n, and an interpolation of unit normals
+ *     is shorter than 1 inside the triangle; unnormalised, the tilted frame draws directions below n's plane, whose
+ *     1 / cos weight is infinite;
+ *   - n replaces the first-vertex normal wherever a scattering surface reads it: the frame of both samplers
+ *     (MathLib.cl:313-366, computed from n as for the first-vertex normal), BRDF_GGX's n, glass's 1/|dot(d, normalize(n))|
+ *     and the cosine factor (Raytracing.cl:86-87), and with bits 0 / 1 the importance sampler, the light sample's cosS
+ *     and the MIS densities.  The emitter side of light sampling (its density) keeps the emitter's geometry; sun and
+ *     shadow rays are unchanged.
+ * Known limits: a direction drawn around the shading normal can leave below the geometric surface (the reference does not
+ * flip normals either); the sun's shadow terminator stays faceted, since the shadow ray tests geometry.
+ * Every render entry point takes the bit, alone or with bits 1, 2 and 8 (b200rt_render_adaptive still refuses 8).
+ * b200rt_gbuffer and b200rt_render_denoised with the bit write the normalised n at the primary hit as the G-buffer
+ * normal, x being cam_pos + unit(d) * k.  b200rt_primary_hits and b200rt_trace_rays ignore it.  b200rt_set_scene
+ * validates n0's index only; a render or G-buffer with the bit refuses (B200RT_ERR_INVALID) a scene in which a
+ * triangle's n1 or n2 index is out of range, and its message names the first such triangle. */
 
 /* output modes */
 #define B200RT_OUT_FINAL 0 /* mean over spp, clamped to [0,1]  (Raytracing.cl:211-219) */
