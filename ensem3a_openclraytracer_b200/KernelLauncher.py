@@ -40,7 +40,12 @@ Differences a caller can observe (all documented in INTEGRATION.md):
   * `smooth_normals = True` shades every hit with the interpolation of its triangle's three vertex normals instead of
     the first vertex's (B200RT_SAMPLING_SMOOTH_NORMALS), so smooth meshes no longer render as facets.
     B200RT_SMOOTH_NORMALS=1 (or 0) sets it for callers that never touch the attribute.  It combines with `adaptive`,
-    `denoise`, `pixel_jitter` and `cuda_devices`.
+    `denoise`, `pixel_jitter` and `cuda_devices`;
+  * `dielectric_glass = True` makes glass (material type 3) a smooth dielectric interface that reflects with the Fresnel
+    probability and refracts by Snell's law with the material's ior, instead of the reference's tinted pass-through
+    (B200RT_SAMPLING_DIELECTRIC_GLASS; an ior slot of 0 means 1.5, of 1 keeps the pass-through).
+    B200RT_DIELECTRIC_GLASS=1 (or 0) sets it for callers that never touch the attribute.  It combines with `adaptive`,
+    `denoise`, `pixel_jitter`, `smooth_normals` and `cuda_devices`.
 """
 import math
 import os
@@ -106,6 +111,14 @@ def pixel_jitter_from_env(text):
     return t == "1"
 
 
+def dielectric_glass_from_env(text):
+    """The `dielectric_glass` flag that B200RT_DIELECTRIC_GLASS=0 or =1 stands for; ValueError otherwise."""
+    t = str(text).strip()
+    if t not in ("0", "1"):
+        raise ValueError(f"B200RT_DIELECTRIC_GLASS={text!r}: expected 0 or 1")
+    return t == "1"
+
+
 def smooth_normals_from_env(text):
     """The `smooth_normals` flag that B200RT_SMOOTH_NORMALS=0 or =1 stands for; ValueError otherwise."""
     t = str(text).strip()
@@ -148,6 +161,9 @@ class KernelLauncher(object):
         # False: the first vertex's normal (the reference's faceted shading); True: smooth shading (module docstring)
         self.smooth_normals = (smooth_normals_from_env(os.environ["B200RT_SMOOTH_NORMALS"])
                                if os.environ.get("B200RT_SMOOTH_NORMALS") else False)
+        # False: the reference's pass-through glass; True: refractive glass (module docstring)
+        self.dielectric_glass = (dielectric_glass_from_env(os.environ["B200RT_DIELECTRIC_GLASS"])
+                                 if os.environ.get("B200RT_DIELECTRIC_GLASS") else False)
         self.last_spp = None
         self.last_stats = None
         self._warned_deep = False
@@ -200,7 +216,8 @@ class KernelLauncher(object):
         opts = _capi.make_opts(rng_mode=self.rng_mode, traversal=traversal, stack_cap=self.stack_cap,
                                seed=self.seed, collect_stats=self.collect_stats, sample_streams=self.sample_streams,
                                sampling=((_capi.SAMPLING_PIXEL_JITTER if self.pixel_jitter else 0) |
-                                         (_capi.SAMPLING_SMOOTH_NORMALS if self.smooth_normals else 0)))
+                                         (_capi.SAMPLING_SMOOTH_NORMALS if self.smooth_normals else 0) |
+                                         (_capi.SAMPLING_DIELECTRIC_GLASS if self.dielectric_glass else 0)))
         out = h_img_out.reshape(-1)[:imgDim * 3]
         if self.adaptive is not None:
             img, self.last_spp, _ = self._ctx.render_adaptive(cam[:10], h_envData, width, height, int(spp), int(maxBounce),

@@ -19,6 +19,7 @@ OUT_FINAL, OUT_SUMS = 0, 1
 SAMPLING_REFERENCE, SAMPLING_IMPORTANCE, SAMPLING_LIGHTS = 0, 1, 2
 SAMPLING_PIXEL_JITTER = 8   # anti-aliasing: changes the integrand to the pixel's area (include/b200rt.h)
 SAMPLING_SMOOTH_NORMALS = 32   # smooth shading: the interpolated vertex normal at the hit (include/b200rt.h)
+SAMPLING_DIELECTRIC_GLASS = 128   # refractive glass: Fresnel reflection and Snell refraction at type 3 (include/b200rt.h)
 
 
 class B200RTError(RuntimeError):

@@ -125,6 +125,7 @@ int fail(Handle *h, int code, const char *fmt, ...) {
 }  // namespace
 
 static_assert(kRefStack == kRefStackMax, "scene_repack.h and rt_trace.cuh disagree on the exact walk's stack");
+static_assert(kGlassDefaultIor == B200RT_GLASS_DEFAULT_IOR, "b200rt.h and rt_shade.cuh disagree on the default ior");
 size_t b200rt::lane_smem_bytes_host(int stack_depth) { return lane_smem_bytes(stack_depth); }
 
 namespace {
@@ -381,21 +382,26 @@ int prepare_trace_t(b200rt_ctx *c, WaveLaunch *w) {
 }
 
 // jitter and adaptive are never both set (b200rt_render_adaptive refuses the jitter bit)
-template <bool SMOOTH>
+template <bool SMOOTH, bool GLASS>
 void pick_shade(bool nee, bool adaptive, bool jitter, WaveLaunch *w) {
-  if (jitter) w->shade = nee ? k_shade<true, false, true, SMOOTH> : k_shade<false, false, true, SMOOTH>;
-  else if (nee) w->shade = adaptive ? k_shade<true, true, false, SMOOTH> : k_shade<true, false, false, SMOOTH>;
-  else w->shade = adaptive ? k_shade<false, true, false, SMOOTH> : k_shade<false, false, false, SMOOTH>;
+  if (jitter) w->shade = nee ? k_shade<true, false, true, SMOOTH, GLASS> : k_shade<false, false, true, SMOOTH, GLASS>;
+  else if (nee) w->shade = adaptive ? k_shade<true, true, false, SMOOTH, GLASS> : k_shade<true, false, false, SMOOTH, GLASS>;
+  else w->shade = adaptive ? k_shade<false, true, false, SMOOTH, GLASS> : k_shade<false, false, false, SMOOTH, GLASS>;
 }
 
 int prepare_wave(b200rt_ctx *c, int trav, bool smem, bool stats, bool nee, bool adaptive, bool jitter, bool smooth,
-                 WaveLaunch *w) {
+                 bool glass, WaveLaunch *w) {
   int per_sm = 0;
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shade<false, false>, kShadeBlock, 0));
   if (per_sm < 1) return fail(c, B200RT_ERR_CUDA, "k_shade does not fit on an SM");
   w->shade_grid = per_sm * c->sm_count;
-  if (!smooth) pick_shade<false>(nee, adaptive, jitter, w);
-  else pick_shade<true>(nee, adaptive, jitter, w);
+  if (glass) {
+    if (!smooth) pick_shade<false, true>(nee, adaptive, jitter, w);
+    else pick_shade<true, true>(nee, adaptive, jitter, w);
+  } else {
+    if (!smooth) pick_shade<false, false>(nee, adaptive, jitter, w);
+    else pick_shade<true, false>(nee, adaptive, jitter, w);
+  }
   return with_variant(c, trav, smem, stats, [&](auto t, auto s, auto st) {
     return prepare_trace_t<decltype(t)::value, decltype(s)::value, decltype(st)::value>(c, w);
   });
@@ -508,7 +514,7 @@ int check_frame_args(b200rt_ctx *c, const float *cam, int width, int height, int
   if (o.traversal < 0 || o.traversal > 2) return fail(c, B200RT_ERR_INVALID, "bad traversal %d", o.traversal);
   if (o.sampling < 0 ||
       (o.sampling & ~(B200RT_SAMPLING_IMPORTANCE | B200RT_SAMPLING_LIGHTS | B200RT_SAMPLING_PIXEL_JITTER |
-                      B200RT_SAMPLING_SMOOTH_NORMALS)) != 0)
+                      B200RT_SAMPLING_SMOOTH_NORMALS | B200RT_SAMPLING_DIELECTRIC_GLASS)) != 0)
     return fail(c, B200RT_ERR_INVALID, "bad sampling mode %d", o.sampling);
   if (o.output != B200RT_OUT_FINAL && o.output != B200RT_OUT_SUMS)
     return fail(c, B200RT_ERR_INVALID, "bad output mode %d", o.output);
@@ -539,6 +545,17 @@ int check_smooth_scene(b200rt_ctx *c, const b200rt_opts &o) {
   return 0;
 }
 
+// Refractive glass reads the ior slot of glass materials, which b200rt_set_materials accepts whatever it holds: a frame
+// with the bit refuses a material set in which a glass material's ior is negative, NaN or infinite.
+int check_glass_materials(b200rt_ctx *c, const b200rt_opts &o) {
+  if ((o.sampling & B200RT_SAMPLING_DIELECTRIC_GLASS) && c->scene.glass_bad >= 0)
+    return fail(c, B200RT_ERR_INVALID,
+                "B200RT_SAMPLING_DIELECTRIC_GLASS: material %d is glass (type 3) with ior %g; the ior must be 0 "
+                "(default %g), 1 (pass-through) or another finite positive value", c->scene.glass_bad,
+                (double)c->scene.glass_bad_ior, (double)B200RT_GLASS_DEFAULT_IOR);
+  return 0;
+}
+
 constexpr int kAdaptBatch = 32;  // adaptive renders: wavefront iterations enqueued between two looks at the list length
 
 // One render on c's stream; render_frame has checked the frame.  ad != NULL: adaptive sampling (b200rt_render_adaptive
@@ -558,6 +575,7 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   const bool nee = (o.sampling & B200RT_SAMPLING_LIGHTS) != 0 && c->n_light > 0;
   const bool jitter = (o.sampling & B200RT_SAMPLING_PIXEL_JITTER) != 0;
   const bool smooth = (o.sampling & B200RT_SAMPLING_SMOOTH_NORMALS) != 0;
+  const bool glass = (o.sampling & B200RT_SAMPLING_DIELECTRIC_GLASS) != 0;
   const long long per_sample = (nee ? 2 * ((long long)max_bounce + 1) + 1 : (long long)max_bounce + 2) + (jitter ? 1 : 0);
   const long long n_iter_ll = (long long)(F.s1 - F.s0) * per_sample;
   if (n_iter_ll > (1 << 22)) return fail(c, B200RT_ERR_UNSUPPORTED, "%lld wavefront iterations exceed 2^22", n_iter_ll);
@@ -589,7 +607,7 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   A.validate = (trav == B200RT_TRAVERSAL_FAST) ? 1 : 0;
   const bool smem = use_smem_scene(c);
   WaveLaunch wl;
-  int rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, jitter, smooth, &wl);
+  int rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, jitter, smooth, glass, &wl);
   if (rc) return rc;
   if (ensure(c, c->d_part_count, (size_t)wl.shade_grid * sizeof(unsigned int))) return B200RT_ERR_CUDA;
   A.part_count = static_cast<unsigned int *>(c->d_part_count.p);
@@ -831,6 +849,7 @@ int render_frame(b200rt_ctx *c, const float *cam, const float *env, int width, i
     return fail(c, B200RT_ERR_INVALID, "bad sample_streams %d (-1 automatic, 0 / 1 off, up to 16)", o.sample_streams);
   int rc = check_frame_args(c, cam, width, height, spp, max_bounce, o, true, env);
   if (!rc) rc = check_smooth_scene(c, o);
+  if (!rc) rc = check_glass_materials(c, o);
   if (rc) return rc;
   if (!c->have_ibl) return fail(c, B200RT_ERR_NO_SCENE, "no environment map: call b200rt_set_ibl first");
   int s0 = o.sample_begin, s1 = o.sample_end;
@@ -989,6 +1008,16 @@ int b200rt_set_materials(b200rt_ctx *c, const float *mat, int64_t n_mat) {
   }
   for (int32_t m : c->tri_mat)
     if (m < 0 || m >= nm) return fail(c, B200RT_ERR_INVALID, "a triangle uses material %d but only %d materials were given", m, nm);
+  // opt-in refractive glass: the first glass material whose ior it cannot use (check_glass_materials)
+  c->scene.glass_bad = -1;
+  for (int m = 0; m < nm; ++m) {
+    const float ior = mat[6 * m + 5];
+    if ((int)mat[6 * m] == 3 && !(std::isfinite(ior) && ior >= 0.0f)) {
+      c->scene.glass_bad = m;
+      c->scene.glass_bad_ior = ior;
+      break;
+    }
+  }
   CU(cudaSetDevice(c->device));
   uint64_t h = hash_bytes(mat, (size_t)n_mat * 4, 0x6d617473ull);
   DevBuf &d_mats = c->d_scene[kMats], &d_light = c->d_scene[kLight];

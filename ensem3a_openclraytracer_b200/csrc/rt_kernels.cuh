@@ -437,8 +437,10 @@ RT_DEV v3 shading_normal(const SceneView &S, int n_tris, int tri, v3 n0, v3 x, b
 // a sample starts with a camera ray through a jittered point of its pixel (phase 3), which phase 2 resolves the way
 // k_primary resolves the cached primary ray, instead of from the cached primary hit.  SMOOTH = opt-in smooth shading
 // (B200RT_SAMPLING_SMOOTH_NORMALS): a hit on a curved triangle is shaded with the interpolated normal and a frame built
-// in registers (shading_normal, tri_frame_at); a flat one keeps its precomputed frame.
-template <bool NEE, bool ADAPT, bool JITTER = false, bool SMOOTH = false>
+// in registers (shading_normal, tri_frame_at); a flat one keeps its precomputed frame.  GLASS = opt-in refractive glass
+// (B200RT_SAMPLING_DIELECTRIC_GLASS): a glass hit whose ior slot is not 1 reflects or refracts (scatter_dielectric)
+// instead of passing through.
+template <bool NEE, bool ADAPT, bool JITTER = false, bool SMOOTH = false, bool GLASS = false>
 __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant__ KernelArgs A, int iter) {
   const FrameParams &F = A.F;
   const SceneView &S = A.S;
@@ -678,10 +680,20 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
       const TriFrame tf = curved ? tri_frame_at(n, which) : load_tri_frame(S.frames, htri, which);
       v3 nd, brdf;
       float inv_pdf;
+      bool dielectric = false, reflected = false;
       if (m.type == 3) {
-        nd = d;
-        brdf = m.color;
-        inv_pdf = 1.0f / fabsf(dot(nd, tf.un));
+        const float v = GLASS ? load_material_ior(S.mats, tri_material(S, htri)) : 1.0f;
+        if (v == 1.0f) {  // the reference's pass-through (always without GLASS)
+          nd = d;
+          brdf = m.color;
+          inv_pdf = 1.0f / fabsf(dot(nd, tf.un));
+        } else {
+          float u;
+          if (F.rng_mode == 0) u = draw1<0>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, F.key0, F.key1);
+          else u = draw1<1>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, F.key0, F.key1);
+          nd = scatter_dielectric(d, tf.un, v == 0.0f ? kGlassDefaultIor : v, u, &reflected);
+          dielectric = true;
+        }
       } else {
         float u0, u1;
         if (F.rng_mode == 0) draw2<0>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, F.key0, F.key1, &u0, &u1);
@@ -698,8 +710,12 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
       if (NEE) pb_ray = m.type == 3 ? 0.0f : bsdf_pdf(m, F.sampling, tf.un, d, unit(nd));
       if (!NEE || !from_light) o = o + unit(d) * hk;  // :79 — no offset along the normal
       d = nd;
-      const float att = inv_pdf * fabsf(dot(nd, tf.un));
-      acc = (acc * brdf) * att;
+      if (GLASS && dielectric) {  // weight 1: reflection keeps the throughput, refraction tints it
+        if (!reflected) acc = acc * m.color;
+      } else {
+        const float att = inv_pdf * fabsf(dot(nd, tf.un));
+        acc = (acc * brdf) * att;
+      }
       seg_type = m.type;
       sun_ray = 0;
     }

@@ -249,6 +249,21 @@ RT_DEV void draw2(rng_state &g, uint32_t pixel, uint32_t sample, uint32_t bounce
   }
 }
 
+// One uniform draw for bounce `j` (opt-in refractive glass): draw2's first value, i.e. the generator's next value in
+// reference mode, word 0 of the Philox block (pixel, sample, bounce, 0) otherwise.
+template <int RNG>
+RT_DEV float draw1(rng_state &g, uint32_t pixel, uint32_t sample, uint32_t bounce, uint32_t k0, uint32_t k1) {
+  if (RNG == 0) {
+    const uint32_t b = 36969u * (g.a & 65535u) + (g.a >> 16);
+    const uint32_t a = 18000u * (b & 65535u) + (b >> 16);
+    g.a = a;
+    return bits_to_unit((b << 16) + a);
+  }
+  uint32_t o[4];
+  philox4x32_10(pixel, sample, bounce, 0u, k0, k1, o);
+  return bits_to_unit(o[0]);
+}
+
 // Three uniform draws for the light sample of bounce `j` (opt-in light sampling): the generator's next three values
 // in reference mode, the second Philox block of (pixel, sample, bounce) otherwise (the first feeds draw2).
 template <int RNG>

@@ -205,6 +205,38 @@ RT_DEV v3 sample_uniform(v3 n, const TriFrame &T, float u, float u2, float *inv_
   return apply_rotor(T.rot, local);
 }
 
+// ---- opt-in: refractive glass (b200rt_opts.sampling bit B200RT_SAMPLING_DIELECTRIC_GLASS) -------------------------------
+constexpr float kGlassDefaultIor = 1.5f;  // B200RT_GLASS_DEFAULT_IOR: the ior of a glass material whose ior slot is 0
+
+// the raw ior slot of material idx (materialData[6 idx + 5]), which the reference's extractMaterial never reads
+RT_DEV float load_material_ior(const float *mats, int idx) { return __ldg(mats + 6 * idx + 5); }
+
+// The smooth dielectric interface of b200rt.h: the next direction of a path that meets glass of index `ior` along d,
+// un the unit normal, u one uniform.  Reflects with Fresnel's probability F (always on total internal reflection),
+// refracts by Snell's law otherwise; *reflected tells which.  The caller keeps the throughput on a reflection and
+// tints it by the colour on a refraction.
+RT_DEV v3 scatter_dielectric(v3 d, v3 un, float ior, float u, bool *reflected) {
+  const v3 w = unit(d);
+  const float c = dot(w, un);
+  const bool enter = c < 0.0f;
+  const float eta = enter ? 1.0f / ior : ior;
+  const float ci = enter ? -c : c;
+  const v3 m = enter ? un : neg3(un);
+  const float k = 1.0f - (eta * eta) * (1.0f - ci * ci);
+  float ct = 0.0f;
+  bool refl = true;
+  if (k >= 0.0f) {
+    ct = sqrtf(k);
+    const float rs = (eta * ci - ct) / (eta * ci + ct);
+    const float rp = (ci - eta * ct) / (ci + eta * ct);
+    const float F = 0.5f * (rs * rs + rp * rp);
+    refl = !(u >= F);
+  }
+  *reflected = refl;
+  if (refl) return w + m * (2.0f * ci);
+  return w * eta + m * (eta * ci - ct);
+}
+
 RT_DEV float ipow(float x, int n) {  // pown: repeated multiply from 1
   float r = 1.0f;
   for (int i = 0; i < n; ++i) r = r * x;

@@ -37,6 +37,8 @@ struct SceneDesc {
   int fast_ok = 0;
   float root_box[6] = {0, 0, 0, 0, 0, 0};  // the caller's root box, bvh[2..7] (min.xyz, max.xyz): the denoiser's scale
   int smooth_bad = -1;          // first triangle whose n1 or n2 index is out of range: smooth-shaded renders refuse it
+  int glass_bad = -1;           // first glass material whose ior is negative, NaN or infinite: renders with refractive
+  float glass_bad_ior = 0.0f;   // glass refuse it (set by b200rt_set_materials, not by the repack)
 };
 
 // .w of the first `nsmooth` record of a triangle (opt-in smooth shading, b200rt.h B200RT_SAMPLING_SMOOTH_NORMALS)

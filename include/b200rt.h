@@ -56,7 +56,7 @@ typedef enum {
 /* Anti-aliasing: every sample traces its own camera ray through a jittered point of its pixel.  Unlike bits 0 and 1
  * this bit CHANGES THE INTEGRAND: the image converges to the box-filtered (pixel-area) image, no longer to the
  * reference's, whose pixel is one point (one camera ray per pixel, whose hit every sample restarts from,
- * Raytracing.cl:184-187).  Its value is 8: 4 and 16 are not assigned and are refused, as is any bit above 32.  The rule, in
+ * Raytracing.cl:184-187).  Its value is 8: 4, 16 and 64 are not assigned and are refused, as is any bit above 128.  The rule, in
  * binary32 with every operation rounded separately (no contraction):
  *   - (ux, uy) are two uniforms in [0, 1): with B200RT_RNG_PHILOX words 0 and 1 of the block at counter (i, s, 0, 2) for
  *     sample s of work-item i (direction sampling uses n = 0, light sampling n = 1); with B200RT_RNG_REFERENCE the pixel
@@ -103,6 +103,44 @@ typedef enum {
  * normal, x being cam_pos + unit(d) * k.  b200rt_primary_hits and b200rt_trace_rays ignore it.  b200rt_set_scene
  * validates n0's index only; a render or G-buffer with the bit refuses (B200RT_ERR_INVALID) a scene in which a
  * triangle's n1 or n2 index is out of range, and its message names the first such triangle. */
+#define B200RT_SAMPLING_DIELECTRIC_GLASS 128
+#define B200RT_GLASS_DEFAULT_IOR 1.5f
+/* Refractive glass: a type-3 surface becomes a smooth dielectric interface that reflects or refracts, instead of the
+ * reference's pass-through (the ray keeps its direction, tinted by the colour: MathLib.cl:391-395, Raytracing.cl:58-78,
+ * which never read the material's ior).  This bit CHANGES THE INTEGRAND.  The rule, in binary32 with every operation
+ * rounded separately (no contraction), true division, correctly rounded sqrtf and dot(a, b) = (a.x*b.x + a.y*b.y) +
+ * a.z*b.z, for a hit on a glass material m by the ray (o, d) at bounce j of sample s of work-item i:
+ *   - the ior: v = materialData[6m + 5]; v == 0 gives ior = B200RT_GLASS_DEFAULT_IOR (every shipped scene has 0 there);
+ *     v == 1 keeps the reference's pass-through bit for bit (nd = d, brdf = colour, inv_pdf = 1 / |dot(d, un)|, the
+ *     cosine factor, and no draw), which is how a pane modelled as one plane stays a window; any other finite v > 0 is the
+ *     ior (below 1 too, e.g. a bubble);
+ *   - un is the unit normal glass uses without the bit: the normalised first-vertex normal, or the smooth-shading normal
+ *     with B200RT_SAMPLING_SMOOTH_NORMALS;
+ *   - w = unit(d), c = dot(w, un).  c < 0 enters: eta = 1 / ior, ci = -c, m = un; otherwise it leaves: eta = ior,
+ *     ci = c, m = -un;
+ *   - k = 1 - (eta*eta) * (1 - ci*ci).  If k >= 0: ct = sqrtf(k), rs = (eta*ci - ct) / (eta*ci + ct),
+ *     rp = (ci - eta*ct) / (ci + eta*ct), F = 0.5 * (rs*rs + rp*rp) (Fresnel's reflectance of unpolarised light);
+ *   - one uniform u: with B200RT_RNG_PHILOX word 0 of the block at counter (i, s, j, 0), the block direction sampling
+ *     of bounce j uses, which a glass hit never draws from; with B200RT_RNG_REFERENCE the pixel generator's next value;
+ *   - the path reflects iff !(k >= 0) (total internal reflection) or !(u >= F), so a NaN F reflects; otherwise it
+ *     refracts.  Reflection: nd = w + m * (2*ci) per component, the throughput unchanged (a dielectric reflects
+ *     untinted).  Refraction: nd = w*eta + m * (eta*ci - ct) per component (Snell's law), throughput = throughput *
+ *     colour per component (the reference's tint per crossing).  No inv_pdf * |cos| factor: the choice between the two
+ *     is drawn with the probability of each, so the estimator's weight is 1;
+ *   - everything else stays as without the bit: the path continues from x = o + unit(d) * k with no offset
+ *     (Raytracing.cl:79; the traversal's k > 0.0001 rejects the surface just left), the segment's type is 3 for both
+ *     outcomes, so the sun-ray rules (Raytracing.cl:115-137: the sun through glass is colour x sun power, no sun after a
+ *     glass segment) and light sampling (glass is not a light-sampling site) are unchanged, and the bounce count j, the
+ *     rays per sample, wave_iterations and kernel_launches keep their formulas.
+ * Known limits: inside and outside are decided per hit from the side of the normal, so an open surface (one plane)
+ * bounds a half-space of glass: give panes ior 1.  No caustics: the sun's shadow ray keeps the reference's tinted
+ * pass-through.  No absorption inside the medium, no dispersion and no rough glass: type 3's roughness stays ignored.
+ * The denoiser's G-buffer describes the glass surface, not what is seen through it.
+ * Every render entry point takes the bit, alone or with bits 1, 2, 8 and 32 (b200rt_render_adaptive still refuses 8).
+ * b200rt_primary_hits, b200rt_gbuffer and b200rt_trace_rays ignore it.  b200rt_set_materials and b200rt_set_scene
+ * accept what they accept without it; a render with the bit refuses (B200RT_ERR_INVALID) a material set in which a glass
+ * material has a negative, NaN or infinite ior, and its message names the first such material.  The ior of a material
+ * of another type is never read. */
 
 /* output modes */
 #define B200RT_OUT_FINAL 0 /* mean over spp, clamped to [0,1]  (Raytracing.cl:211-219) */
