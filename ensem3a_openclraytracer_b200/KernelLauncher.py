@@ -45,7 +45,12 @@ Differences a caller can observe (all documented in INTEGRATION.md):
     probability and refracts by Snell's law with the material's ior, instead of the reference's tinted pass-through
     (B200RT_SAMPLING_DIELECTRIC_GLASS; an ior slot of 0 means 1.5, of 1 keeps the pass-through).
     B200RT_DIELECTRIC_GLASS=1 (or 0) sets it for callers that never touch the attribute.  It combines with `adaptive`,
-    `denoise`, `pixel_jitter`, `smooth_normals` and `cuda_devices`.
+    `denoise`, `pixel_jitter`, `smooth_normals` and `cuda_devices`;
+  * `textures = {material index: image}` (the argument of Context.set_textures) binds albedo textures and renders with
+    B200RT_SAMPLING_TEXTURES: a diffuse or glossy surface takes its colour from its material's image at the hit's
+    interpolated UV (the scene's V_uv), times the material colour.  B200RT_TEXTURES=<material>=<path>[,...] loads the
+    files with PIL for callers that never touch the attribute.  It combines with `adaptive`, `denoise`, `pixel_jitter`,
+    `smooth_normals`, `dielectric_glass` and `cuda_devices`.
 """
 import math
 import os
@@ -127,6 +132,23 @@ def smooth_normals_from_env(text):
     return t == "1"
 
 
+def textures_from_env(text):
+    """The `textures` dict that B200RT_TEXTURES=<material>=<path>[,<material>=<path>...] stands for, the images loaded
+    with PIL; ValueError if malformed (OSError if a file cannot be read)."""
+    usage = f"B200RT_TEXTURES={text!r}: expected <material>=<path>[,<material>=<path>...], e.g. 4=wood.png,0=brick.png"
+    out = {}
+    for item in str(text).split(","):
+        m, sep, path = item.partition("=")
+        m, path = m.strip(), path.strip()
+        if not sep or not path or not m.isdigit():
+            raise ValueError(usage)
+        if int(m) in out:
+            raise ValueError(usage + f" (material {int(m)} given twice)")
+        out[int(m)] = path
+    from PIL import Image
+    return {m: Image.open(path).convert("RGBA") for m, path in out.items()}
+
+
 class KernelLauncher(object):
 
     def __init__(self, context=None, platform=None, device=None, queue=None, cuda_device=0, cuda_devices=None):
@@ -164,6 +186,9 @@ class KernelLauncher(object):
         # False: the reference's pass-through glass; True: refractive glass (module docstring)
         self.dielectric_glass = (dielectric_glass_from_env(os.environ["B200RT_DIELECTRIC_GLASS"])
                                  if os.environ.get("B200RT_DIELECTRIC_GLASS") else False)
+        # None: the material colours (the reference's image); a dict: albedo textures (module docstring)
+        self.textures = textures_from_env(os.environ["B200RT_TEXTURES"]) if os.environ.get("B200RT_TEXTURES") else None
+        self._textures_bound = False
         self.last_spp = None
         self.last_stats = None
         self._warned_deep = False
@@ -202,6 +227,9 @@ class KernelLauncher(object):
             self._ctx.set_ibl(h_IBL.tobytes(), w, h)
         else:
             self._ctx.set_ibl(np.asarray(h_IBL))
+        if self.textures or self._textures_bound:   # the default path makes no call; an emptied dict unbinds
+            self._ctx.set_textures(self.textures)
+            self._textures_bound = bool(self.textures)
 
         traversal = self.traversal
         need = self._ctx.stats()["ref_stack_need"]
@@ -217,7 +245,8 @@ class KernelLauncher(object):
                                seed=self.seed, collect_stats=self.collect_stats, sample_streams=self.sample_streams,
                                sampling=((_capi.SAMPLING_PIXEL_JITTER if self.pixel_jitter else 0) |
                                          (_capi.SAMPLING_SMOOTH_NORMALS if self.smooth_normals else 0) |
-                                         (_capi.SAMPLING_DIELECTRIC_GLASS if self.dielectric_glass else 0)))
+                                         (_capi.SAMPLING_DIELECTRIC_GLASS if self.dielectric_glass else 0) |
+                                         (_capi.SAMPLING_TEXTURES if self.textures else 0)))
         out = h_img_out.reshape(-1)[:imgDim * 3]
         if self.adaptive is not None:
             img, self.last_spp, _ = self._ctx.render_adaptive(cam[:10], h_envData, width, height, int(spp), int(maxBounce),

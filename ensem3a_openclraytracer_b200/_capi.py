@@ -20,6 +20,7 @@ SAMPLING_REFERENCE, SAMPLING_IMPORTANCE, SAMPLING_LIGHTS = 0, 1, 2
 SAMPLING_PIXEL_JITTER = 8   # anti-aliasing: changes the integrand to the pixel's area (include/b200rt.h)
 SAMPLING_SMOOTH_NORMALS = 32   # smooth shading: the interpolated vertex normal at the hit (include/b200rt.h)
 SAMPLING_DIELECTRIC_GLASS = 128   # refractive glass: Fresnel reflection and Snell refraction at type 3 (include/b200rt.h)
+SAMPLING_TEXTURES = 512   # albedo textures: diffuse / glossy colour from the bound image at the hit's UV (include/b200rt.h)
 
 
 class B200RTError(RuntimeError):
@@ -72,13 +73,13 @@ def _denoise_params(passes=DENOISE_DEFAULTS["passes"], sigma_color=DENOISE_DEFAU
 # every symbol include/b200rt.h declares (tests/test_abi.py checks the header against this list)
 SYMBOLS = [
     "b200rt_default_opts", "b200rt_create", "b200rt_destroy", "b200rt_last_error", "b200rt_set_scene",
-    "b200rt_set_materials", "b200rt_set_ibl", "b200rt_render", "b200rt_render_adaptive", "b200rt_gbuffer", "b200rt_denoise", "b200rt_render_denoised", "b200rt_render_rgb8", "b200rt_render_device", "b200rt_finalize_device",
+    "b200rt_set_materials", "b200rt_set_ibl", "b200rt_set_textures", "b200rt_render", "b200rt_render_adaptive", "b200rt_gbuffer", "b200rt_denoise", "b200rt_render_denoised", "b200rt_render_rgb8", "b200rt_render_device", "b200rt_finalize_device",
     "b200rt_reduce_finalize_device", "b200rt_sync", "b200rt_set_stream", "b200rt_invalidate", "b200rt_primary_hits", "b200rt_trace_rays",
     "b200rt_img_processing", "b200rt_get_stats", "b200rt_math_probe", "b200rt_texel_probe", "b200rt_philox_probe", "b200rt_alloc",
     "b200rt_free", "b200rt_ipc_export",
     "b200rt_ipc_open", "b200rt_ipc_close", "b200rt_build_bvh", "b200rt_repack_probe", "b200rt_version", "b200rt_device_count",
     "b200rt_multi_create", "b200rt_multi_destroy", "b200rt_multi_last_error", "b200rt_multi_device_count",
-    "b200rt_multi_context", "b200rt_multi_set_scene", "b200rt_multi_set_ibl", "b200rt_multi_invalidate",
+    "b200rt_multi_context", "b200rt_multi_set_scene", "b200rt_multi_set_ibl", "b200rt_multi_set_textures", "b200rt_multi_invalidate",
     "b200rt_multi_render", "b200rt_multi_render_denoised", "b200rt_multi_get_stats",
 ]
 
@@ -112,6 +113,8 @@ def load_library():
     lib.b200rt_set_scene.argtypes = [vp, vp, i64, vp, i64, vp, i64, vp, i64, vp, i64, vp, i64, vp, i64]
     lib.b200rt_set_materials.argtypes = [vp, vp, i64]
     lib.b200rt_set_ibl.argtypes = [vp, vp, i32, i32]
+    lib.b200rt_set_textures.argtypes = [vp, vp, i64, vp, i32, vp, i64]
+    lib.b200rt_multi_set_textures.argtypes = lib.b200rt_set_textures.argtypes
     lib.b200rt_render.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), vp]
     lib.b200rt_render_adaptive.argtypes = [vp, vp, vp, i32, i32, i32, i32, ctypes.POINTER(Opts), ctypes.POINTER(Adaptive),
                                            vp, vp, vp]
@@ -188,6 +191,20 @@ def make_opts(rng_mode=RNG_REFERENCE, traversal=TRAVERSAL_FAST, stack_cap=20, ou
     o.sample_streams = int(sample_streams)
     o.sampling = int(sampling)
     return o
+
+
+def texture_rgba(image):
+    """(H, W, 4) uint8 RGBA of an albedo texture given as an (H, W, 4) or (H, W, 3) uint8 array (alpha 255 added) or a
+    PIL image (converted to RGBA); row 0 is the top row."""
+    if not isinstance(image, np.ndarray) and hasattr(image, "convert"):
+        image = image.convert("RGBA")
+    a = np.asarray(image)
+    if a.dtype != np.uint8 or a.ndim != 3 or a.shape[2] not in (3, 4) or a.shape[0] < 1 or a.shape[1] < 1:
+        raise B200RTError(f"a texture must be an (H, W, 4) or (H, W, 3) uint8 array or a PIL image "
+                          f"(got {a.dtype} {a.shape})")
+    if a.shape[2] == 3:
+        a = np.concatenate([a, np.full(a.shape[:2] + (1,), 255, np.uint8)], axis=2)
+    return np.ascontiguousarray(a)
 
 
 def build_bvh(face_data, vertex_p, return_depth=False):
@@ -274,6 +291,27 @@ class _Handle:
         if arr.size != int(width) * int(height) * 4:
             raise B200RTError(f"environment map: {arr.size} bytes for {width}x{height} RGBA")
         self._call("set_ibl", _ptr(arr), int(width), int(height))
+
+    def set_textures(self, textures):
+        """Binds the albedo textures of SAMPLING_TEXTURES: `textures` maps a material index to an (H, W, 4) or
+        (H, W, 3) uint8 array or a PIL image (texture_rgba).  Identical images are uploaded once; None or {} unbinds.
+        Bindings survive set_scene and set_materials."""
+        images, index = [], {}
+        for m, img in sorted((textures or {}).items()):
+            if int(m) != m or m < 0:
+                raise B200RTError(f"texture key {m!r}: expected a material index >= 0")
+            a = texture_rgba(img)
+            k = next((i for i, b in enumerate(images) if b.shape == a.shape and np.array_equal(b, a)), None)
+            if k is None:
+                k = len(images)
+                images.append(a)
+            index[int(m)] = k
+        mat_tex = np.full(max(index) + 1 if index else 0, -1, np.int32)
+        for m, k in index.items():
+            mat_tex[m] = k
+        texels = np.concatenate([a.reshape(-1) for a in images]) if images else np.zeros(0, np.uint8)
+        dims = np.array([[a.shape[1], a.shape[0]] for a in images], np.int32).reshape(-1)
+        self._call("set_textures", _ptr(texels), texels.size, _ptr(dims), len(images), _ptr(mat_tex), mat_tex.size)
 
     def invalidate(self):
         self._call("invalidate")

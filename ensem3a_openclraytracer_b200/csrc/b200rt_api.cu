@@ -31,7 +31,9 @@ struct DevBuf {
 };
 
 // the scene's device buffers, which sample-stream helpers borrow as a set
-enum SceneBuf { kNodes, kTris, kCtris, kNormals, kTboxes, kFrames, kMats, kBvh9, kLeafcnt, kLight, kSceneBufs };
+// kTex: the bound albedo textures (b200rt_set_textures, layout in rt_kernels.cuh surface_albedo), which survive a scene
+// upload
+enum SceneBuf { kNodes, kTris, kCtris, kNormals, kTboxes, kFrames, kMats, kBvh9, kLeafcnt, kLight, kTex, kSceneBufs };
 
 // Resident k_trace CTAs per SM while three or more sample streams share the GPU.  A k_trace that fills every SM's
 // register file leaves the other streams' kernels nothing but its tail to run in; capped, one stream's shading and
@@ -66,6 +68,8 @@ struct b200rt_ctx : Handle {
   int frame_trace_cap = 0; // resident k_trace CTAs per SM in the frame being enqueued (0 = what fits; set by render_frame)
   std::vector<int32_t> tri_mat;  // for re-validating material edits
   DevBuf d_pS, d_pL, d_pR;       // light sampling: three more float4 of path state
+  uint64_t tex_hash = 0;         // of the bound albedo textures (b200rt_set_textures); 0 = none cached
+  int n_mat_tex = 0, n_tex = 0;  // materials and textures d_scene[kTex] holds; n_mat_tex 0 = no texture bound
 
   // environment map
   bool have_ibl = false;
@@ -285,6 +289,16 @@ void fill_args(b200rt_ctx *c, const FrameParams &F, const b200rt_opts &o, float 
   A->ad = AdaptArgs();
 }
 
+// The texture header after the UV records in the normals buffer (rt_kernels.cuh surface_albedo), on c's stream: where the
+// bound textures are, or that none is.  Written by every scene upload and every texture binding.
+int write_tex_header(b200rt_ctx *c, int n_tris) {
+  const uint64_t p = reinterpret_cast<uint64_t>(c->d_scene[kTex].p);
+  const uint4 hd = make_uint4((uint32_t)p, (uint32_t)(p >> 32), (uint32_t)c->n_mat_tex, (uint32_t)c->n_tex);
+  CU(cudaMemcpyAsync(static_cast<float4 *>(c->d_scene[kNormals].p) + 5 * (size_t)n_tris, &hd, sizeof hd,
+                     cudaMemcpyHostToDevice, c->stream));
+  return 0;
+}
+
 // The fast path needs a strict two-child tree with nested boxes; any other tree is walked in reference order.  When
 // the caller asked for FAST (a walk that never drops a push) the substitute keeps that promise as far as its
 // thread-local stack reaches: it runs with the largest cap instead of the reference's 20.
@@ -382,25 +396,28 @@ int prepare_trace_t(b200rt_ctx *c, WaveLaunch *w) {
 }
 
 // jitter and adaptive are never both set (b200rt_render_adaptive refuses the jitter bit)
-template <bool SMOOTH, bool GLASS>
+template <bool SMOOTH, bool GLASS, bool TEX>
 void pick_shade(bool nee, bool adaptive, bool jitter, WaveLaunch *w) {
-  if (jitter) w->shade = nee ? k_shade<true, false, true, SMOOTH, GLASS> : k_shade<false, false, true, SMOOTH, GLASS>;
-  else if (nee) w->shade = adaptive ? k_shade<true, true, false, SMOOTH, GLASS> : k_shade<true, false, false, SMOOTH, GLASS>;
-  else w->shade = adaptive ? k_shade<false, true, false, SMOOTH, GLASS> : k_shade<false, false, false, SMOOTH, GLASS>;
+  if (jitter) w->shade = nee ? k_shade<true, false, true, SMOOTH, GLASS, TEX> : k_shade<false, false, true, SMOOTH, GLASS, TEX>;
+  else if (nee) w->shade = adaptive ? k_shade<true, true, false, SMOOTH, GLASS, TEX> : k_shade<true, false, false, SMOOTH, GLASS, TEX>;
+  else w->shade = adaptive ? k_shade<false, true, false, SMOOTH, GLASS, TEX> : k_shade<false, false, false, SMOOTH, GLASS, TEX>;
 }
 
 int prepare_wave(b200rt_ctx *c, int trav, bool smem, bool stats, bool nee, bool adaptive, bool jitter, bool smooth,
-                 bool glass, WaveLaunch *w) {
+                 bool glass, bool tex, WaveLaunch *w) {
   int per_sm = 0;
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shade<false, false>, kShadeBlock, 0));
   if (per_sm < 1) return fail(c, B200RT_ERR_CUDA, "k_shade does not fit on an SM");
   w->shade_grid = per_sm * c->sm_count;
-  if (glass) {
-    if (!smooth) pick_shade<false, true>(nee, adaptive, jitter, w);
-    else pick_shade<true, true>(nee, adaptive, jitter, w);
-  } else {
-    if (!smooth) pick_shade<false, false>(nee, adaptive, jitter, w);
-    else pick_shade<true, false>(nee, adaptive, jitter, w);
+  switch ((smooth ? 1 : 0) | (glass ? 2 : 0) | (tex ? 4 : 0)) {
+    case 0: pick_shade<false, false, false>(nee, adaptive, jitter, w); break;
+    case 1: pick_shade<true, false, false>(nee, adaptive, jitter, w); break;
+    case 2: pick_shade<false, true, false>(nee, adaptive, jitter, w); break;
+    case 3: pick_shade<true, true, false>(nee, adaptive, jitter, w); break;
+    case 4: pick_shade<false, false, true>(nee, adaptive, jitter, w); break;
+    case 5: pick_shade<true, false, true>(nee, adaptive, jitter, w); break;
+    case 6: pick_shade<false, true, true>(nee, adaptive, jitter, w); break;
+    default: pick_shade<true, true, true>(nee, adaptive, jitter, w); break;
   }
   return with_variant(c, trav, smem, stats, [&](auto t, auto s, auto st) {
     return prepare_trace_t<decltype(t)::value, decltype(s)::value, decltype(st)::value>(c, w);
@@ -514,7 +531,7 @@ int check_frame_args(b200rt_ctx *c, const float *cam, int width, int height, int
   if (o.traversal < 0 || o.traversal > 2) return fail(c, B200RT_ERR_INVALID, "bad traversal %d", o.traversal);
   if (o.sampling < 0 ||
       (o.sampling & ~(B200RT_SAMPLING_IMPORTANCE | B200RT_SAMPLING_LIGHTS | B200RT_SAMPLING_PIXEL_JITTER |
-                      B200RT_SAMPLING_SMOOTH_NORMALS | B200RT_SAMPLING_DIELECTRIC_GLASS)) != 0)
+                      B200RT_SAMPLING_SMOOTH_NORMALS | B200RT_SAMPLING_DIELECTRIC_GLASS | B200RT_SAMPLING_TEXTURES)) != 0)
     return fail(c, B200RT_ERR_INVALID, "bad sampling mode %d", o.sampling);
   if (o.output != B200RT_OUT_FINAL && o.output != B200RT_OUT_SUMS)
     return fail(c, B200RT_ERR_INVALID, "bad output mode %d", o.output);
@@ -556,6 +573,16 @@ int check_glass_materials(b200rt_ctx *c, const b200rt_opts &o) {
   return 0;
 }
 
+// Albedo textures read all three UV indices of a triangle, which b200rt_set_scene does not validate: a frame or G-buffer
+// with the bit refuses a scene that has an out-of-range one.
+int check_uv_scene(b200rt_ctx *c, const b200rt_opts &o) {
+  if ((o.sampling & B200RT_SAMPLING_TEXTURES) && c->scene.uv_bad >= 0)
+    return fail(c, B200RT_ERR_INVALID,
+                "B200RT_SAMPLING_TEXTURES: triangle %d has a UV index (faceData[10t+1 .. 10t+3]) out of range",
+                c->scene.uv_bad);
+  return 0;
+}
+
 constexpr int kAdaptBatch = 32;  // adaptive renders: wavefront iterations enqueued between two looks at the list length
 
 // One render on c's stream; render_frame has checked the frame.  ad != NULL: adaptive sampling (b200rt_render_adaptive
@@ -576,6 +603,7 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   const bool jitter = (o.sampling & B200RT_SAMPLING_PIXEL_JITTER) != 0;
   const bool smooth = (o.sampling & B200RT_SAMPLING_SMOOTH_NORMALS) != 0;
   const bool glass = (o.sampling & B200RT_SAMPLING_DIELECTRIC_GLASS) != 0;
+  const bool tex = (o.sampling & B200RT_SAMPLING_TEXTURES) != 0 && c->n_mat_tex > 0;   // nothing bound: the plain kernels
   const long long per_sample = (nee ? 2 * ((long long)max_bounce + 1) + 1 : (long long)max_bounce + 2) + (jitter ? 1 : 0);
   const long long n_iter_ll = (long long)(F.s1 - F.s0) * per_sample;
   if (n_iter_ll > (1 << 22)) return fail(c, B200RT_ERR_UNSUPPORTED, "%lld wavefront iterations exceed 2^22", n_iter_ll);
@@ -607,7 +635,7 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   A.validate = (trav == B200RT_TRAVERSAL_FAST) ? 1 : 0;
   const bool smem = use_smem_scene(c);
   WaveLaunch wl;
-  int rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, jitter, smooth, glass, &wl);
+  int rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, jitter, smooth, glass, tex, &wl);
   if (rc) return rc;
   if (ensure(c, c->d_part_count, (size_t)wl.shade_grid * sizeof(unsigned int))) return B200RT_ERR_CUDA;
   A.part_count = static_cast<unsigned int *>(c->d_part_count.p);
@@ -825,6 +853,7 @@ void borrow_scene(b200rt_ctx *p, b200rt_ctx *h) {
   h->n_light = p->n_light;
   h->have_scene = p->have_scene;
   h->ibl_tex = p->ibl_tex; h->ibl_w = p->ibl_w; h->ibl_h = p->ibl_h; h->have_ibl = p->have_ibl;
+  h->n_mat_tex = p->n_mat_tex;
   h->shared_epoch = p->scene_epoch;
 }
 
@@ -850,6 +879,7 @@ int render_frame(b200rt_ctx *c, const float *cam, const float *env, int width, i
   int rc = check_frame_args(c, cam, width, height, spp, max_bounce, o, true, env);
   if (!rc) rc = check_smooth_scene(c, o);
   if (!rc) rc = check_glass_materials(c, o);
+  if (!rc) rc = check_uv_scene(c, o);
   if (rc) return rc;
   if (!c->have_ibl) return fail(c, B200RT_ERR_NO_SCENE, "no environment map: call b200rt_set_ibl first");
   int s0 = o.sample_begin, s1 = o.sample_end;
@@ -1051,6 +1081,7 @@ namespace {
 struct SceneArgs {
   const float *vp; int64_t n_vp;
   const float *vn; int64_t n_vn;
+  const float *vuv; int64_t n_vuv;   // not validated (may be NULL): only textured renders read the UVs (repack_uvs)
   const int32_t *face; int64_t n_face;
   const float *mat; int64_t n_mat;
   const float *bvh; int64_t n_bvh;
@@ -1072,6 +1103,7 @@ uint64_t scene_hash_of(const SceneArgs &a) {
   uint64_t h = 0x7363656e65ull;
   h = hash_bytes(a.vp, (size_t)a.n_vp * 4, h);
   h = hash_bytes(a.vn, (size_t)a.n_vn * 4, h);
+  if (a.vuv && a.n_vuv > 0) h = hash_bytes(a.vuv, (size_t)a.n_vuv * 4, h);
   h = hash_bytes(a.face, (size_t)a.n_face * 4, h);
   h = hash_bytes(a.bvh, (size_t)a.n_bvh * 4, h);
   return h;
@@ -1092,8 +1124,9 @@ int upload_scene(b200rt_ctx *c, const Repacked &R, const SceneArgs &a, uint64_t 
   CU(cudaSetDevice(c->device));
   if (ensure(c, B[kTris], R.tris.size() * sizeof(float4))) return B200RT_ERR_CUDA;
   if (ensure(c, B[kCtris], R.ctris.size() * sizeof(float4))) return B200RT_ERR_CUDA;
-  // the first-vertex normals, then the other two vertex normals of opt-in smooth shading (rt_trace.cuh)
-  if (ensure(c, B[kNormals], (R.normals.size() + R.nsmooth.size()) * sizeof(float4))) return B200RT_ERR_CUDA;
+  // the first-vertex normals, then the other two vertex normals of opt-in smooth shading (rt_trace.cuh), then the UV
+  // records and the texture header of opt-in albedo textures (rt_kernels.cuh surface_albedo)
+  if (ensure(c, B[kNormals], (R.normals.size() + R.nsmooth.size() + R.uvs.size() + 1) * sizeof(float4))) return B200RT_ERR_CUDA;
   if (ensure(c, B[kTboxes], R.tboxes.size() * sizeof(float4))) return B200RT_ERR_CUDA;
   if (ensure(c, B[kFrames], (size_t)n_tris * kFrameVec * sizeof(float4))) return B200RT_ERR_CUDA;
   if (ensure(c, B[kNodes], R.nodes.size() * sizeof(uint4))) return B200RT_ERR_CUDA;
@@ -1105,6 +1138,9 @@ int upload_scene(b200rt_ctx *c, const Repacked &R, const SceneArgs &a, uint64_t 
   CU(cudaMemcpyAsync(B[kNormals].p, R.normals.data(), R.normals.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
   CU(cudaMemcpyAsync(static_cast<float4 *>(B[kNormals].p) + R.normals.size(), R.nsmooth.data(), R.nsmooth.size() * sizeof(float4),
                      cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(static_cast<float4 *>(B[kNormals].p) + R.normals.size() + R.nsmooth.size(), R.uvs.data(),
+                     R.uvs.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+  if (write_tex_header(c, n_tris)) return B200RT_ERR_CUDA;
   CU(cudaMemcpyAsync(B[kTboxes].p, R.tboxes.data(), R.tboxes.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
   if (!R.nodes.empty())
     CU(cudaMemcpyAsync(B[kNodes].p, R.nodes.data(), R.nodes.size() * sizeof(uint4), cudaMemcpyHostToDevice, c->stream));
@@ -1213,7 +1249,9 @@ int launch_gbuffer(b200rt_ctx *c, const float *cam, int width, int height, const
   float *k = static_cast<float *>(c->d_dn_k.p);
   int rc = launch_primary(c, A, effective_traversal(c, og), use_smem_scene(c), true, og.collect_stats != 0, tri, k);
   if (rc) return rc;
-  auto kg = (o.sampling & B200RT_SAMPLING_SMOOTH_NORMALS) ? k_gbuffer<true> : k_gbuffer<false>;
+  const bool smooth = (o.sampling & B200RT_SAMPLING_SMOOTH_NORMALS) != 0;
+  const bool tex = (o.sampling & B200RT_SAMPLING_TEXTURES) != 0 && c->n_mat_tex > 0;
+  auto kg = tex ? (smooth ? k_gbuffer<true, true> : k_gbuffer<false, true>) : (smooth ? k_gbuffer<true> : k_gbuffer<false>);
   kg<<<(unsigned)((npix + kBlock - 1) / kBlock), kBlock, 0, c->stream>>>(A, tri, k, gbuffer_view(c), d_rgb,
                                                                           static_cast<float4 *>(c->d_dn_col[0].p));
   CU(cudaGetLastError());
@@ -1264,10 +1302,10 @@ extern "C" {
 int b200rt_set_scene(b200rt_ctx *c, const float *vp, int64_t n_vp, const float *vn, int64_t n_vn, const float *vuv,
                      int64_t n_vuv, const int32_t *face, int64_t n_face, const float *mat, int64_t n_mat,
                      const int32_t *light, int64_t n_light, const float *bvh, int64_t n_bvh) {
-  (void)vuv; (void)n_vuv; (void)light; (void)n_light;  // fetched / passed but never used by the kernel (MathLib.cl:217, Raytracing.cl:163)
+  (void)light; (void)n_light;  // passed but never used by the kernel (Raytracing.cl:163)
   if (!c) return B200RT_ERR_INVALID;
   auto t0 = std::chrono::steady_clock::now();
-  const SceneArgs a{vp, n_vp, vn, n_vn, face, n_face, mat, n_mat, bvh, n_bvh};
+  const SceneArgs a{vp, n_vp, vn, n_vn, vuv, n_vuv, face, n_face, mat, n_mat, bvh, n_bvh};
   int rc = check_scene_args(c, a);
   if (rc) return rc;
   const uint64_t h = scene_hash_of(a);
@@ -1283,6 +1321,7 @@ int b200rt_set_scene(b200rt_ctx *c, const float *vp, int64_t n_vp, const float *
       c->scene_hash = 0;
       return fail(c, rc, "%s", msg.c_str());
     }
+    repack_uvs(vuv, n_vuv, face, &R);
     rc = upload_scene(c, R, a, h);
   }
   c->stats.upload_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -1331,6 +1370,64 @@ int b200rt_set_ibl(b200rt_ctx *c, const uint8_t *rgba, int width, int height) {
   c->ibl_hash = h;
   ++c->scene_epoch;
   c->have_ibl = true;
+  c->stats.upload_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  return 0;
+}
+
+int b200rt_set_textures(b200rt_ctx *c, const uint8_t *texels, int64_t n_texel_bytes, const int32_t *dims, int n_textures,
+                        const int32_t *material_texture, int64_t n_materials) {
+  if (!c) return B200RT_ERR_INVALID;
+  if (n_textures < 0 || n_texel_bytes < 0 || n_materials < 0)
+    return fail(c, B200RT_ERR_INVALID, "negative texture count (%d textures, %lld bytes, %lld materials)", n_textures,
+                (long long)n_texel_bytes, (long long)n_materials);
+  if ((!texels && n_texel_bytes) || (!dims && n_textures) || (!material_texture && n_materials))
+    return fail(c, B200RT_ERR_INVALID, "NULL texture buffer with a nonzero count");
+  if (n_materials > 0x7fffffffLL) return fail(c, B200RT_ERR_UNSUPPORTED, "%lld materials", (long long)n_materials);
+  // per texture: index of its first texel, w, h; every texel index must fit the kernels' int32 arithmetic
+  std::vector<int4> info((size_t)n_textures);
+  long long total = 0;
+  for (int i = 0; i < n_textures; ++i) {
+    const int w = dims[2 * i], h = dims[2 * i + 1];
+    if (w < 1 || h < 1) return fail(c, B200RT_ERR_INVALID, "texture %d is %d x %d texels", i, w, h);
+    if (w > (1 << 24) || h > (1 << 24))
+      return fail(c, B200RT_ERR_UNSUPPORTED, "texture %d is %d x %d texels: at most 2^24 a side", i, w, h);
+    info[(size_t)i] = make_int4((int)total, w, h, 0);
+    total += (long long)w * h;
+    if (total > 0x7fffffffLL) return fail(c, B200RT_ERR_UNSUPPORTED, "textures of more than 2^31 - 1 texels in all");
+  }
+  if (n_texel_bytes != total * 4)
+    return fail(c, B200RT_ERR_INVALID, "%lld texel bytes for textures of %lld texels (4 bytes each)",
+                (long long)n_texel_bytes, total);
+  for (int64_t m = 0; m < n_materials; ++m)
+    if (material_texture[m] < -1 || material_texture[m] >= n_textures)
+      return fail(c, B200RT_ERR_INVALID, "material %lld has texture %d; expected -1 or an index below %d", (long long)m,
+                  (int)material_texture[m], n_textures);
+  auto t0 = std::chrono::steady_clock::now();
+  uint64_t h = hash_bytes(texels, (size_t)n_texel_bytes, 0x746578ull);
+  h = hash_bytes(dims, (size_t)n_textures * 2 * sizeof(int32_t), h);
+  h = hash_bytes(material_texture, (size_t)n_materials * sizeof(int32_t), h);
+  if (c->tex_hash != 0 && h == c->tex_hash) return 0;
+  CU(cudaSetDevice(c->device));
+  c->tex_hash = 0;    // nothing bound until every copy has succeeded
+  c->n_mat_tex = 0;
+  ++c->scene_epoch;
+  if (n_textures > 0) {   // one buffer: the int4 per texture, the int32 per material (padded to 4), the texels
+    DevBuf &d_tex = c->d_scene[kTex];
+    const size_t mat_off = info.size() * sizeof(int4);
+    const size_t texel_off = mat_off + (((size_t)n_materials + 3) & ~(size_t)3) * sizeof(int32_t);
+    if (ensure(c, d_tex, texel_off + (size_t)n_texel_bytes)) return B200RT_ERR_CUDA;
+    char *base = static_cast<char *>(d_tex.p);
+    CU(cudaMemcpyAsync(base, info.data(), mat_off, cudaMemcpyHostToDevice, c->stream));
+    if (n_materials > 0)
+      CU(cudaMemcpyAsync(base + mat_off, material_texture, (size_t)n_materials * sizeof(int32_t), cudaMemcpyHostToDevice,
+                         c->stream));
+    CU(cudaMemcpyAsync(base + texel_off, texels, (size_t)n_texel_bytes, cudaMemcpyHostToDevice, c->stream));
+    c->n_mat_tex = (int)n_materials;
+    c->n_tex = n_textures;
+  }
+  if (c->have_scene && write_tex_header(c, c->scene.n_tris)) return B200RT_ERR_CUDA;
+  CU(cudaStreamSynchronize(c->stream));
+  c->tex_hash = h;
   c->stats.upload_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
   return 0;
 }
@@ -1420,6 +1517,7 @@ int b200rt_gbuffer(b200rt_ctx *c, const float *cam, int width, int height, const
   if (!rc && (o.pixel_end > 0 || o.tile_row_mod > 1))
     rc = fail(c, B200RT_ERR_INVALID, "the G-buffer covers the whole frame: no pixel range or tile rows");
   if (!rc) rc = check_smooth_scene(c, o);
+  if (!rc) rc = check_uv_scene(c, o);
   if (rc) return rc;
   CU(cudaSetDevice(c->device));
   const size_t npix = (size_t)width * height;
@@ -1521,6 +1619,7 @@ int b200rt_invalidate(b200rt_ctx *c) {
   c->scene_hash = 0;
   c->mat_hash = 0;
   c->ibl_hash = 0;
+  c->tex_hash = 0;
   c->have_scene_cached = false;
   return 0;
 }
@@ -1833,10 +1932,10 @@ b200rt_ctx *b200rt_multi_context(b200rt_multi *m, int index) {
 int b200rt_multi_set_scene(b200rt_multi *m, const float *vp, int64_t n_vp, const float *vn, int64_t n_vn, const float *vuv,
                            int64_t n_vuv, const int32_t *face, int64_t n_face, const float *mat, int64_t n_mat,
                            const int32_t *light, int64_t n_light, const float *bvh, int64_t n_bvh) {
-  (void)vuv; (void)n_vuv; (void)light; (void)n_light;
+  (void)light; (void)n_light;
   if (!m) return B200RT_ERR_INVALID;
   auto t0 = std::chrono::steady_clock::now();
-  const SceneArgs a{vp, n_vp, vn, n_vn, face, n_face, mat, n_mat, bvh, n_bvh};
+  const SceneArgs a{vp, n_vp, vn, n_vn, vuv, n_vuv, face, n_face, mat, n_mat, bvh, n_bvh};
   int rc = check_scene_args(m->ctx[0], a);
   if (rc) { m->err = m->ctx[0]->err; return rc; }
   const uint64_t h = scene_hash_of(a);
@@ -1850,6 +1949,7 @@ int b200rt_multi_set_scene(b200rt_multi *m, const float *vp, int64_t n_vp, const
       for (b200rt_ctx *c : m->ctx) { c->have_scene = false; c->have_scene_cached = false; c->scene_hash = 0; }
       return fail(m, rc, "%s", msg.c_str());
     }
+    repack_uvs(vuv, n_vuv, face, &R);
   }
   int bad = 0;
   rc = run_parts((int)m->ctx.size(), &bad, [&](int i) {
@@ -1866,6 +1966,17 @@ int b200rt_multi_set_ibl(b200rt_multi *m, const uint8_t *rgba, int width, int he
   if (!m) return B200RT_ERR_INVALID;
   int bad = 0;
   const int rc = run_parts((int)m->ctx.size(), &bad, [&](int i) { return b200rt_set_ibl(m->ctx[i], rgba, width, height); });
+  if (rc) return fail(m, rc, "GPU %d: %s", m->ctx[bad]->device, m->ctx[bad]->err.c_str());
+  return 0;
+}
+
+int b200rt_multi_set_textures(b200rt_multi *m, const uint8_t *texels, int64_t n_texel_bytes, const int32_t *dims,
+                              int n_textures, const int32_t *material_texture, int64_t n_materials) {
+  if (!m) return B200RT_ERR_INVALID;
+  int bad = 0;
+  const int rc = run_parts((int)m->ctx.size(), &bad, [&](int i) {
+    return b200rt_set_textures(m->ctx[i], texels, n_texel_bytes, dims, n_textures, material_texture, n_materials);
+  });
   if (rc) return fail(m, rc, "GPU %d: %s", m->ctx[bad]->device, m->ctx[bad]->err.c_str());
   return 0;
 }

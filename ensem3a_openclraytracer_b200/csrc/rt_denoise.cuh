@@ -22,8 +22,9 @@ struct GBufferView {
 };
 
 // SMOOTH (B200RT_SAMPLING_SMOOTH_NORMALS): the normal of a hit on a curved triangle is the normalised shading normal at
-// the render's point cam_pos + unit(d) * k
-template <bool SMOOTH>
+// the render's point cam_pos + unit(d) * k.  TEX (B200RT_SAMPLING_TEXTURES): the albedo of a type-1 or type-2 hit is
+// surface_albedo at that point.
+template <bool SMOOTH, bool TEX = false>
 __global__ void __launch_bounds__(kBlock) k_gbuffer(const __grid_constant__ KernelArgs A, const int *__restrict__ tri,
                                                     const float *__restrict__ k, GBufferView G,
                                                     const float *__restrict__ rgb, float4 *__restrict__ col) {
@@ -50,6 +51,8 @@ __global__ void __launch_bounds__(kBlock) k_gbuffer(const __grid_constant__ Kern
         nrm = (isfinite(un.x) && isfinite(un.y) && isfinite(un.z)) ? un : mk3(0.0f, 0.0f, 0.0f);
       }
     }
+    if (TEX && (m.type == 1 || m.type == 2))
+      alb = surface_albedo(S, A.n_tris, t, tri_material(S, t), m.color, A.F.cam_pos + unit(d) * __ldg(k + i));
     pos = A.F.cam_pos + d * __ldg(k + i);
   }
   G.gn[i] = make_float4(nrm.x, nrm.y, nrm.z, kind);

@@ -404,6 +404,20 @@ __global__ void __launch_bounds__(kCompactBlock) k_compact(const int *__restrict
 // normals buffer holds n_tris first-vertex normals, then 2 float4 per triangle: (n1.xyz, flat / curved flag), (n2.xyz, -)
 // (scene_repack.h).  *curved: the triangle is not flat, so its precomputed frame does not apply and tri_frame_at builds
 // one.
+// The barycentrics (b0, b1, b2) of point x on triangle `tri` by the rule b200rt.h states for smooth shading, which
+// albedo textures share.
+RT_DEV v3 barycentrics(const SceneView &S, int tri, v3 x) {
+  const Tri t = load_tri(S.tris, tri);
+  const v3 p = x - t.A;
+  const float d00 = dot(t.e1, t.e1), d01 = dot(t.e1, t.e2), d11 = dot(t.e2, t.e2);
+  const float d20 = dot(p, t.e1), d21 = dot(p, t.e2);
+  const float den = d00 * d11 - d01 * d01;
+  const float b1 = (d11 * d20 - d01 * d21) / den;
+  const float b2 = (d00 * d21 - d01 * d20) / den;
+  const float b0 = (1.0f - b1) - b2;
+  return mk3(b0, b1, b2);
+}
+
 template <bool SMOOTH>
 RT_DEV v3 shading_normal(const SceneView &S, int n_tris, int tri, v3 n0, v3 x, bool *curved) {
   *curved = false;
@@ -413,17 +427,35 @@ RT_DEV v3 shading_normal(const SceneView &S, int n_tris, int tri, v3 n0, v3 x, b
   if (!(c1.w > 0.0f)) return n0;   // flat (scene_repack.h kSmoothFlat; kSmoothBadIndex never reaches a render)
   *curved = true;
   const float4 c2 = __ldg(nsmooth + 2 * (size_t)tri + 1);
-  const Tri t = load_tri(S.tris, tri);
-  const v3 p = x - t.A;
-  const float d00 = dot(t.e1, t.e1), d01 = dot(t.e1, t.e2), d11 = dot(t.e2, t.e2);
-  const float d20 = dot(p, t.e1), d21 = dot(p, t.e2);
-  const float den = d00 * d11 - d01 * d01;
-  const float b1 = (d11 * d20 - d01 * d21) / den;
-  const float b2 = (d00 * d21 - d01 * d20) / den;
-  const float b0 = (1.0f - b1) - b2;
-  const v3 n = unit(((n0 * b0) + (mk3(c1.x, c1.y, c1.z) * b1)) + (mk3(c2.x, c2.y, c2.z) * b2));
+  const v3 b = barycentrics(S, tri, x);
+  const v3 n = unit(((n0 * b.x) + (mk3(c1.x, c1.y, c1.z) * b.y)) + (mk3(c2.x, c2.y, c2.z) * b.z));
   if (!isfinite(n.x) || !isfinite(n.y) || !isfinite(n.z) || !(dot(n, n) > 0.0f)) return n0;
   return n;
+}
+
+// ---- opt-in albedo textures (b200rt_opts.sampling bit B200RT_SAMPLING_TEXTURES) -----------------------------------------
+// The albedo of a type-1 or type-2 hit on triangle `tri` (material `mat`, colour `color`) at point x, by the rule b200rt.h
+// states: color times the texture factor at the interpolated UV, or color itself when the material has no texture.  The
+// normals buffer holds, after the smooth-shading records, 2 float4 of UVs per triangle, (u0, v0, u1, v1), (u2, v2, -, -),
+// and then one texture header (b200rt_api.cu write_tex_header): the address of the texture buffer (low, high word), the
+// materials it covers, the textures it holds.  That buffer holds an int4 per texture (first texel, w, h, -), an int32 per
+// material (its texture or -1, padded to a multiple of 4), then the texels.  Kept out of KernelArgs, so that no existing
+// kernel's parameters move.
+RT_DEV v3 surface_albedo(const SceneView &S, int n_tris, int tri, int mat, v3 color, v3 x) {
+  const float4 *uv = S.normals + 3 * (size_t)n_tris;
+  const uint4 hd = __ldg(reinterpret_cast<const uint4 *>(uv + 2 * (size_t)n_tris));
+  if ((unsigned)mat >= hd.z) return color;
+  TexView T;
+  T.info = reinterpret_cast<const int4 *>(((unsigned long long)hd.y << 32) | hd.x);
+  const int *mat_tex = reinterpret_cast<const int *>(T.info + hd.w);
+  const int tex = __ldg(mat_tex + mat);
+  if (tex < 0) return color;
+  T.texels = reinterpret_cast<const uchar4 *>(mat_tex + ((hd.z + 3u) & ~3u));
+  const float4 q0 = __ldg(uv + 2 * (size_t)tri), q1 = __ldg(uv + 2 * (size_t)tri + 1);
+  const v3 b = barycentrics(S, tri, x);
+  const float u = (q0.x * b.x + q0.z * b.y) + q1.x * b.z;
+  const float v = (q0.y * b.x + q0.w * b.y) + q1.y * b.z;
+  return color * texture_factor(T, tex, u, v);
 }
 
 // ---- shading ----------------------------------------------------------------------------------------------------
@@ -439,8 +471,9 @@ RT_DEV v3 shading_normal(const SceneView &S, int n_tris, int tri, v3 n0, v3 x, b
 // (B200RT_SAMPLING_SMOOTH_NORMALS): a hit on a curved triangle is shaded with the interpolated normal and a frame built
 // in registers (shading_normal, tri_frame_at); a flat one keeps its precomputed frame.  GLASS = opt-in refractive glass
 // (B200RT_SAMPLING_DIELECTRIC_GLASS): a glass hit whose ior slot is not 1 reflects or refracts (scatter_dielectric)
-// instead of passing through.
-template <bool NEE, bool ADAPT, bool JITTER = false, bool SMOOTH = false, bool GLASS = false>
+// instead of passing through.  TEX = opt-in albedo textures (B200RT_SAMPLING_TEXTURES): a diffuse or glossy surface
+// whose material has a texture takes surface_albedo for its colour in the light sample (phase 3b) and the scatter (4).
+template <bool NEE, bool ADAPT, bool JITTER = false, bool SMOOTH = false, bool GLASS = false, bool TEX = false>
 __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant__ KernelArgs A, int iter) {
   const FrameParams &F = A.F;
   const SceneView &S = A.S;
@@ -643,7 +676,7 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
     if (NEE && want_light) {
       const float4 nn = __ldg(S.normals + htri);
       v3 n = mk3(nn.x, nn.y, nn.z);
-      const Material m = load_material(S.mats, tri_material(S, htri));
+      Material m = load_material(S.mats, tri_material(S, htri));
       v3 un = unit(n);
       float ul, ua, ub;
       if (F.rng_mode == 0) draw3_light<0>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, F.key0, F.key1, &ul, &ua, &ub);
@@ -660,6 +693,7 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
         n = shading_normal<true>(S, A.n_tris, htri, n, x, &curved);
         un = unit(n);
       }
+      if (TEX) m.color = surface_albedo(S, A.n_tris, htri, tri_material(S, htri), m.color, x);
       v3 w;
       const v3 direct = sample_light(m, F.sampling, n, un, x, d, acc, l.A, l.e1, l.e2, Le, A.n_light, ua, ub, &w);
       A.pS[pix] = make_float4(d.x, d.y, d.z, __int_as_float(htri));
@@ -675,7 +709,9 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
       const float4 nn = __ldg(S.normals + htri);
       bool curved;   // the surface point: o itself when the light ray is back at it (phase 3b moved o there)
       const v3 n = shading_normal<SMOOTH>(S, A.n_tris, htri, mk3(nn.x, nn.y, nn.z), (NEE && from_light) ? o : o + unit(d) * hk, &curved);
-      const Material m = load_material(S.mats, tri_material(S, htri));
+      Material m = load_material(S.mats, tri_material(S, htri));
+      if (TEX && (m.type == 1 || m.type == 2))
+        m.color = surface_albedo(S, A.n_tris, htri, tri_material(S, htri), m.color, (NEE && from_light) ? o : o + unit(d) * hk);
       const int which = m.type == 3 ? 0 : (m.type == 1 ? 1 : 2);
       const TriFrame tf = curved ? tri_frame_at(n, which) : load_tri_frame(S.frames, htri, which);
       v3 nd, brdf;

@@ -237,6 +237,43 @@ RT_DEV v3 scatter_dielectric(v3 d, v3 un, float ior, float u, bool *reflected) {
   return w * eta + m * (eta * ci - ct);
 }
 
+// ---- opt-in: albedo textures (b200rt_opts.sampling bit B200RT_SAMPLING_TEXTURES) ---------------------------------------
+// The bound textures (b200rt_set_textures) are read through the read-only data path.  The texture unit's bilinear filter
+// is not used: its 8-bit fractional weights are not the float weights b200rt.h states.
+struct TexView {
+  const int4 *info;       // per texture: index of its first texel, w, h, -
+  const uchar4 *texels;   // every texture's texels back to back, row-major, top row first
+};
+
+RT_DEV float lerpf(float a, float b, float t) { return a + (b - a) * t; }
+
+RT_DEV v3 texel_value(const TexView &T, int base, int w, int x, int y) {
+  const uchar4 c = __ldg(T.texels + base + y * w + x);
+  return mk3(__fdiv_rn((float)c.x, 255.0f), __fdiv_rn((float)c.y, 255.0f), __fdiv_rn((float)c.z, 255.0f));
+}
+
+RT_DEV int wrap_index(int i, int n) {
+  const int r = i % n;
+  return r < 0 ? r + n : r;
+}
+
+// The texture factor f of b200rt.h at (u, v): repeat wrap, bilinear as lerps between the four texels around the point.
+RT_DEV v3 texture_factor(const TexView &T, int tex, float u, float v) {
+  if (!isfinite(u) || !isfinite(v)) return mk3(1.0f, 1.0f, 1.0f);
+  const int4 info = __ldg(T.info + tex);
+  const int w = info.y, h = info.z;
+  const float fu = u - floorf(u), fv = v - floorf(v);
+  const float tx = fu * (float)w - 0.5f, ty = (1.0f - fv) * (float)h - 0.5f;
+  const int x0 = (int)floorf(tx), y0 = (int)floorf(ty);
+  const float ax = tx - (float)x0, ay = ty - (float)y0;
+  const int xa = wrap_index(x0, w), xb = wrap_index(x0 + 1, w), ya = wrap_index(y0, h), yb = wrap_index(y0 + 1, h);
+  const v3 c00 = texel_value(T, info.x, w, xa, ya), c10 = texel_value(T, info.x, w, xb, ya);
+  const v3 c01 = texel_value(T, info.x, w, xa, yb), c11 = texel_value(T, info.x, w, xb, yb);
+  const v3 top = mk3(lerpf(c00.x, c10.x, ax), lerpf(c00.y, c10.y, ax), lerpf(c00.z, c10.z, ax));
+  const v3 bot = mk3(lerpf(c01.x, c11.x, ax), lerpf(c01.y, c11.y, ax), lerpf(c01.z, c11.z, ax));
+  return mk3(lerpf(top.x, bot.x, ay), lerpf(top.y, bot.y, ay), lerpf(top.z, bot.z, ay));
+}
+
 RT_DEV float ipow(float x, int n) {  // pown: repeated multiply from 1
   float r = 1.0f;
   for (int i = 0; i < n; ++i) r = r * x;

@@ -92,6 +92,29 @@ struct HostThreads {
 
 }  // namespace
 
+void repack_uvs(const float *vuv, int64_t n_vuv, const int32_t *face, Repacked *out) {
+  HostThreads host_threads;
+  Repacked &R = *out;
+  const int n_tris = R.n_tris;
+  const int64_t nuv = vuv && n_vuv > 0 ? n_vuv / 2 : 0;
+  R.uvs.resize((size_t)n_tris * 2);
+  int uv_bad = n_tris;
+#pragma omp parallel for schedule(static) reduction(min : uv_bad)
+  for (int t = 0; t < n_tris; ++t) {
+    const int32_t *f = face + 10 * (size_t)t;
+    if (f[1] >= 0 && f[1] < nuv && f[2] >= 0 && f[2] < nuv && f[3] >= 0 && f[3] < nuv) {
+      const float *a = vuv + 2 * (size_t)f[1], *b = vuv + 2 * (size_t)f[2], *c = vuv + 2 * (size_t)f[3];
+      R.uvs[2 * (size_t)t] = Repacked::f4{a[0], a[1], b[0], b[1]};
+      R.uvs[2 * (size_t)t + 1] = Repacked::f4{c[0], c[1], 0.0f, 0.0f};
+    } else {
+      R.uvs[2 * (size_t)t] = Repacked::f4{0.0f, 0.0f, 0.0f, 0.0f};
+      R.uvs[2 * (size_t)t + 1] = Repacked::f4{0.0f, 0.0f, 0.0f, 0.0f};
+      if (t < uv_bad) uv_bad = t;
+    }
+  }
+  R.uv_bad = uv_bad < n_tris ? uv_bad : -1;
+}
+
 int repack_scene(const float *vp, int64_t n_vp, const float *vn, int64_t n_vn, const int32_t *face, int64_t n_face,
                  int64_t n_materials, const float *bvh, int64_t n_bvh, Repacked *out, std::string *err, bool own_tree) {
   HostThreads host_threads;

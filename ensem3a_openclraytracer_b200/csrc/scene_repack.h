@@ -39,6 +39,7 @@ struct SceneDesc {
   int smooth_bad = -1;          // first triangle whose n1 or n2 index is out of range: smooth-shaded renders refuse it
   int glass_bad = -1;           // first glass material whose ior is negative, NaN or infinite: renders with refractive
   float glass_bad_ior = 0.0f;   // glass refuse it (set by b200rt_set_materials, not by the repack)
+  int uv_bad = -1;              // first triangle with a UV index out of range: textured renders refuse it (repack_uvs)
 };
 
 // .w of the first `nsmooth` record of a triangle (opt-in smooth shading, b200rt.h B200RT_SAMPLING_SMOOTH_NORMALS)
@@ -52,6 +53,7 @@ struct Repacked : SceneDesc {
   raw_vector<u4> nodes;         // node_f4 x 16 bytes per interior node (rt_trace.cuh "repacked scene")
   raw_vector<f4> tris, normals, tboxes;
   raw_vector<f4> nsmooth;       // 2 per triangle: (n1.xyz, kSmooth* flag), (n2.xyz, 0)
+  raw_vector<f4> uvs;           // 2 per triangle: (u0, v0, u1, v1), (u2, v2, 0, 0) — opt-in albedo textures (repack_uvs)
   raw_vector<f4> ctris;         // the triangle records in the order of the culling tree's leaves (what leaf refs index); .w of the
                                 // third vector = the triangle's id
   std::vector<int32_t> tri_mat;
@@ -81,5 +83,10 @@ size_t lane_smem_bytes_host(int stack_depth);
 // own_tree: build the culling tree here (cull_tree.cpp) instead of taking the caller's topology over.
 int repack_scene(const float *vp, int64_t n_vp, const float *vn, int64_t n_vn, const int32_t *face, int64_t n_face,
                  int64_t n_materials, const float *bvh, int64_t n_bvh, Repacked *out, std::string *err, bool own_tree = true);
+
+// The UV records of a repacked scene (opt-in albedo textures, b200rt.h B200RT_SAMPLING_TEXTURES): out->uvs from V_uv
+// (n_vuv floats, may be NULL) and faceData[10t+1 .. 10t+3]; a triangle with an index out of range gets zeros and the
+// first such one goes to out->uv_bad.  Never refuses: only textured renders read the records.
+void repack_uvs(const float *vuv, int64_t n_vuv, const int32_t *face, Repacked *out);
 
 }  // namespace b200rt

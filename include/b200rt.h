@@ -56,7 +56,7 @@ typedef enum {
 /* Anti-aliasing: every sample traces its own camera ray through a jittered point of its pixel.  Unlike bits 0 and 1
  * this bit CHANGES THE INTEGRAND: the image converges to the box-filtered (pixel-area) image, no longer to the
  * reference's, whose pixel is one point (one camera ray per pixel, whose hit every sample restarts from,
- * Raytracing.cl:184-187).  Its value is 8: 4, 16 and 64 are not assigned and are refused, as is any bit above 128.  The rule, in
+ * Raytracing.cl:184-187).  Its value is 8: 4, 16, 64 and 256 are not assigned and are refused, as is any bit above 512.  The rule, in
  * binary32 with every operation rounded separately (no contraction):
  *   - (ux, uy) are two uniforms in [0, 1): with B200RT_RNG_PHILOX words 0 and 1 of the block at counter (i, s, 0, 2) for
  *     sample s of work-item i (direction sampling uses n = 0, light sampling n = 1); with B200RT_RNG_REFERENCE the pixel
@@ -141,6 +141,35 @@ typedef enum {
  * accept what they accept without it; a render with the bit refuses (B200RT_ERR_INVALID) a material set in which a glass
  * material has a negative, NaN or infinite ior, and its message names the first such material.  The ior of a material
  * of another type is never read. */
+#define B200RT_SAMPLING_TEXTURES 512
+/* Albedo textures: a diffuse or glossy surface takes its colour from an RGBA8 image bound to its material
+ * (b200rt_set_textures), sampled at the hit's interpolated texture coordinates, instead of the flat material colour.
+ * The reference reads every OBJ `vt` record into V_uv and keeps three UV indices per triangle (faceData[10t+1 .. 10t+3])
+ * but never uses them (MathLib.cl:203-228).  This bit CHANGES THE INTEGRAND.  The rule, in binary32 with every operation
+ * rounded separately (no contraction) and true division, for a hit on triangle t whose material m is of type 1 or 2 and
+ * has a bound texture T (w x h texels, RGBA8, row 0 at the top):
+ *   - x and the barycentrics b0, b1, b2 are those of B200RT_SAMPLING_SMOOTH_NORMALS (x = o + unit(d) * k; on a light
+ *     ray's return the stored surface point; for the G-buffer cam_pos + unit(d) * k);
+ *   - uv_k = V_uv[2 * faceData[10t+1+k] .. +1]; u = (u0*b0 + u1*b1) + u2*b2, and v likewise; if u or v is not finite the
+ *     texture factor is f = (1, 1, 1);
+ *   - repeat wrap: fu = u - floorf(u), fv = v - floorf(v); tx = fu*(float)w - 0.5f, ty = (1.0f - fv)*(float)h - 0.5f
+ *     (1 - fv puts OBJ's v = 1 on the top row); x0 = (int)floorf(tx), ax = tx - (float)x0, y0 and ay likewise; the
+ *     texel columns x0 and x0+1 and rows y0 and y0+1 are each taken modulo the extent into [0, extent);
+ *   - a texel's value is c = byte / 255.0f per channel, as for the environment map (no sRGB decode); alpha is ignored;
+ *   - bilinear as lerps, lerp(a, b, t) = a + (b - a)*t: first along x for both rows, then along y, so that a uniform
+ *     texture returns its value exactly (a white one exactly 1.0f);
+ *   - albedo = m.color * f per component.  It replaces m.color wherever a type-1 or type-2 surface reads its colour:
+ *     the diffuse BRDF (Raytracing.cl:58-66), BRDF_GGX's diffuse term, the light sample's BRDF with
+ *     B200RT_SAMPLING_LIGHTS, and the G-buffer albedo of kind-1 pixels.  The texture of a type-0 or type-3 material is
+ *     never read (emitters, glass tint and the sun through glass keep the colour).  No direction, density or path length
+ *     depends on the albedo, so rays, samples, wave_iterations and kernel_launches are those of the render without the
+ *     bit, whatever texture is bound; with no texture bound the image is too.
+ * Known limits: no mipmapping (a minified texture aliases until enough samples average it), no sRGB decode, no alpha,
+ * no normal or roughness maps.
+ * Every render entry point takes the bit, alone or with bits 1, 2, 8, 32 and 128 (b200rt_render_adaptive still refuses 8);
+ * b200rt_gbuffer and b200rt_render_denoised use it for the albedo; b200rt_primary_hits and b200rt_trace_rays ignore it.
+ * b200rt_set_scene keeps the scene's UVs and accepts a triangle whose UV index is out of range; a render or G-buffer with
+ * the bit refuses (B200RT_ERR_INVALID) such a scene, and its message names the first such triangle. */
 
 /* output modes */
 #define B200RT_OUT_FINAL 0 /* mean over spp, clamped to [0,1]  (Raytracing.cl:211-219) */
@@ -221,6 +250,16 @@ int b200rt_set_materials(b200rt_ctx *ctx, const float *material_data, int64_t n_
 
 /* RGBA8 environment map, row-major, top row first.  Replaces cl.Image(...), KernelLauncher.py:71-72. */
 int b200rt_set_ibl(b200rt_ctx *ctx, const uint8_t *rgba, int width, int height);
+
+/* Albedo textures of B200RT_SAMPLING_TEXTURES.  The textures lie back to back in `texels` (w*h*4 bytes each, RGBA8,
+ * row-major, top row first); dims holds 2 int32 per texture (w, h), each >= 1; material_texture[m] is -1 (untextured)
+ * or the index of material m's texture, for the n_materials first materials (the others are untextured).  n_textures == 0
+ * unbinds.  Refused (B200RT_ERR_INVALID): a NULL pointer with a nonzero count, a negative count, w or h < 1, a byte count
+ * that is not the sum of w*h*4, an index outside [-1, n_textures); B200RT_ERR_UNSUPPORTED: w or h above 2^24 or more than
+ * 2^31 - 1 texels in all.  The upload is cached by content (b200rt_invalidate forgets it).  Bindings survive
+ * b200rt_set_scene and b200rt_set_materials. */
+int b200rt_set_textures(b200rt_ctx *ctx, const uint8_t *texels, int64_t n_texel_bytes, const int32_t *dims,
+                        int n_textures, const int32_t *material_texture, int64_t n_materials);
 
 /* The `Raytracing` kernel + blocking read-back, KernelLauncher.py:76-78.  cam = 10 floats, env = 5
  * floats (main.py:59-61,72-73).  width must equal (int)cam[6]; the frame has width*height work-items
@@ -417,6 +456,8 @@ int b200rt_multi_set_scene(b200rt_multi *m, const float *vertex_p, int64_t n_ver
                            int64_t n_face_data, const float *material_data, int64_t n_material_data,
                            const int32_t *light_data, int64_t n_light_data, const float *bvh, int64_t n_bvh);
 int b200rt_multi_set_ibl(b200rt_multi *m, const uint8_t *rgba, int width, int height);
+int b200rt_multi_set_textures(b200rt_multi *m, const uint8_t *texels, int64_t n_texel_bytes, const int32_t *dims,
+                              int n_textures, const int32_t *material_texture, int64_t n_materials);
 int b200rt_multi_invalidate(b200rt_multi *m);
 int b200rt_multi_render(b200rt_multi *m, const float *cam, const float *env, int width, int height, int spp,
                         int max_bounce, const b200rt_opts *opts, float *out_rgb);
