@@ -50,7 +50,11 @@ Differences a caller can observe (all documented in INTEGRATION.md):
     B200RT_SAMPLING_TEXTURES: a diffuse or glossy surface takes its colour from its material's image at the hit's
     interpolated UV (the scene's V_uv), times the material colour.  B200RT_TEXTURES=<material>=<path>[,...] loads the
     files with PIL for callers that never touch the attribute.  It combines with `adaptive`, `denoise`, `pixel_jitter`,
-    `smooth_normals`, `dielectric_glass` and `cuda_devices`.
+    `smooth_normals`, `dielectric_glass` and `cuda_devices`;
+  * `rough_glass = True` (with `dielectric_glass = True`, which it roughens) makes a glass material whose roughness slot
+    is > 0 a rough interface of GGX microfacets, so frosted glass blurs what is behind it (B200RT_SAMPLING_ROUGH_GLASS;
+    roughness 0 keeps the smooth interface).  B200RT_ROUGH_GLASS=1 (or 0) sets it for callers that never touch the
+    attribute.  It combines with `adaptive`, `denoise`, `pixel_jitter`, `smooth_normals`, `textures` and `cuda_devices`.
 """
 import math
 import os
@@ -124,6 +128,14 @@ def dielectric_glass_from_env(text):
     return t == "1"
 
 
+def rough_glass_from_env(text):
+    """The `rough_glass` flag that B200RT_ROUGH_GLASS=0 or =1 stands for; ValueError otherwise."""
+    t = str(text).strip()
+    if t not in ("0", "1"):
+        raise ValueError(f"B200RT_ROUGH_GLASS={text!r}: expected 0 or 1")
+    return t == "1"
+
+
 def smooth_normals_from_env(text):
     """The `smooth_normals` flag that B200RT_SMOOTH_NORMALS=0 or =1 stands for; ValueError otherwise."""
     t = str(text).strip()
@@ -186,6 +198,9 @@ class KernelLauncher(object):
         # False: the reference's pass-through glass; True: refractive glass (module docstring)
         self.dielectric_glass = (dielectric_glass_from_env(os.environ["B200RT_DIELECTRIC_GLASS"])
                                  if os.environ.get("B200RT_DIELECTRIC_GLASS") else False)
+        # False: glass roughness ignored; True: rough glass, with dielectric_glass (module docstring)
+        self.rough_glass = (rough_glass_from_env(os.environ["B200RT_ROUGH_GLASS"])
+                            if os.environ.get("B200RT_ROUGH_GLASS") else False)
         # None: the material colours (the reference's image); a dict: albedo textures (module docstring)
         self.textures = textures_from_env(os.environ["B200RT_TEXTURES"]) if os.environ.get("B200RT_TEXTURES") else None
         self._textures_bound = False
@@ -202,6 +217,9 @@ class KernelLauncher(object):
         if self.adaptive is not None and self.pixel_jitter:
             raise ValueError("adaptive sampling and pixel jitter cannot be combined: set launcher.adaptive = None or "
                              "launcher.pixel_jitter = False")
+        if self.rough_glass and not self.dielectric_glass:
+            raise ValueError("rough glass roughens refractive glass: set launcher.dielectric_glass = True as well, or "
+                             "launcher.rough_glass = False")
         if self.adaptive is not None and isinstance(self._ctx, _capi.MultiContext):
             raise ValueError("adaptive sampling renders on one GPU: its stopping rule needs each pixel's samples in one "
                              f"sequence, which a split over cuda_devices={self._ctx.devices} would cut apart; set "
@@ -246,7 +264,8 @@ class KernelLauncher(object):
                                sampling=((_capi.SAMPLING_PIXEL_JITTER if self.pixel_jitter else 0) |
                                          (_capi.SAMPLING_SMOOTH_NORMALS if self.smooth_normals else 0) |
                                          (_capi.SAMPLING_DIELECTRIC_GLASS if self.dielectric_glass else 0) |
-                                         (_capi.SAMPLING_TEXTURES if self.textures else 0)))
+                                         (_capi.SAMPLING_TEXTURES if self.textures else 0) |
+                                         (_capi.SAMPLING_ROUGH_GLASS if self.rough_glass else 0)))
         out = h_img_out.reshape(-1)[:imgDim * 3]
         if self.adaptive is not None:
             img, self.last_spp, _ = self._ctx.render_adaptive(cam[:10], h_envData, width, height, int(spp), int(maxBounce),

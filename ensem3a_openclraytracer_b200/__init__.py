@@ -8,7 +8,7 @@ from ._capi import (Adaptive, B200RTError, Context, Denoise, DENOISE_DEFAULTS, M
                     RNG_REFERENCE, RNG_PHILOX, TRAVERSAL_FAST, TRAVERSAL_REFERENCE, TRAVERSAL_VERIFY,
                     OUT_FINAL, OUT_SUMS, SAMPLING_REFERENCE, SAMPLING_IMPORTANCE, SAMPLING_LIGHTS,
                     SAMPLING_PIXEL_JITTER, SAMPLING_SMOOTH_NORMALS,
-                    SAMPLING_DIELECTRIC_GLASS, SAMPLING_TEXTURES)
+                    SAMPLING_DIELECTRIC_GLASS, SAMPLING_TEXTURES, SAMPLING_ROUGH_GLASS)
 from .KernelLauncher import KernelLauncher
 from .BVH import BVH
 from .progressive import ProgressiveRender
@@ -16,4 +16,5 @@ from .progressive import ProgressiveRender
 __all__ = ["Adaptive", "B200RTError", "Context", "Denoise", "DENOISE_DEFAULTS", "MultiContext", "Opts", "Stats", "make_opts", "build_library", "load_library", "LIB_PATH",
            "KernelLauncher", "BVH", "ProgressiveRender", "build_bvh", "device_count", "RNG_REFERENCE", "RNG_PHILOX", "TRAVERSAL_FAST", "TRAVERSAL_REFERENCE",
            "TRAVERSAL_VERIFY", "OUT_FINAL", "OUT_SUMS", "SAMPLING_REFERENCE", "SAMPLING_IMPORTANCE", "SAMPLING_LIGHTS",
-           "SAMPLING_PIXEL_JITTER", "SAMPLING_SMOOTH_NORMALS", "SAMPLING_DIELECTRIC_GLASS", "SAMPLING_TEXTURES"]
+           "SAMPLING_PIXEL_JITTER", "SAMPLING_SMOOTH_NORMALS", "SAMPLING_DIELECTRIC_GLASS", "SAMPLING_TEXTURES",
+           "SAMPLING_ROUGH_GLASS"]

@@ -21,6 +21,7 @@ SAMPLING_PIXEL_JITTER = 8   # anti-aliasing: changes the integrand to the pixel'
 SAMPLING_SMOOTH_NORMALS = 32   # smooth shading: the interpolated vertex normal at the hit (include/b200rt.h)
 SAMPLING_DIELECTRIC_GLASS = 128   # refractive glass: Fresnel reflection and Snell refraction at type 3 (include/b200rt.h)
 SAMPLING_TEXTURES = 512   # albedo textures: diffuse / glossy colour from the bound image at the hit's UV (include/b200rt.h)
+SAMPLING_ROUGH_GLASS = 2048   # rough glass: GGX microfacet glass with the roughness, needs 128 (include/b200rt.h)
 
 
 class B200RTError(RuntimeError):

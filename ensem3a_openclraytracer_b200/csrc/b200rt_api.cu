@@ -396,20 +396,28 @@ int prepare_trace_t(b200rt_ctx *c, WaveLaunch *w) {
 }
 
 // jitter and adaptive are never both set (b200rt_render_adaptive refuses the jitter bit)
-template <bool SMOOTH, bool GLASS, bool TEX>
+template <bool SMOOTH, bool GLASS, bool TEX, bool ROUGH = false>
 void pick_shade(bool nee, bool adaptive, bool jitter, WaveLaunch *w) {
-  if (jitter) w->shade = nee ? k_shade<true, false, true, SMOOTH, GLASS, TEX> : k_shade<false, false, true, SMOOTH, GLASS, TEX>;
-  else if (nee) w->shade = adaptive ? k_shade<true, true, false, SMOOTH, GLASS, TEX> : k_shade<true, false, false, SMOOTH, GLASS, TEX>;
-  else w->shade = adaptive ? k_shade<false, true, false, SMOOTH, GLASS, TEX> : k_shade<false, false, false, SMOOTH, GLASS, TEX>;
+  if (jitter) w->shade = nee ? k_shade<true, false, true, SMOOTH, GLASS, TEX, ROUGH> : k_shade<false, false, true, SMOOTH, GLASS, TEX, ROUGH>;
+  else if (nee) w->shade = adaptive ? k_shade<true, true, false, SMOOTH, GLASS, TEX, ROUGH> : k_shade<true, false, false, SMOOTH, GLASS, TEX, ROUGH>;
+  else w->shade = adaptive ? k_shade<false, true, false, SMOOTH, GLASS, TEX, ROUGH> : k_shade<false, false, false, SMOOTH, GLASS, TEX, ROUGH>;
 }
 
+// rough: rough glass, which render_impl sets only together with glass
 int prepare_wave(b200rt_ctx *c, int trav, bool smem, bool stats, bool nee, bool adaptive, bool jitter, bool smooth,
-                 bool glass, bool tex, WaveLaunch *w) {
+                 bool glass, bool tex, bool rough, WaveLaunch *w) {
   int per_sm = 0;
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shade<false, false>, kShadeBlock, 0));
   if (per_sm < 1) return fail(c, B200RT_ERR_CUDA, "k_shade does not fit on an SM");
   w->shade_grid = per_sm * c->sm_count;
-  switch ((smooth ? 1 : 0) | (glass ? 2 : 0) | (tex ? 4 : 0)) {
+  if (rough) {
+    switch ((smooth ? 1 : 0) | (tex ? 2 : 0)) {
+      case 0: pick_shade<false, true, false, true>(nee, adaptive, jitter, w); break;
+      case 1: pick_shade<true, true, false, true>(nee, adaptive, jitter, w); break;
+      case 2: pick_shade<false, true, true, true>(nee, adaptive, jitter, w); break;
+      default: pick_shade<true, true, true, true>(nee, adaptive, jitter, w); break;
+    }
+  } else switch ((smooth ? 1 : 0) | (glass ? 2 : 0) | (tex ? 4 : 0)) {
     case 0: pick_shade<false, false, false>(nee, adaptive, jitter, w); break;
     case 1: pick_shade<true, false, false>(nee, adaptive, jitter, w); break;
     case 2: pick_shade<false, true, false>(nee, adaptive, jitter, w); break;
@@ -531,8 +539,13 @@ int check_frame_args(b200rt_ctx *c, const float *cam, int width, int height, int
   if (o.traversal < 0 || o.traversal > 2) return fail(c, B200RT_ERR_INVALID, "bad traversal %d", o.traversal);
   if (o.sampling < 0 ||
       (o.sampling & ~(B200RT_SAMPLING_IMPORTANCE | B200RT_SAMPLING_LIGHTS | B200RT_SAMPLING_PIXEL_JITTER |
-                      B200RT_SAMPLING_SMOOTH_NORMALS | B200RT_SAMPLING_DIELECTRIC_GLASS | B200RT_SAMPLING_TEXTURES)) != 0)
+                      B200RT_SAMPLING_SMOOTH_NORMALS | B200RT_SAMPLING_DIELECTRIC_GLASS | B200RT_SAMPLING_TEXTURES |
+                      B200RT_SAMPLING_ROUGH_GLASS)) != 0)
     return fail(c, B200RT_ERR_INVALID, "bad sampling mode %d", o.sampling);
+  if ((o.sampling & B200RT_SAMPLING_ROUGH_GLASS) && !(o.sampling & B200RT_SAMPLING_DIELECTRIC_GLASS))
+    return fail(c, B200RT_ERR_INVALID,
+                "bad sampling mode %d: B200RT_SAMPLING_ROUGH_GLASS roughens refractive glass and needs "
+                "B200RT_SAMPLING_DIELECTRIC_GLASS too", o.sampling);
   if (o.output != B200RT_OUT_FINAL && o.output != B200RT_OUT_SUMS)
     return fail(c, B200RT_ERR_INVALID, "bad output mode %d", o.output);
   if (o.sample_end > 0) {
@@ -573,6 +586,17 @@ int check_glass_materials(b200rt_ctx *c, const b200rt_opts &o) {
   return 0;
 }
 
+// Rough glass reads the roughness slot of glass materials, which b200rt_set_materials accepts whatever it holds: a frame
+// with the bit refuses a material set in which a glass material that is not a pass-through (ior slot != 1) has a
+// negative, NaN or infinite roughness.
+int check_rough_materials(b200rt_ctx *c, const b200rt_opts &o) {
+  if ((o.sampling & B200RT_SAMPLING_ROUGH_GLASS) && c->scene.rough_bad >= 0)
+    return fail(c, B200RT_ERR_INVALID,
+                "B200RT_SAMPLING_ROUGH_GLASS: material %d is glass (type 3) with roughness %g; the roughness must be "
+                "finite and >= 0", c->scene.rough_bad, (double)c->scene.rough_bad_r);
+  return 0;
+}
+
 // Albedo textures read all three UV indices of a triangle, which b200rt_set_scene does not validate: a frame or G-buffer
 // with the bit refuses a scene that has an out-of-range one.
 int check_uv_scene(b200rt_ctx *c, const b200rt_opts &o) {
@@ -604,6 +628,8 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   const bool smooth = (o.sampling & B200RT_SAMPLING_SMOOTH_NORMALS) != 0;
   const bool glass = (o.sampling & B200RT_SAMPLING_DIELECTRIC_GLASS) != 0;
   const bool tex = (o.sampling & B200RT_SAMPLING_TEXTURES) != 0 && c->n_mat_tex > 0;   // nothing bound: the plain kernels
+  // no rough glass material: the refractive-glass kernels, which render such a material set the same
+  const bool rough = glass && (o.sampling & B200RT_SAMPLING_ROUGH_GLASS) != 0 && c->scene.rough_any;
   const long long per_sample = (nee ? 2 * ((long long)max_bounce + 1) + 1 : (long long)max_bounce + 2) + (jitter ? 1 : 0);
   const long long n_iter_ll = (long long)(F.s1 - F.s0) * per_sample;
   if (n_iter_ll > (1 << 22)) return fail(c, B200RT_ERR_UNSUPPORTED, "%lld wavefront iterations exceed 2^22", n_iter_ll);
@@ -635,7 +661,7 @@ int render_impl(b200rt_ctx *c, const float *cam, const float *env, int width, in
   A.validate = (trav == B200RT_TRAVERSAL_FAST) ? 1 : 0;
   const bool smem = use_smem_scene(c);
   WaveLaunch wl;
-  int rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, jitter, smooth, glass, tex, &wl);
+  int rc = prepare_wave(c, trav, smem, o.collect_stats != 0, nee, ad != nullptr, jitter, smooth, glass, tex, rough, &wl);
   if (rc) return rc;
   if (ensure(c, c->d_part_count, (size_t)wl.shade_grid * sizeof(unsigned int))) return B200RT_ERR_CUDA;
   A.part_count = static_cast<unsigned int *>(c->d_part_count.p);
@@ -879,6 +905,7 @@ int render_frame(b200rt_ctx *c, const float *cam, const float *env, int width, i
   int rc = check_frame_args(c, cam, width, height, spp, max_bounce, o, true, env);
   if (!rc) rc = check_smooth_scene(c, o);
   if (!rc) rc = check_glass_materials(c, o);
+  if (!rc) rc = check_rough_materials(c, o);
   if (!rc) rc = check_uv_scene(c, o);
   if (rc) return rc;
   if (!c->have_ibl) return fail(c, B200RT_ERR_NO_SCENE, "no environment map: call b200rt_set_ibl first");
@@ -1046,6 +1073,22 @@ int b200rt_set_materials(b200rt_ctx *c, const float *mat, int64_t n_mat) {
       c->scene.glass_bad = m;
       c->scene.glass_bad_ior = ior;
       break;
+    }
+  }
+  // opt-in rough glass: the first glass material whose roughness it cannot use (check_rough_materials), and whether any
+  // glass material is rough at all
+  c->scene.rough_bad = -1;
+  c->scene.rough_any = false;
+  for (int m = 0; m < nm; ++m) {
+    const float r = mat[6 * m + 4];
+    if ((int)mat[6 * m] != 3 || mat[6 * m + 5] == 1.0f) continue;
+    if (!(std::isfinite(r) && r >= 0.0f)) {
+      if (c->scene.rough_bad < 0) {
+        c->scene.rough_bad = m;
+        c->scene.rough_bad_r = r;
+      }
+    } else if (r > 0.0f) {
+      c->scene.rough_any = true;
     }
   }
   CU(cudaSetDevice(c->device));

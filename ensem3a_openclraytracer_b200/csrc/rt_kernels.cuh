@@ -473,7 +473,10 @@ RT_DEV v3 surface_albedo(const SceneView &S, int n_tris, int tri, int mat, v3 co
 // (B200RT_SAMPLING_DIELECTRIC_GLASS): a glass hit whose ior slot is not 1 reflects or refracts (scatter_dielectric)
 // instead of passing through.  TEX = opt-in albedo textures (B200RT_SAMPLING_TEXTURES): a diffuse or glossy surface
 // whose material has a texture takes surface_albedo for its colour in the light sample (phase 3b) and the scatter (4).
-template <bool NEE, bool ADAPT, bool JITTER = false, bool SMOOTH = false, bool GLASS = false, bool TEX = false>
+// ROUGH = opt-in rough glass (B200RT_SAMPLING_ROUGH_GLASS, only with GLASS): a glass hit whose ior slot is not 1 and
+// whose roughness is > 0 scatters off a GGX microfacet (scatter_rough_dielectric) and weighs the throughput by G1.
+template <bool NEE, bool ADAPT, bool JITTER = false, bool SMOOTH = false, bool GLASS = false, bool TEX = false,
+          bool ROUGH = false>
 __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant__ KernelArgs A, int iter) {
   const FrameParams &F = A.F;
   const SceneView &S = A.S;
@@ -679,8 +682,8 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
       Material m = load_material(S.mats, tri_material(S, htri));
       v3 un = unit(n);
       float ul, ua, ub;
-      if (F.rng_mode == 0) draw3_light<0>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, F.key0, F.key1, &ul, &ua, &ub);
-      else draw3_light<1>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, F.key0, F.key1, &ul, &ua, &ub);
+      if (F.rng_mode == 0) draw3<0>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, 1u, F.key0, F.key1, &ul, &ua, &ub);
+      else draw3<1>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, 1u, F.key0, F.key1, &ul, &ua, &ub);
       int idx = (int)(ul * (float)A.n_light);
       if (idx > A.n_light - 1) idx = A.n_light - 1;
       const int lt = __ldg(A.light + idx);
@@ -717,12 +720,20 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
       v3 nd, brdf;
       float inv_pdf;
       bool dielectric = false, reflected = false;
+      float wt = 1.0f;   // rough glass: G1 of the microfacet scatter, 0 for a direction on the wrong side
       if (m.type == 3) {
         const float v = GLASS ? load_material_ior(S.mats, tri_material(S, htri)) : 1.0f;
         if (v == 1.0f) {  // the reference's pass-through (always without GLASS)
           nd = d;
           brdf = m.color;
           inv_pdf = 1.0f / fabsf(dot(nd, tf.un));
+        } else if (ROUGH && m.roughness > 0.0f) {
+          float uf, u1, u2;
+          if (F.rng_mode == 0) draw3<0>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, 0u, F.key0, F.key1, &uf, &u1, &u2);
+          else draw3<1>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, 0u, F.key0, F.key1, &uf, &u1, &u2);
+          nd = scatter_rough_dielectric(d, tf.un, v == 0.0f ? kGlassDefaultIor : v, m.roughness, uf, u1, u2, &reflected,
+                                        &wt);
+          dielectric = true;
         } else {
           float u;
           if (F.rng_mode == 0) u = draw1<0>(g, (uint32_t)pix, (uint32_t)s, (uint32_t)j, F.key0, F.key1);
@@ -746,8 +757,9 @@ __global__ void __launch_bounds__(kShadeBlock, 8) k_shade(const __grid_constant_
       if (NEE) pb_ray = m.type == 3 ? 0.0f : bsdf_pdf(m, F.sampling, tf.un, d, unit(nd));
       if (!NEE || !from_light) o = o + unit(d) * hk;  // :79 — no offset along the normal
       d = nd;
-      if (GLASS && dielectric) {  // weight 1: reflection keeps the throughput, refraction tints it
+      if (GLASS && dielectric) {  // reflection keeps the throughput, refraction tints it; rough glass then weighs by G1
         if (!reflected) acc = acc * m.color;
+        if (ROUGH) acc = wt == 0.0f ? mk3(0.0f, 0.0f, 0.0f) : acc * wt;
       } else {
         const float att = inv_pdf * fabsf(dot(nd, tf.un));
         acc = (acc * brdf) * att;

@@ -264,11 +264,12 @@ RT_DEV float draw1(rng_state &g, uint32_t pixel, uint32_t sample, uint32_t bounc
   return bits_to_unit(o[0]);
 }
 
-// Three uniform draws for the light sample of bounce `j` (opt-in light sampling): the generator's next three values
-// in reference mode, the second Philox block of (pixel, sample, bounce) otherwise (the first feeds draw2).
+// Three uniform draws for bounce `j`: the generator's next three values in reference mode, words 0, 1 and 2 of the
+// Philox block (pixel, sample, bounce, n) otherwise.  The light sample (opt-in light sampling) uses n = 1, the block
+// after the one draw2 reads; rough glass (opt-in) n = 0, the block draw2 reads, which a glass hit never draws from.
 template <int RNG>
-RT_DEV void draw3_light(rng_state &g, uint32_t pixel, uint32_t sample, uint32_t bounce, uint32_t k0, uint32_t k1,
-                        float *u0, float *u1, float *u2) {
+RT_DEV void draw3(rng_state &g, uint32_t pixel, uint32_t sample, uint32_t bounce, uint32_t n, uint32_t k0, uint32_t k1,
+                  float *u0, float *u1, float *u2) {
   if (RNG == 0) {
     float u[3];
 #pragma unroll
@@ -281,7 +282,7 @@ RT_DEV void draw3_light(rng_state &g, uint32_t pixel, uint32_t sample, uint32_t 
     *u0 = u[0]; *u1 = u[1]; *u2 = u[2];
   } else {
     uint32_t o[4];
-    philox4x32_10(pixel, sample, bounce, 1u, k0, k1, o);
+    philox4x32_10(pixel, sample, bounce, n, k0, k1, o);
     *u0 = bits_to_unit(o[0]);
     *u1 = bits_to_unit(o[1]);
     *u2 = bits_to_unit(o[2]);

@@ -205,11 +205,54 @@ RT_DEV v3 sample_uniform(v3 n, const TriFrame &T, float u, float u2, float *inv_
   return apply_rotor(T.rot, local);
 }
 
+// ---- GGX microfacet pieces shared by the importance sampler of glossy surfaces and rough glass -------------------------
+// orthonormal basis (T, B) around the unit vector N (Duff et al. 2017)
+RT_DEV void basis_duff(v3 N, v3 *T, v3 *B) {
+  const float sg = copysignf(1.0f, N.z);
+  const float a = -1.0f / (sg + N.z);
+  const float b = N.x * N.y * a;
+  *T = mk3(1.0f + sg * N.x * N.x * a, sg * b, -sg * N.x);
+  *B = mk3(b, sg + N.y * N.y * a, -N.y);
+}
+
+// A normal of the GGX distribution of visible normals [Heitz 2018] of roughness al around N (basis T, B from basis_duff)
+// seen from the unit direction Vw, ndv = dot(N, Vw); (r, sp, cp) is the radius, sine and cosine of the polar point of
+// the unit disc it is drawn with.  The importance sampler of glossy surfaces and rough glass share these statements.
+RT_DEV v3 ggx_visible_normal(float al, v3 N, v3 T, v3 B, v3 Vw, float ndv, float r, float sp, float cp) {
+  const v3 Vh = unit(mk3(al * dot(Vw, T), al * dot(Vw, B), ndv));
+  const float lensq = Vh.x * Vh.x + Vh.y * Vh.y;
+  v3 T1 = mk3(1.0f, 0.0f, 0.0f);
+  if (lensq > 0.0f) {
+    const float inv = 1.0f / sqrtf(lensq);
+    T1 = mk3(-Vh.y * inv, Vh.x * inv, 0.0f);
+  }
+  const v3 T2 = cross(Vh, T1);
+  const float t1 = r * cp;
+  float t2 = r * sp;
+  const float s = 0.5f * (1.0f + Vh.z);
+  t2 = (1.0f - s) * sqrtf(fmaxf(0.0f, 1.0f - t1 * t1)) + s * t2;
+  const float t3 = sqrtf(fmaxf(0.0f, 1.0f - t1 * t1 - t2 * t2));
+  const v3 Nh = ((T1 * t1) + (T2 * t2)) + (Vh * t3);
+  const v3 hl = unit(mk3(al * Nh.x, al * Nh.y, fmaxf(0.0f, Nh.z)));
+  return ((T * hl.x) + (B * hl.y)) + (N * hl.z);
+}
+
+// Smith's separable masking term of GGX for a direction at cosine c > 0 to the normal, a2 = alpha^2
+RT_DEV float smith_g1(float a2, float c) { return (2.0f * c) / (c + sqrtf(a2 + (1.0f - a2) * c * c)); }
+
 // ---- opt-in: refractive glass (b200rt_opts.sampling bit B200RT_SAMPLING_DIELECTRIC_GLASS) -------------------------------
 constexpr float kGlassDefaultIor = 1.5f;  // B200RT_GLASS_DEFAULT_IOR: the ior of a glass material whose ior slot is 0
 
 // the raw ior slot of material idx (materialData[6 idx + 5]), which the reference's extractMaterial never reads
 RT_DEV float load_material_ior(const float *mats, int idx) { return __ldg(mats + 6 * idx + 5); }
+
+// Fresnel's reflectance of unpolarised light at an interface of relative index eta, ci the cosine on the incident side,
+// ct = sqrtf(k) the cosine of the refracted direction
+RT_DEV float fresnel(float eta, float ci, float ct) {
+  const float rs = (eta * ci - ct) / (eta * ci + ct);
+  const float rp = (ci - eta * ct) / (ci + eta * ct);
+  return 0.5f * (rs * rs + rp * rp);
+}
 
 // The smooth dielectric interface of b200rt.h: the next direction of a path that meets glass of index `ior` along d,
 // un the unit normal, u one uniform.  Reflects with Fresnel's probability F (always on total internal reflection),
@@ -227,14 +270,50 @@ RT_DEV v3 scatter_dielectric(v3 d, v3 un, float ior, float u, bool *reflected) {
   bool refl = true;
   if (k >= 0.0f) {
     ct = sqrtf(k);
-    const float rs = (eta * ci - ct) / (eta * ci + ct);
-    const float rp = (ci - eta * ct) / (ci + eta * ct);
-    const float F = 0.5f * (rs * rs + rp * rp);
-    refl = !(u >= F);
+    refl = !(u >= fresnel(eta, ci, ct));
   }
   *reflected = refl;
   if (refl) return w + m * (2.0f * ci);
   return w * eta + m * (eta * ci - ct);
+}
+
+// ---- opt-in: rough glass (b200rt_opts.sampling bit B200RT_SAMPLING_ROUGH_GLASS, on top of refractive glass) ------------
+// The GGX microfacet interface of b200rt.h [Walter et al. 2007] with alpha = roughness > 0, met along d (un the unit
+// normal, ior != 1): a microfacet normal h drawn from the visible normals seen from the incident side with (u1, u2), then
+// scatter_dielectric's Fresnel choice at h with uf.  *reflected tells which; *weight is Smith's G1 of the outgoing
+// direction, or 0 when that direction leaves on the wrong side of the surface.  c == 0, a non-finite c (un) or a
+// non-finite h take scatter_dielectric with uf and weight 1.  The caller tints a refraction by the colour, then
+// multiplies the throughput by the weight (a weight of 0 zeroes it).
+RT_DEV v3 scatter_rough_dielectric(v3 d, v3 un, float ior, float al, float uf, float u1, float u2, bool *reflected,
+                                   float *weight) {
+  const float kTwoPi = 6.2831853f;
+  const v3 w = unit(d);
+  const float c = dot(w, un);
+  const bool enter = c < 0.0f;
+  const float eta = enter ? 1.0f / ior : ior;
+  const v3 m = enter ? un : neg3(un);
+  const v3 Vw = neg3(w);
+  v3 T, B;
+  basis_duff(m, &T, &B);
+  float sp, cp;
+  cr_sincos(kTwoPi * u2, &sp, &cp);
+  const v3 h = ggx_visible_normal(al, m, T, B, Vw, dot(m, Vw), sqrtf(u1), sp, cp);
+  *weight = 1.0f;
+  if (c == 0.0f || !isfinite(c) || !isfinite(h.x) || !isfinite(h.y) || !isfinite(h.z))
+    return scatter_dielectric(d, un, ior, uf, reflected);
+  const float ch = dot(Vw, h);
+  const float k = 1.0f - (eta * eta) * (1.0f - ch * ch);
+  float ct = 0.0f;
+  bool refl = true;
+  if (k >= 0.0f) {
+    ct = sqrtf(k);
+    refl = !(uf >= fresnel(eta, ch, ct));
+  }
+  *reflected = refl;
+  const v3 nd = refl ? w + h * (2.0f * ch) : w * eta + h * (eta * ch - ct);
+  const float co = dot(nd, m);
+  *weight = (refl ? co > 0.0f : co < 0.0f) ? smith_g1(al * al, fabsf(co)) : 0.0f;
+  return nd;
 }
 
 // ---- opt-in: albedo textures (b200rt_opts.sampling bit B200RT_SAMPLING_TEXTURES) ---------------------------------------
@@ -320,7 +399,7 @@ RT_DEV float glossy_mix_pdf(float al, v3 N, v3 Vw, v3 l) {
     const float a2 = al * al;
     const float dden = ndh * ndh * (a2 - 1.0f) + 1.0f;
     const float D = a2 / (kPi * dden * dden);
-    const float G1 = (2.0f * ndv) / (ndv + sqrtf(a2 + (1.0f - a2) * ndv * ndv));
+    const float G1 = smith_g1(a2, ndv);
     pdf_spec = (G1 * D) / (4.0f * ndv);
   }
   const float ps = ndv > 0.0f ? 0.5f : 0.0f;
@@ -332,12 +411,8 @@ RT_DEV v3 sample_glossy_importance(float roughness, v3 un, v3 d_in, float u0, fl
   const v3 N = un;
   const v3 Vw = unit(neg3(d_in));
   const float ndv = dot(N, Vw);
-  // orthonormal basis around N (Duff et al. 2017)
-  const float sg = copysignf(1.0f, N.z);
-  const float a = -1.0f / (sg + N.z);
-  const float b = N.x * N.y * a;
-  const v3 T = mk3(1.0f + sg * N.x * N.x * a, sg * b, -sg * N.x);
-  const v3 B = mk3(b, sg + N.y * N.y * a, -N.y);
+  v3 T, B;
+  basis_duff(N, &T, &B);
   const bool spec = ndv > 0.0f && u0 < 0.5f;
   const float u0r = u0 < 0.5f ? u0 * 2.0f : u0 * 2.0f - 1.0f;
   const float al = roughness;
@@ -346,22 +421,7 @@ RT_DEV v3 sample_glossy_importance(float roughness, v3 un, v3 d_in, float u0, fl
   const float r = sqrtf(u0r);
   v3 l;
   if (spec) {
-    const v3 Vh = unit(mk3(al * dot(Vw, T), al * dot(Vw, B), ndv));
-    const float lensq = Vh.x * Vh.x + Vh.y * Vh.y;
-    v3 T1 = mk3(1.0f, 0.0f, 0.0f);
-    if (lensq > 0.0f) {
-      const float inv = 1.0f / sqrtf(lensq);
-      T1 = mk3(-Vh.y * inv, Vh.x * inv, 0.0f);
-    }
-    const v3 T2 = cross(Vh, T1);
-    const float t1 = r * cp;
-    float t2 = r * sp;
-    const float s = 0.5f * (1.0f + Vh.z);
-    t2 = (1.0f - s) * sqrtf(fmaxf(0.0f, 1.0f - t1 * t1)) + s * t2;
-    const float t3 = sqrtf(fmaxf(0.0f, 1.0f - t1 * t1 - t2 * t2));
-    const v3 Nh = ((T1 * t1) + (T2 * t2)) + (Vh * t3);
-    const v3 hl = unit(mk3(al * Nh.x, al * Nh.y, fmaxf(0.0f, Nh.z)));
-    const v3 h = ((T * hl.x) + (B * hl.y)) + (N * hl.z);
+    const v3 h = ggx_visible_normal(al, N, T, B, Vw, ndv, r, sp, cp);
     l = (h * (2.0f * dot(Vw, h))) - Vw;
   } else {
     l = ((T * (r * cp)) + (B * (r * sp))) + (N * sqrtf(fmaxf(0.0f, 1.0f - u0r)));

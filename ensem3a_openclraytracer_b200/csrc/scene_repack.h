@@ -39,6 +39,9 @@ struct SceneDesc {
   int smooth_bad = -1;          // first triangle whose n1 or n2 index is out of range: smooth-shaded renders refuse it
   int glass_bad = -1;           // first glass material whose ior is negative, NaN or infinite: renders with refractive
   float glass_bad_ior = 0.0f;   // glass refuse it (set by b200rt_set_materials, not by the repack)
+  int rough_bad = -1;           // first glass material with ior slot != 1 whose roughness is negative, NaN or infinite:
+  float rough_bad_r = 0.0f;     // renders with rough glass refuse it (set by b200rt_set_materials)
+  bool rough_any = false;       // some glass material has ior slot != 1 and roughness > 0: rough glass runs its kernels
   int uv_bad = -1;              // first triangle with a UV index out of range: textured renders refuse it (repack_uvs)
 };
 

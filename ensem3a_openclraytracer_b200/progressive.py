@@ -13,8 +13,8 @@ edge-avoiding à-trous filter of include/b200rt.h, with the G-buffer computed on
 
 `sampling` (a mask of the SAMPLING_* bits, e.g. SAMPLING_PIXEL_JITTER) goes into every slice's options and into the
 denoiser's G-buffer (with SAMPLING_SMOOTH_NORMALS its normal is the interpolated one, with SAMPLING_TEXTURES its albedo
-the textured one of the textures bound on `ctx`; the G-buffer ignores SAMPLING_DIELECTRIC_GLASS and describes a glass
-surface, not what is seen through it).
+the textured one of the textures bound on `ctx`; the G-buffer ignores SAMPLING_DIELECTRIC_GLASS and SAMPLING_ROUGH_GLASS
+and describes a glass surface, not what is seen through it).
 """
 import numpy as np
 

@@ -56,7 +56,7 @@ typedef enum {
 /* Anti-aliasing: every sample traces its own camera ray through a jittered point of its pixel.  Unlike bits 0 and 1
  * this bit CHANGES THE INTEGRAND: the image converges to the box-filtered (pixel-area) image, no longer to the
  * reference's, whose pixel is one point (one camera ray per pixel, whose hit every sample restarts from,
- * Raytracing.cl:184-187).  Its value is 8: 4, 16, 64 and 256 are not assigned and are refused, as is any bit above 512.  The rule, in
+ * Raytracing.cl:184-187).  Its value is 8: 4, 16, 64, 256 and 1024 are not assigned and are refused, as is any bit above 2048.  The rule, in
  * binary32 with every operation rounded separately (no contraction):
  *   - (ux, uy) are two uniforms in [0, 1): with B200RT_RNG_PHILOX words 0 and 1 of the block at counter (i, s, 0, 2) for
  *     sample s of work-item i (direction sampling uses n = 0, light sampling n = 1); with B200RT_RNG_REFERENCE the pixel
@@ -134,7 +134,8 @@ typedef enum {
  *     rays per sample, wave_iterations and kernel_launches keep their formulas.
  * Known limits: inside and outside are decided per hit from the side of the normal, so an open surface (one plane)
  * bounds a half-space of glass: give panes ior 1.  No caustics: the sun's shadow ray keeps the reference's tinted
- * pass-through.  No absorption inside the medium, no dispersion and no rough glass: type 3's roughness stays ignored.
+ * pass-through.  No absorption inside the medium and no dispersion.  Type 3's roughness is read only with
+ * B200RT_SAMPLING_ROUGH_GLASS.
  * The denoiser's G-buffer describes the glass surface, not what is seen through it.
  * Every render entry point takes the bit, alone or with bits 1, 2, 8 and 32 (b200rt_render_adaptive still refuses 8).
  * b200rt_primary_hits, b200rt_gbuffer and b200rt_trace_rays ignore it.  b200rt_set_materials and b200rt_set_scene
@@ -166,10 +167,55 @@ typedef enum {
  *     bit, whatever texture is bound; with no texture bound the image is too.
  * Known limits: no mipmapping (a minified texture aliases until enough samples average it), no sRGB decode, no alpha,
  * no normal or roughness maps.
- * Every render entry point takes the bit, alone or with bits 1, 2, 8, 32 and 128 (b200rt_render_adaptive still refuses 8);
+ * Every render entry point takes the bit, alone or with bits 1, 2, 8, 32, 128 and 2048 (b200rt_render_adaptive still
+ * refuses 8);
  * b200rt_gbuffer and b200rt_render_denoised use it for the albedo; b200rt_primary_hits and b200rt_trace_rays ignore it.
  * b200rt_set_scene keeps the scene's UVs and accepts a triangle whose UV index is out of range; a render or G-buffer with
  * the bit refuses (B200RT_ERR_INVALID) such a scene, and its message names the first such triangle. */
+#define B200RT_SAMPLING_ROUGH_GLASS 2048
+/* Rough glass: on top of B200RT_SAMPLING_DIELECTRIC_GLASS, a glass surface whose roughness slot is > 0 becomes a rough
+ * dielectric interface of GGX microfacets [Walter et al. 2007], so that frosted and etched glass blurs what is seen
+ * through it.  Without this bit type 3's roughness is ignored.  The bit needs bit 128: a mask that has 2048 without 128 is
+ * refused (B200RT_ERR_INVALID).  This bit CHANGES THE INTEGRAND.  The rule, in the conventions of bit 128 (binary32,
+ * every operation rounded separately, true division, correctly rounded sqrtf), at a hit on a glass material m whose ior
+ * slot v is not 1, with r = materialData[6m + 4]:
+ *   - r == 0: the bit-128 rule bit for bit, with its single draw (v == 1 is the pass-through, and r is not read);
+ *   - r > 0: alpha = r (BRDF_GGX's convention, a2 = roughness^2, and the importance sampler's).  w = unit(d); un, c =
+ *     dot(w, un), eta and m (the normal on the incident side) are those of bit 128; Vw = -w;
+ *   - three uniforms uf, u1, u2: with B200RT_RNG_PHILOX words 0, 1 and 2 of the block at counter (i, s, j, 0) (the block
+ *     whose word 0 bit 128 draws); with B200RT_RNG_REFERENCE the pixel generator's next three values in that order.  All
+ *     three are drawn whatever follows;
+ *   - the microfacet normal h: the GGX visible normal around m with alpha seen from Vw [Heitz 2018], in the statements of
+ *     B200RT_SAMPLING_IMPORTANCE's visible-normal draw: sg = copysignf(1, m.z), a = -1 / (sg + m.z), b = (m.x*m.y)*a,
+ *     T = (1 + ((sg*m.x)*m.x)*a, sg*b, -sg*m.x), B = (b, sg + (m.y*m.y)*a, -m.y) (Duff et al. 2017); Vh =
+ *     unit((alpha*dot(Vw, T), alpha*dot(Vw, B), dot(m, Vw))); lensq = Vh.x*Vh.x + Vh.y*Vh.y; T1 = (1, 0, 0), or
+ *     (-Vh.y*inv, Vh.x*inv, 0) with inv = 1 / sqrtf(lensq) if lensq > 0; T2 = cross(Vh, T1); rr = sqrtf(u1), (sp, cp) the
+ *     correctly rounded sine and cosine of 6.2831853f*u2; t1 = rr*cp; t2 = rr*sp; s = 0.5*(1 + Vh.z); t2 = (1 - s)*
+ *     sqrtf(fmaxf(0, 1 - t1*t1)) + s*t2; t3 = sqrtf(fmaxf(0, (1 - t1*t1) - t2*t2)); Nh = ((T1*t1) + (T2*t2)) + (Vh*t3);
+ *     hl = unit((alpha*Nh.x, alpha*Nh.y, fmaxf(0, Nh.z))); h = ((T*hl.x) + (B*hl.y)) + (m*hl.z);
+ *   - if c == 0, c is not finite (a non-finite un) or a component of h is not finite, the bit-128 rule applies with u =
+ *     uf (weight 1);
+ *   - otherwise ch = dot(Vw, h), k = 1 - (eta*eta)*(1 - ch*ch), and F is bit 128's formula with ch in place of ci; the
+ *     path reflects iff !(k >= 0) or !(uf >= F).  Reflection: nd = w + h*(2*ch); refraction: nd = w*eta + h*(eta*ch - ct),
+ *     ct = sqrtf(k).  With co = dot(nd, m), a reflection with !(co > 0) or a refraction with !(co < 0) has weight 0;
+ *     otherwise the weight is Smith's separable masking term of the outgoing direction, G1 = (2*a) / (a + sqrtf(a2 +
+ *     ((1 - a2)*a)*a)) with a = fabsf(co), a2 = alpha*alpha;
+ *   - the throughput: a refraction first tints it by the colour as with bit 128; then a weight of 0 sets it to (0, 0, 0)
+ *     and any other weight multiplies it per component.  h is drawn with the visible-normal density and the branch with
+ *     probability F, so Walter et al.'s BSDF times |cos| over that density is G2 / G1(Vw) = G1(nd): the estimator is
+ *     unbiased for the single-scattering microfacet BSDF.  No eta^2 radiance factor (bit 128 has none);
+ *   - everything else stays as with bit 128 alone: the segment's type is 3, the path goes on from x (a weight-0 path too,
+ *     so no path ends in a new way), the sun-ray rules and light sampling are unchanged (glass is not a light-sampling
+ *     site) and the rays per sample, wave_iterations and kernel_launches keep their formulas.
+ * Known limits: no light sampling at rough glass (a rough pane lit by small emitters is noisy); no multiple-scattering
+ * compensation (the separable Smith term loses energy at high roughness); no caustics (the sun's shadow ray keeps the
+ * tinted pass-through); a one-plane pane with ior 1 cannot be frosted; no eta^2 radiance scaling; no roughness textures,
+ * absorption or dispersion.
+ * Every render entry point takes the bit with 128, alone or with bits 1, 2, 8, 32 and 512 (b200rt_render_adaptive still
+ * refuses 8).  b200rt_primary_hits, b200rt_gbuffer and b200rt_trace_rays ignore it.  b200rt_set_materials and
+ * b200rt_set_scene accept what they accept without it; a render with the bit refuses (B200RT_ERR_INVALID) a material set
+ * in which a glass material whose ior slot is not 1 has a negative, NaN or infinite roughness, and its message names the
+ * first such material.  Any finite r >= 0 is allowed (above 1 too). */
 
 /* output modes */
 #define B200RT_OUT_FINAL 0 /* mean over spp, clamped to [0,1]  (Raytracing.cl:211-219) */
