@@ -76,7 +76,7 @@ SYMBOLS = [
     "b200rt_default_opts", "b200rt_create", "b200rt_destroy", "b200rt_last_error", "b200rt_set_scene",
     "b200rt_set_materials", "b200rt_set_ibl", "b200rt_set_textures", "b200rt_render", "b200rt_render_adaptive", "b200rt_gbuffer", "b200rt_denoise", "b200rt_render_denoised", "b200rt_render_rgb8", "b200rt_render_device", "b200rt_finalize_device",
     "b200rt_reduce_finalize_device", "b200rt_sync", "b200rt_set_stream", "b200rt_invalidate", "b200rt_primary_hits", "b200rt_trace_rays",
-    "b200rt_img_processing", "b200rt_get_stats", "b200rt_math_probe", "b200rt_texel_probe", "b200rt_philox_probe", "b200rt_alloc",
+    "b200rt_img_processing", "b200rt_get_stats", "b200rt_math_probe", "b200rt_texel_probe", "b200rt_rule_probe", "b200rt_philox_probe", "b200rt_alloc",
     "b200rt_free", "b200rt_ipc_export",
     "b200rt_ipc_open", "b200rt_ipc_close", "b200rt_build_bvh", "b200rt_repack_probe", "b200rt_version", "b200rt_device_count",
     "b200rt_multi_create", "b200rt_multi_destroy", "b200rt_multi_last_error", "b200rt_multi_device_count",
@@ -137,6 +137,7 @@ def load_library():
     lib.b200rt_get_stats.argtypes = [vp, ctypes.POINTER(Stats)]
     lib.b200rt_math_probe.argtypes = [vp, i32, vp, vp, i64, vp]
     lib.b200rt_texel_probe.argtypes = [vp, i32, vp, vp, i64, i32, vp]
+    lib.b200rt_rule_probe.argtypes = [vp, i32, vp, i64, vp]
     lib.b200rt_philox_probe.argtypes = [vp, ctypes.POINTER(u32 * 4), u32, u32, ctypes.POINTER(u32 * 4)]
     lib.b200rt_alloc.argtypes = [vp, i64, ctypes.POINTER(vp)]
     lib.b200rt_free.argtypes = [vp, vp]
@@ -510,6 +511,18 @@ class Context(_Handle):
         else:
             self._check(self._lib.b200rt_texel_probe(self._h, int(fn), _ptr(a_), _ptr(b_), a_.size, int(extent),
                                                      _ptr(out)), "b200rt_texel_probe")
+        return out
+
+    def rule_probe(self, rule, records):
+        """b200rt_rule_probe: records (m, 16) of any 4-byte type, taken as bit patterns (float fields as float32, integer
+        fields and uniform words as int32 / uint32) -> (m, 8) float32"""
+        rec = np.ascontiguousarray(records)
+        if rec.ndim != 2 or rec.shape[1] != 16 or rec.dtype.itemsize != 4:
+            raise B200RTError(f"rule_probe records must be (m, 16) of a 4-byte type, not {rec.shape} {rec.dtype}")
+        rec = rec.view(np.float32)
+        out = np.zeros((rec.shape[0], 8), np.float32)
+        self._check(self._lib.b200rt_rule_probe(self._h, int(rule), _ptr(rec), rec.shape[0], _ptr(out)),
+                    "b200rt_rule_probe")
         return out
 
     def philox_probe(self, ctr, key0, key1):

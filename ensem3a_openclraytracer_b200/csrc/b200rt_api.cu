@@ -1820,6 +1820,63 @@ int b200rt_texel_probe(b200rt_ctx *c, int fn, const float *a, const float *b, in
   return math_probe(c, fn, a, b, n, extent, out);
 }
 
+int b200rt_rule_probe(b200rt_ctx *c, int rule, const float *in, int64_t n, float *out) {
+  if (!c) return B200RT_ERR_INVALID;
+  if (!in || !out || n <= 0 || n > 0x7fffffffLL || rule < 0 || rule > 11)
+    return fail(c, B200RT_ERR_INVALID, "bad rule_probe arguments");
+  if (rule >= 8 && rule <= 10 && !c->have_scene) return fail(c, B200RT_ERR_NO_SCENE, "no scene: call b200rt_set_scene first");
+  const int n_tex = c->n_mat_tex > 0 ? c->n_tex : 0;   // textures the kernels can reach
+  const int n_tris = c->have_scene ? c->scene.n_tris : 0;
+  // every index field is checked here, so that no record makes the kernel read out of bounds
+  for (int64_t i = 0; i < n; ++i) {
+    int32_t f[3];
+    memcpy(f, in + 16 * i + 9, sizeof f);
+    const bool bad_tri = (rule >= 8 && rule <= 10) && (f[0] < 0 || f[0] >= n_tris);
+    const bool bad_mat = (rule == 8 || rule == 10) && (f[1] < 0 || f[1] >= c->n_mats);
+    if (bad_tri || bad_mat || (rule == 8 && f[2] < 1) || (rule == 11 && (f[0] < 0 || f[0] >= n_tex)))
+      return fail(c, B200RT_ERR_INVALID,
+                  "rule_probe record %lld: index fields %d %d %d out of range (%d triangles, %d materials, %d textures)",
+                  (long long)i, f[0], f[1], f[2], n_tris, c->n_mats, n_tex);
+  }
+  CU(cudaSetDevice(c->device));
+  const bool framed = rule == 2 || rule == 4 || rule == 6;
+  if (ensure(c, c->d_tmp_a, (size_t)n * 16 * sizeof(float))) return B200RT_ERR_CUDA;
+  if (ensure(c, c->d_misc, (size_t)n * 8 * sizeof(float))) return B200RT_ERR_CUDA;
+  CU(cudaMemcpyAsync(c->d_tmp_a.p, in, (size_t)n * 16 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  const unsigned grid = (unsigned)((n + 255) / 256);
+  float4 *frames = nullptr;
+  std::vector<float4> normals;
+  if (framed) {   // the records' normals, framed by the kernel that frames a scene's normals at upload
+    normals.resize((size_t)n);
+    for (int64_t i = 0; i < n; ++i) normals[(size_t)i] = make_float4(in[16 * i + 3], in[16 * i + 4], in[16 * i + 5], 0.0f);
+    if (ensure(c, c->d_tmp_b, (size_t)n * (kFrameVec + 1) * sizeof(float4))) return B200RT_ERR_CUDA;
+    frames = static_cast<float4 *>(c->d_tmp_b.p);
+    float4 *d_normals = frames + (size_t)n * kFrameVec;
+    CU(cudaMemcpyAsync(d_normals, normals.data(), (size_t)n * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
+    k_tri_frames<<<grid, 256, 0, c->stream>>>(d_normals, (int)n, frames);
+    CU(cudaGetLastError());
+  }
+  SceneView S = SceneView();
+  if (c->have_scene) {
+    S.tris = static_cast<const float4 *>(c->d_scene[kTris].p);
+    S.normals = static_cast<const float4 *>(c->d_scene[kNormals].p);
+    S.mats = static_cast<const float *>(c->d_scene[kMats].p);
+  }
+  TexView T = TexView();
+  if (n_tex > 0) {   // the layout b200rt_set_textures uploads
+    const char *base = static_cast<const char *>(c->d_scene[kTex].p);
+    T.info = reinterpret_cast<const int4 *>(base);
+    T.texels = reinterpret_cast<const uchar4 *>(base + (size_t)c->n_tex * sizeof(int4) +
+                                                (((size_t)c->n_mat_tex + 3) & ~(size_t)3) * sizeof(int32_t));
+  }
+  k_rule_probe<<<grid, 256, 0, c->stream>>>(rule, static_cast<const float *>(c->d_tmp_a.p), (long long)n, frames, S, n_tris,
+                                            T, static_cast<float *>(c->d_misc.p));
+  CU(cudaGetLastError());
+  CU(cudaMemcpyAsync(out, c->d_misc.p, (size_t)n * 8 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return 0;
+}
+
 int b200rt_philox_probe(b200rt_ctx *c, const uint32_t ctr[4], uint32_t key0, uint32_t key1, uint32_t out[4]) {
   if (!c) return B200RT_ERR_INVALID;
   if (!ctr || !out) return fail(c, B200RT_ERR_INVALID, "NULL argument");

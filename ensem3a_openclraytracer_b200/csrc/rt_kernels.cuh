@@ -1033,6 +1033,78 @@ __global__ void k_math_probe(int fn, const float *a, const float *b, long long n
   out[i] = r;
 }
 
+// One record of b200rt_rule_probe per thread: 16 floats in, 8 out (rule codes and layout in b200rt.h).  Every rule calls
+// the functions k_shade calls and restates none of their statements.  What k_shade computes inline arrives as an input:
+// the hit point x (o + unit(d) * k), the emitter triangle it picks with the light sample's first uniform, and the
+// surface's material.  frames: per record, the frame k_tri_frames made of the record's normal (rules 2, 4, 6).
+// b200rt_rule_probe has checked every index field.
+__global__ void k_rule_probe(int rule, const float *__restrict__ in, long long n, const float4 *__restrict__ frames,
+                             const SceneView S, int n_tris, const TexView T, float *__restrict__ out) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float *a = in + 16 * i;
+  const v3 d = mk3(a[0], a[1], a[2]), nr = mk3(a[3], a[4], a[5]), x = mk3(a[6], a[7], a[8]);
+  const int i9 = __float_as_int(a[9]), i10 = __float_as_int(a[10]), i11 = __float_as_int(a[11]);
+  const float u0 = bits_to_unit(__float_as_uint(a[12])), u1 = bits_to_unit(__float_as_uint(a[13]));
+  const float u2 = bits_to_unit(__float_as_uint(a[14]));
+  float r[8] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
+  v3 v = mk3(0.0f, 0.0f, 0.0f);
+  bool flag = false;
+  switch (rule) {
+    case 0: v = scatter_dielectric(d, nr, a[6], u0, &flag); r[3] = flag ? 1.0f : 0.0f; break;
+    case 1: v = scatter_rough_dielectric(d, nr, a[6], a[7], u0, u1, u2, &flag, &r[4]); r[3] = flag ? 1.0f : 0.0f; break;
+    case 2: v = sample_cosine(nr, load_tri_frame(frames, (int)i, 1), u0, u1, &r[3]); break;
+    case 3: v = sample_cosine(nr, tri_frame_at(nr, 1), u0, u1, &r[3]); break;
+    case 4: v = sample_uniform(nr, load_tri_frame(frames, (int)i, 2), u0, u1, &r[3]); break;
+    case 5: v = sample_uniform(nr, tri_frame_at(nr, 2), u0, u1, &r[3]); break;
+    case 6: {
+      const TriFrame tf = load_tri_frame(frames, (int)i, 2);
+      Material m;
+      m.type = 2;
+      m.color = mk3(1.0f, 1.0f, 1.0f);
+      m.roughness = a[6];
+      v = sample_glossy_importance(m.roughness, tf.un, d, u0, u1, &r[3]);
+      r[4] = bsdf_pdf(m, 1, tf.un, d, unit(v));
+      break;
+    }
+    case 7: {
+      Material m;
+      m.type = 2;
+      m.color = mk3(a[9], a[10], a[11]);
+      m.roughness = a[12];
+      v = bsdf_ggx(m, d, x, nr);
+      break;
+    }
+    case 8: {
+      const Material m = load_material(S.mats, i10);
+      const Tri l = load_tri(S.tris, i9);
+      const Material ml = load_material(S.mats, l.mat);
+      const float Le = ml.type == 0 ? ml.roughness : 0.0f;
+      const v3 un = unit(nr);
+      const int sampling = __float_as_int(a[15]);
+      v3 w;
+      v = sample_light(m, sampling, nr, un, x, d, mk3(1.0f, 1.0f, 1.0f), l.A, l.e1, l.e2, Le, i11, u1, u2, &w);
+      const float dist2 = dot(w, w);
+      const v3 wi = w / sqrtf(dist2);
+      r[3] = w.x; r[4] = w.y; r[5] = w.z;
+      r[6] = light_pdf(l.e1, l.e2, i11, wi, dist2);
+      r[7] = bsdf_pdf(m, sampling, un, d, wi);
+      break;
+    }
+    case 9: {
+      const float4 nn = __ldg(S.normals + i9);
+      v = shading_normal<true>(S, n_tris, i9, mk3(nn.x, nn.y, nn.z), x, &flag);
+      r[3] = flag ? 1.0f : 0.0f;
+      break;
+    }
+    case 10: v = surface_albedo(S, n_tris, i9, i10, d, x); break;
+    case 11: v = texture_factor(T, i9, a[6], a[7]); break;
+  }
+  r[0] = v.x; r[1] = v.y; r[2] = v.z;
+  float *o = out + 8 * i;
+  for (int k = 0; k < 8; ++k) o[k] = r[k];
+}
+
 __global__ void k_philox_probe(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1, uint32_t *out) {
   uint32_t o[4];
   philox4x32_10(c0, c1, c2, c3, k0, k1, o);

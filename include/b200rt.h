@@ -460,6 +460,34 @@ int b200rt_math_probe(b200rt_ctx *ctx, int fn, const float *a, const float *b, i
 /* fn 11-14 of b200rt_math_probe for an environment map of any size: `extent` is its width (11/12) or height (13/14). */
 int b200rt_texel_probe(b200rt_ctx *ctx, int fn, const float *a, const float *b, int64_t n, int extent, float *out);
 
+/* The per-hit shading rules of the kernels, one record at a time, so that tests can compare them value by value with the
+ * oracle and histogram their draws.  Each record is 16 floats of `in` and 8 of `out`; integer fields are int32 bit
+ * patterns, and a uniform is a uint32 word that the device turns into [0, 1) as its generators do.  Fields: d = in[0..2]
+ * (a direction), n = in[3..5] (a normal), x = in[6..8] (a point), i9 i10 i11 = in[9], in[10], in[11] (integers),
+ * w12 w13 w14 = in[12], in[13], in[14] (uniform words).  Unlisted outputs are 0; a flag is 1.0 or 0.0.
+ *   0 smooth dielectric (bit 128): ior = in[6], u = w12                 -> out[0..2] direction, out[3] reflected
+ *     (rules 0 and 1 take the ior itself: a render first maps slot 0 to B200RT_GLASS_DEFAULT_IOR)
+ *   1 rough dielectric (bit 2048): ior = in[6], alpha = in[7], (uf, u1, u2) = (w12, w13, w14)
+ *                                                                        -> direction, reflected, out[4] weight
+ *   2 / 3 cosine sampler about n, (u, u2) = (w12, w13), with the frame precomputed per triangle (2) or built at the
+ *         hit as for a smooth-shaded triangle (3)                        -> out[0..2] l, out[3] inv_pdf
+ *   4 / 5 the same for the uniform hemisphere sampler
+ *   6 glossy importance sampler (bit 1): roughness = in[6], incoming d, (u0, u1) = (w12, w13)
+ *                                                                        -> l, out[3] inv_pdf, out[4] density at l
+ *   7 BRDF_GGX: v = d, l = x, colour = in[9..11], roughness = in[12]     -> out[0..2]
+ *   8 light sample (bit 2) at surface point x with normal n, incoming d, surface material i10, throughput (1, 1, 1),
+ *     towards emitter triangle i9 of n_light = i11 emitters, (ua, ub) = (w13, w14), sampling bits = in[15] (the picking
+ *     uniform w12 is not read: the emitter is given)
+ *                                      -> contribution, out[3..5] shadow-ray direction w, out[6..7] the light and
+ *                                         surface densities at unit(w)
+ *   9 shading normal (bit 32) of triangle i9 at x                        -> normal, out[3] curved
+ *  10 albedo (bit 512) of triangle i9 with material i10 and colour d at x -> out[0..2]
+ *  11 texture factor of bound texture i9 at (u, v) = (in[6], in[7])      -> out[0..2]
+ * Rules 8-10 read the uploaded scene, rules 10 and 11 the bound textures.  B200RT_ERR_INVALID for a triangle outside
+ * [0, n_tris), a material outside the material set, a texture outside the bound ones or n_light < 1 (checked before the
+ * launch); NaN, infinite and huge floats are inputs the rules define. */
+int b200rt_rule_probe(b200rt_ctx *ctx, int rule, const float *in, int64_t n, float *out);
+
 /* Philox4x32-10 block of the device implementation (known-answer tests). */
 int b200rt_philox_probe(b200rt_ctx *ctx, const uint32_t ctr[4], uint32_t key0, uint32_t key1, uint32_t out[4]);
 
